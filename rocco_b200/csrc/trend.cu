@@ -153,18 +153,34 @@ __device__ __forceinline__ void cta_range(long long rows, long long n, long long
 }
 
 // ------------------------------------------------------------------ T1 fused with the rolling AR(1) variance
-// One CTA streams a CHUNK of one row in tiles of RV_T bins: the tile (+ w-1 halo) is staged in shared memory in a
-// padded layout (position i + i/8, so that 8-bin-per-thread accesses are bank-conflict free), every thread
-// produces 8 consecutive variances (direct 31-term window sums for the first, sliding updates for the next 7 --
-// far less drift than the reference's whole-row slide), results go back through shared memory for coalesced
+// One CTA streams RV_CHUNK bins of one row in tiles of RV_T bins: the tile (+ w-1 halo) is staged in shared memory in a
+// padded layout (position i + i/8, so that 8-bin-per-block accesses are bank-conflict free), every block of 8
+// consecutive variances gets direct 31-term window sums for the first and sliding updates for the next 7 (far less
+// drift than the reference's whole-row slide), each thread computes two such blocks with their dependent sum chains
+// interleaved (worth 1.6 ms per step against one block per thread), results go back through shared memory for coalesced
 // stores, and the same pass feeds the |C| histogram.  Replaces wls_backend.c:610-742 + the T1 pass.
+// Staging is asynchronous and double-buffered: tile t+1 arrives by 8-byte cp.async copies (the padded layout keeps
+// no 16-byte alignment) while tile t computes.  Interior tiles histogram each block's own 8 bins from the registers
+// that hold them for the window sums; edge tiles (first / last of a row, a partial tail) read them back from shared
+// memory.  The histogram keeps 16-bit counts, two buckets per word, so that two CTAs with two tile buffers each fit
+// an SM and the barrier and store phases of one overlap the window arithmetic of the other.
 constexpr int RV_T = 4096;                   // bins per CTA iteration
-constexpr int RV_K = 8;
-constexpr int RV_THREADS = RV_T / RV_K;      // 512: two CTAs per SM (64 KB histogram + 37 KB tile each), so that the staging
-                                             // loads of one overlap the window arithmetic of the other
+constexpr int RV_K = 8;                      // outputs per block (direct window sums for the first, slides for the rest)
+constexpr int RV_B = 2;                      // blocks per thread: blocks tid and tid + RV_THREADS, computed interleaved
+constexpr int RV_THREADS = RV_T / (RV_K * RV_B);   // 256 at <= 128 registers: two CTAs per SM (32 KB histogram + two tile
+                                                   // buffers of 37 KB at w = 31 each)
+constexpr int RV_CHUNK = 15 * RV_T;          // bins per CTA: every bucket count fits the 16-bit halves of the shared histogram
+static_assert(RV_CHUNK < 65536, "16-bit histogram counters");
 constexpr int RV_MAXW = 1025;
 
 __host__ __device__ __forceinline__ int padpos(int i) { return i + (i >> 3); }
+// doubles per tile buffer (span <= RV_T + w - 1), even so that the second buffer starts 16-byte aligned
+__host__ __device__ __forceinline__ int rv_buf(int w) { return (padpos(RV_T + w) + 1) & ~1; }
+
+__device__ __forceinline__ void cp_async8(double *dst, const double *src)
+{
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
+}
 
 // W > 0: compile-time window (31 = the reference default): interior tiles run fully unrolled from registers.
 template <int W>
@@ -173,73 +189,98 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
 {
     extern __shared__ int s_dyn[];
     const int w = W > 0 ? W : w_rt;
-    int *s_h = s_dyn;                                              // NBX
-    double *s_in = reinterpret_cast<double *>(s_dyn + NBX);        // padpos(RV_T + w)
-    double *s_out = s_in;                                          // the results reuse the tile's slots (after a barrier)
+    unsigned *s_h = reinterpret_cast<unsigned *>(s_dyn);           // NBX / 2: bucket b counts in the 16-bit half b & 1 of word b / 2
+    double *s_buf = reinterpret_cast<double *>(s_dyn + NBX / 2);  // 2 x rv_buf(w): tile t in buffer t & 1
     const long long row = blockIdx.y;
     const double *c = C + row * row_stride;
     double *v = V + row * row_stride;
-    const long long c0 = (long long)blockIdx.x * CHUNK, c1 = min(n, c0 + CHUNK);
+    const long long c0 = (long long)blockIdx.x * RV_CHUNK, c1 = min(n, c0 + RV_CHUNK);
     const long long half = w / 2, last = n - w;
     const double wd = (double)w, pairs = (double)(w - 1), rwd = 1.0 / wd, shrink = 1.0 + 1.0 / (wd + 1.0) + 1.0e-4;      // c1 of ar1_window_variance
     const int tid = threadIdx.x;
-    for (int k = tid; k < NBX; k += RV_THREADS) s_h[k] = 0;
-    __syncthreads();
+    auto count = [&](double x) { const int b = xbucket(fabs(x), G); atomicAdd(&s_h[b >> 1], 1u << ((b & 1) << 4)); };
+    const int bstride = rv_buf(w);
+    // staged range of the tile starting at j0: [tlo, tlo + span)
+    auto tile_range = [&](long long j0, long long *tlo, int *span) {
+        const long long j1 = min(c1, j0 + RV_T);
+        long long lo = j0 - half; if (lo < 0) lo = 0; else if (lo > last) lo = last;
+        long long hi = (j1 - 1) - half; if (hi < 0) hi = 0; else if (hi > last) hi = last;
+        *tlo = lo;
+        *span = (int)(hi - lo) + w;
+    };
+    auto stage = [&](long long j0, double *buf) {
+        long long tlo; int span;
+        tile_range(j0, &tlo, &span);
+        const double *src = c + tlo;
+#pragma unroll 4
+        for (int e = tid; e < span; e += RV_THREADS) cp_async8(buf + padpos(e), src + e);
+        asm volatile("cp.async.commit_group;" ::: "memory");
+    };
+    double *s_in = s_buf, *s_next = s_buf + bstride;
+    stage(c0, s_in);
+    for (int k = tid; k < NBX / 2; k += RV_THREADS) s_h[k] = 0;
     for (long long j0 = c0; j0 < c1; j0 += RV_T) {
         const long long j1 = min(c1, j0 + RV_T);
-        long long tlo = j0 - half; if (tlo < 0) tlo = 0; else if (tlo > last) tlo = last;
-        long long thi = (j1 - 1) - half; if (thi < 0) thi = 0; else if (thi > last) thi = last;
-        const int span = (int)(thi - tlo) + w;                     // bins staged: [tlo, tlo + span)
-        const int own0 = (int)(j0 - tlo), own1 = (int)(j1 - tlo);  // staged positions of the tile's own bins
-        const double *src = c + tlo;
-#pragma unroll 1
-        for (int e0 = tid; e0 < span; e0 += 4 * RV_THREADS) {          // four loads in flight per thread
-            double val[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) { const int e = e0 + u * RV_THREADS; val[u] = (e < span) ? src[e] : 0.0; }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int e = e0 + u * RV_THREADS;
-                if (e >= span) break;
-                s_in[padpos(e)] = val[u];
-                if (e >= own0 && e < own1) atomicAdd(&s_h[xbucket(fabs(val[u]), G)], 1);
-            }
-        }
-        __syncthreads();
+        long long tlo; int span;
+        tile_range(j0, &tlo, &span);
+        asm volatile("cp.async.wait_group 0;" ::: "memory");
+        __syncthreads();                                           // this tile has landed; the other buffer has been copied out
+        if (j0 + RV_T < c1) stage(j0 + RV_T, s_next);
         const bool interior = (j0 - half >= 0) && ((j1 - 1) - half <= last) && (j1 - j0 == RV_T);
-        double res[RV_K];
+        double res[RV_B][RV_K];
         if (W > 0 && interior) {
-            // window of output k starts at staged position tid*8 + k; padded address = tid*9 + q + (q >> 3)
-            const double *base = s_in + tid * 9;
-            double y[W + RV_K - 1];
+            // window of output k of block b starts at staged position b*8 + k; padded address = b*9 + q + (q >> 3).  The
+            // blocks' sums are independent chains, interleaved here so that each thread keeps RV_B of them in flight.
+            double y[RV_B][W + RV_K - 1];
 #pragma unroll
-            for (int q = 0; q < W + RV_K - 1; ++q) y[q] = base[q + (q >> 3)];
-            double s1 = 0.0, s2 = 0.0, sl = 0.0;
+            for (int h = 0; h < RV_B; ++h) {
+                const double *base = s_in + (tid + h * RV_THREADS) * 9;
+#pragma unroll
+                for (int q = 0; q < W + RV_K - 1; ++q) y[h][q] = base[q + (q >> 3)];
+            }
+            double s1[RV_B], s2[RV_B], sl[RV_B];
+#pragma unroll
+            for (int h = 0; h < RV_B; ++h) s1[h] = s2[h] = sl[h] = 0.0;
 #pragma unroll
             for (int q = 0; q < W; ++q) {
-                s1 = __dadd_rn(s1, y[q]);
-                s2 = __fma_rn(y[q], y[q], s2);
-                if (q + 1 < W) sl = __fma_rn(y[q], y[q + 1], sl);
+#pragma unroll
+                for (int h = 0; h < RV_B; ++h) {
+                    s1[h] = __dadd_rn(s1[h], y[h][q]);
+                    s2[h] = __fma_rn(y[h][q], y[h][q], s2[h]);
+                    if (q + 1 < W) sl[h] = __fma_rn(y[h][q], y[h][q + 1], sl[h]);
+                }
             }
 #pragma unroll
             for (int k = 0; k < RV_K; ++k) {
-                if (k > 0) {
-                    const double out_v = y[k - 1], nx = y[k - 1 + W];
-                    s1 = __dadd_rn(__dsub_rn(s1, out_v), nx);
-                    s2 = __fma_rn(nx, nx, __fma_rn(-out_v, out_v, s2));
-                    sl = __fma_rn(y[k - 2 + W], nx, __fma_rn(-out_v, y[k], sl));
+#pragma unroll
+                for (int h = 0; h < RV_B; ++h) {
+                    if (k > 0) {
+                        const double out_v = y[h][k - 1], nx = y[h][k - 1 + W];
+                        s1[h] = __dadd_rn(__dsub_rn(s1[h], out_v), nx);
+                        s2[h] = __fma_rn(nx, nx, __fma_rn(-out_v, out_v, s2[h]));
+                        sl[h] = __fma_rn(y[h][k - 2 + W], nx, __fma_rn(-out_v, y[h][k], sl[h]));
+                    }
+                    const double cur = ar1_window_variance(s1[h], s2[h], sl[h], y[h][k], y[h][k + W - 1], wd, rwd, pairs, shrink);
+                    res[h][k] = dmax(cur, 1.0e-8);                                 // wls_backend.c:869
                 }
-                const double cur = ar1_window_variance(s1, s2, sl, y[k], y[k + W - 1], wd, rwd, pairs, shrink);
-                res[k] = dmax(cur, 1.0e-8);                                        // wls_backend.c:869
             }
+#pragma unroll
+            for (int h = 0; h < RV_B; ++h)
+#pragma unroll
+                for (int k = 0; k < RV_K; ++k) count(y[h][W / 2 + k]);         // own bins: staged b*8 + half + k
         } else {
-            const long long jt = j0 + (long long)tid * RV_K;
+#pragma unroll
+          for (int h = 0; h < RV_B; ++h) {
+            const long long jt = j0 + (long long)(tid + h * RV_THREADS) * RV_K;
+#pragma unroll
+            for (int k = 0; k < RV_K; ++k)
+                if (jt + k < j1) count(s_in[padpos((int)(jt + k - tlo))]);
             double s1 = 0.0, s2 = 0.0, sl = 0.0, cur = 0.0;
             long long tprev = -1;
 #pragma unroll
             for (int k = 0; k < RV_K; ++k) {
                 const long long j = jt + k;
-                res[k] = 0.0;
+                res[h][k] = 0.0;
                 if (j >= j1) continue;
                 long long t = j - half;
                 if (t < 0) t = 0; else if (t > last) t = last;
@@ -265,24 +306,30 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
                     cur = ar1_window_variance(s1, s2, sl, s_in[padpos(r)], s_in[padpos(r + w - 1)], wd, rwd, pairs, shrink);
                     tprev = t;
                 }
-                res[k] = dmax(cur, 1.0e-8);
+                res[h][k] = dmax(cur, 1.0e-8);
             }
+          }
         }
         __syncthreads();                                           // every window has been read: the slots can take the results
-        {
-            double *ob = s_out + tid * 9;                          // padpos(tid * 8 + k) = tid * 9 + k
+        double *const s_out = s_in;
 #pragma unroll
-            for (int k = 0; k < RV_K; ++k) ob[k] = res[k];
+        for (int h = 0; h < RV_B; ++h) {
+            double *ob = s_out + (tid + h * RV_THREADS) * 9;       // padpos(b * 8 + k) = b * 9 + k
+#pragma unroll
+            for (int k = 0; k < RV_K; ++k) ob[k] = res[h][k];
         }
         __syncthreads();
+        // plain stores: nothing waits for them; the next iteration's barrier orders these shared reads before the
+        // buffer is staged again
         double *dst = v + j0;
         for (int e = tid; e < (int)(j1 - j0); e += RV_THREADS) dst[e] = s_out[padpos(e)];
-        __syncthreads();
+        double *const t = s_in; s_in = s_next; s_next = t;
     }
     int *g = xhist + row * NBX;
-    for (int k = tid; k < NBX; k += RV_THREADS) {
-        const int val = s_h[k];
-        if (val) atomicAdd(&g[k], val);
+    for (int k = tid; k < NBX / 2; k += RV_THREADS) {
+        const unsigned val = s_h[k];
+        if (val & 0xFFFFu) atomicAdd(&g[2 * k], (int)(val & 0xFFFFu));
+        if (val >> 16) atomicAdd(&g[2 * k + 1], (int)(val >> 16));
     }
 }
 
@@ -1032,20 +1079,21 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
     const unsigned chunks = (unsigned)((n + CHUNK - 1) / CHUNK);
     const dim3 gstream(chunks, (unsigned)m);
     if (fused_window > 0) {
-        const size_t sm_fused = sizeof(int) * NBX + sizeof(double) * (padpos(RV_T + fused_window) + 8);
+        const size_t sm_fused = sizeof(int) * NBX / 2 + 2 * sizeof(double) * rv_buf(fused_window);
         static bool attr2_dev[64] = {false};
     int attr2_d = 0;
     cudaGetDevice(&attr2_d);
     bool &attr2 = attr2_dev[attr2_d & 63];
         if (!attr2) {
-            const int mx = (int)(sizeof(int) * NBX + sizeof(double) * (padpos(RV_T + RV_MAXW) + 8));
+            const int mx = (int)(sizeof(int) * NBX / 2 + 2 * sizeof(double) * rv_buf(RV_MAXW));
             RB_CUDA(cudaFuncSetAttribute(k_rollvar_xhist<31>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
             RB_CUDA(cudaFuncSetAttribute(k_rollvar_xhist<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
             attr2 = true;
         }
         RB_PROF("k_rollvar_xhist", st, (double)m * n * 16.0);
-        if (fused_window == 31) k_rollvar_xhist<31><<<gstream, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom);
-        else k_rollvar_xhist<0><<<gstream, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom);
+        const dim3 grv((unsigned)((n + RV_CHUNK - 1) / RV_CHUNK), (unsigned)m);
+        if (fused_window == 31) k_rollvar_xhist<31><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom);
+        else k_rollvar_xhist<0><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom);
         RB_LAUNCH_CHECK();
     } else {
         RB_PROF("trend_xhist", st, (double)m * n * 8.0);
