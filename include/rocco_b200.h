@@ -218,7 +218,9 @@ typedef struct rocco_b200_score_params {
 void rocco_b200_default_score_params(rocco_b200_score_params *p);
 
 /* Order statistics of the variance trend: 0 = histogram multi-select with a sort fallback for rows whose
- * buckets overflow (default), 1 = sort every row.  Both are exact; returns the previous mode. */
+ * buckets overflow (default), 1 = sort every row, 2 = as 0 but without the 32-bit pair keys the rolling-variance
+ * pass leaves the slot collection (it reads the signal and the variances instead; for A/B timing).  Any other
+ * value means 0.  All are exact; returns the previous mode. */
 int rocco_b200_trend_set_mode(int mode);
 long long rocco_b200_trend_fallback_rows(void);   /* rows that took the sort path since load */
 void rocco_b200_trend_fallback_reasons(long long *out8);   /* per-reason counts (diagnostics) */

@@ -68,6 +68,14 @@ __device__ __forceinline__ int ybucket(double y, int yb0, const BucketGeom &G)
     const int b = u - yb0;
     return b < 0 ? 0 : (b >= NBY ? NBY - 1 : b);
 }
+// T3's 32-bit key of a pair, written by the fused rolling-variance pass: |signal| bucket << 18 | variance bits >> yshift.
+// V is floored at 1e-8 (a NaN window gives the floor), so its sign bit is clear and a shift by 45 or 46 leaves at most
+// 18 bits; T3 then finds both buckets of a pair without reading C or V (ybucket(v) == clamp((key & 0x3FFFF) - yb0)).
+constexpr int KEY_YBITS = 18;
+__device__ __forceinline__ unsigned pair_key(int xb, double v, const BucketGeom &G)
+{
+    return ((unsigned)xb << KEY_YBITS) | ((unsigned)__double2hiint(v) >> (G.yshift - 32));
+}
 __device__ __forceinline__ int bin_of_rank(long long p, long long N, int B)
 {
     int b = (int)((p * B) / N);
@@ -113,6 +121,7 @@ struct TrendBuffers {
     int *ycand_cnt;        // [m][MAXB][2]
     unsigned long long *yover_min, *yover_max;   // [m][MAXB][2]  bit-pattern range of the variances that did not fit their slot
     unsigned short *codes;  // [m][code_stride]  T3 -> T6: bin << 10 | variance bucket of every pair (0xFFFF: not T6's business)
+    unsigned *keys;         // [m][code_stride]  fused rolling variance -> T3: pair_key of every pair (nullptr: T3 reads C and V)
     long long code_stride;  // n rounded up to a multiple of 8 (128-bit loads)
     long long rows;
     BucketGeom geom;
@@ -164,6 +173,9 @@ __device__ __forceinline__ void cta_range(long long rows, long long n, long long
 // that hold them for the window sums; edge tiles (first / last of a row, a partial tail) read them back from shared
 // memory.  The histogram keeps 16-bit counts, two buckets per word, so that two CTAs with two tile buffers each fit
 // an SM and the barrier and store phases of one overlap the window arithmetic of the other.
+// With `keys` given, the pass also leaves T3 the pair_key of every bin, built from the bucket just counted and the
+// variance just computed: interior tiles store each block's 8 keys as two 128-bit stores straight from registers (block
+// starts are multiples of 8 bins, so 32-byte aligned), edge tiles one key per bin.
 constexpr int RV_T = 4096;                   // bins per CTA iteration
 constexpr int RV_K = 8;                      // outputs per block (direct window sums for the first, slides for the rest)
 constexpr int RV_B = 2;                      // blocks per thread: blocks tid and tid + RV_THREADS, computed interleaved
@@ -185,7 +197,8 @@ __device__ __forceinline__ void cp_async8(double *dst, const double *src)
 // W > 0: compile-time window (31 = the reference default): interior tiles run fully unrolled from registers.
 template <int W>
 __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *__restrict__ C, long long n, long long row_stride, int w_rt,
-                                                               double *__restrict__ V, int *xhist, BucketGeom G)
+                                                               double *__restrict__ V, int *xhist, BucketGeom G,
+                                                               unsigned *__restrict__ keys, long long key_stride)
 {
     extern __shared__ int s_dyn[];
     const int w = W > 0 ? W : w_rt;
@@ -194,11 +207,12 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
     const long long row = blockIdx.y;
     const double *c = C + row * row_stride;
     double *v = V + row * row_stride;
+    unsigned *const kr = keys ? keys + row * key_stride : nullptr;
     const long long c0 = (long long)blockIdx.x * RV_CHUNK, c1 = min(n, c0 + RV_CHUNK);
     const long long half = w / 2, last = n - w;
     const double wd = (double)w, pairs = (double)(w - 1), rwd = 1.0 / wd, shrink = 1.0 + 1.0 / (wd + 1.0) + 1.0e-4;      // c1 of ar1_window_variance
     const int tid = threadIdx.x;
-    auto count = [&](double x) { const int b = xbucket(fabs(x), G); atomicAdd(&s_h[b >> 1], 1u << ((b & 1) << 4)); };
+    auto count = [&](double x) { const int b = xbucket(fabs(x), G); atomicAdd(&s_h[b >> 1], 1u << ((b & 1) << 4)); return b; };
     const int bstride = rv_buf(w);
     // staged range of the tile starting at j0: [tlo, tlo + span)
     auto tile_range = [&](long long j0, long long *tlo, int *span) {
@@ -264,17 +278,20 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
                     res[h][k] = dmax(cur, 1.0e-8);                                 // wls_backend.c:869
                 }
             }
+            // own bins (staged b*8 + half + k): histogram, and the keys four at a time so that no more than four are live
 #pragma unroll
             for (int h = 0; h < RV_B; ++h)
 #pragma unroll
-                for (int k = 0; k < RV_K; ++k) count(y[h][W / 2 + k]);         // own bins: staged b*8 + half + k
+                for (int k4 = 0; k4 < RV_K; k4 += 4) {
+                    unsigned kk[4];
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) kk[q] = pair_key(count(y[h][W / 2 + k4 + q]), res[h][k4 + q], G);
+                    if (kr) *reinterpret_cast<uint4 *>(kr + j0 + (tid + h * RV_THREADS) * RV_K + k4) = make_uint4(kk[0], kk[1], kk[2], kk[3]);
+                }
         } else {
 #pragma unroll
           for (int h = 0; h < RV_B; ++h) {
             const long long jt = j0 + (long long)(tid + h * RV_THREADS) * RV_K;
-#pragma unroll
-            for (int k = 0; k < RV_K; ++k)
-                if (jt + k < j1) count(s_in[padpos((int)(jt + k - tlo))]);
             double s1 = 0.0, s2 = 0.0, sl = 0.0, cur = 0.0;
             long long tprev = -1;
 #pragma unroll
@@ -308,6 +325,12 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
                 }
                 res[h][k] = dmax(cur, 1.0e-8);
             }
+#pragma unroll
+            for (int k = 0; k < RV_K; ++k)
+                if (jt + k < j1) {
+                    const int b = count(s_in[padpos((int)(jt + k - tlo))]);
+                    if (kr) kr[jt + k] = pair_key(b, res[h][k], G);
+                }
           }
         }
         __syncthreads();                                           // every window has been read: the slots can take the results
@@ -503,6 +526,123 @@ __global__ void __launch_bounds__(XC_THREADS) k_xcollect(const double *__restric
                 codes[jb + u * XC_THREADS + threadIdx.x] = code;    // T6 reads two bytes per pair instead of sixteen
             }
         }
+        __syncthreads();
+        int *gh = T.yhist + (size_t)row * MAXB * NBY;
+        for (int k = threadIdx.x; k < B * NBY; k += XC_THREADS) {
+            const int val = s_yh[k];
+            if (val) atomicAdd(&gh[k], val);
+        }
+    }
+}
+
+// T3 from the keys the fused rolling-variance pass left (pair_key): 4 bytes per pair instead of C and V's 16, no
+// per-pair bucketing of doubles, and C and V gathered only for the pairs of slot buckets (~2 %).  The same histogram
+// updates, codes and candidates as k_xcollect.  A thread takes groups of four consecutive pairs -- one 128-bit key load,
+// one 64-bit store of their codes -- XK_R groups 4 * XC_THREADS pairs apart.  Ranges start at a multiple of 1024 pairs
+// and end at one or at n, so a group never straddles two CTAs; keys at or past c1 are row padding and are masked.
+constexpr int XK_R = 2;
+
+__global__ void __launch_bounds__(XC_THREADS) k_xcollect_keys(const double *__restrict__ C, const double *__restrict__ V, long long n,
+                                                              long long row_stride, TrendBuffers T, int B)
+{
+    extern __shared__ int s_raw[];
+    int *s_yh = s_raw;                                              // [B][NBY]
+    unsigned short *s_tab = reinterpret_cast<unsigned short *>(s_raw + B * NBY);    // per |signal| bucket: bin | boundary << 7 | slot << 8
+    long long g0, g1;
+    cta_range(T.rows, n, &g0, &g1);
+    const long long np = padded_row(n);
+    for (long long g = g0; g < g1;) {
+        const long long row = g / np, c0 = g - row * np, seg = min(np - c0, g1 - g), c1 = min(n, c0 + seg);
+        g += seg;
+        const RowPlan &P = T.plan[row];
+        if (P.fallback || c0 >= c1) continue;
+        __syncthreads();                                            // the previous row's flush is done
+        for (int k = threadIdx.x; k < B * NBY; k += XC_THREADS) s_yh[k] = 0;
+        bucket_table(s_tab, T.lut + row * NBX, T.binlo + row * NBX, P, XC_THREADS);
+        __syncthreads();
+        const double *c = C + row * row_stride, *v = V + row * row_stride;
+        const unsigned *keys = T.keys + row * T.code_stride;
+        double2 *cand = T.cand + (size_t)row * MAXSLOT * CAPX;
+        int *ccnt = T.cand_cnt + row * MAXSLOT;
+        unsigned short *codes = T.codes + row * T.code_stride;
+        const int yb0 = P.yb0;
+        constexpr int U = 4 * XK_R;
+        constexpr long long STEP = 4LL * XC_THREADS * XK_R;
+        // Software-pipelined over iterations so that no iteration waits on a global round trip: the keys of iteration
+        // i + 1 are loaded during iteration i, and a thread's first two slot pairs of iteration i (~2 % of the pairs: some
+        // lane of a warp nearly always has one) get their slot counters bumped and their C and V gathered at the top of
+        // iteration i + 1, to be filed at its end.  A third or later slot pair of one iteration (rows with heavy ties) is
+        // filed on the spot after the loop body.
+        auto load_keys = [&](long long jb0, uint4 *ks) {
+#pragma unroll
+            for (int r = 0; r < XK_R; ++r) {
+                const long long jb = jb0 + 4LL * XC_THREADS * r;
+                ks[r] = jb < c1 ? *reinterpret_cast<const uint4 *>(keys + jb) : make_uint4(0u, 0u, 0u, 0u);
+            }
+        };
+        auto file_pair = [&](int off, unsigned sl) {               // one slot pair, filed with its own round trip
+            const long long j = c0 + off;
+            const int p = atomicAdd(&ccnt[sl], 1);
+            if (p < CAPX) cand[(size_t)sl * CAPX + p] = make_double2(fabs(c[j]), v[j]);
+        };
+        uint4 kn[XK_R];
+        load_keys(c0 + 4LL * threadIdx.x, kn);
+        int oc0 = -1, oc1 = -1;                                     // carried slot pairs: offset from c0 (-1: none), slot
+        unsigned sc0 = 0u, sc1 = 0u;
+        for (long long jb0 = c0 + 4LL * threadIdx.x; jb0 < c1; jb0 += STEP) {
+            uint4 ks[XK_R];
+#pragma unroll
+            for (int r = 0; r < XK_R; ++r) ks[r] = kn[r];
+            load_keys(jb0 + STEP, kn);
+            int pc0 = CAPX, pc1 = CAPX;
+            double xc0 = 0.0, yc0 = 0.0, xc1 = 0.0, yc1 = 0.0;
+            if (oc0 >= 0) { pc0 = atomicAdd(&ccnt[sc0], 1); xc0 = fabs(c[c0 + oc0]); yc0 = v[c0 + oc0]; }
+            if (oc1 >= 0) { pc1 = atomicAdd(&ccnt[sc1], 1); xc1 = fabs(c[c0 + oc1]); yc1 = v[c0 + oc1]; }
+            const int o = (int)(jb0 - c0);
+            auto off_at = [&](int u) { return o + 4 * XC_THREADS * (u >> 2) + (u & 3); };
+            int na = 0, on0 = -1, on1 = -1;
+            unsigned sn0 = 0u, sn1 = 0u, more = 0u;
+            unsigned cw[XK_R][2];
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const int r = u >> 2, q = u & 3;
+                const unsigned key = q == 0 ? ks[r].x : q == 1 ? ks[r].y : q == 2 ? ks[r].z : ks[r].w;
+                unsigned code = 0xFFFFu;
+                if (jb0 + 4LL * XC_THREADS * r + q < c1) {
+                    const unsigned e = s_tab[key >> KEY_YBITS];
+                    const bool slot = e < 0xFF00u;
+                    if (slot) {
+                        const unsigned sl = e >> 8;
+                        if (na == 0) { on0 = off_at(u); sn0 = sl; }
+                        else if (na == 1) { on1 = off_at(u); sn1 = sl; }
+                        else more |= 1u << u;
+                        ++na;
+                    }
+                    if (!(slot && (e & 0x80u))) {                   // (boundary bucket: its bin is settled by T4)
+                        const unsigned bin = e & 31u;
+                        const unsigned yb = (unsigned)min(max((int)(key & ((1u << KEY_YBITS) - 1u)) - yb0, 0), NBY - 1);
+                        atomicAdd(&s_yh[bin * NBY + yb], 1);
+                        code = (bin << 10) | yb;
+                    }
+                }
+                unsigned &word = cw[r][(u >> 1) & 1];
+                word = (u & 1) ? (word | (code << 16)) : code;
+            }
+#pragma unroll
+            for (int r = 0; r < XK_R; ++r) {
+                const long long jb = jb0 + 4LL * XC_THREADS * r;
+                if (jb < c1) *reinterpret_cast<uint2 *>(codes + jb) = make_uint2(cw[r][0], cw[r][1]);
+            }
+            if (pc0 < CAPX) cand[(size_t)sc0 * CAPX + pc0] = make_double2(xc0, yc0);
+            if (pc1 < CAPX) cand[(size_t)sc1 * CAPX + pc1] = make_double2(xc1, yc1);
+            for (; more; more &= more - 1) {                        // (the slot is looked up again from the key)
+                const int off = off_at(__ffs(more) - 1);
+                file_pair(off, (unsigned)s_tab[keys[c0 + off] >> KEY_YBITS] >> 8);
+            }
+            oc0 = on0; sc0 = sn0; oc1 = on1; sc1 = sn1;
+        }
+        if (oc0 >= 0) file_pair(oc0, sc0);                          // the last iteration's carried pairs
+        if (oc1 >= 0) file_pair(oc1, sc1);
         __syncthreads();
         int *gh = T.yhist + (size_t)row * MAXB * NBY;
         for (int k = threadIdx.x; k < B * NBY; k += XC_THREADS) {
@@ -1026,9 +1166,10 @@ __global__ void k_knots_serial(const double *bx, const double *by, const double 
 
 // ------------------------------------------------------------------ host driver
 int trend_knots_select(const double *d_C, double *d_V, long long m, long long n, long long row_stride, Knots *d_knots,
-                       int *d_row_fallback, int fused_window, cudaStream_t st)
+                       int *d_row_fallback, int fused_window, bool pair_keys, cudaStream_t st)
 {
-    // fused_window > 0: V is not computed yet -- the first pass produces it together with the |C| histogram
+    // fused_window > 0: V is not computed yet -- the first pass produces it together with the |C| histogram (and, with
+    // pair_keys, T3's 32-bit key of every pair)
     const int B = (int)fmax(4.0, floor(1.0 + (log((double)n + 1.0) / log(2.0))));      // wls_backend.c:456
     if (B > MAXB) return ST_INVALID;
     Arena ar(st);
@@ -1047,6 +1188,7 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
     RB_TRY(ar.alloc(&T.ycand_cnt, (size_t)m * MAXB * 2));
     T.code_stride = (n + 7) & ~7LL;
     RB_TRY(ar.alloc(&T.codes, (size_t)m * (size_t)T.code_stride));
+    if (fused_window > 0 && pair_keys) RB_TRY(ar.alloc(&T.keys, (size_t)m * (size_t)T.code_stride));
     RB_CUDA(cudaMemsetAsync(T.xhist, 0, sizeof(int) * (size_t)m * NBX, st));
     RB_CUDA(cudaMemsetAsync(T.cand_cnt, 0, sizeof(int) * (size_t)m * MAXSLOT, st));
     RB_CUDA(cudaMemsetAsync(T.yhist, 0, sizeof(int) * (size_t)m * MAXB * NBY, st));
@@ -1068,6 +1210,7 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
         RB_CUDA(cudaFuncSetAttribute(k_xhist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_xhist));
         RB_CUDA(cudaFuncSetAttribute(k_ycollect, cudaFuncAttributeMaxDynamicSharedMemorySize, 32768));
         RB_CUDA(cudaFuncSetAttribute(k_xcollect, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(int) * MAXB * NBY + 2 * NBX)));
+        RB_CUDA(cudaFuncSetAttribute(k_xcollect_keys, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(int) * MAXB * NBY + 2 * NBX)));
         RB_CUDA(cudaFuncSetAttribute(k_xresolve<512, 4096, CAPX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_resolve));
         RB_CUDA(cudaFuncSetAttribute(k_xresolve<512, 2048, 4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double2) * 4096)));
         RB_CUDA(cudaFuncSetAttribute(k_xplan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_plan));
@@ -1090,10 +1233,12 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
             RB_CUDA(cudaFuncSetAttribute(k_rollvar_xhist<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
             attr2 = true;
         }
-        RB_PROF("k_rollvar_xhist", st, (double)m * n * 16.0);
+        RB_PROF("k_rollvar_xhist", st, (double)m * n * (T.keys ? 20.0 : 16.0));
         const dim3 grv((unsigned)((n + RV_CHUNK - 1) / RV_CHUNK), (unsigned)m);
-        if (fused_window == 31) k_rollvar_xhist<31><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom);
-        else k_rollvar_xhist<0><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom);
+        if (fused_window == 31)
+            k_rollvar_xhist<31><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom, T.keys, T.code_stride);
+        else
+            k_rollvar_xhist<0><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom, T.keys, T.code_stride);
         RB_LAUNCH_CHECK();
     } else {
         RB_PROF("trend_xhist", st, (double)m * n * 8.0);
@@ -1106,8 +1251,10 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
         RB_LAUNCH_CHECK();
     }
     {
-        RB_PROF("trend_xcollect", st, (double)m * n * 18.0);
-        k_xcollect<<<(unsigned)sm_count(), XC_THREADS, sm_collect, st>>>(d_C, d_V, n, row_stride, T, B);
+        // with keys: 4 B of keys + 2 B of codes per pair (the gathers of slot pairs are not counted); else C, V and codes
+        RB_PROF("trend_xcollect", st, (double)m * n * (T.keys ? 6.0 : 18.0));
+        if (T.keys) k_xcollect_keys<<<(unsigned)sm_count(), XC_THREADS, sm_collect, st>>>(d_C, d_V, n, row_stride, T, B);
+        else k_xcollect<<<(unsigned)sm_count(), XC_THREADS, sm_collect, st>>>(d_C, d_V, n, row_stride, T, B);
         RB_LAUNCH_CHECK();
     }
     {
