@@ -218,17 +218,11 @@ typedef struct rocco_b200_score_params {
 void rocco_b200_default_score_params(rocco_b200_score_params *p);
 
 /* Order statistics of the variance trend: 0 = histogram multi-select with a sort fallback for rows whose
- * buckets overflow (default), 1 = sort every row, 2 = as 0 but without the 32-bit pair keys the rolling-variance
- * pass leaves the slot collection (it reads the signal and the variances instead; for A/B timing).  Any other
- * value means 0.  All are exact; returns the previous mode. */
+ * buckets overflow (default), 1 = sort every row.  Any other value means 0.  Both are exact; returns the
+ * previous mode. */
 int rocco_b200_trend_set_mode(int mode);
 long long rocco_b200_trend_fallback_rows(void);   /* rows that took the sort path since load */
 void rocco_b200_trend_fallback_reasons(long long *out8);   /* per-reason counts (diagnostics) */
-
-/* Kernel used for the interior ("steady") tiles of the Whittaker baseline: 0 = the streaming cluster-pair kernel
- * (default); 1 = the round-1 single-CTA kernel; 2 = one-shot pair kernel; 3 = same as 0.  All solve the same regions;
- * results agree to rounding.  Returns the previous mode. */
-int rocco_b200_whittaker_set_mode(int mode);
 
 /* Optional per-locus detail outputs (device or host according to the entry point); any may be NULL. */
 typedef struct rocco_b200_score_outputs {

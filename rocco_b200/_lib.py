@@ -150,7 +150,6 @@ def _declare(lib):
         "rocco_b200_default_score_params": (None, [POINTER(ScoreParams)]),
         "rocco_b200_trim_pools": (c_int, [c_size_t]),
         "rocco_b200_trend_set_mode": (c_int, [c_int]),
-        "rocco_b200_whittaker_set_mode": (c_int, [c_int]),
         "rocco_b200_trend_fallback_rows": (c_longlong, []),
         "rocco_b200_trend_fallback_reasons": (None, [c_void_p]),
         "rocco_score_loci_wls_f64": (c_int, [c_void_p, c_size_t, c_size_t, POINTER(ScoreParams), POINTER(ScoreOutputs)]),

@@ -10,9 +10,6 @@ namespace score {
 int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double *d_pilot, long long rows, long long n,
                    long long row_stride, double lam, int write_baseline, double *d_out, int *d_bad, cudaStream_t st);
 
-// 0: cluster-pair kernel for the steady tiles (default), 1: single-CTA kernel; returns the previous mode.
-int whittaker_set_mode(int mode);
-
 // Pilot offsets: per-row median of log2(max(x,0)+1) -- exact for n <= 4096, else the median of a
 // 4096-point strided sample (the offset cancels in  y - baseline(y)  up to the solver's noise).
 // exact != 0: np.median for any n (one radix sort per row).

@@ -121,7 +121,7 @@ struct TrendBuffers {
     int *ycand_cnt;        // [m][MAXB][2]
     unsigned long long *yover_min, *yover_max;   // [m][MAXB][2]  bit-pattern range of the variances that did not fit their slot
     unsigned short *codes;  // [m][code_stride]  T3 -> T6: bin << 10 | variance bucket of every pair (0xFFFF: not T6's business)
-    unsigned *keys;         // [m][code_stride]  fused rolling variance -> T3: pair_key of every pair (nullptr: T3 reads C and V)
+    unsigned *keys;         // [m][code_stride]  fused rolling variance -> T3: pair_key of every pair (fused pass only; nullptr: T3 reads C and V)
     long long code_stride;  // n rounded up to a multiple of 8 (128-bit loads)
     long long rows;
     BucketGeom geom;
@@ -173,7 +173,7 @@ __device__ __forceinline__ void cta_range(long long rows, long long n, long long
 // that hold them for the window sums; edge tiles (first / last of a row, a partial tail) read them back from shared
 // memory.  The histogram keeps 16-bit counts, two buckets per word, so that two CTAs with two tile buffers each fit
 // an SM and the barrier and store phases of one overlap the window arithmetic of the other.
-// With `keys` given, the pass also leaves T3 the pair_key of every bin, built from the bucket just counted and the
+// The pass also leaves T3 the pair_key of every bin, built from the bucket just counted and the
 // variance just computed: interior tiles store each block's 8 keys as two 128-bit stores straight from registers (block
 // starts are multiples of 8 bins, so 32-byte aligned), edge tiles one key per bin.
 constexpr int RV_T = 4096;                   // bins per CTA iteration
@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
     const long long row = blockIdx.y;
     const double *c = C + row * row_stride;
     double *v = V + row * row_stride;
-    unsigned *const kr = keys ? keys + row * key_stride : nullptr;
+    unsigned *const kr = keys + row * key_stride;
     const long long c0 = (long long)blockIdx.x * RV_CHUNK, c1 = min(n, c0 + RV_CHUNK);
     const long long half = w / 2, last = n - w;
     const double wd = (double)w, pairs = (double)(w - 1), rwd = 1.0 / wd, shrink = 1.0 + 1.0 / (wd + 1.0) + 1.0e-4;      // c1 of ar1_window_variance
@@ -286,7 +286,7 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
                     unsigned kk[4];
 #pragma unroll
                     for (int q = 0; q < 4; ++q) kk[q] = pair_key(count(y[h][W / 2 + k4 + q]), res[h][k4 + q], G);
-                    if (kr) *reinterpret_cast<uint4 *>(kr + j0 + (tid + h * RV_THREADS) * RV_K + k4) = make_uint4(kk[0], kk[1], kk[2], kk[3]);
+                    *reinterpret_cast<uint4 *>(kr + j0 + (tid + h * RV_THREADS) * RV_K + k4) = make_uint4(kk[0], kk[1], kk[2], kk[3]);
                 }
         } else {
 #pragma unroll
@@ -329,7 +329,7 @@ __global__ void __launch_bounds__(RV_THREADS, 2) k_rollvar_xhist(const double *_
             for (int k = 0; k < RV_K; ++k)
                 if (jt + k < j1) {
                     const int b = count(s_in[padpos((int)(jt + k - tlo))]);
-                    if (kr) kr[jt + k] = pair_key(b, res[h][k], G);
+                    kr[jt + k] = pair_key(b, res[h][k], G);
                 }
           }
         }
@@ -1166,10 +1166,10 @@ __global__ void k_knots_serial(const double *bx, const double *by, const double 
 
 // ------------------------------------------------------------------ host driver
 int trend_knots_select(const double *d_C, double *d_V, long long m, long long n, long long row_stride, Knots *d_knots,
-                       int *d_row_fallback, int fused_window, bool pair_keys, cudaStream_t st)
+                       int *d_row_fallback, int fused_window, cudaStream_t st)
 {
-    // fused_window > 0: V is not computed yet -- the first pass produces it together with the |C| histogram (and, with
-    // pair_keys, T3's 32-bit key of every pair)
+    // fused_window > 0: V is not computed yet -- the first pass produces it together with the |C| histogram and T3's
+    // 32-bit key of every pair
     const int B = (int)fmax(4.0, floor(1.0 + (log((double)n + 1.0) / log(2.0))));      // wls_backend.c:456
     if (B > MAXB) return ST_INVALID;
     Arena ar(st);
@@ -1188,7 +1188,7 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
     RB_TRY(ar.alloc(&T.ycand_cnt, (size_t)m * MAXB * 2));
     T.code_stride = (n + 7) & ~7LL;
     RB_TRY(ar.alloc(&T.codes, (size_t)m * (size_t)T.code_stride));
-    if (fused_window > 0 && pair_keys) RB_TRY(ar.alloc(&T.keys, (size_t)m * (size_t)T.code_stride));
+    if (fused_window > 0) RB_TRY(ar.alloc(&T.keys, (size_t)m * (size_t)T.code_stride));
     RB_CUDA(cudaMemsetAsync(T.xhist, 0, sizeof(int) * (size_t)m * NBX, st));
     RB_CUDA(cudaMemsetAsync(T.cand_cnt, 0, sizeof(int) * (size_t)m * MAXSLOT, st));
     RB_CUDA(cudaMemsetAsync(T.yhist, 0, sizeof(int) * (size_t)m * MAXB * NBY, st));
@@ -1233,7 +1233,7 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
             RB_CUDA(cudaFuncSetAttribute(k_rollvar_xhist<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
             attr2 = true;
         }
-        RB_PROF("k_rollvar_xhist", st, (double)m * n * (T.keys ? 20.0 : 16.0));
+        RB_PROF("k_rollvar_xhist", st, (double)m * n * 20.0);
         const dim3 grv((unsigned)((n + RV_CHUNK - 1) / RV_CHUNK), (unsigned)m);
         if (fused_window == 31)
             k_rollvar_xhist<31><<<grv, RV_THREADS, sm_fused, st>>>(d_C, n, row_stride, fused_window, d_V, T.xhist, T.geom, T.keys, T.code_stride);
@@ -1251,7 +1251,7 @@ int trend_knots_select(const double *d_C, double *d_V, long long m, long long n,
         RB_LAUNCH_CHECK();
     }
     {
-        // with keys: 4 B of keys + 2 B of codes per pair (the gathers of slot pairs are not counted); else C, V and codes
+        // fused pass: 4 B of keys + 2 B of codes per pair (the gathers of slot pairs are not counted); else C, V and codes
         RB_PROF("trend_xcollect", st, (double)m * n * (T.keys ? 6.0 : 18.0));
         if (T.keys) k_xcollect_keys<<<(unsigned)sm_count(), XC_THREADS, sm_collect, st>>>(d_C, d_V, n, row_stride, T, B);
         else k_xcollect<<<(unsigned)sm_count(), XC_THREADS, sm_collect, st>>>(d_C, d_V, n, row_stride, T, B);

@@ -14,11 +14,10 @@ __device__ void knots_from_bins(const double *bx, const double *by, const double
 
 // Histogram multi-select for all m rows; rows it cannot handle (a bucket over capacity) get row_fallback = 1.
 // fused_window > 0: d_V is an OUTPUT -- the rolling AR(1) variance (window `fused_window`, already resolved) is
-// computed in the same pass as the first histogram; fused_window == 0: d_V is an input.  pair_keys (fused pass only):
-// that pass also writes a 32-bit key per pair (4 B per sample-bin of scratch), and the slot collection reads those
-// instead of C and V.
+// computed in the same pass as the first histogram, which also writes a 32-bit key per pair (4 B per sample-bin of
+// scratch) that the slot collection reads instead of C and V; fused_window == 0: d_V is an input.
 int trend_knots_select(const double *d_C, double *d_V, long long m, long long n, long long row_stride, Knots *d_knots,
-                       int *d_row_fallback, int fused_window, bool pair_keys, cudaStream_t st);
+                       int *d_row_fallback, int fused_window, cudaStream_t st);
 int trend_fused_max_window();
 
 }  // namespace score

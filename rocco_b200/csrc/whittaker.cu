@@ -9,14 +9,21 @@
 //    itself) and only the last two rows deviate.  The host computes a short head table, the steady
 //    pair and a 4-entry tail once per (n, lambda);
 //  * forward / backward substitution are second-order linear recurrences, i.e. IIR filters whose
-//    impulse response decays like 0.9775^k for the default window.  Each CTA solves one tile plus a
+//    impulse response decays like 0.9775^k for the default window.  Each tile is solved with a
 //    halo of HALO bins on both sides from a zero state; the truncation error at the tile is
 //    0.9775^1280 ~ 2e-13 of the signal, below the reference's own ~1e-10 noise floor;
-//  * inside a CTA every thread owns ITEMS consecutive bins: a zero-state local sweep, a
-//    Kogge-Stone scan of the 2-vector carry across threads, then the true sweep.  Both parities run
-//    interleaved in the same thread (two independent dependency chains).
+//  * every thread owns ITEMS consecutive bins: a zero-state local sweep, a scan of the 2-vector
+//    carry across threads, then the true sweep.  Both parities run interleaved in the same thread
+//    (two independent dependency chains).
 //
-// The same kernel fuses the reference's Python prologue: y = log2(max(x,0)+1) - pilot_row
+// Kernels:
+//  * k_whittaker_stream: interior ("steady") tiles, whose coefficients are the period-2 steady state.  A
+//    persistent grid of two-CTA clusters, one cluster per tile region at a time;
+//  * k_whittaker: the first and last tile(s) of a row, which read the head and tail tables.  One CTA per
+//    region, with a general carry scan over per-chunk transitions;
+//  * k_small_rows: rows shorter than 25 bins.
+//
+// Both tile kernels fuse the reference's Python prologue: y = log2(max(x,0)+1) - pilot_row
 // (inference.py:40-47, 333-334) and the epilogue  centered = y - baseline  (inference.py:338).
 #include "common.cuh"
 #include "score.cuh"
@@ -35,11 +42,7 @@ namespace score {
 constexpr int WT_REGION = 12288;                   // bins solved per CTA
 constexpr int WT_HALO = 1280;
 constexpr int WT_OUT = WT_REGION - 2 * WT_HALO;    // 9728 bins written per CTA
-// two thread geometries over the same region: steady (interior) tiles use 1024 threads x 12 bins (32 warps per SM to
-// hide the FP64 dependency chains), edge tiles 512 x 24 (the general carry scan needs the extra shared memory)
-constexpr int WT_THREADS_S = 1024, WT_ITEMS_S = 12;
-constexpr int WT_THREADS_G = 512, WT_ITEMS_G = 24;
-constexpr int WT_LEVELS = 10;                      // log2(max threads)
+constexpr int WT_THREADS_G = 512, WT_ITEMS_G = 24; // edge tiles (k_whittaker): one CTA per region
 constexpr int HEAD_LEN = 4096;
 
 // ------------------------------------------------------------------ host: factor tables
@@ -73,16 +76,14 @@ static void host_factor(long long n_true, long long len, int parity, double lam,
     }
 }
 
-// Tables of the cluster-pair kernel for one alignment shift parity `ap` (region position 0 has index parity ap):
+// Tables of the streaming kernel for one alignment shift parity `ap` (region position 0 has index parity ap):
 // chain A carries the rhs of the even region positions (parity p = ap), chain B the odd ones (p = 1 - ap).
 constexpr int WP_HALF = 6144;                      // bins per CTA, two CTAs per region
 constexpr int WP_MAXWARPS = 16;
 constexpr int WP_LEVELS = 9;                       // 5 in-warp levels + 4 across the warps of a CTA
-// thread geometry of the pair kernels (threads x bins per thread = WP_HALF): 512 x 12 (384 x 16 and a cluster of four
+// thread geometry of the streaming kernel (threads x bins per thread = WP_HALF): 512 x 12 (384 x 16 and a cluster of four
 // 256-thread CTAs were measured slower: fewer resident warps / no gain from the finer phases)
-constexpr int WP_NGEOM = 1;
-constexpr int WP_GEOM_THREADS[WP_NGEOM] = {512};
-constexpr int WP_GEOM_ITEMS[WP_NGEOM] = {12};
+constexpr int WP_GEOM_THREADS = 512, WP_GEOM_ITEMS = 12;
 struct PairTab {
     double cf[2][3][2];                            // [chain][dinv, l1, l2][position parity]
     double trans[2][2][WP_LEVELS][4];              // [chain][fwd/bwd][level]: transition over ITEMS * 2^level bins
@@ -96,13 +97,11 @@ struct PairPow {
 
 struct FactorHost {
     int head_len = 0;
-    PairTab pair_tab[WP_NGEOM][2];                 // [geometry][alignment shift parity]
-    PairPow pair_pow[WP_NGEOM][2];
+    PairTab pair_tab[2];                           // [alignment shift parity]
+    PairPow pair_pow[2];
     std::vector<double> head[2][3];      // [parity][dinv,l1,l2][head_len]
     double steady[2][3][2];              // [parity][coef][index parity]
     double tail[2][3][4];                // rows n-4 .. n-1
-    double trans[2][2][WT_LEVELS + 1][4];  // [parity][fwd/bwd][level] 2x2 transition over WT_ITEMS_S * 2^level bins
-    double lanepow[2][2][32][4];           // [parity][fwd/bwd][k] transition over (k+1) chunks: T^(k+1)
 };
 
 static void mat2_mul(const double *a, const double *b, double *c)   // c = a*b (row-major 2x2)
@@ -151,41 +150,12 @@ static void build_factor(long long n, double lam, FactorHost &F)
         } else {
             for (int k = 0; k < 4; ++k) F.tail[p][0][k] = F.tail[p][1][k] = F.tail[p][2][k] = 0.0;
         }
-        // transition matrices of the homogeneous recurrences over one thread chunk (ITEMS bins, steady state)
-        // forward state (f[i], f[i-1]):  f[i] = -l1[i-1] f[i-1] - l2[i-2] f[i-2]
-        // backward state (x[i], x[i+1]): x[i] = -l1[i] x[i+1] - l2[i] x[i+2]
-        // chunks start on an even index (region starts are even), so index parity == position parity
-        double Tf[4] = {1, 0, 0, 1}, Tb[4] = {1, 0, 0, 1};
-        for (int j = 0; j < WT_ITEMS_S; ++j) {                // forward: j = position in chunk, index parity j&1
-            const double c1 = F.steady[p][1][(j + 1) & 1];    // l1[i-1]
-            const double c2 = F.steady[p][2][j & 1];          // l2[i-2]
-            const double S[4] = {-c1, -c2, 1.0, 0.0};
-            mat2_mul(S, Tf, Tf);
-        }
-        for (int j = WT_ITEMS_S - 1; j >= 0; --j) {           // backward
-            const double c1 = F.steady[p][1][j & 1], c2 = F.steady[p][2][j & 1];
-            const double S[4] = {-c1, -c2, 1.0, 0.0};
-            mat2_mul(S, Tb, Tb);
-        }
-        for (int k = 0; k < 4; ++k) { F.trans[p][0][0][k] = Tf[k]; F.trans[p][1][0][k] = Tb[k]; }
-        for (int l = 1; l <= WT_LEVELS; ++l) {
-            mat2_mul(F.trans[p][0][l - 1], F.trans[p][0][l - 1], F.trans[p][0][l]);
-            mat2_mul(F.trans[p][1][l - 1], F.trans[p][1][l - 1], F.trans[p][1][l]);
-        }
-        for (int dct = 0; dct < 2; ++dct) {
-            double acc[4] = {1, 0, 0, 1};
-            for (int k = 0; k < 32; ++k) {
-                mat2_mul(F.trans[p][dct][0], acc, acc);
-                for (int q = 0; q < 4; ++q) F.lanepow[p][dct][k][q] = acc[q];
-            }
-        }
     }
-    // cluster-pair kernel: chains by region-position parity, for both alignment shift parities
-    for (int gm = 0; gm < WP_NGEOM; ++gm)
+    // streaming kernel: chains by region-position parity, for both alignment shift parities
+    constexpr int WP_ITEMS = WP_GEOM_ITEMS, WP_WARPS = WP_GEOM_THREADS / 32;
     for (int ap = 0; ap < 2; ++ap) {
-        const int WP_ITEMS = WP_GEOM_ITEMS[gm], WP_WARPS = WP_GEOM_THREADS[gm] / 32;
-        PairTab &T = F.pair_tab[gm][ap];
-        PairPow &W = F.pair_pow[gm][ap];
+        PairTab &T = F.pair_tab[ap];
+        PairPow &W = F.pair_pow[ap];
         for (int ch = 0; ch < 2; ++ch) {
             const int p = ch ^ ap;                                  // parity mask served by this chain
             for (int k = 0; k < 3; ++k)
@@ -276,7 +246,7 @@ __device__ __forceinline__ double fast_log2_ge1(double v, const double *s_inv, c
 }
 
 
-// Leaner variant for the pair kernel: a 32-entry interleaved table {inv[i], tab[i]} (one 128-bit shared load; 512 bytes, so
+// Leaner variant for the streaming kernel: a 32-entry interleaved table {inv[i], tab[i]} (one 128-bit shared load; 512 bytes, so
 // that the 32 lanes' lookups rarely collide on a bank), |r| <= 2^-6 and the degree-7 polynomial above (truncation
 // r^8 / (8 ln 2) < 1e-15 absolute, five orders below the solver's noise floor), exponent converted with the 2^52 trick
 // instead of I2F.  Exact for powers of two (zero counts give 0.0) like the function above.
@@ -305,8 +275,6 @@ struct WhitParams {
     const double *head[2][3];   // device head tables
     double steady[2][3][2];
     double tail[2][3][4];
-    double trans[2][2][WT_LEVELS + 1][4];
-    const double *lanepow;      // device copy of FactorHost::lanepow, [parity][dir][32][4]
     const double *log2tab;      // device copy of Log2Tables (inv[128], tab[128])
     long long n;
     long long row_stride;       // elements between rows of x / out
@@ -338,56 +306,6 @@ __device__ __forceinline__ double coef(const WhitParams &P, int p, int k, long l
     if (i < P.head_len) return P.head[p][k][i];
     if (i >= P.n - 4) return P.tail[p][k][i - (P.n - 4)];
     return P.steady[p][k][i & 1];
-}
-
-// Carry scan for the uniform (steady) case: state_t = r_t + T r_{t-1} + T^2 r_{t-2} + ...
-// `v` holds the chunk's zero-state end vector on entry, the inclusive carry on exit.
-//   1. Kogge-Stone inside each warp with T^(2^l);  2. warp 0 scans the warp totals with T^(32 * 2^l);
-//   3. every lane adds T^(lane+1) applied to the state entering its warp (table `lp`, staged in shared memory).
-template <int THREADS>
-__device__ __forceinline__ void carry_scan_uniform(double &v0, double &v1, const double (*T)[4], const double *lp /* [32][4] */,
-                                                   bool reverse, double2 *s_warp /* [THREADS/32] */)
-{
-    constexpr int NW = THREADS / 32;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int lpos = reverse ? 31 - lane : lane;
-#pragma unroll
-    for (int l = 0; l < 5; ++l) {
-        const int dlt = 1 << l;
-        const double o0 = reverse ? __shfl_down_sync(0xffffffffu, v0, dlt) : __shfl_up_sync(0xffffffffu, v0, dlt);
-        const double o1 = reverse ? __shfl_down_sync(0xffffffffu, v1, dlt) : __shfl_up_sync(0xffffffffu, v1, dlt);
-        if (lpos >= dlt) {
-            v0 += T[l][0] * o0 + T[l][1] * o1;
-            v1 += T[l][2] * o0 + T[l][3] * o1;
-        }
-    }
-    const int wpos = reverse ? NW - 1 - wid : wid;            // position of this warp in scan order
-    if (lpos == 31) s_warp[wpos] = make_double2(v0, v1);
-    __syncthreads();
-    if (wid == 0) {
-        double a0 = 0.0, a1 = 0.0;
-        if (lane < NW) { const double2 t = s_warp[lane]; a0 = t.x; a1 = t.y; }
-#pragma unroll
-        for (int l = 0; (1 << l) < NW; ++l) {
-            const int dlt = 1 << l;
-            const double o0 = __shfl_up_sync(0xffffffffu, a0, dlt), o1 = __shfl_up_sync(0xffffffffu, a1, dlt);
-            if (lane >= dlt) {
-                a0 += T[5 + l][0] * o0 + T[5 + l][1] * o1;
-                a1 += T[5 + l][2] * o0 + T[5 + l][3] * o1;
-            }
-        }
-        // exclusive: the state entering warp w is the inclusive value of warp w-1
-        const double e0 = __shfl_up_sync(0xffffffffu, a0, 1), e1 = __shfl_up_sync(0xffffffffu, a1, 1);
-        if (lane < NW) s_warp[lane] = (lane == 0) ? make_double2(0.0, 0.0) : make_double2(e0, e1);
-    }
-    __syncthreads();
-    {
-        const double2 e = s_warp[wpos];
-        const double *m = lp + lpos * 4;
-        v0 += m[0] * e.x + m[1] * e.y;
-        v1 += m[2] * e.x + m[3] * e.y;
-    }
-    __syncthreads();
 }
 
 // General carry scan (chunks with their own transition matrices: first / last tile of a row).
@@ -423,21 +341,18 @@ __device__ __forceinline__ void carry_scan_general(double &v0, double &v1, doubl
     }
 }
 
-template <bool STEADY, int WT_THREADS, int WT_ITEMS>
+// First and last tile(s) of a row: the coefficients vary along the region (head table, tail rows, row ends) and the
+// region may be short, so every chunk builds its own transition and the carry scan is the general one.
+template <int WT_THREADS, int WT_ITEMS>
 __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
 {
     constexpr int WT_PAD = WT_ITEMS + 1;
     extern __shared__ double smem[];
     double *s_f0 = smem;                             // WT_THREADS * WT_PAD
     double *s_f1 = smem + WT_THREADS * WT_PAD;
-    __shared__ double2 s_warp[WT_THREADS / 32];
-    __shared__ double s_lp[STEADY ? 4 * 32 * 4 : 1];  // T^(k+1) tables: [parity][dir][32][4]
     __shared__ double s_log[256];                     // fast-log2 tables: inv[128], tab[128]
     for (int k = threadIdx.x; k < 256; k += WT_THREADS) s_log[k] = P.log2tab[k];
     __syncthreads();
-    if (STEADY) {
-        for (int k = threadIdx.x; k < 4 * 32 * 4; k += WT_THREADS) s_lp[k] = P.lanepow[k];
-    }
 
     const int tid = threadIdx.x;
     const long long row = blockIdx.x / P.span_tiles;
@@ -447,7 +362,6 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
     long long r0 = out0 - WT_HALO; if (r0 < 0) r0 = 0;               // region solved (even start)
     long long r1 = out1 + WT_HALO; if (r1 > P.n) r1 = P.n;
     const int rlen = (int)(r1 - r0);
-    // STEADY instantiation is only launched for CTAs whose region lies in [head_len, n-4)
 
     // ---- stage rhs (masked y) for both parities, coalesced; four loads in flight per thread before any arithmetic
     int bad = 0;
@@ -459,24 +373,21 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
     double *outp = P.out + rbase;
     const double pil = (P.log_transform && P.pilot) ? P.pilot[row] : 0.0;
     const bool par0 = ((r0 & 1) == 0);
-    // STEADY: the region is always complete (rlen == WT_REGION) and all twelve loads of a thread are issued before
-    // any arithmetic; every bin is stored once, into the array of its own parity -- the other array's slot would hold the
-    // masked zero, which the forward sweeps below supply as a literal instead of loading it.
-    constexpr int LD = STEADY ? WT_ITEMS : 4;
+    constexpr int LD = 4;
 #pragma unroll 1
     for (int e0 = tid; e0 < WT_REGION; e0 += LD * WT_THREADS) {
         double raw[LD];
 #pragma unroll
         for (int u = 0; u < LD; ++u) {
             const int e = e0 + u * WT_THREADS;
-            raw[u] = (STEADY || e < rlen) ? (P.in_f32 ? (double)xf[e] : xd[e]) : 0.0;
+            raw[u] = (e < rlen) ? (P.in_f32 ? (double)xf[e] : xd[e]) : 0.0;
         }
 #pragma unroll
         for (int u = 0; u < LD; ++u) {
             const int e = e0 + u * WT_THREADS;
-            if (!STEADY && e >= WT_REGION) break;
+            if (e >= WT_REGION) break;
             double y = 0.0;
-            if (STEADY || e < rlen) {
+            if (e < rlen) {
                 y = raw[u];
                 // inference.py:45-46 rejects non-finite input (fmax would swallow NaN / -inf); a finite input gives a
                 // finite y, so one test serves both the input check and the result check
@@ -489,12 +400,8 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
             }
             const int a = e + e / WT_ITEMS;
             const bool even = (((e & 1) == 0) == par0);
-            if (STEADY) {
-                if (even) s_f0[a] = y; else s_f1[a] = y;
-            } else {
-                s_f0[a] = even ? y : 0.0;
-                s_f1[a] = even ? 0.0 : y;
-            }
+            s_f0[a] = even ? y : 0.0;
+            s_f1[a] = even ? 0.0 : y;
         }
     }
     if (bad) *P.bad = 1;
@@ -504,42 +411,29 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
     const long long i0 = r0 + base;                                   // global index of that bin
     double *f0 = s_f0 + tid * WT_PAD, *f1 = s_f1 + tid * WT_PAD;
     const int cnt = max(0, min(WT_ITEMS, rlen - base));
-
-    // per-parity steady coefficients by position parity (i0 is even)
-    double c_l1[2][2], c_l2[2][2], c_di[2][2];
-    if (STEADY) {
-#pragma unroll
-        for (int p = 0; p < 2; ++p)
-#pragma unroll
-            for (int q = 0; q < 2; ++q) { c_di[p][q] = P.steady[p][0][q]; c_l1[p][q] = P.steady[p][1][q]; c_l2[p][q] = P.steady[p][2][q]; }
-    }
+    double *s_buf = reinterpret_cast<double *>(smem + 2 * WT_THREADS * WT_PAD);
 
     // ================= forward substitution  L f = rhs
-    // pass A: zero-state sweep -> end vector (f[last], f[last-1]); general case also builds the chunk transition
+    // pass A: zero-state sweep -> end vector (f[last], f[last-1]) and the chunk transition
     double e00 = 0.0, e01 = 0.0, e10 = 0.0, e11 = 0.0;        // parity0: (f, fprev) ; parity1: (f, fprev)
-    double ha[2][4];                                          // general: homogeneous solutions per parity
-    if (!STEADY) { for (int p = 0; p < 2; ++p) { ha[p][0] = 1.0; ha[p][1] = 0.0; ha[p][2] = 0.0; ha[p][3] = 1.0; } }
+    double ha[2][4];                                          // homogeneous solutions per parity
+    for (int p = 0; p < 2; ++p) { ha[p][0] = 1.0; ha[p][1] = 0.0; ha[p][2] = 0.0; ha[p][3] = 1.0; }
     {
         double a1 = 0.0, a2 = 0.0, b1 = 0.0, b2 = 0.0;        // f[i-1], f[i-2] per parity
 #pragma unroll
         for (int j = 0; j < WT_ITEMS; ++j) {
-            if (STEADY || j < cnt) {
-                double l1a, l2a, l1b, l2b;
-                if (STEADY) { l1a = c_l1[0][(j + 1) & 1]; l2a = c_l2[0][j & 1]; l1b = c_l1[1][(j + 1) & 1]; l2b = c_l2[1][j & 1]; }
-                else {
-                    const long long i = i0 + j;
-                    l1a = i >= 1 ? coef(P, 0, 1, i - 1) : 0.0; l2a = i >= 2 ? coef(P, 0, 2, i - 2) : 0.0;
-                    l1b = i >= 1 ? coef(P, 1, 1, i - 1) : 0.0; l2b = i >= 2 ? coef(P, 1, 2, i - 2) : 0.0;
-                    // homogeneous: h[i] = -l1 h[i-1] - l2 h[i-2] for the two unit start states
-                    for (int p = 0; p < 2; ++p) {
-                        const double l1 = p ? l1b : l1a, l2 = p ? l2b : l2a;
-                        const double n0 = -l1 * ha[p][0] - l2 * ha[p][2], n1 = -l1 * ha[p][1] - l2 * ha[p][3];
-                        ha[p][2] = ha[p][0]; ha[p][3] = ha[p][1]; ha[p][0] = n0; ha[p][1] = n1;
-                    }
+            if (j < cnt) {
+                const long long i = i0 + j;
+                const double l1a = i >= 1 ? coef(P, 0, 1, i - 1) : 0.0, l2a = i >= 2 ? coef(P, 0, 2, i - 2) : 0.0;
+                const double l1b = i >= 1 ? coef(P, 1, 1, i - 1) : 0.0, l2b = i >= 2 ? coef(P, 1, 2, i - 2) : 0.0;
+                // homogeneous: h[i] = -l1 h[i-1] - l2 h[i-2] for the two unit start states
+                for (int p = 0; p < 2; ++p) {
+                    const double l1 = p ? l1b : l1a, l2 = p ? l2b : l2a;
+                    const double n0 = -l1 * ha[p][0] - l2 * ha[p][2], n1 = -l1 * ha[p][1] - l2 * ha[p][3];
+                    ha[p][2] = ha[p][0]; ha[p][3] = ha[p][1]; ha[p][0] = n0; ha[p][1] = n1;
                 }
-                const double ra = (STEADY && (j & 1)) ? 0.0 : f0[j], rb_ = (STEADY && !(j & 1)) ? 0.0 : f1[j];
-                const double na = fma(-l2a, a2, fma(-l1a, a1, ra));
-                const double nb = fma(-l2b, b2, fma(-l1b, b1, rb_));
+                const double na = fma(-l2a, a2, fma(-l1a, a1, f0[j]));
+                const double nb = fma(-l2b, b2, fma(-l1b, b1, f1[j]));
                 a2 = a1; a1 = na; b2 = b1; b1 = nb;
             }
         }
@@ -547,14 +441,8 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
     }
     // carry: state entering chunk t = inclusive scan value of chunk t-1
     double in00, in01, in10, in11;
-    if (STEADY) {
-        carry_scan_uniform<WT_THREADS>(e00, e01, P.trans[0][0], s_lp + (0 * 2 + 0) * 128, false, s_warp);
-        carry_scan_uniform<WT_THREADS>(e10, e11, P.trans[1][0], s_lp + (1 * 2 + 0) * 128, false, s_warp);
-    } else {
-        double *s_buf = reinterpret_cast<double *>(smem + 2 * WT_THREADS * WT_PAD);
-        carry_scan_general<WT_THREADS>(e00, e01, ha[0][0], ha[0][1], ha[0][2], ha[0][3], false, s_buf);
-        carry_scan_general<WT_THREADS>(e10, e11, ha[1][0], ha[1][1], ha[1][2], ha[1][3], false, s_buf);
-    }
+    carry_scan_general<WT_THREADS>(e00, e01, ha[0][0], ha[0][1], ha[0][2], ha[0][3], false, s_buf);
+    carry_scan_general<WT_THREADS>(e10, e11, ha[1][0], ha[1][1], ha[1][2], ha[1][3], false, s_buf);
     in00 = __shfl_up_sync(0xffffffffu, e00, 1); in01 = __shfl_up_sync(0xffffffffu, e01, 1);
     in10 = __shfl_up_sync(0xffffffffu, e10, 1); in11 = __shfl_up_sync(0xffffffffu, e11, 1);
     {
@@ -572,20 +460,13 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
         double a1 = in00, a2 = in01, b1 = in10, b2 = in11;
 #pragma unroll
         for (int j = 0; j < WT_ITEMS; ++j) {
-            if (STEADY || j < cnt) {
-                double l1a, l2a, l1b, l2b, da, db;
-                if (STEADY) {
-                    l1a = c_l1[0][(j + 1) & 1]; l2a = c_l2[0][j & 1]; l1b = c_l1[1][(j + 1) & 1]; l2b = c_l2[1][j & 1];
-                    da = c_di[0][j & 1]; db = c_di[1][j & 1];
-                } else {
-                    const long long i = i0 + j;
-                    l1a = i >= 1 ? coef(P, 0, 1, i - 1) : 0.0; l2a = i >= 2 ? coef(P, 0, 2, i - 2) : 0.0;
-                    l1b = i >= 1 ? coef(P, 1, 1, i - 1) : 0.0; l2b = i >= 2 ? coef(P, 1, 2, i - 2) : 0.0;
-                    da = coef(P, 0, 0, i); db = coef(P, 1, 0, i);
-                }
-                const double ra = (STEADY && (j & 1)) ? 0.0 : f0[j], rb_ = (STEADY && !(j & 1)) ? 0.0 : f1[j];
-                const double na = fma(-l2a, a2, fma(-l1a, a1, ra));
-                const double nb = fma(-l2b, b2, fma(-l1b, b1, rb_));
+            if (j < cnt) {
+                const long long i = i0 + j;
+                const double l1a = i >= 1 ? coef(P, 0, 1, i - 1) : 0.0, l2a = i >= 2 ? coef(P, 0, 2, i - 2) : 0.0;
+                const double l1b = i >= 1 ? coef(P, 1, 1, i - 1) : 0.0, l2b = i >= 2 ? coef(P, 1, 2, i - 2) : 0.0;
+                const double da = coef(P, 0, 0, i), db = coef(P, 1, 0, i);
+                const double na = fma(-l2a, a2, fma(-l1a, a1, f0[j]));
+                const double nb = fma(-l2b, b2, fma(-l1b, b1, f1[j]));
                 a2 = a1; a1 = na; b2 = b1; b1 = nb;
                 f0[j] = na * da; f1[j] = nb * db;
             }
@@ -593,23 +474,19 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
     }
 
     // ================= backward substitution  L' x = z   (right to left)
-    if (!STEADY) { for (int p = 0; p < 2; ++p) { ha[p][0] = 1.0; ha[p][1] = 0.0; ha[p][2] = 0.0; ha[p][3] = 1.0; } }
+    for (int p = 0; p < 2; ++p) { ha[p][0] = 1.0; ha[p][1] = 0.0; ha[p][2] = 0.0; ha[p][3] = 1.0; }
     {
         double a1 = 0.0, a2 = 0.0, b1 = 0.0, b2 = 0.0;        // x[i+1], x[i+2]
 #pragma unroll
         for (int j = WT_ITEMS - 1; j >= 0; --j) {
-            if (STEADY || j < cnt) {
-                double l1a, l2a, l1b, l2b;
-                if (STEADY) { l1a = c_l1[0][j & 1]; l2a = c_l2[0][j & 1]; l1b = c_l1[1][j & 1]; l2b = c_l2[1][j & 1]; }
-                else {
-                    const long long i = i0 + j;
-                    l1a = (i + 1 < P.n) ? coef(P, 0, 1, i) : 0.0; l2a = (i + 2 < P.n) ? coef(P, 0, 2, i) : 0.0;
-                    l1b = (i + 1 < P.n) ? coef(P, 1, 1, i) : 0.0; l2b = (i + 2 < P.n) ? coef(P, 1, 2, i) : 0.0;
-                    for (int p = 0; p < 2; ++p) {
-                        const double l1 = p ? l1b : l1a, l2 = p ? l2b : l2a;
-                        const double n0 = -l1 * ha[p][0] - l2 * ha[p][2], n1 = -l1 * ha[p][1] - l2 * ha[p][3];
-                        ha[p][2] = ha[p][0]; ha[p][3] = ha[p][1]; ha[p][0] = n0; ha[p][1] = n1;
-                    }
+            if (j < cnt) {
+                const long long i = i0 + j;
+                const double l1a = (i + 1 < P.n) ? coef(P, 0, 1, i) : 0.0, l2a = (i + 2 < P.n) ? coef(P, 0, 2, i) : 0.0;
+                const double l1b = (i + 1 < P.n) ? coef(P, 1, 1, i) : 0.0, l2b = (i + 2 < P.n) ? coef(P, 1, 2, i) : 0.0;
+                for (int p = 0; p < 2; ++p) {
+                    const double l1 = p ? l1b : l1a, l2 = p ? l2b : l2a;
+                    const double n0 = -l1 * ha[p][0] - l2 * ha[p][2], n1 = -l1 * ha[p][1] - l2 * ha[p][3];
+                    ha[p][2] = ha[p][0]; ha[p][3] = ha[p][1]; ha[p][0] = n0; ha[p][1] = n1;
                 }
                 const double na = fma(-l2a, a2, fma(-l1a, a1, f0[j]));
                 const double nb = fma(-l2b, b2, fma(-l1b, b1, f1[j]));
@@ -618,14 +495,8 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
         }
         e00 = a1; e01 = a2; e10 = b1; e11 = b2;
     }
-    if (STEADY) {
-        carry_scan_uniform<WT_THREADS>(e00, e01, P.trans[0][1], s_lp + (0 * 2 + 1) * 128, true, s_warp);
-        carry_scan_uniform<WT_THREADS>(e10, e11, P.trans[1][1], s_lp + (1 * 2 + 1) * 128, true, s_warp);
-    } else {
-        double *s_buf = reinterpret_cast<double *>(smem + 2 * WT_THREADS * WT_PAD);
-        carry_scan_general<WT_THREADS>(e00, e01, ha[0][0], ha[0][1], ha[0][2], ha[0][3], true, s_buf);
-        carry_scan_general<WT_THREADS>(e10, e11, ha[1][0], ha[1][1], ha[1][2], ha[1][3], true, s_buf);
-    }
+    carry_scan_general<WT_THREADS>(e00, e01, ha[0][0], ha[0][1], ha[0][2], ha[0][3], true, s_buf);
+    carry_scan_general<WT_THREADS>(e10, e11, ha[1][0], ha[1][1], ha[1][2], ha[1][3], true, s_buf);
     in00 = __shfl_down_sync(0xffffffffu, e00, 1); in01 = __shfl_down_sync(0xffffffffu, e01, 1);
     in10 = __shfl_down_sync(0xffffffffu, e10, 1); in11 = __shfl_down_sync(0xffffffffu, e11, 1);
     {
@@ -642,14 +513,10 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
         double a1 = in00, a2 = in01, b1 = in10, b2 = in11;
 #pragma unroll
         for (int j = WT_ITEMS - 1; j >= 0; --j) {
-            if (STEADY || j < cnt) {
-                double l1a, l2a, l1b, l2b;
-                if (STEADY) { l1a = c_l1[0][j & 1]; l2a = c_l2[0][j & 1]; l1b = c_l1[1][j & 1]; l2b = c_l2[1][j & 1]; }
-                else {
-                    const long long i = i0 + j;
-                    l1a = (i + 1 < P.n) ? coef(P, 0, 1, i) : 0.0; l2a = (i + 2 < P.n) ? coef(P, 0, 2, i) : 0.0;
-                    l1b = (i + 1 < P.n) ? coef(P, 1, 1, i) : 0.0; l2b = (i + 2 < P.n) ? coef(P, 1, 2, i) : 0.0;
-                }
+            if (j < cnt) {
+                const long long i = i0 + j;
+                const double l1a = (i + 1 < P.n) ? coef(P, 0, 1, i) : 0.0, l2a = (i + 2 < P.n) ? coef(P, 0, 2, i) : 0.0;
+                const double l1b = (i + 1 < P.n) ? coef(P, 1, 1, i) : 0.0, l2b = (i + 2 < P.n) ? coef(P, 1, 2, i) : 0.0;
                 const double na = fma(-l2a, a2, fma(-l1a, a1, f0[j]));
                 const double nb = fma(-l2b, b2, fma(-l1b, b1, f1[j]));
                 a2 = a1; a1 = na; b2 = b1; b1 = nb;
@@ -661,7 +528,7 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
 
     // ---- write the tile (coalesced); y comes back from where the staging loop parked it (an L2 hit)
     int bad2 = 0;
-    constexpr int LDE = STEADY ? 5 : 4;                       // steady tiles: 9728 own bins = 9.5 per thread -> two rounds of five
+    constexpr int LDE = 4;
 #pragma unroll 1
     for (int e0 = o_lo + tid; e0 < o_hi; e0 += LDE * WT_THREADS) {
         double yv[LDE];
@@ -684,24 +551,31 @@ __global__ void __launch_bounds__(WT_THREADS, 1) k_whittaker(WhitParams P)
 }
 
 
-// ------------------------------------------------------------------ steady tiles, cluster-pair form
-// The same 12288-bin region (9728 own bins + two 1280-bin halos) is solved by a CLUSTER of two CTAs, each holding one
-// half (6144 bins, ~113 KB of shared memory), so that two CTAs of different tiles are resident per SM and the
-// barrier-separated phases of one overlap the sweeps of the other:
-//   * the half's raw input and the scan tables arrive by bulk async copies (cp.async.bulk, completion on an mbarrier);
-//     the raw bins land in the shared memory that later holds the second chain's forward solution.  Every thread reads
-//     its own consecutive bins with 128-bit shared loads and keeps y = log2(max(x,0)+1) - pilot in registers;
-//   * the carry scan runs inside the warp (shuffles), across the warps (warp 0), and across the two CTAs: the left CTA
-//     hands its total to the right one for the forward substitution, the right CTA to the left one for the backward
-//     substitution, with st.async into the peer's shared memory (DSMEM) completing on the peer's mbarrier -- only the
-//     receiver waits, and there is no cluster-scope fence after start-up (which would also invalidate L1);
-//   * centered = y - baseline is laid out contiguously in shared memory and leaves as ONE bulk store per CTA
-//     (whole lines; a scalar head/tail element where the row start is only 8-byte aligned).
+// ------------------------------------------------------------------ steady tiles: streaming cluster-pair kernel
+// A 12288-bin region (9728 own bins + two 1280-bin halos) is solved by a CLUSTER of two CTAs, each holding one half
+// (6144 bins), and two CTAs are resident per SM, so that the barrier-separated phases of one overlap the sweeps of the
+// other.  The grid is PERSISTENT: as many clusters as are co-resident walk the (row, tile) list, and the raw input of a
+// cluster's next tile is in flight (bulk async copy, cp.async.bulk completing on an mbarrier, into the second of two
+// landing buffers) while the current one is solved, so that neither the load latency at the start of a tile nor the
+// drain of its bulk store at the end is exposed; the scan tables are loaded once per CTA.
+//   * every thread reads its own consecutive bins with 128-bit shared loads and keeps y = log2(max(x,0)+1) - pilot in
+//     registers;
+//   * the carry scan runs inside the warp (shuffles), across the warps, and across the two CTAs: the left CTA hands its
+//     total to the right one for the forward substitution, the right CTA to the left one for the backward substitution,
+//     with st.async into the peer's shared memory (DSMEM) completing on the peer's mbarrier -- only the receiver waits,
+//     and there is no cluster-scope fence after start-up (which would also invalidate L1);
+//   * the true forward sweep also accumulates the zero-state end vector of the chunk's backward sweep, which is linear
+//     in the z_j (table g), so the backward substitution needs one sweep instead of two;
+//   * the forward solution is not stored: the backward sweep re-derives it by running the forward recurrence right to
+//     left from the chunk's final state (n_{j-2} = (r_j - n_j - l1 n_{j-1}) / l2; twelve steps of a recurrence whose
+//     reverse growth is 1/0.9775 per bin, i.e. ~1e-16 relative);
+//   * the result is written over the thread's own slots of the landing buffer and leaves from there as ONE bulk store
+//     per CTA (whole lines; a scalar head/tail element where the row start is only 8-byte aligned).
 // A bulk copy needs a 16-byte aligned source: the region starts `shift` bins left of the tile's nominal (even) start.
 // An odd shift swaps which parity mask sits on the even region positions, hence the per-launch chain tables.
 struct PairParams {
     const void *x; const double *pilot; double *out; int *bad;
-    const double *pow_tab;      // PairPow of this geometry and shift parity (device)
+    const double *pow_tab;      // PairPow of this shift parity (device)
     const double *log2tab;      // LOG2_V2_ENTRIES x {inv, tab} interleaved (device)
     PairTab tab;
     long long n, row_stride;
@@ -709,8 +583,8 @@ struct PairParams {
     int tile_offset, span_tiles;
     int shift;
     int log_transform, write_baseline;
-    int total_pairs;            // streaming form: (row, tile) pairs of this launch
-    double w_y, w_b;            // streaming form: output = w_b * (b_even + b_odd) + w_y * y  ((1, -0.5) centred, (0, 0.5) baseline)
+    int total_pairs;            // (row, tile) pairs of this launch
+    double w_y, w_b;            // output = w_b * (b_even + b_odd) + w_y * y  ((1, -0.5) centred, (0, 0.5) baseline)
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -769,10 +643,10 @@ __device__ __forceinline__ void warp_entry_state(double (&E)[4], int target, int
     }
 }
 
-template <bool REV, int WP_WARPS, int CL = 2>
+template <bool REV, int WP_WARPS, int CL>
 __device__ __forceinline__ void pair_scan(double (&v)[4], double (&in)[4], const PairParams &P, double (*s_wex)[4],
                                           const double *s_pow, double (*s_nbr)[4], unsigned long long *s_cbar, int rank,
-                                          unsigned cpar = 0)
+                                          unsigned cpar)
 {
     constexpr int D = REV ? 1 : 0;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -840,178 +714,6 @@ __device__ __forceinline__ void pair_scan(double (&v)[4], double (&in)[4], const
     }
 }
 
-template <bool F32, int WP_THREADS, int WP_ITEMS>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WP_THREADS, 2) k_whittaker_pair(const __grid_constant__ PairParams P)
-{
-    namespace cg = cooperative_groups;
-    static_assert(WP_THREADS * WP_ITEMS == WP_HALF && WP_ITEMS % 4 == 0 && WP_ITEMS <= 16, "pair geometry");
-    constexpr int WP_WARPS = WP_THREADS / 32;
-    constexpr int PAD = WP_ITEMS + 1;                     // thread stride in 16-byte units: odd, so 128-bit accesses are conflict-free
-    extern __shared__ __align__(128) double smem_pair[];
-    // forward solutions of both chains, interleaved {zA_j, zB_j}, thread-blocked with one pad unit; the same memory is
-    // first the landing zone of the raw input and last the contiguous output stage
-    double2 *s_z = reinterpret_cast<double2 *>(smem_pair);
-    double *s_pow = smem_pair + 2 * WP_THREADS * PAD;     // PairPow (lane + warp tables)
-    const double2 *s_log = reinterpret_cast<const double2 *>(s_pow + sizeof(PairPow) / sizeof(double));   // {inv[i], tab[i]}
-    __shared__ __align__(8) unsigned long long s_mbar;    // input + tables
-    __shared__ __align__(8) unsigned long long s_cbar[2]; // carry from the peer CTA: [forward, backward]
-    __shared__ __align__(16) double s_nbr[2][4];
-    __shared__ __align__(16) double s_wex[2][WP_MAXWARPS][4];   // warp totals, one array per scan direction (no reuse, no hazard)
-
-    const int rank = (int)cg::this_cluster().block_rank();
-    const int tid = threadIdx.x;
-    const int pair_idx = blockIdx.x >> 1;
-    const long long row = P.row0 + (long long)(pair_idx / P.span_tiles) * P.row_step;
-    const int tile = P.tile_offset + pair_idx % P.span_tiles;
-    const long long r0 = (long long)tile * WT_OUT - WT_HALO - P.shift;               // region start (inside the row: steady tiles only)
-    const long long hbase = row * P.row_stride + r0 + (long long)rank * WP_HALF;     // first element of this CTA's half
-    constexpr unsigned BYTES = WP_HALF * (F32 ? 4u : 8u);
-    constexpr unsigned LOG_BYTES = 16u * LOG2_V2_ENTRIES;
-    constexpr unsigned TAB_BYTES = (unsigned)sizeof(PairPow) + LOG_BYTES;
-
-    const unsigned mbar = smem_u32(&s_mbar);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mbar));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&s_cbar[0])));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&s_cbar[1])));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        const char *src = reinterpret_cast<const char *>(P.x) + hbase * (F32 ? 4 : 8);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(BYTES + TAB_BYTES) : "memory");
-        bulk_load(smem_u32(s_z), src, BYTES, mbar);
-        bulk_load(smem_u32(s_pow), P.pow_tab, (unsigned)sizeof(PairPow), mbar);
-        bulk_load(smem_u32(s_log), P.log2tab, LOG_BYTES, mbar);
-        // this CTA receives one 32-byte carry: the right half in the forward scan, the left half in the backward scan
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], 32;" ::"r"(smem_u32(&s_cbar[rank == 1 ? 0 : 1])) : "memory");
-    }
-    // both CTAs' barriers must exist before anything is sent to them: fence.mbarrier_init + a RELAXED cluster arrive (no
-    // memory fence: nothing else has to be published) and the matching wait, whose latency hides under the bulk copy
-    asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
-    const double pil = (P.log_transform && P.pilot) ? P.pilot[row] : 0.0;
-    asm volatile("barrier.cluster.wait.aligned;" ::: "memory");
-    mbar_wait(mbar, 0);
-
-    // ---- this thread's bins: raw -> y (registers)
-    double y[WP_ITEMS];
-    if (F32) {
-        const float4 *rp = reinterpret_cast<const float4 *>(smem_pair) + tid * (WP_ITEMS / 4);
-#pragma unroll
-        for (int u = 0; u < WP_ITEMS / 4; ++u) {
-            const float4 q = rp[u];
-            y[4 * u + 0] = (double)q.x; y[4 * u + 1] = (double)q.y; y[4 * u + 2] = (double)q.z; y[4 * u + 3] = (double)q.w;
-        }
-    } else {
-        const double2 *rp = reinterpret_cast<const double2 *>(smem_pair) + tid * (WP_ITEMS / 2);
-#pragma unroll
-        for (int u = 0; u < WP_ITEMS / 2; ++u) { const double2 q = rp[u]; y[2 * u] = q.x; y[2 * u + 1] = q.y; }
-    }
-    // inference.py:45-46 rejects non-finite input: the largest exponent field seen decides at the end (a flagged call
-    // returns ST_NONFINITE and its output is discarded, so the transform need not special-case those bins)
-    int expmax = 0;
-#pragma unroll
-    for (int j = 0; j < WP_ITEMS; ++j) expmax = max(expmax, __double2hiint(y[j]) & 0x7FF00000);
-    int bad = (expmax == 0x7FF00000);
-    if (P.log_transform) {
-#pragma unroll
-        for (int j = 0; j < WP_ITEMS; ++j) y[j] = fast_log2_ge1_v2(dmax(y[j], 0.0) + 1.0, s_log) - pil;
-    }
-
-    const double (*cfA)[2] = P.tab.cf[0];                 // [dinv, l1, l2][position parity]
-    const double (*cfB)[2] = P.tab.cf[1];
-    double2 *fz = s_z + tid * PAD;
-    double v[4], in[4];
-    // own bins in region positions; the left CTA's threads that lie entirely in the left halo only feed the forward
-    // scan: nothing downstream reads their forward solution, so they skip everything after it
-    const int p0 = rank * WP_HALF + tid * WP_ITEMS;
-    const int o_lo = WT_HALO + P.shift, o_hi = o_lo + WT_OUT;
-    const bool dead = (p0 + WP_ITEMS <= o_lo);
-
-    // ================= forward substitution: zero-state sweep, carry scan, true sweep (scaled by 1/d on the way out)
-    {
-        double a1 = 0.0, a2 = 0.0, b1 = 0.0, b2 = 0.0;
-#pragma unroll
-        for (int j = 0; j < WP_ITEMS; ++j) {
-            const double ra = (j & 1) ? 0.0 : y[j], rb_ = (j & 1) ? y[j] : 0.0;
-            const double na = fma(-cfA[2][j & 1], a2, fma(-cfA[1][(j + 1) & 1], a1, ra));
-            const double nb = fma(-cfB[2][j & 1], b2, fma(-cfB[1][(j + 1) & 1], b1, rb_));
-            a2 = a1; a1 = na; b2 = b1; b1 = nb;
-        }
-        v[0] = a1; v[1] = a2; v[2] = b1; v[3] = b2;
-    }
-    pair_scan<false, WP_WARPS>(v, in, P, s_wex[0], s_pow, s_nbr, s_cbar, rank);   // (its barriers also order the raw reads before the writes below)
-    // The true sweep also accumulates the zero-state END VECTOR of the chunk's backward sweep, which is linear in the z_j
-    // (table g): the backward substitution then needs one pass over shared memory instead of two.
-    v[0] = v[1] = v[2] = v[3] = 0.0;
-    if (!dead) {
-        double a1 = in[0], a2 = in[1], b1 = in[2], b2 = in[3];
-#pragma unroll
-        for (int j = 0; j < WP_ITEMS; ++j) {
-            const double ra = (j & 1) ? 0.0 : y[j], rb_ = (j & 1) ? y[j] : 0.0;
-            const double na = fma(-cfA[2][j & 1], a2, fma(-cfA[1][(j + 1) & 1], a1, ra));
-            const double nb = fma(-cfB[2][j & 1], b2, fma(-cfB[1][(j + 1) & 1], b1, rb_));
-            a2 = a1; a1 = na; b2 = b1; b1 = nb;
-            const double za = na * cfA[0][j & 1], zb = nb * cfB[0][j & 1];
-            fz[j] = make_double2(za, zb);
-            v[0] = fma(P.tab.g[0][j][0], za, v[0]); v[1] = fma(P.tab.g[0][j][1], za, v[1]);
-            v[2] = fma(P.tab.g[1][j][0], zb, v[2]); v[3] = fma(P.tab.g[1][j][1], zb, v[3]);
-        }
-    }
-    // ================= backward substitution (right to left)
-    pair_scan<true, WP_WARPS>(v, in, P, s_wex[1], s_pow, s_nbr, s_cbar, rank);
-    if (!dead) {
-        double a1 = in[0], a2 = in[1], b1 = in[2], b2 = in[3];
-#pragma unroll
-        for (int j = WP_ITEMS - 1; j >= 0; --j) {
-            const double2 z = fz[j];
-            const double na = fma(-cfA[2][j & 1], a2, fma(-cfA[1][j & 1], a1, z.x));
-            const double nb = fma(-cfB[2][j & 1], b2, fma(-cfB[1][j & 1], b1, z.y));
-            a2 = a1; a1 = na; b2 = b1; b1 = nb;
-            const double bsl = 0.5 * (na + nb);                       // cross-fit average (baseline_backend.c:296-299)
-            y[j] = P.write_baseline ? bsl : y[j] - bsl;
-        }
-    }
-    expmax = 0;
-#pragma unroll
-    for (int j = 0; j < WP_ITEMS; ++j) expmax = max(expmax, __double2hiint(y[j]) & 0x7FF00000);
-    bad |= (expmax == 0x7FF00000);
-    if (bad) *P.bad = 1;
-
-    // ---- epilogue: the half's results contiguous in shared memory (the forward solutions are dead), own bins out in bulk
-    __syncthreads();                                                  // every thread is done reading its z slots
-    if (!dead) {
-        double2 *sp = reinterpret_cast<double2 *>(smem_pair) + tid * (WP_ITEMS / 2);
-#pragma unroll
-        for (int u = 0; u < WP_ITEMS / 2; ++u) sp[u] = make_double2(y[2 * u], y[2 * u + 1]);
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // generic-proxy writes -> visible to the bulk (async proxy) read
-    __syncthreads();
-    const int q0 = max(o_lo, rank * WP_HALF) - rank * WP_HALF, q1 = min(o_hi, (rank + 1) * WP_HALF) - rank * WP_HALF;   // own bins in half positions
-    double *outp = P.out + hbase;
-    if ((reinterpret_cast<uintptr_t>(outp) & 15) == 0) {
-        if (tid == 0) {
-            const int b0 = (q0 + 1) & ~1, b1 = q1 & ~1;               // 16-byte aligned middle part
-            if (q0 < b0) outp[q0] = smem_pair[q0];
-            if (b1 < q1) outp[b1] = smem_pair[b1];
-            if (b1 > b0) {
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                             ::"l"(outp + b0), "r"(smem_u32(smem_pair + b0)), "r"((unsigned)(b1 - b0) * 8u) : "memory");
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // shared memory must outlive the read
-            }
-        }
-    } else {
-        for (int q = q0 + tid; q < q1; q += WP_THREADS) outp[q] = smem_pair[q];       // coalesced fallback
-    }
-}
-
-// ------------------------------------------------------------------ steady tiles, streaming cluster-pair form
-// The pair kernel above made PERSISTENT: 148 clusters walk the (row, tile) list, and the raw input of a cluster's next tile
-// is in flight (bulk async copy into the second of two landing buffers) while the current one is solved, so that neither
-// the load latency at the start of a tile nor the drain of its bulk store at the end is exposed; the scan tables are
-// loaded once per CTA.  Shared memory has room for the second buffer because the forward solution is no longer stored:
-// the backward sweep re-derives it by running the forward recurrence right to left from the chunk's final state
-// (n_{j-2} = (r_j - n_j - l1 n_{j-1}) / l2; twelve steps of a recurrence whose reverse growth is 1/0.9775 per bin, i.e.
-// ~1e-16 relative).  y stays in registers, the result is written over the thread's own slots of the landing buffer and
-// leaves from there as one bulk store.
 template <bool F32, int WP_THREADS, int WP_ITEMS, int CL>
 __global__ void __launch_bounds__(WP_THREADS, 1024 / WP_THREADS) k_whittaker_stream(const __grid_constant__ PairParams P)
 {
@@ -1234,10 +936,9 @@ __global__ void k_small_rows(WhitParams P)
 struct FactorDev {
     FactorHost host;
     double *d_head[2][3] = {{nullptr, nullptr, nullptr}, {nullptr, nullptr, nullptr}};
-    double *d_lanepow = nullptr;
     double *d_log2 = nullptr;
-    double *d_log2i = nullptr;                       // the same tables interleaved {inv[i], tab[i]} (pair kernel)
-    double *d_pairpow[WP_NGEOM][2] = {};       // PairPow per geometry and shift parity
+    double *d_log2i = nullptr;                       // the same tables interleaved {inv[i], tab[i]} (streaming kernel)
+    double *d_pairpow[2] = {};                       // PairPow per shift parity
     int device = 0;
     unsigned long long last_use = 0;
     FactorDev() = default;
@@ -1247,9 +948,8 @@ struct FactorDev {
     {
         for (int p = 0; p < 2; ++p) {
             for (int k = 0; k < 3; ++k) if (d_head[p][k]) cudaFree(d_head[p][k]);
-            for (int gm = 0; gm < WP_NGEOM; ++gm) if (d_pairpow[gm][p]) cudaFree(d_pairpow[gm][p]);
+            if (d_pairpow[p]) cudaFree(d_pairpow[p]);
         }
-        if (d_lanepow) cudaFree(d_lanepow);
         if (d_log2) cudaFree(d_log2);
         if (d_log2i) cudaFree(d_log2i);
     }
@@ -1281,13 +981,10 @@ static int upload_factor(FactorDev &F)
         RB_CUDA(cudaMalloc(&F.d_log2i, sizeof(il)));
         RB_CUDA(cudaMemcpy(F.d_log2i, il, sizeof(il), cudaMemcpyHostToDevice));
     }
-    RB_CUDA(cudaMalloc(&F.d_lanepow, sizeof(F.host.lanepow)));
-    RB_CUDA(cudaMemcpy(F.d_lanepow, F.host.lanepow, sizeof(F.host.lanepow), cudaMemcpyHostToDevice));
-    for (int gm = 0; gm < WP_NGEOM; ++gm)
-        for (int ap = 0; ap < 2; ++ap) {
-            RB_CUDA(cudaMalloc(&F.d_pairpow[gm][ap], sizeof(PairPow)));
-            RB_CUDA(cudaMemcpy(F.d_pairpow[gm][ap], &F.host.pair_pow[gm][ap], sizeof(PairPow), cudaMemcpyHostToDevice));
-        }
+    for (int ap = 0; ap < 2; ++ap) {
+        RB_CUDA(cudaMalloc(&F.d_pairpow[ap], sizeof(PairPow)));
+        RB_CUDA(cudaMemcpy(F.d_pairpow[ap], &F.host.pair_pow[ap], sizeof(PairPow), cudaMemcpyHostToDevice));
+    }
     return 0;
 }
 
@@ -1322,30 +1019,6 @@ static int get_factor(long long n, double lam, FactorRef *out)
     F->last_use = ++g_fclock;
     cache[key] = F;
     *out = F;
-    return 0;
-}
-
-// steady tiles: 0 = the streaming cluster-pair kernel (default, both input types: float32 storage of the same values
-// must give the same bits as float64 storage, so both take the same arithmetic), 1 = the single-CTA kernel, 2 = one-shot
-// pair kernel, 3 = streaming pair kernel (1-3 kept for A/B checks)
-static std::atomic<int> g_whit_mode{0};
-int whittaker_set_mode(int mode) { return g_whit_mode.exchange((mode >= 0 && mode <= 3) ? mode : 0); }
-
-template <bool F32, int THREADS, int ITEMS>
-static int launch_pair(const PairParams &R, unsigned grid, cudaStream_t st)
-{
-    constexpr size_t sm = sizeof(double) * 2 * THREADS * (ITEMS + 1) + sizeof(PairPow) + 16 * LOG2_V2_ENTRIES;
-    static bool attr_dev[64] = {false};
-    int d = 0;
-    cudaGetDevice(&d);
-    bool &attr = attr_dev[d & 63];
-    if (!attr) {
-        RB_CUDA(cudaFuncSetAttribute(k_whittaker_pair<F32, THREADS, ITEMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-        RB_CUDA(cudaFuncSetAttribute(k_whittaker_pair<F32, THREADS, ITEMS>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        attr = true;
-    }
-    k_whittaker_pair<F32, THREADS, ITEMS><<<grid, THREADS, sm, st>>>(R);
-    RB_LAUNCH_CHECK();
     return 0;
 }
 
@@ -1396,6 +1069,8 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
                    long long row_stride, double lam, int write_baseline, double *d_out, int *d_bad, cudaStream_t st)
 {
     if (rows <= 0 || n <= 0) return ST_INVALID;
+    const size_t esz = in_f32 ? 4 : 8;
+    if (reinterpret_cast<uintptr_t>(d_x) % esz != 0) return ST_INVALID;      // every kernel loads whole elements
     WhitParams P{};
     P.x = d_x; P.pilot = d_pilot; P.out = d_out; P.bad = d_bad; P.n = n; P.row_stride = row_stride;
     P.rows = (int)rows; P.in_f32 = in_f32; P.log_transform = log_transform; P.write_baseline = write_baseline;
@@ -1413,21 +1088,17 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
         for (int k = 0; k < 3; ++k) P.head[p][k] = F->d_head[p][k];
     memcpy(P.steady, F->host.steady, sizeof(P.steady));
     memcpy(P.tail, F->host.tail, sizeof(P.tail));
-    memcpy(P.trans, F->host.trans, sizeof(P.trans));
-    P.lanepow = F->d_lanepow;
     P.log2tab = F->d_log2;
     P.tiles_per_row = (int)((n + WT_OUT - 1) / WT_OUT);
-    // Interior tiles (region inside [head_len, n-4)) take the steady instantiation; the first and last
-    // tile(s) of each row take the general one.  Two launches over disjoint tile sets.
-    const size_t sm_steady = sizeof(double) * 2 * WT_THREADS_S * (WT_ITEMS_S + 1);
+    // Interior tiles (region inside [head_len, n-4)) take the streaming kernel; the first and last tile(s) of each row
+    // take k_whittaker.  Launches over disjoint tile sets.
     const size_t sm_general = sizeof(double) * 2 * WT_THREADS_G * (WT_ITEMS_G + 1) + sizeof(double) * 6 * WT_THREADS_G;
     static bool attr_dev[64] = {false};
     int attr_d = 0;
     cudaGetDevice(&attr_d);
     bool &attr = attr_dev[attr_d & 63];
     if (!attr) {
-        RB_CUDA(cudaFuncSetAttribute(k_whittaker<true, WT_THREADS_S, WT_ITEMS_S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_steady));
-        RB_CUDA(cudaFuncSetAttribute(k_whittaker<false, WT_THREADS_G, WT_ITEMS_G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_general));
+        RB_CUDA(cudaFuncSetAttribute(k_whittaker<WT_THREADS_G, WT_ITEMS_G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_general));
         attr = true;
     }
     // classify tiles
@@ -1435,7 +1106,7 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
     for (int t = 0; t < P.tiles_per_row; ++t) {
         const long long o0 = (long long)t * WT_OUT, o1 = std::min(n, o0 + WT_OUT);
         const long long r0 = std::max<long long>(0, o0 - WT_HALO), r1 = std::min(n, o1 + WT_HALO);
-        const bool steady = (r0 >= P.head_len + 8) && (r1 <= n - 6) && (r1 - r0 == WT_REGION);      // (+8: room for the pair kernel's alignment shift)
+        const bool steady = (r0 >= P.head_len + 8) && (r1 <= n - 6) && (r1 - r0 == WT_REGION);      // (+8: room for the streaming kernel's alignment shift)
         if (steady) { first_steady = std::min(first_steady, t); last_steady = std::max(last_steady, t); }
     }
     // general tiles: [0, first_steady) and (last_steady, tiles); steady tiles are contiguous in between
@@ -1448,11 +1119,6 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
     } else {
         spans.push_back({0, P.tiles_per_row, false});
     }
-    const size_t esz = in_f32 ? 4 : 8;
-    const int mode = g_whit_mode.load();
-    const int gm = 0;
-    const bool stream = mode == 3 || mode == 0;
-    const bool pair_ok = mode != 1 && (reinterpret_cast<uintptr_t>(d_x) % esz) == 0;
     for (const Span &sp : spans) {
         WhitParams Q = P;
         Q.tile_offset = sp.t0;
@@ -1462,7 +1128,7 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
         // algorithmic bytes of this launch: read the input once, write the centered matrix once
         const double span_bins = (double)std::min<long long>(n, (long long)sp.t1 * WT_OUT) - (double)sp.t0 * WT_OUT;
         RB_PROF(sp.steady ? "k_whittaker_steady" : "k_whittaker_edge", st, (double)rows * span_bins * ((in_f32 ? 4.0 : 8.0) + 8.0));
-        if (sp.steady && pair_ok) {
+        if (sp.steady) {
             // rows whose start has the same offset inside a 16-byte unit share a launch (the bulk copy needs an aligned source)
             const long long M = 16 / (long long)esz;
             const long long base_off = (long long)((reinterpret_cast<uintptr_t>(d_x) / esz) % (uintptr_t)M);
@@ -1473,19 +1139,15 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
                 R.row0 = (int)p; R.row_step = (int)period; R.tile_offset = sp.t0; R.span_tiles = Q.span_tiles;
                 R.shift = (int)((base_off + p * (row_stride % M)) % M);
                 R.log_transform = log_transform; R.write_baseline = write_baseline;
-                R.tab = F->host.pair_tab[gm][R.shift & 1];
-                R.pow_tab = F->d_pairpow[gm][R.shift & 1];
+                R.tab = F->host.pair_tab[R.shift & 1];
+                R.pow_tab = F->d_pairpow[R.shift & 1];
                 R.log2tab = F->d_log2i;
                 const long long nrows = (rows - p + period - 1) / period;
-                const unsigned grid = (unsigned)(nrows * Q.span_tiles * 2);
-                if (stream) RB_TRY(in_f32 ? (launch_stream<true, 512, 12, 2>(R, nrows * Q.span_tiles, st)) : (launch_stream<false, 512, 12, 2>(R, nrows * Q.span_tiles, st)));
-                else RB_TRY(in_f32 ? (launch_pair<true, 512, 12>(R, grid, st)) : (launch_pair<false, 512, 12>(R, grid, st)));
+                RB_TRY(in_f32 ? (launch_stream<true, WP_GEOM_THREADS, WP_GEOM_ITEMS, 2>(R, nrows * Q.span_tiles, st))
+                              : (launch_stream<false, WP_GEOM_THREADS, WP_GEOM_ITEMS, 2>(R, nrows * Q.span_tiles, st)));
             }
-        } else if (sp.steady) {
-            k_whittaker<true, WT_THREADS_S, WT_ITEMS_S><<<(unsigned)blocks, WT_THREADS_S, sm_steady, st>>>(Q);
-            RB_LAUNCH_CHECK();
         } else {
-            k_whittaker<false, WT_THREADS_G, WT_ITEMS_G><<<(unsigned)blocks, WT_THREADS_G, sm_general, st>>>(Q);
+            k_whittaker<WT_THREADS_G, WT_ITEMS_G><<<(unsigned)blocks, WT_THREADS_G, sm_general, st>>>(Q);
             RB_LAUNCH_CHECK();
         }
     }

@@ -279,8 +279,7 @@ static int trend_knots_sorted(const double *d_C, const double *d_V, const std::v
     return 0;
 }
 
-// 0: histogram multi-select with sort fallback, the fused rolling variance leaving the slot collection 32-bit pair keys
-// (default); 1: force the sort-based path (tests); 2: as 0, but the slot collection reads C and V (A/B of the keys)
+// 0: histogram multi-select with sort fallback (default); 1: force the sort-based path (tests)
 static std::atomic<int> g_trend_mode{0};
 static std::atomic<long long> g_trend_fallback_rows{0};
 static std::atomic<long long> g_trend_fb_reason[8];
@@ -475,7 +474,7 @@ struct WlsRun {
     long long m = 0, n = 0;
     int w = 0;
     double ldf = 0, pdf = 0, tdf = 0, pfr = 0;
-    bool const_rows = false, fused = false, sort_all = false, keys = false;
+    bool const_rows = false, fused = false, sort_all = false;
     double *d_V = nullptr, *d_rc = nullptr;
     Knots *d_knots = nullptr;
     KnotTable *d_tables = nullptr;
@@ -502,10 +501,8 @@ static int wls_prepare(Arena &ar, long long m, long long n, const rocco_b200_sco
         RB_TRY(ar.alloc(&R.d_knots, (size_t)m));
         RB_TRY(ar.alloc(&R.d_tables, (size_t)m));
         RB_TRY(ar.alloc(&R.d_fb, (size_t)m));
-        const int mode = g_trend_mode.load();
-        R.sort_all = mode == 1;
+        R.sort_all = g_trend_mode.load() == 1;
         R.fused = !R.sort_all && (R.w <= trend_fused_max_window());
-        R.keys = R.fused && mode != 2;
     }
     return 0;
 }
@@ -527,7 +524,7 @@ static int wls_rows(const double *d_centered, WlsRun &R, long long r0, long long
         k_rollvar<<<grid, 256, 0, st>>>(c, n, n, R.w, v);
         RB_LAUNCH_CHECK();
     }
-    if (!R.sort_all) RB_TRY(trend_knots_select(c, v, g, n, n, R.d_knots + r0, R.d_fb + r0, R.fused ? R.w : 0, R.keys, st));
+    if (!R.sort_all) RB_TRY(trend_knots_select(c, v, g, n, n, R.d_knots + r0, R.d_fb + r0, R.fused ? R.w : 0, st));
     return 0;
 }
 
@@ -845,9 +842,8 @@ using namespace rb;
 
 RB_API int rocco_b200_trend_set_mode(int mode)
 {
-    return score::g_trend_mode.exchange(mode == 1 || mode == 2 ? mode : 0);
+    return score::g_trend_mode.exchange(mode == 1 ? 1 : 0);
 }
-RB_API int rocco_b200_whittaker_set_mode(int mode) { return score::whittaker_set_mode(mode); }
 RB_API long long rocco_b200_trend_fallback_rows(void) { return score::g_trend_fallback_rows.load(); }
 RB_API void rocco_b200_trend_fallback_reasons(long long *out8) { for (int k = 0; k < 8; ++k) out8[k] = score::g_trend_fb_reason[k].load(); }
 

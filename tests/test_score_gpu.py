@@ -158,21 +158,21 @@ def test_baseline_matches_oracle_across_tile_and_table_edges(rb, oracle, n):
     assert got1.shape == (n,) and np.max(np.abs(got1 - want[0])) <= 2e-9
 
 
-@pytest.mark.parametrize("mode", [1, 2, 3])
-@pytest.mark.parametrize("rows,n", [(3, 140001), (5, 60002), (2, 300007)])
-def test_every_steady_tile_kernel_matches_the_oracle(rb, oracle, mode, rows, n):
-    """the single-CTA kernel, the one-shot cluster pair and the streaming cluster pair (the default for float64 input) solve
-    the same regions: each within 2e-9 of the oracle, odd row lengths (every 16-byte alignment class of the bulk copies)"""
-    from rocco_b200 import _baseline, _lib
-    rng = np.random.default_rng(100 * mode + rows)
+# (3, 20741) has no steady tile and (3, 20742) exactly one; one row gives a single alignment group; 24 rows of 300007 or
+# 300008 bins and 4 rows of 1000003 give each persistent cluster several tiles, so both landing buffers and both phases
+# of every mbarrier are used (odd n: two row groups with different bulk-copy shifts, even n: one)
+@pytest.mark.parametrize("rows,n", [(3, 140001), (5, 60002), (2, 300007), (1, 140001), (3, 20741), (3, 20742),
+                                    (24, 300007), (24, 300008), (4, 1000003)])
+def test_streaming_steady_tile_kernel_matches_the_oracle(rb, oracle, rows, n):
+    """the streaming cluster-pair kernel of the interior tiles within 2e-9 of the oracle, odd row lengths (every 16-byte
+    alignment class of the bulk copies), the row lengths at which the first steady tile appears, and launches in which
+    each cluster walks several tiles"""
+    from rocco_b200 import _baseline
+    rng = np.random.default_rng(300 + rows)
     y = rng.normal(size=(rows, n)) + 2.0 * np.sin(np.arange(n) / 900.0) + (rng.random((rows, n)) < 0.01) * 6.0
     lam = oracle.whittaker_lambda(oracle.resolve_local_baseline_window(n))
     want = oracle.native("port").crossfit_whittaker_baseline(y, lam)
-    prev = _lib.load().rocco_b200_whittaker_set_mode(mode)
-    try:
-        got = _baseline.crossfit_whittaker_baseline(y, lam)
-    finally:
-        _lib.load().rocco_b200_whittaker_set_mode(prev)
+    got = _baseline.crossfit_whittaker_baseline(y, lam)
     assert np.max(np.abs(got - want)) <= 2e-9, float(np.max(np.abs(got - want)))
 
 

@@ -261,10 +261,6 @@ def _reason_text(rs):
     return ",".join(f"{FB_NAMES[1 << k]}:{int(rs[k])}" for k in range(5) if rs[k]) or "-"
 
 
-def _modes(w):
-    return (0, 1, 2) if w <= 1025 else (0, 1)
-
-
 # ------------------------------------------------------------------ A on the GPU
 def _a_lengths(w):
     h = w // 2
@@ -288,7 +284,7 @@ def _check_a(c, window, label, gate=True, score_tol=TIGHT):
         from oracle import oracle as orc
         want_s, want = orc.score_centered_wls_matrix(c, spatial_window=window)
     worst, worst_own = 0.0, 0.0
-    for mode in _modes(w):
+    for mode in (0, 1):
         sc, det, fb, rs = _gpu(c, mode, spatial_window=window)
         assert det["prior_spatial_window"] == w
         raw = det["raw_variance"]

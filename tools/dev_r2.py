@@ -1,6 +1,5 @@
 """Round-2 development probes (run on the GPU box): A/B checks and timings of the reworked kernels.
 
-    python tools/dev_r2.py whit        # Whittaker steady-tile kernels: pair modes vs the round-1 kernel vs the oracle
     python tools/dev_r2.py scopes      # per-scope times of one chromosome set (profile scopes)
 
 Results go to stdout and gpurun_out/dev_<cmd>.json.
@@ -10,7 +9,6 @@ import os
 import sys
 import time
 
-import numpy as np
 import torch
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,64 +32,6 @@ def scopes_of(fn, reps=3):
     rep = _lib.profile_report()
     _lib.profile_enable(False)
     return {k: {"ms": v[0] / reps, "GBps": (v[2] / 1e9) / (v[0] / 1e3) if v[0] > 0 else 0.0} for k, v in rep.items()}
-
-
-def cmd_whit():
-    lib = _lib.load()
-    res = {"parity": [], "timing": []}
-    prm = pipeline.score_params(prior_df=6.0)
-    from oracle import oracle as orc
-    shapes = [(3, 60000, torch.float64, True), (3, 60001, torch.float64, True), (4, 934200, torch.float64, False),
-              (5, 250001, torch.float32, False), (5, 250002, torch.float32, False), (6, 250003, torch.float32, False),
-              (3, 1000001, torch.float64, False)]
-    for m, n, dt, use_oracle in shapes:
-        x = chrom_matrix_torch(m, n, 11 + n % 7, DEV, dt)
-        out = {}
-        for mode in (1, 2, 3):
-            prev = lib.rocco_b200_whittaker_set_mode(mode)
-            s, d = pipeline.score_loci_wls_device(x, params=prm, details=True)
-            torch.cuda.synchronize()
-            out[mode] = (s.clone(), d["centered_matrix"].clone())
-            lib.rocco_b200_whittaker_set_mode(prev)
-        row = {"m": m, "n": n, "dtype": str(dt)}
-        for mode in (2, 3):
-            row[f"centered_maxabs_mode{mode}_vs_old"] = float((out[mode][1] - out[1][1]).abs().max())
-            row[f"scores_maxabs_mode{mode}_vs_old"] = float((out[mode][0] - out[1][0]).abs().max())
-        if use_oracle:
-            want_s, want_d = orc.score_loci_wls(x.cpu().numpy(), prior_df=6.0, return_details=True,
-                                                kind="reference" if orc.reference_available() else "port")
-            for mode in (1, 2, 3):
-                row[f"centered_maxabs_mode{mode}_vs_oracle"] = float(np.max(np.abs(out[mode][1].cpu().numpy() - want_d["centered_matrix"])))
-                ref = np.maximum(np.abs(want_s), 1e-3)
-                row[f"scores_maxrel_mode{mode}_vs_oracle"] = float(np.max(np.abs(out[mode][0].cpu().numpy() - want_s) / ref))
-        print(json.dumps(row), flush=True)
-        res["parity"].append(row)
-        del x, out
-    # non-finite input is still reported
-    x = chrom_matrix_torch(3, 60000, 5, DEV, torch.float64)
-    x[1, 30000] = float("nan")
-    try:
-        pipeline.score_loci_wls_device(x, params=prm)
-        res["nonfinite_raises"] = False
-    except ValueError:
-        res["nonfinite_raises"] = True
-    print("nonfinite raises:", res["nonfinite_raises"], flush=True)
-    # timings
-    for name, m, dt in (("chr21", 100, torch.float64), ("chr21", 100, torch.float32), ("chr1", 100, torch.float64)):
-        n = chrom_bins(name)
-        x = chrom_matrix_torch(m, n, chrom_seed(name), DEV, dt)
-        sc = torch.empty(n, dtype=torch.float64, device=DEV)
-        for mode in (1, 2, 3):
-            prev = lib.rocco_b200_whittaker_set_mode(mode)
-            sp = scopes_of(lambda: pipeline.score_loci_wls_device(x, out_scores=sc, params=prm))
-            lib.rocco_b200_whittaker_set_mode(prev)
-            row = {"chrom": name, "m": m, "dtype": str(dt), "mode": mode,
-                   "steady_ms": sp.get("k_whittaker_steady", {}).get("ms"), "steady_GBps": sp.get("k_whittaker_steady", {}).get("GBps"),
-                   "edge_ms": sp.get("k_whittaker_edge", {}).get("ms"), "all": {k: round(v["ms"], 3) for k, v in sp.items()}}
-            print(json.dumps(row), flush=True)
-            res["timing"].append(row)
-        del x
-    json.dump(res, open(os.path.join(OUT, "dev_whit.json"), "w"), indent=1)
 
 
 def cmd_scopes():
@@ -167,4 +107,4 @@ def cmd_timeline():
 
 
 if __name__ == "__main__":
-    {"whit": cmd_whit, "scopes": cmd_scopes, "fallback": cmd_fallback, "timeline": cmd_timeline}[sys.argv[1]]()
+    {"scopes": cmd_scopes, "fallback": cmd_fallback, "timeline": cmd_timeline}[sys.argv[1]]()
