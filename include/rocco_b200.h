@@ -255,6 +255,11 @@ int rocco_b200_score_loci_wls_dev(const void *d_matrix, int dtype, size_t m, siz
  * the TOTAL sample count (wls_backend.c:915-937). */
 int rocco_b200_score_partial_dev(const void *d_matrix, int dtype, size_t m_local, size_t n,
                                  const rocco_b200_score_params *params, double *d_acc, void *cuda_stream);
+/* The same, also keeping this rank's centred rows in d_centered_out [m_local][n] (device, NULL: not kept) -- the input of
+ * rocco_b200_budget_nonnull_fraction_sharded_dev. */
+int rocco_b200_score_partial_ex_dev(const void *d_matrix, int dtype, size_t m_local, size_t n,
+                                    const rocco_b200_score_params *params, double *d_centered_out, double *d_acc,
+                                    void *cuda_stream);
 int rocco_b200_score_finalize_dev(const double *d_acc, size_t m_total, size_t n, const rocco_b200_score_params *params,
                                   rocco_b200_score_outputs *out, void *cuda_stream);
 int rocco_b200_crossfit_baseline_dev(const double *d_rows, size_t m, size_t n, double penalty_lambda,
@@ -274,11 +279,13 @@ typedef struct rocco_b200_budget_params {
     int dependence_lag_hint;        /* <= 0: none (bandwidth round(n^(1/3)), ESS scale 101); rocco.py:1035 passes >= 25 */
     int num_null_draws;             /* 25                                                                        */
     int min_null_draws;             /* <= 0: 8 (inference.py:795-797)                                            */
-    int reserved;
+    int sample_offset;              /* global index of the first local sample (sample sharding; 0 = unsharded): row r
+                                       draws the Philox stream of sample sample_offset + r                          */
     double stability_abs_tol;       /* 5e-3                                                                      */
     double stability_rel_tol;       /* 5e-2                                                                      */
     unsigned long long random_seed;
-    const double *d_innovations;    /* optional DEVICE buffer [num_null_draws][m][n + 2*bandwidth] of iid N(0,1)  */
+    const double *d_innovations;    /* optional DEVICE buffer [num_null_draws][m][n + 2*bandwidth] of iid N(0,1)
+                                       (sharded: [num_null_draws][m_local][n + 2*bandwidth], this rank's rows)       */
 } rocco_b200_budget_params;
 
 typedef struct rocco_b200_budget_result {
@@ -303,6 +310,27 @@ int rocco_b200_budget_ess_max_lag(size_t n, int dependence_lag_hint);    /* infe
 int rocco_b200_budget_nonnull_fraction_dev(const double *d_centered, size_t m, size_t n, const double *d_observed_scores,
                                            const rocco_b200_budget_params *params, rocco_b200_budget_result *result,
                                            void *cuda_stream);
+/* Sum over ranks for the sample-sharded estimator, built by the caller (NCCL is not linked into this library): replace
+ * d_buf[0 .. count) (device, float64) by its sum over all ranks, in place, ordered after the work already queued on
+ * `cuda_stream` and before anything queued on it later (e.g. ncclAllReduce on that stream, or a collective on a stream
+ * that waits for it and that it then waits for).  Every rank calls it with the same count, the same number of times.
+ * Return 0 on success; any other value aborts the call with -3 on that rank. */
+typedef int (*rocco_b200_allreduce_fn)(double *d_buf, size_t count, void *cuda_stream, void *user);
+/* The estimator with the SAMPLES sharded over ranks (BASELINE.json config 5): each rank passes its m_local centred rows
+ * (global rows params->sample_offset .. + m_local of m_total) and the same n, observed scores and params.  The template, the
+ * multiplier field and the per-row WLS stages stay local; each of the 2 + K scoring passes (fit, reference field, K draws)
+ * reduces 2n column sums {sum y/post, sum 1/post} plus 4 status slots through `allreduce` (16 B/bin); everything after
+ * a score track exists is recomputed by every rank from the reduced, bit-identical track, so all ranks return the same
+ * result and the same status.  A rank-local failure (an allocation, a degenerate multiplier row, a non-finite local row)
+ * is carried to the next reduce: every rank then returns that status; the failing rank keeps its
+ * rocco_b200_last_error() text.  Not covered: a failure to allocate the 16 B/bin reduce buffer itself (the first
+ * allocation of the call) and a sticky CUDA context error, after which no collective can run.  Shapes must be checked
+ * across ranks before the call.  With m_local == m_total the result equals rocco_b200_budget_nonnull_fraction_dev's
+ * bit for bit (allreduce may then be NULL). */
+int rocco_b200_budget_nonnull_fraction_sharded_dev(const double *d_centered_local, size_t m_local, size_t n, size_t m_total,
+                                                   const double *d_observed_scores, const rocco_b200_budget_params *params,
+                                                   rocco_b200_allreduce_fn allreduce, void *user,
+                                                   rocco_b200_budget_result *result, void *cuda_stream);
 /* Building block of one draw (inference.py:653-662): d_out = d_template x W, W the Bartlett multiplier field of
  * (random_seed, draw_index), or of d_innovations [m][n + 2*bandwidth] when given.  d_out may not alias d_template. */
 int rocco_b200_wild_multiply_dev(const double *d_template, size_t m, size_t n, int bandwidth,

@@ -54,9 +54,13 @@ class ScoreOutputs(Structure):
 class BudgetParams(Structure):
     _fields_ = [
         ("score", ScoreParams), ("dependence_lag_hint", c_int), ("num_null_draws", c_int), ("min_null_draws", c_int),
-        ("reserved", c_int), ("stability_abs_tol", c_double), ("stability_rel_tol", c_double),
+        ("sample_offset", c_int), ("stability_abs_tol", c_double), ("stability_rel_tol", c_double),
         ("random_seed", c_ulonglong), ("d_innovations", c_void_p),
     ]
+
+
+# rocco_b200_allreduce_fn: sum d_buf[0:count) over ranks in place, stream-ordered; 0 = success
+ALLREDUCE_FN = ctypes.CFUNCTYPE(c_int, c_void_p, c_size_t, c_void_p, c_void_p)
 
 
 _BUDGET_DOUBLES = (
@@ -115,6 +119,9 @@ def _declare(lib):
         "rocco_b200_budget_ess_max_lag": (c_int, [c_size_t, c_int]),
         "rocco_b200_budget_nonnull_fraction_dev": (c_int, [c_void_p, c_size_t, c_size_t, c_void_p, POINTER(BudgetParams),
                                                            POINTER(BudgetResult), c_void_p]),
+        "rocco_b200_budget_nonnull_fraction_sharded_dev": (
+            c_int, [c_void_p, c_size_t, c_size_t, c_size_t, c_void_p, POINTER(BudgetParams), c_void_p, c_void_p,
+                    POINTER(BudgetResult), c_void_p]),
         "rocco_budget_nonnull_fraction_f64": (c_int, [c_void_p, c_size_t, c_size_t, c_void_p, POINTER(BudgetParams), c_void_p,
                                                       POINTER(BudgetResult)]),
         "rocco_b200_wild_multiply_dev": (c_int, [c_void_p, c_size_t, c_size_t, c_int, c_ulonglong, ctypes.c_uint, c_void_p, c_void_p,
@@ -157,6 +164,8 @@ def _declare(lib):
         "rocco_b200_score_loci_wls_dev": (
             c_int, [c_void_p, c_int, c_size_t, c_size_t, POINTER(ScoreParams), POINTER(ScoreOutputs), c_void_p]),
         "rocco_b200_score_partial_dev": (c_int, [c_void_p, c_int, c_size_t, c_size_t, POINTER(ScoreParams), c_void_p, c_void_p]),
+        "rocco_b200_score_partial_ex_dev": (
+            c_int, [c_void_p, c_int, c_size_t, c_size_t, POINTER(ScoreParams), c_void_p, c_void_p, c_void_p]),
         "rocco_b200_score_finalize_dev": (c_int, [c_void_p, c_size_t, c_size_t, POINTER(ScoreParams), POINTER(ScoreOutputs), c_void_p]),
         "rocco_b200_crossfit_baseline_dev": (c_int, [c_void_p, c_size_t, c_size_t, c_double, c_void_p, c_void_p]),
         "rocco_b200_score_centered_wls_dev": (

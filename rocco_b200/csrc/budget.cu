@@ -10,6 +10,14 @@
 // in double -- so a draw is reproducible and independent of tiling, but the streams differ from NumPy's: parity with
 // the reference is statistical.  For bit-level checks the caller may pass the innovations themselves
 // (`d_innovations`), which is how tests replay the reference's own streams through these kernels.
+//
+// Sample sharding: the estimator also runs with the samples split over ranks (the layout of the sample-sharded scoring).
+// Everything per sample -- the template, the multiplier field (row r of a shard draws the stream of global sample
+// sample_offset + r), the per-row WLS stages -- stays on the rank; the only cross-sample step of a scoring pass, the column
+// sums of the combine, goes through the caller's all-reduce (2n sums + status slots); everything after a score track exists
+// (sort, centre/scale, track sums, adaptive stop, ESS, positive median) is recomputed by every rank from the bit-identical
+// reduced track.  Every decision taken after a reduce depends only on reduced data, and a rank-local failure is carried to
+// the next reduce in the status slots, so all ranks leave together with the same status.
 #include <cub/cub.cuh>
 
 #include <cmath>
@@ -76,10 +84,11 @@ __global__ void __launch_bounds__(256) k_template(const double *__restrict__ C, 
 //   L_j = z[j] + .. + z[j+b],   R_j = z[j+b+1] + .. + z[j+2b+1]:
 // every thread forms its first output (and L, R) directly -- K fused multiply-adds -- and slides the next 15, which
 // keeps the rounding of a slide chain at 15 steps (~1e-15) instead of the row length.
+// The Philox stream of row r is that of sample sample_offset + r: a shard's field equals those rows of the whole field.
 __global__ void __launch_bounds__(FIR_THREADS, 2) k_wild_fir(const double *__restrict__ innov, long long innov_stride, uint2 key,
-                                                          unsigned draw, long long n, int K, const double *__restrict__ taps,
-                                                          double h, double *__restrict__ raw, double2 *__restrict__ partial,
-                                                          int tiles)
+                                                          unsigned draw, unsigned sample_offset, long long n, int K,
+                                                          const double *__restrict__ taps, double h, double *__restrict__ raw,
+                                                          double2 *__restrict__ partial, int tiles)
 {
     extern __shared__ double s_fir[];
     double *s_x = s_fir;                                   // padpos(FIR_T + K + 8)
@@ -100,7 +109,7 @@ __global__ void __launch_bounds__(FIR_THREADS, 2) k_wild_fir(const double *__res
         for (int p = tid; 2 * p < staged; p += FIR_THREADS) {
             const int e = 2 * p;
             double2 z = make_double2(0.0, 0.0);
-            if (e < span) z = normal_pair((unsigned long long)(j0 / 2 + p), (unsigned)row, draw, key);
+            if (e < span) z = normal_pair((unsigned long long)(j0 / 2 + p), sample_offset + (unsigned)row, draw, key);
             s_x[padpos(e)] = z.x;
             if (e + 1 < staged) s_x[padpos(e + 1)] = (e + 1 < span) ? z.y : 0.0;
         }
@@ -326,13 +335,33 @@ __global__ void __launch_bounds__(256) k_autocov_final(const double *__restrict_
     if (threadIdx.x == 0) acov[l] = sh[0] / (double)(n - l);
 }
 
+// ------------------------------------------------------------------ sample sharding: status slots of a reduce
+// After the 2n column sums of a sharded reduce: slot k counts the ranks that failed with status -(k + 1) (ST_NOMEM,
+// ST_INVALID, ST_CUDA, ST_NONFINITE).  Summed, the slots are the same on every rank, and so is the status they return.
+constexpr int NSTATUS = 4;
+
+__global__ void k_shard_status(double *slots, int local_status, const int *bad)
+{
+    const int k = threadIdx.x;
+    if (k >= NSTATUS) return;
+    const int cls = (local_status >= -NSTATUS && local_status < 0) ? -local_status - 1 : (local_status ? -ST_CUDA - 1 : -1);
+    double v = (k == cls) ? 1.0 : 0.0;
+    if (k == -ST_NONFINITE - 1 && bad && *bad) v += 1.0;        // degenerate multiplier row of this rank
+    slots[k] = v;
+}
+
 // ------------------------------------------------------------------ host side
-static int sort_track(Arena &ar, const double *d_in, double *d_sorted, long long n, cudaStream_t st)
+static size_t sort_track_bytes(long long n)
 {
     size_t bytes = 0;
-    RB_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, bytes, d_in, d_sorted, (int)n, 0, 64, st));
-    char *tmp = nullptr;
-    RB_TRY(ar.alloc(&tmp, bytes));
+    cub::DeviceRadixSort::SortKeys(nullptr, bytes, (const double *)nullptr, (double *)nullptr, (int)n, 0, 64);
+    return bytes;
+}
+
+// `tmp` holds sort_track_bytes(n)
+static int sort_track(char *tmp, const double *d_in, double *d_sorted, long long n, cudaStream_t st)
+{
+    size_t bytes = sort_track_bytes(n);
     RB_CUDA(cub::DeviceRadixSort::SortKeys(tmp, bytes, d_in, d_sorted, (int)n, 0, 64, st));
     count_launch(4);
     return 0;
@@ -385,9 +414,21 @@ struct Welford {
     double stderr_() const { return std::sqrt(var() / (double)std::max(n, 1)); }
 };
 
-// one multiplier field applied to the template:  d_out = template x W   (inference.py:656-662)
-static int wild_multiply(Arena &ar, const double *d_template, long long m, long long n, int bandwidth, const double *d_taps, double h,
-                         unsigned long long seed, unsigned draw, const double *d_innov, double *d_out, int *d_bad, cudaStream_t st)
+// scratch of wild_multiply: per-(row, tile) partial moments, then per-row (mean, sd)
+struct WildScratch {
+    double2 *part = nullptr, *stats = nullptr;
+    int alloc(Arena &ar, long long m, long long n)
+    {
+        RB_TRY(ar.alloc(&part, (size_t)m * (size_t)((n + FIR_T - 1) / FIR_T)));
+        return ar.alloc(&stats, (size_t)m);
+    }
+};
+
+// one multiplier field applied to the template:  d_out = template x W   (inference.py:656-662); row r draws the stream of
+// sample sample_offset + r
+static int wild_multiply(const WildScratch &ws, const double *d_template, long long m, long long n, int bandwidth, const double *d_taps,
+                         double h, unsigned long long seed, unsigned draw, unsigned sample_offset, const double *d_innov, double *d_out,
+                         int *d_bad, cudaStream_t st)
 {
     if (n == 1) {                                         // weights are exactly one (inference.py:556-557)
         RB_CUDA(cudaMemcpyAsync(d_out, d_template, sizeof(double) * (size_t)m, cudaMemcpyDeviceToDevice, st));
@@ -395,9 +436,7 @@ static int wild_multiply(Arena &ar, const double *d_template, long long m, long 
     }
     const int K = 2 * bandwidth + 1;
     const int tiles = (int)((n + FIR_T - 1) / FIR_T);
-    double2 *d_part = nullptr, *d_stats = nullptr;
-    RB_TRY(ar.alloc(&d_part, (size_t)m * tiles));
-    RB_TRY(ar.alloc(&d_stats, (size_t)m));
+    double2 *d_part = ws.part, *d_stats = ws.stats;
     const size_t smem = sizeof(double) * ((size_t)padpos(FIR_T + K + 8) + 8 + (size_t)K);
     static bool attr_dev[64] = {false};
     int dev = 0;
@@ -410,8 +449,8 @@ static int wild_multiply(Arena &ar, const double *d_template, long long m, long 
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
     {
         RB_PROF("k_wild_fir", st, (double)m * n * 8.0);
-        k_wild_fir<<<dim3((unsigned)tiles, (unsigned)m), FIR_THREADS, smem, st>>>(d_innov, n + K - 1, key, draw, n, K, d_taps, h, d_out,
-                                                                                  d_part, tiles);
+        k_wild_fir<<<dim3((unsigned)tiles, (unsigned)m), FIR_THREADS, smem, st>>>(d_innov, n + K - 1, key, draw, sample_offset, n, K,
+                                                                                  d_taps, h, d_out, d_part, tiles);
         RB_LAUNCH_CHECK();
     }
     k_row_moments<<<(unsigned)m, 256, 0, st>>>(d_part, tiles, n, d_stats, d_bad);
@@ -481,8 +520,63 @@ static int effective_sample_size(Arena &ar, const double *d_s, long long n, int 
     return 0;
 }
 
-static int budget_core(const double *d_centered, long long m, long long n, const double *d_observed,
-                       const rocco_b200_budget_params &P, rocco_b200_budget_result *R, cudaStream_t st)
+// Sample sharding of one estimator call.  reduce == nullptr: one rank holds every sample and each step runs as written.
+struct Shard {
+    rocco_b200_allreduce_fn reduce = nullptr;
+    void *user = nullptr;
+    long long m_total = 0;
+    double *d_red = nullptr;      // [2n column sums][NSTATUS status slots], the buffer every pass reduces
+    int *d_fin_bad = nullptr;     // non-finite flag of the finalisation
+    int failed = 0;               // first rank-local failure; the rank's local work stops until the next reduce reports it
+
+    // A rank-local step.  Unsharded its failure is returned at once; sharded it is kept for the next reduce (all ranks must
+    // get there) and 0 is returned.
+    int local(int status)
+    {
+        if (status == 0 || !reduce) return status;
+        if (!failed) failed = status;
+        return 0;
+    }
+};
+
+// One scoring pass over this rank's rows -> d_scores (and d_mean when not null).  Unsharded: the centred-WLS chain.  Sharded:
+// the per-row stages and the partial column sums (skipped after a local failure), the status slots, the reduce, and the
+// finalisation of the summed sums; every rank returns the same status.
+static int score_pass(Shard &S, const double *d_rows, long long m, long long n, const rocco_b200_score_params &prm, double *d_scores,
+                      double *d_mean, const int *d_bad, cudaStream_t st)
+{
+    rocco_b200_score_outputs so{};
+    so.scores = d_scores; so.mean = d_mean;
+    if (!S.reduce) return score::centered_wls(d_rows, m, n, prm, &so, st);
+    if (!S.failed) {
+        rocco_b200_score_outputs none{};
+        S.local(score::centered_wls(d_rows, m, n, prm, &none, st, S.d_red));
+    }
+    k_shard_status<<<1, 32, 0, st>>>(S.d_red + 2 * n, S.failed, d_bad);
+    count_launch();
+    S.local(cudaGetLastError() == cudaSuccess ? 0 : ST_CUDA);
+    if (S.reduce(S.d_red, (size_t)(2 * n + NSTATUS), (void *)st, S.user) != 0) {
+        set_error("sample-sharded budget null: the all-reduce callback failed");
+        return ST_CUDA;
+    }
+    RB_TRY(score::finalize_acc(S.d_red, n, false, S.m_total, prm, &so, S.d_fin_bad, st));
+    double slots[NSTATUS];
+    int flags[2] = {0, 0};
+    RB_CUDA(cudaMemcpyAsync(slots, S.d_red + 2 * n, sizeof(slots), cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(&flags[0], S.d_fin_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    if (d_bad) RB_CUDA(cudaMemcpyAsync(&flags[1], d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    for (int k = 0; k < NSTATUS; ++k) {
+        if (!(slots[k] > 0.0)) continue;
+        if (flags[1]) set_error("degenerate multiplier field");
+        else if (!S.failed) set_error("sample-sharded budget null: another rank failed with status %d", -(k + 1));
+        return -(k + 1);
+    }
+    return flags[0] ? ST_NONFINITE : 0;
+}
+
+static int budget_core(const double *d_centered, long long m, long long n, const double *d_observed, const rocco_b200_budget_params &P,
+                       Shard &S, rocco_b200_budget_result *R, cudaStream_t st)
 {
     if (!d_centered || !R || m <= 0 || n <= 0) return ST_INVALID;
     RB_TRY(ensure_device());
@@ -492,31 +586,45 @@ static int budget_core(const double *d_centered, long long m, long long n, const
     if (bandwidth > MAX_BANDWIDTH) { set_error("bootstrap bandwidth %d exceeds %d", bandwidth, MAX_BANDWIDTH); return ST_INVALID; }
     double *d_fit = nullptr, *d_mean = nullptr, *d_tmpl = nullptr, *d_boot = nullptr, *d_ref = nullptr, *d_sorted = nullptr;
     double *d_part = nullptr, *d_small = nullptr, *d_taps = nullptr;
+    char *d_sort_tmp = nullptr;
     int *d_bad = nullptr;
-    RB_TRY(ar.alloc(&d_fit, (size_t)n));
-    RB_TRY(ar.alloc(&d_mean, (size_t)n));
-    RB_TRY(ar.alloc(&d_ref, (size_t)n));
-    RB_TRY(ar.alloc(&d_sorted, (size_t)n));
-    RB_TRY(ar.alloc(&d_tmpl, (size_t)m * n));
-    RB_TRY(ar.alloc(&d_boot, (size_t)m * n));
-    RB_TRY(ar.alloc(&d_part, (size_t)RED_BLOCKS * 6));
-    RB_TRY(ar.alloc(&d_small, 16));
-    RB_TRY(ar.alloc(&d_bad, 1));
-    RB_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
+    WildScratch wild;
+    if (S.reduce) {
+        // the buffers every pass needs to take part in a reduce (a failure here cannot be reported to the other ranks)
+        RB_TRY(ar.alloc(&S.d_red, (size_t)(2 * n + NSTATUS)));
+        RB_TRY(ar.alloc(&S.d_fin_bad, 1));
+        RB_CUDA(cudaMemsetAsync(S.d_fin_bad, 0, sizeof(int), st));
+    }
     std::vector<double> taps;
     const double tap_step = bartlett_taps(bandwidth, taps);
-    RB_TRY(ar.alloc(&d_taps, taps.size()));
-    RB_CUDA(cudaMemcpyAsync(d_taps, taps.data(), sizeof(double) * taps.size(), cudaMemcpyHostToDevice, st));
+    // everything the passes and the draw loop need, before the first reduce
+    auto setup = [&]() -> int {
+        RB_TRY(ar.alloc(&d_bad, 1));
+        RB_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
+        RB_TRY(ar.alloc(&d_fit, (size_t)n));
+        RB_TRY(ar.alloc(&d_mean, (size_t)n));
+        RB_TRY(ar.alloc(&d_ref, (size_t)n));
+        RB_TRY(ar.alloc(&d_sorted, (size_t)n));
+        RB_TRY(ar.alloc(&d_tmpl, (size_t)m * n));
+        RB_TRY(ar.alloc(&d_boot, (size_t)m * n));
+        RB_TRY(ar.alloc(&d_part, (size_t)RED_BLOCKS * 6));
+        RB_TRY(ar.alloc(&d_small, 16));
+        RB_TRY(ar.alloc(&d_sort_tmp, sort_track_bytes(n)));
+        RB_TRY(wild.alloc(ar, m, n));
+        RB_TRY(ar.alloc(&d_taps, taps.size()));
+        RB_CUDA(cudaMemcpyAsync(d_taps, taps.data(), sizeof(double) * taps.size(), cudaMemcpyHostToDevice, st));
+        return 0;
+    };
+    RB_TRY(S.local(setup()));
 
     // ---- fit, template, fitted-null score field
-    rocco_b200_score_outputs so{};
-    so.scores = d_fit; so.mean = d_mean;
-    RB_TRY(score::centered_wls(d_centered, m, n, P.score, &so, st));
-    {
+    RB_TRY(score_pass(S, d_centered, m, n, P.score, d_fit, d_mean, d_bad, st));
+    if (!S.failed) {
         const long long total = m * n;
         const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, 148LL * 32);
         k_template<<<grid, 256, 0, st>>>(d_centered, d_mean, m, n, d_tmpl);
-        RB_LAUNCH_CHECK();
+        count_launch();
+        RB_TRY(S.local(cudaGetLastError() == cudaSuccess ? 0 : ST_CUDA));
     }
     double h[8];
     {
@@ -530,10 +638,8 @@ static int budget_core(const double *d_centered, long long m, long long n, const
         R->null_reference_mean_positive_consensus = h[0] / (double)n;
         R->null_reference_max_positive_consensus = h[1];
     }
-    rocco_b200_score_outputs so2{};
-    so2.scores = d_ref;
-    RB_TRY(score::centered_wls(d_tmpl, m, n, P.score, &so2, st));
-    RB_TRY(sort_track(ar, d_ref, d_sorted, n, st));
+    RB_TRY(score_pass(S, d_tmpl, m, n, P.score, d_ref, nullptr, d_bad, st));
+    RB_TRY(sort_track(d_sort_tmp, d_ref, d_sorted, n, st));
     k_center_scale<<<1, 32, 0, st>>>(d_sorted, n, d_small);
     RB_LAUNCH_CHECK();
     RB_CUDA(cudaMemcpyAsync(h, d_small, 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -553,10 +659,11 @@ static int budget_core(const double *d_centered, long long m, long long n, const
     const size_t innov_per_draw = (size_t)m * (size_t)(n + 2 * bandwidth);
     for (int d = 0; d < draws; ++d) {
         const double *innov = P.d_innovations ? P.d_innovations + (size_t)d * innov_per_draw : nullptr;
-        RB_TRY(wild_multiply(ar, d_tmpl, m, n, bandwidth, d_taps, tap_step, P.random_seed, (unsigned)d, innov, d_boot, d_bad, st));
-        rocco_b200_score_outputs sd{};
-        sd.scores = d_ref;                                        // the reference field is no longer needed: reuse its buffer
-        RB_TRY(score::centered_wls(d_boot, m, n, P.score, &sd, st));
+        if (!S.failed)
+            RB_TRY(S.local(wild_multiply(wild, d_tmpl, m, n, bandwidth, d_taps, tap_step, P.random_seed, (unsigned)d,
+                                         (unsigned)P.sample_offset, innov, d_boot, d_bad, st)));
+        // the reference field is no longer needed: reuse its buffer
+        RB_TRY(score_pass(S, d_boot, m, n, P.score, d_ref, nullptr, d_bad, st));
         RB_TRY(track_sums(d_ref, n, center, soft, threshold, d_part, d_small, h, st));
         if (h[5] != 0.0) return ST_NONFINITE;
         for (int q = 0; q < 4; ++q) acc[q].add(h[q] / (double)n);
@@ -590,7 +697,7 @@ static int budget_core(const double *d_centered, long long m, long long n, const
     R->effective_count = R->nonnull_fraction * R->effective_total_count;
     R->num_loci = n;
     // ---- automatic gamma inputs (rocco.py:762-769)
-    RB_TRY(sort_track(ar, d_obs, d_sorted, n, st));
+    RB_TRY(sort_track(d_sort_tmp, d_obs, d_sorted, n, st));
     k_positive_median<<<1, 32, 0, st>>>(d_sorted, n, d_small);
     RB_LAUNCH_CHECK();
     RB_CUDA(cudaMemcpyAsync(h, d_small, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -632,7 +739,26 @@ RB_API int rocco_b200_budget_nonnull_fraction_dev(const double *d_centered, size
 {
     rocco_b200_budget_params P;
     if (params) P = *params; else rocco_b200_default_budget_params(&P);
-    return budget::budget_core(d_centered, (long long)m, (long long)n, d_observed_scores, P, result, (cudaStream_t)cuda_stream);
+    if (P.sample_offset < 0) return ST_INVALID;
+    budget::Shard whole;
+    return budget::budget_core(d_centered, (long long)m, (long long)n, d_observed_scores, P, whole, result, (cudaStream_t)cuda_stream);
+}
+
+RB_API int rocco_b200_budget_nonnull_fraction_sharded_dev(const double *d_centered_local, size_t m_local, size_t n, size_t m_total,
+                                                          const double *d_observed_scores, const rocco_b200_budget_params *params,
+                                                          rocco_b200_allreduce_fn allreduce, void *user, rocco_b200_budget_result *result,
+                                                          void *cuda_stream)
+{
+    rocco_b200_budget_params P;
+    if (params) P = *params; else rocco_b200_default_budget_params(&P);
+    if (m_local == 0 || P.sample_offset < 0 || (size_t)P.sample_offset + m_local > m_total) return ST_INVALID;
+    if (!allreduce && m_local != m_total) return ST_INVALID;
+    budget::Shard shard;
+    shard.reduce = allreduce;
+    shard.user = user;
+    shard.m_total = (long long)m_total;
+    return budget::budget_core(d_centered_local, (long long)m_local, (long long)n, d_observed_scores, P, shard, result,
+                               (cudaStream_t)cuda_stream);
 }
 
 // One bootstrap draw's input (inference.py:653-662): d_out[i][j] = d_template[i][j] * W_ij with W the unit-variance
@@ -648,11 +774,13 @@ RB_API int rocco_b200_wild_multiply_dev(const double *d_template, size_t m, size
     const double tap_step = budget::bartlett_taps(bandwidth, taps);
     double *d_taps = nullptr;
     int *d_bad = nullptr;
+    budget::WildScratch ws;
+    RB_TRY(ws.alloc(ar, (long long)m, (long long)n));
     RB_TRY(ar.alloc(&d_taps, taps.size()));
     RB_TRY(ar.alloc(&d_bad, 1));
     RB_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
     RB_CUDA(cudaMemcpyAsync(d_taps, taps.data(), sizeof(double) * taps.size(), cudaMemcpyHostToDevice, st));
-    RB_TRY(budget::wild_multiply(ar, d_template, (long long)m, (long long)n, bandwidth, d_taps, tap_step, random_seed, draw_index,
+    RB_TRY(budget::wild_multiply(ws, d_template, (long long)m, (long long)n, bandwidth, d_taps, tap_step, random_seed, draw_index, 0,
                                  d_innovations, d_out, d_bad, st));
     int bad = 0;
     RB_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -686,7 +814,9 @@ RB_API int rocco_budget_nonnull_fraction_f64(const double *centered, size_t m, s
         RB_CUDA(cudaMemcpyAsync(d_i, innovations, sizeof(double) * cnt, cudaMemcpyHostToDevice, st));
     }
     P.d_innovations = d_i;
-    const int status = budget::budget_core(d_c, (long long)m, (long long)n, d_o, P, result, st);
+    if (P.sample_offset < 0) return ST_INVALID;
+    budget::Shard whole;
+    const int status = budget::budget_core(d_c, (long long)m, (long long)n, d_o, P, whole, result, st);
     cudaStreamSynchronize(st);
     return status;
 }
@@ -722,11 +852,13 @@ RB_API int rocco_positive_score_median_f64(const double *scores, size_t n, doubl
     cudaStream_t st = lease.stream();
     Arena ar(st);
     double *d_s = nullptr, *d_sorted = nullptr, *d_out = nullptr;
+    char *d_tmp = nullptr;
     RB_TRY(ar.alloc(&d_s, n));
     RB_TRY(ar.alloc(&d_sorted, n));
     RB_TRY(ar.alloc(&d_out, 2));
+    RB_TRY(ar.alloc(&d_tmp, budget::sort_track_bytes((long long)n)));
     RB_CUDA(cudaMemcpyAsync(d_s, scores, sizeof(double) * n, cudaMemcpyHostToDevice, st));
-    RB_TRY(budget::sort_track(ar, d_s, d_sorted, (long long)n, st));
+    RB_TRY(budget::sort_track(d_tmp, d_s, d_sorted, (long long)n, st));
     budget::k_positive_median<<<1, 32, 0, st>>>(d_sorted, (long long)n, d_out);
     RB_LAUNCH_CHECK();
     double h[2];

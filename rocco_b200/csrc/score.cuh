@@ -16,9 +16,15 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
 int pilot_offsets(const void *d_x, int in_f32, long long rows, long long n, long long row_stride, double *d_pilot,
                   cudaStream_t st, int exact = 0);
 
-// Centered matrix -> per-locus WLS outputs (wls_backend.c:744-947).
+// Centered matrix -> per-locus WLS outputs (wls_backend.c:744-947).  d_acc2 != nullptr: stop at the column sums of these
+// rows instead, d_acc2[2][n] = {sum y/post, sum 1/post} (what scores and mean need), for finalize_acc after a cross-rank sum.
 int centered_wls(const double *d_centered, long long m, long long n, const rocco_b200_score_params &prm,
-                 rocco_b200_score_outputs *out, cudaStream_t st);
+                 rocco_b200_score_outputs *out, cudaStream_t st, double *d_acc2 = nullptr);
+
+// Per-bin outputs from column sums over m_total samples (wls_backend.c:915-937): d_acc [4][n], or [2][n] without has_rq (the
+// raw / prior variance outputs must then be NULL).  Sets *d_bad on a non-finite result.
+int finalize_acc(const double *d_acc, long long n, bool has_rq, long long m_total, const rocco_b200_score_params &prm,
+                 rocco_b200_score_outputs *out, int *d_bad, cudaStream_t st);
 
 // a / b from a correctly rounded reciprocal rb = RN(1/b): Markstein's final step (q = RN(a*rb), r = a - q*b exactly by
 // FMA, RN(q + r*rb)) gives the correctly rounded quotient for operands in the normal range without the generic

@@ -345,7 +345,7 @@ struct CombineParams {
     double ldf, pdf, tdf, pfr, lower_bound_z, min_effect;
     int use_min_effect; int const_rows;
     double *scores, *mean, *raw, *prior, *mod, *se;
-    double *acc;          // != nullptr: sample-sharded mode, write the four per-bin sums [4][n] and stop
+    double *acc;          // != nullptr: sample-sharded mode, write the per-bin sums [4][n] ([2][n] without WANT_RQ) and stop
     int *bad;
 };
 
@@ -424,7 +424,8 @@ __global__ void __launch_bounds__(CB_THREADS, 2) k_combine(CombineParams P)
     }
     if (!live) return;
     if (P.acc) {                                   // partial sums of this rank's samples (summed across ranks by the caller)
-        P.acc[j] = wsum; P.acc[P.n + j] = psum; P.acc[2 * P.n + j] = rsum; P.acc[3 * P.n + j] = qsum;
+        P.acc[j] = wsum; P.acc[P.n + j] = psum;
+        if (WANT_RQ) { P.acc[2 * P.n + j] = rsum; P.acc[3 * P.n + j] = qsum; }
         return;
     }
     // wls_backend.c:915-937
@@ -445,14 +446,16 @@ __global__ void __launch_bounds__(CB_THREADS, 2) k_combine(CombineParams P)
     if (P.se) P.se[j] = se;
 }
 
-// finalisation of summed accumulators (sample-sharded scoring): wls_backend.c:915-937 on [4][n] sums
-__global__ void __launch_bounds__(256) k_finalize_acc(const double *acc, long long n, double m_total, double lower_bound_z,
+// finalisation of summed accumulators (sample-sharded scoring): wls_backend.c:915-937 on [4][n] sums, or on [2][n] when
+// only the scores and the mean are wanted (has_rq = 0: the raw / prior variance rows are absent)
+__global__ void __launch_bounds__(256) k_finalize_acc(const double *acc, long long n, int has_rq, double m_total, double lower_bound_z,
                                                       double min_effect, int use_min_effect, double *scores, double *mean_o,
                                                       double *raw, double *prior, double *mod, double *se_o, int *bad)
 {
     const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n) return;
-    const double wsum = acc[j], psum = acc[n + j], rsum = acc[2 * n + j], qsum = acc[3 * n + j];
+    const double wsum = acc[j], psum = acc[n + j];
+    const double rsum = has_rq ? acc[2 * n + j] : 1.0, qsum = has_rq ? acc[3 * n + j] : 1.0;
     const double Pj = fmax(psum, 1.0e-8);
     const double mean = wsum / Pj;
     const double se = sqrt(1.0 / Pj);
@@ -529,8 +532,9 @@ static int wls_rows(const double *d_centered, WlsRun &R, long long r0, long long
 }
 
 // after every row went through wls_rows: sort-path for flagged rows, then the fused column reduction
+// d_acc != nullptr: write the per-bin sums instead of the outputs -- all four rows with acc_rq, else {sum y/post, sum 1/post}
 static int wls_finish(const double *d_centered, WlsRun &R, const rocco_b200_score_params &prm, rocco_b200_score_outputs *out,
-                      cudaStream_t st, double *d_acc = nullptr)
+                      cudaStream_t st, double *d_acc = nullptr, bool acc_rq = true)
 {
     const long long m = R.m, n = R.n;
     CombineParams P{};
@@ -566,7 +570,7 @@ static int wls_finish(const double *d_centered, WlsRun &R, const rocco_b200_scor
     {
         RB_PROF("k_combine", st, (double)m * (double)n * (P.const_rows ? 8.0 : 16.0) + 48.0 * (double)n);
         const unsigned grid = (unsigned)((n + CB_THREADS - 1) / CB_THREADS);
-        const bool want_rq = (P.raw != nullptr) || (P.prior != nullptr) || (P.acc != nullptr);   // raw / prior variance sums only when asked for
+        const bool want_rq = P.acc ? acc_rq : (P.raw != nullptr) || (P.prior != nullptr);   // raw / prior variance sums only when asked for
         if (P.const_rows) {
             if (want_rq) k_combine<true, true><<<grid, CB_THREADS, 0, st>>>(P); else k_combine<true, false><<<grid, CB_THREADS, 0, st>>>(P);
         } else {
@@ -582,14 +586,25 @@ static int wls_finish(const double *d_centered, WlsRun &R, const rocco_b200_scor
 }
 
 int centered_wls(const double *d_centered, long long m, long long n, const rocco_b200_score_params &prm,
-                 rocco_b200_score_outputs *out, cudaStream_t st)
+                 rocco_b200_score_outputs *out, cudaStream_t st, double *d_acc2)
 {
     if (!d_centered || !out || m <= 0 || n <= 0) return ST_INVALID;
     Arena ar(st);
     WlsRun R;
     RB_TRY(wls_prepare(ar, m, n, prm, out, R, st));
     RB_TRY(wls_rows(d_centered, R, 0, m, st));
-    return wls_finish(d_centered, R, prm, out, st);
+    return wls_finish(d_centered, R, prm, out, st, d_acc2, false);
+}
+
+int finalize_acc(const double *d_acc, long long n, bool has_rq, long long m_total, const rocco_b200_score_params &prm,
+                 rocco_b200_score_outputs *out, int *d_bad, cudaStream_t st)
+{
+    k_finalize_acc<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_acc, n, has_rq ? 1 : 0, (double)m_total, prm.lower_bound_z,
+                                                                prm.min_effect, prm.use_min_effect, out->scores, out->mean,
+                                                                out->raw_variance, out->prior_variance, out->moderated_variance,
+                                                                out->standard_error, d_bad);
+    RB_LAUNCH_CHECK();
+    return 0;
 }
 
 // ------------------------------------------------------------------ the full chain (inference.py:302-379)
@@ -860,13 +875,22 @@ RB_API int rocco_b200_score_loci_wls_dev(const void *d_matrix, int dtype, size_t
     return score::score_loci_dev(d_matrix, dtype, (long long)m, (long long)n, params, out, (cudaStream_t)cuda_stream);
 }
 
-/* Sample-sharded scoring: this rank's rows -> four per-bin sums [4][n]; sum them over ranks, then finalise. */
-RB_API int rocco_b200_score_partial_dev(const void *d_matrix, int dtype, size_t m_local, size_t n,
-                                        const rocco_b200_score_params *params, double *d_acc, void *cuda_stream)
+/* Sample-sharded scoring: this rank's rows -> four per-bin sums [4][n]; sum them over ranks, then finalise.  The _ex form
+ * also leaves the rank's centred rows in d_centered_out [m_local][n] (NULL: not kept). */
+RB_API int rocco_b200_score_partial_ex_dev(const void *d_matrix, int dtype, size_t m_local, size_t n,
+                                           const rocco_b200_score_params *params, double *d_centered_out, double *d_acc,
+                                           void *cuda_stream)
 {
     if (!d_acc) return ST_INVALID;
     rocco_b200_score_outputs out{};
+    out.centered_matrix = d_centered_out;
     return score::score_loci_core(d_matrix, nullptr, dtype, (long long)m_local, (long long)n, params, &out, (cudaStream_t)cuda_stream, d_acc);
+}
+
+RB_API int rocco_b200_score_partial_dev(const void *d_matrix, int dtype, size_t m_local, size_t n,
+                                        const rocco_b200_score_params *params, double *d_acc, void *cuda_stream)
+{
+    return rocco_b200_score_partial_ex_dev(d_matrix, dtype, m_local, n, params, nullptr, d_acc, cuda_stream);
 }
 
 RB_API int rocco_b200_score_finalize_dev(const double *d_acc, size_t m_total, size_t n, const rocco_b200_score_params *params,
@@ -881,10 +905,7 @@ RB_API int rocco_b200_score_finalize_dev(const double *d_acc, size_t m_total, si
     int *d_bad = nullptr;
     RB_TRY(ar.alloc(&d_bad, 1));
     RB_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
-    score::k_finalize_acc<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_acc, (long long)n, (double)m_total, prm.lower_bound_z, prm.min_effect,
-                                                                      prm.use_min_effect, out->scores, out->mean, out->raw_variance,
-                                                                      out->prior_variance, out->moderated_variance, out->standard_error, d_bad);
-    RB_LAUNCH_CHECK();
+    RB_TRY(score::finalize_acc(d_acc, (long long)n, true, (long long)m_total, prm, out, d_bad, st));
     const int w = score::resolve_spatial_window((long long)n, prm.spatial_window);
     out->resolved_spatial_window = w;
     out->total_df = (w > 0 ? fmax(4.0, (double)w - 3.0) : 1.0) + fmax(prm.prior_df, 0.0);

@@ -469,19 +469,24 @@ def sweep_multipliers(scores, gamma: float, lambdas):
     return counts, pen, obj
 
 
-def score_partial_device(d_matrix_local, params=None):
-    """Per-sample stages of this rank's rows -> the four per-bin accumulators, a [4, bins] float64 CUDA tensor."""
+def score_partial_device(d_matrix_local, params=None, centered_out=None):
+    """Per-sample stages of this rank's rows -> the four per-bin accumulators, a [4, bins] float64 CUDA tensor.
+    ``centered_out`` (a contiguous float64 CUDA tensor shaped like the rows) also receives the rows' centred values."""
     torch = _torch()
     lib = _lib.load()
     if d_matrix_local.dim() != 2 or not d_matrix_local.is_cuda or not d_matrix_local.is_contiguous():
         raise ValueError("`d_matrix_local` must be a contiguous two-dimensional CUDA tensor")
     m, n = d_matrix_local.shape
+    if centered_out is not None and (tuple(centered_out.shape) != (m, n) or centered_out.dtype != torch.float64
+                                     or centered_out.device != d_matrix_local.device or not centered_out.is_contiguous()):
+        raise ValueError("`centered_out` must be a contiguous float64 tensor shaped like `d_matrix_local` on its device")
     acc = torch.empty((4, n), dtype=torch.float64, device=d_matrix_local.device)
     prm = params if params is not None else score_params()
     with torch.cuda.device(d_matrix_local.device):
-        st = lib.rocco_b200_score_partial_dev(
+        st = lib.rocco_b200_score_partial_ex_dev(
             ctypes.c_void_p(d_matrix_local.data_ptr()), 1 if d_matrix_local.dtype == torch.float32 else 0, m, n,
-            ctypes.byref(prm), ctypes.c_void_p(acc.data_ptr()), ctypes.c_void_p(_stream_ptr(d_matrix_local.device)))
+            ctypes.byref(prm), None if centered_out is None else ctypes.c_void_p(centered_out.data_ptr()),
+            ctypes.c_void_p(acc.data_ptr()), ctypes.c_void_p(_stream_ptr(d_matrix_local.device)))
     if st == _lib.ST_NONFINITE:
         raise ValueError("Locus scoring produced non-finite values (or `chrom_matrix` contains non-finite values)")
     _lib.check(st, "score_partial")
@@ -509,15 +514,30 @@ def score_finalize_device(acc, m_total: int, params=None, details: bool = False)
     return res if details else res["scores"]
 
 
-def score_loci_wls_sample_sharded(d_matrix_local, m_total: int, params=None, group=None, details: bool = False):
+def score_loci_wls_sample_sharded(d_matrix_local, m_total: int, params=None, group=None, details: bool = False,
+                                  keep_centered: bool = False):
     """score_loci_wls with the SAMPLES sharded over ranks (every rank holds [m_local, bins] of the same bins):
     per-sample stages stay local; one all-reduce(sum, float64) of the [4, bins] accumulators; every rank then
-    finishes the per-bin combine (SURVEY.md section 8e(2))."""
+    finishes the per-bin combine (SURVEY.md section 8e(2)).
+
+    With ``keep_centered`` returns ``(result, d_centered_local, baseline_window)``: this rank's centred rows (float64,
+    the input of ``budget_null_sample_sharded``) and the resolved Whittaker window, which is the
+    ``dependence_lag_hint`` the reference's CLI hands the budget null (rocco.py:1035)."""
     import torch.distributed as dist
-    acc = score_partial_device(d_matrix_local, params)
+    torch = _torch()
+    centered = None
+    if keep_centered:
+        centered = torch.empty(tuple(d_matrix_local.shape), dtype=torch.float64, device=d_matrix_local.device)
+    acc = score_partial_device(d_matrix_local, params, centered_out=centered)
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
         dist.all_reduce(acc, group=group)
-    return score_finalize_device(acc, m_total, params, details=details)
+    result = score_finalize_device(acc, m_total, params, details=details)
+    if not keep_centered:
+        return result
+    from .inference import _resolve_local_baseline_window
+    prm = params if params is not None else score_params()
+    window = _resolve_local_baseline_window(d_matrix_local.shape[1], prm.baseline_window if prm.baseline_window > 0 else 101)
+    return result, centered, window
 
 
 # ------------------------------------------------------------------ budget null on device tensors (SURVEY.md 8(f) rank 1)
@@ -559,3 +579,131 @@ def budget_null_device(d_centered, d_observed_scores=None, params=None, dependen
         raise ValueError("Budget initialization produced non-finite values")
     _lib.check(st, "budget null")
     return float(res.nonnull_fraction), _budget_details(res)
+
+
+# ------------------------------------------------------------------ budget null with the samples sharded over ranks
+class _DeviceBuffer:
+    """A raw float64 device buffer as a torch tensor (``__cuda_array_interface__``, no copy)."""
+
+    def __init__(self, ptr: int, count: int):
+        self.__cuda_array_interface__ = {"shape": (int(count),), "typestr": "<f8", "data": (int(ptr), False),
+                                          "strides": None, "version": 2}
+
+
+def _budget_null_sharded(d_centered_local, m_total: int, sample_offset: int, reduce_fn, d_observed_scores=None, params=None,
+                         dependence_lag_hint=None, num_null_draws=25, random_seed=0, min_null_draws=None,
+                         stability_abs_tol=5.0e-3, stability_rel_tol=5.0e-2, innovations=None):
+    """One rank's part of the sample-sharded estimator, shapes already agreed between the ranks.  ``reduce_fn(buf)`` sums
+    the float64 CUDA tensor ``buf`` over all ranks in place, ordered on torch's current stream; it is called with the same
+    length on every rank, 2 + (draws used) times.  An exception in it becomes a failed call on this rank.  ``reduce_fn=None``
+    (one rank holding every sample) is the unsharded estimator."""
+    from .inference import _budget_details, _hint
+    torch = _torch()
+    lib = _lib.load()
+    m, n = d_centered_local.shape
+    dev = d_centered_local.device
+    prm = _lib.BudgetParams()
+    lib.rocco_b200_default_budget_params(ctypes.byref(prm))
+    if params is not None:
+        prm.score = params
+    prm.dependence_lag_hint = _hint(dependence_lag_hint)
+    prm.num_null_draws = int(max(1, num_null_draws))
+    prm.min_null_draws = 0 if min_null_draws is None else int(max(1, min_null_draws))
+    prm.stability_abs_tol = float(stability_abs_tol)
+    prm.stability_rel_tol = float(stability_rel_tol)
+    prm.random_seed = int(random_seed) & 0xFFFFFFFFFFFFFFFF
+    prm.sample_offset = int(sample_offset)
+    prm.d_innovations = None if innovations is None else innovations.data_ptr()
+    failure = []
+
+    def _reduce(ptr, count, _stream, _user):
+        try:
+            reduce_fn(torch.as_tensor(_DeviceBuffer(ptr, count), device=dev))
+            return 0
+        except BaseException as exc:          # never let it unwind through the C frames
+            failure.append(exc)
+            return 1
+
+    cb = None if reduce_fn is None else _lib.ALLREDUCE_FN(_reduce)
+    res = _lib.BudgetResult()
+    with torch.cuda.device(dev):
+        st = lib.rocco_b200_budget_nonnull_fraction_sharded_dev(
+            ctypes.c_void_p(d_centered_local.data_ptr()), m, n, int(m_total),
+            None if d_observed_scores is None else ctypes.c_void_p(d_observed_scores.data_ptr()),
+            ctypes.byref(prm), cb, None, ctypes.byref(res), ctypes.c_void_p(_stream_ptr(dev)))
+    if failure:
+        raise RuntimeError(f"budget null: the all-reduce failed: {failure[0]!r}") from failure[0]
+    if st == _lib.ST_NONFINITE:
+        raise ValueError("Budget initialization produced non-finite values")
+    _lib.check(st, "budget null")
+    return float(res.nonnull_fraction), _budget_details(res)
+
+
+def _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint):
+    """This rank's own argument errors (checked before the ranks compare shapes), or None."""
+    from .inference import _resolve_budget_bootstrap_bandwidth
+    torch = _torch()
+    x = d_centered_local
+    if x.dim() != 2 or not x.is_cuda or not x.is_contiguous() or x.dtype != torch.float64:
+        return "`d_centered_local` must be a contiguous two-dimensional float64 CUDA tensor"
+    m, n = x.shape
+    if m == 0 or n == 0:
+        return "`centered_matrix` must contain at least one sample and one locus on every rank"
+    for name, t, shape in (("observed_scores", d_observed_scores, (n,)),
+                           ("innovations", innovations, (int(max(1, num_null_draws)), m,
+                                                         n + 2 * _resolve_budget_bootstrap_bandwidth(n, dependence_lag_hint)))):
+        if t is not None and (tuple(t.shape) != shape or t.dtype != torch.float64 or t.device != x.device or not t.is_contiguous()):
+            return f"`{name}` must be a contiguous float64 tensor of shape {shape} on the device of `d_centered_local`"
+    return None
+
+
+def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=None, group=None, dependence_lag_hint=None,
+                               num_null_draws=25, random_seed=0, min_null_draws=None, stability_abs_tol=5.0e-3,
+                               stability_rel_tol=5.0e-2, innovations=None):
+    """``budget_null_device`` with the SAMPLES sharded over the ranks of ``group`` (BASELINE.json config 5): every rank
+    passes its centred rows ``[m_local, bins]`` (e.g. from ``score_loci_wls_sample_sharded(..., keep_centered=True)``, ranks
+    in sample order) and the same observed scores and arguments.  Each scoring pass all-reduces 2 x bins float64 column
+    sums (plus four status slots); every rank returns the same ``(nonnull_fraction, details)``, with the keys of
+    ``budget_null_device``, and raises the same exception.  ``innovations``: this rank's rows,
+    ``[draws, m_local, bins + 2*bandwidth]`` float64 on the device."""
+    import torch.distributed as dist
+    torch = _torch()
+    problem = _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint)
+    sharded = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+    if not sharded:
+        if problem:
+            raise ValueError(problem)
+        m = d_centered_local.shape[0]
+        return _budget_null_sharded(d_centered_local, m, 0, None, d_observed_scores, params, dependence_lag_hint,
+                                    num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations)
+    dev = d_centered_local.device if d_centered_local.is_cuda else torch.device("cuda", torch.cuda.current_device())
+    m, n = (d_centered_local.shape if d_centered_local.dim() == 2 else (0, 0))
+    # the reduce workspace is allocated before the ranks compare notes, so that its failure is one more problem reported
+    workspace = None
+    if problem is None:
+        try:
+            workspace = torch.empty(2 * n + 4, dtype=torch.float64, device=dev)
+        except RuntimeError as exc:
+            problem = f"could not allocate the reduce workspace: {exc}"
+    world = dist.get_world_size(group)
+    mine = torch.tensor([int(m), int(n), 0 if problem is None else 1], dtype=torch.int64, device=dev)
+    every = [torch.empty_like(mine) for _ in range(world)]
+    dist.all_gather(every, mine, group=group)
+    rows = torch.stack(every).cpu().tolist()
+    if problem is not None:
+        raise ValueError(problem)
+    if any(r[2] for r in rows):
+        raise ValueError("budget null: another rank rejected its arguments")
+    if any(r[1] != n for r in rows):
+        raise ValueError(f"budget null: every rank must hold the same loci, got bins {[r[1] for r in rows]}")
+    rank = dist.get_rank(group)
+    offset, m_total = sum(r[0] for r in rows[:rank]), sum(r[0] for r in rows)
+
+    def reduce_fn(buf):
+        w = workspace[: buf.numel()]
+        w.copy_(buf)
+        dist.all_reduce(w, group=group)
+        buf.copy_(w)
+
+    return _budget_null_sharded(d_centered_local, m_total, offset, reduce_fn, d_observed_scores, params, dependence_lag_hint,
+                                num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations)

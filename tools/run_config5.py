@@ -3,7 +3,12 @@ over the ranks (125 per GPU at 8), one all-reduce of the four per-bin accumulato
 per chromosome on the rank that owns it (LPT).  Chromosomes are generated, scored and dropped one at a time, so a rank never
 holds more than one chromosome's matrix + scratch (~35 GB).
 
-    torchrun --nproc-per-node 8 tools/run_config5.py [--samples 1000] [--step-bp 20] [--chroms chr1,chr2]
+    torchrun --nproc-per-node 8 tools/run_config5.py [--samples 1000] [--step-bp 20] [--chroms chr1,chr2] [--budget-null]
+
+--budget-null replaces the sweep by the default CLI flow on the same layout: per chromosome the sharded scoring keeps each
+rank's centred rows, the wild-bootstrap budget null runs with the samples still sharded (2n column sums all-reduced per
+scoring pass), the fractions go through the empirical-Bayes budgets and the automatic gamma (host, identical on every
+rank), and the owner rank solves each chromosome at its budget.
 """
 import argparse, json, math, os, sys, time
 import numpy as np, torch, torch.distributed as dist
@@ -16,6 +21,8 @@ ap.add_argument("--samples", type=int, default=1000)
 ap.add_argument("--step-bp", type=int, default=20)
 ap.add_argument("--chroms", default="")
 ap.add_argument("--multipliers", type=int, default=256)
+ap.add_argument("--budget-null", action="store_true", help="budget null + EB budgets + solve instead of the sweep")
+ap.add_argument("--null-draws", type=int, default=25)
 args = ap.parse_args()
 rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 local = int(os.environ.get("LOCAL_RANK", 0))
@@ -32,6 +39,82 @@ for r, part in enumerate(pipeline.lpt_partition(bins, world)):
         owner[k] = r
 prm = pipeline.score_params(prior_df=6.0)
 ev = lambda: torch.cuda.Event(enable_timing=True)
+
+
+def budget_null_run():
+    from rocco_b200.rocco import _resolve_budgets, _resolve_chrom_gamma
+    per_chrom, owned = {}, {}
+    for k, (c, n) in enumerate(zip(names, bins)):
+        x = chrom_matrix_torch(m_local, n, chrom_seed(c), dev, torch.float32, sample_stream=rank + 1)
+        if world > 1:
+            dist.barrier()
+        e = [ev() for _ in range(3)]
+        e[0].record()
+        scores, cent, window = pipeline.score_loci_wls_sample_sharded(x, m_local * world, prm, keep_centered=True)
+        del x
+        e[1].record()
+        frac, det = pipeline.budget_null_sample_sharded(cent, scores, params=prm, dependence_lag_hint=window,
+                                                        num_null_draws=args.null_draws)
+        e[2].record()
+        del cent
+        # the collective alone, at the estimator's size (2n sums + 4 status slots), timed after the call
+        buf = torch.zeros(2 * n + 4, dtype=torch.float64, device=dev)
+        r = [ev() for _ in range(2)]
+        if world > 1:
+            dist.all_reduce(buf)
+        r[0].record()
+        for _ in range(5):
+            if world > 1:
+                dist.all_reduce(buf)
+        r[1].record()
+        torch.cuda.synchronize()
+        passes = 2 + int(det["num_null_draws"])
+        per_chrom[c] = {"bins": n, "score_ms": e[0].elapsed_time(e[1]), "budget_null_ms": e[1].elapsed_time(e[2]),
+                        "passes": passes, "ms_per_pass": e[1].elapsed_time(e[2]) / passes,
+                        "all_reduce_ms": r[0].elapsed_time(r[1]) / 5, "nonnull_fraction": frac, "details": det}
+        if owner[k] == rank:
+            owned[c] = scores
+        del scores
+    cache = {c: {"budget_count_hat": v["details"]["effective_count"], "total_count": v["details"]["effective_total_count"]}
+             for c, v in per_chrom.items()}
+    budgets, _ = _resolve_budgets(cache, {"budget": None, "scale_chrom_budgets": 1.0, "budget_posterior_quantile": 0.01})
+    gammas = {c: _resolve_chrom_gamma(c, {"gamma": None}, None, v["details"])[0] for c, v in per_chrom.items()}
+    t_solve = 0.0
+    solved = {}
+    if owned:
+        s0, s1 = ev(), ev()
+        s0.record()
+        res = pipeline.solve_chromosomes(list(owned.values()), [budgets[c] for c in owned], [gammas[c] for c in owned])
+        s1.record()
+        torch.cuda.synchronize()
+        t_solve = s0.elapsed_time(s1)
+        solved = {c: int(r["selected_count"]) for c, r in zip(owned, res)}
+    keys = ("score_ms", "budget_null_ms", "ms_per_pass", "all_reduce_ms")
+    t = torch.tensor([[per_chrom[c][q] for q in keys] + [per_chrom[c]["passes"]] for c in names], dtype=torch.float64, device=dev)
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    gathered = [None] * world
+    if world > 1:
+        dist.all_gather_object(gathered, solved)
+    else:
+        gathered = [solved]
+    if rank == 0:
+        mx = t.tolist()
+        print(json.dumps({
+            "config": f"hg38 @ {args.step_bp} bp x {m_local * world} samples f32, sample-sharded over {world} GPUs, budget null + "
+                      "EB budgets + auto gamma + solve", "gpu": torch.cuda.get_device_name(dev),
+            "chroms": {c: {"bins": per_chrom[c]["bins"], "budget": budgets[c], "gamma": gammas[c],
+                           "nonnull_fraction": per_chrom[c]["nonnull_fraction"],
+                           "ms_max_over_ranks": dict(zip(keys, mx[i][:4])), "passes_max_over_ranks": int(mx[i][4]),
+                           "selected": next((g[c] for g in gathered if c in g), None)} for i, c in enumerate(names)},
+            "solve_ms_rank0": t_solve}))
+
+
+if args.budget_null:
+    budget_null_run()
+    if world > 1:
+        dist.destroy_process_group()
+    sys.exit(0)
 t_score = t_reduce = t_final = t_sweep = 0.0
 gen = 0.0
 selected = {}
