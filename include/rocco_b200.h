@@ -124,6 +124,49 @@ int rocco_b200_chain_solve_batch_dev(
     int levels_per_round,                 /* bisection levels evaluated per launch (1..8); 0 = default */
     void *cuda_stream);
 
+/* Genome-wide budget (opt-in; not a behaviour of the reference, which searches one multiplier per chromosome, dp.py:197-207):
+ * ONE multiplier for a genome spread over this call's chromosomes and those of every other rank that takes part.  The
+ * search is dp.py:89-164 applied to the concatenated chain S = s_1 || s_2 || ... with switch costs c_1 || 0 || c_2 || 0 ...
+ * (a zero cost at each junction decouples the chromosomes, so its mask at any multiplier is the per-chromosome masks laid
+ * end to end): target = floor(N * budget) over N = sum n_c, bracket min(S) - cost_sum - 1 .. max(S) + cost_sum + 1, then
+ * `max_iter` bisection levels on the genome's count; every chromosome is solved at the returned upper end.  All fields
+ * are agreed by the ranks before the call (like the shapes of the sharded budget null).  cost_sum is the correctly rounded
+ * sum of the genome's switch costs, so it does not depend on how chromosomes are ordered or spread over ranks. */
+typedef struct rocco_b200_genome_search {
+    long long total_bins;        /* N over all ranks                                                           */
+    long long target_count;      /* floor(N * budget)                                                          */
+    double cost_sum;             /* correctly rounded sum of every switch cost                                 */
+    double cost_max;             /* largest switch cost of the genome                                          */
+    double score_min, score_max; /* genome extremes; NaN: from this call's chromosomes (valid only without a reducer) */
+    int max_iter;
+    int reserved;
+} rocco_b200_genome_search;
+
+typedef struct rocco_b200_genome_result {
+    double selection_penalty;    /* the genome's multiplier (0.0 when target >= N)                              */
+    long long selected_count;    /* selected bins of the whole genome                                          */
+    int dp_passes;               /* DP passes the reference's search would spend (62 by default)                */
+    int search_rounds;           /* batched launch sets, each followed by one reduce                           */
+    int status;
+    int reserved;
+} rocco_b200_genome_result;
+
+/* `tasks` as for rocco_b200_chain_solve_batch_dev; their mode, target_count and selection_penalty are ignored.  task_count
+ * may be 0 on a rank that holds no chromosome (it still takes part in every reduce).  `allreduce` (rocco_b200_allreduce_fn,
+ * below; NULL when this call holds the whole genome) is called once per search round on 2^L + 1 doubles, L the largest tree
+ * depth (levels_per_round, which every rank passes alike): the counts of the round's multipliers summed over this rank's
+ * chromosomes, its live-tile count and a status slot; every rank then takes the same decision on the same integers.  One
+ * last reduce sums the selected counts of the final masks.  A rank-local failure after the first allocation (the reduce
+ * buffer) is carried to the next reduce, and every rank returns that status.  Argument errors are returned at once:
+ * check them across ranks first.  Exact search (rocco_b200_chain_set_exact_search) is rejected with -2. */
+int rocco_b200_chain_solve_genome_dev(
+    const double *d_scores, const double *d_switch_costs,
+    const rocco_b200_chain_task *tasks, int task_count,
+    const rocco_b200_genome_search *search,
+    int (*allreduce)(double *d_buf, size_t count, void *cuda_stream, void *user), void *user,
+    uint8_t *d_masks_out, rocco_b200_chain_result *results_out, rocco_b200_genome_result *genome_out,
+    int levels_per_round, void *cuda_stream);
+
 /* Chromosomes of at most `max_bins` (<= 4096, the default) bins are solved by replaying the
  * reference's sequential recurrence operation for operation (bit-identical value / count / mask);
  * longer ones use the parallel scan.  Returns the previous setting.  0 forces the scan everywhere. */

@@ -34,6 +34,20 @@ class ChainTask(Structure):
     ]
 
 
+class GenomeSearch(Structure):
+    _fields_ = [
+        ("total_bins", c_longlong), ("target_count", c_longlong), ("cost_sum", c_double), ("cost_max", c_double),
+        ("score_min", c_double), ("score_max", c_double), ("max_iter", c_int), ("reserved", c_int),
+    ]
+
+
+class GenomeResult(Structure):
+    _fields_ = [
+        ("selection_penalty", c_double), ("selected_count", c_longlong), ("dp_passes", c_int), ("search_rounds", c_int),
+        ("status", c_int), ("reserved", c_int),
+    ]
+
+
 class ScoreParams(Structure):
     _fields_ = [
         ("lower_bound_z", c_double), ("prior_df", c_double), ("min_effect", c_double),
@@ -138,6 +152,9 @@ def _declare(lib):
             c_int, [c_void_p, c_void_p, c_size_t, c_longlong, c_int, dp, c_void_p, dp, llp]),
         "rocco_b200_chain_solve_batch_dev": (
             c_int, [c_void_p, c_void_p, POINTER(ChainTask), c_int, c_void_p, POINTER(ChainResult), c_int, c_void_p]),
+        "rocco_b200_chain_solve_genome_dev": (
+            c_int, [c_void_p, c_void_p, POINTER(ChainTask), c_int, POINTER(GenomeSearch), c_void_p, c_void_p, c_void_p,
+                    POINTER(ChainResult), POINTER(GenomeResult), c_int, c_void_p]),
         "rocco_b200_chain_set_seq_max": (c_int, [c_int]),
         "rocco_b200_chain_set_exact_search": (c_int, [c_int]),
         "rocco_b200_chain_set_tile_freezing": (c_int, [c_int]),

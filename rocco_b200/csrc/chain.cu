@@ -21,6 +21,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <cmath>
 
 namespace rb {
 namespace chain {
@@ -172,6 +173,7 @@ struct Params {
     int round_id;
     int levels_base;
     int live_threshold;
+    int group;                  // 1: genome mode, the members' search is driven by the group controller (k_genome_control)
 };
 
 // ------------------------------------------------------------------ the tile kernel
@@ -672,22 +674,26 @@ __global__ void __launch_bounds__(MAX_SLOTS) k_chain_replay(Params P)
 // The reference's bracket (dp.py:110-111) is min(s) - sum(c) - 1 .. max(s) + sum(c) + 1, about 2 sum(c) wide, while
 // counts only vary on [min(s) - 2c, max(s)]: the first ~log2(sum(c) / range(s)) bisection levels land in these two
 // regions and are resolved here, with the margins (1/2, strict) far above any rounding of either implementation.
-// +1: count = n, -1: count = 0, 0: evaluate.
-__device__ __forceinline__ int known_side(const ChromDev &cd, double smin, double smax, double lam, int vec)
+// +1: count = n, -1: count = 0, 0: evaluate.  `cb` bounds every switch cost of the chain (c_max above).
+__device__ __forceinline__ int known_side(double smin, double smax, double cb, double lam)
 {
     if (!(smin == smin)) return 0;
     if (lam > smax) return -1;
-    const double cb = cd.n >= 2 ? (vec ? cd.cost_sum : cd.gamma) : 0.0;
     if (smin - lam > 2.0 * cb + 0.5) return +1;
     return 0;
 }
+// a chromosome's bound: gamma, or (vector costs) their sum
+__device__ __forceinline__ double known_cost_bound(const ChromDev &cd, int vec)
+{
+    return cd.n >= 2 ? (vec ? cd.cost_sum : cd.gamma) : 0.0;
+}
 
 // Walk the bisection (dp.py:141-162) through every level whose midpoint has a known count.
-__device__ void skip_known_levels(const ChromDev &cd, SearchDev &sd, int vec)
+__device__ void skip_known_levels(SearchDev &sd, double cb)
 {
     while (sd.iters_left > 0) {
         const double mid = (sd.lower + sd.upper) / 2.0;
-        const int k = known_side(cd, sd.smin, sd.smax, mid, vec);
+        const int k = known_side(sd.smin, sd.smax, cb, mid);
         if (k == 0) break;
         if (k > 0) sd.lower = mid; else sd.upper = mid;           // count = n > target / count = 0 <= target
         sd.iters_left -= 1;
@@ -708,6 +714,70 @@ __device__ void gen_tree(const SearchDev &sd, double *lam, int levels)
         if (2 * i + 1 <= nodes) {
             lo[2 * i] = lo[i]; hi[2 * i] = mid;
             lo[2 * i + 1] = mid; hi[2 * i + 1] = hi[i];
+        }
+    }
+}
+
+// Bracket lower = min(s) - sum(c) - 1, upper = max(s) + sum(c) + 1 (dp.py:110-111) and the first tree.  Both bracket ends
+// usually have known counts (n > target and 0 <= target): the two bracket solves of dp.py:113-138 and the leading bisection
+// levels then need no DP pass.
+__device__ void search_start(SearchDev &sd, double *lam, double lo, double hi, double cost_sum, int max_iter, double cb, int levels)
+{
+    sd.lower = lo - cost_sum - 1.0;
+    sd.upper = hi + cost_sum + 1.0;
+    sd.phase = PH_BRACKET; sd.iters_left = max_iter; sd.levels = levels; sd.nslots = 2;
+    lam[0] = sd.lower; lam[1] = sd.upper;
+    if (known_side(sd.smin, sd.smax, cb, sd.lower) > 0 && known_side(sd.smin, sd.smax, cb, sd.upper) < 0) {
+        sd.phase = PH_BISECT;
+        sd.passes = 2;
+        skip_known_levels(sd, cb);
+        if (sd.iters_left <= 0) {
+            sd.phase = PH_DONE; sd.nslots = 1; lam[0] = sd.upper;
+        } else {
+            const int lv = min(levels, sd.iters_left);
+            sd.levels = lv; sd.nslots = (1 << lv) - 1;
+            gen_tree(sd, lam, lv);
+        }
+    }
+}
+
+// One controller step after a search round: `cnt` holds the counts at the round's multipliers `lam`.  live >= 0: the tiles
+// that did real work in the round (adaptive depth), -1: fixed depth.
+__device__ void search_advance(SearchDev &sd, const long long *cnt, double *lam, long long target, double cb, int live,
+                               int levels_base, int live_threshold)
+{
+    // reference-equivalent pass count (dp.py: 2 bracket solves + one per bisection level)
+    sd.passes += (sd.phase == PH_BISECT) ? sd.levels : sd.nslots;
+    sd.rounds += 1;
+    if (sd.phase == PH_BRACKET) {
+        // dp.py:113-138: the bracket ends must give count > target (lower) and count <= target (upper)
+        if (cnt[0] <= target || cnt[1] > target) {
+            sd.phase = PH_HOST;                           // expansion loop handled by the host driver
+        } else {
+            sd.phase = PH_BISECT;
+        }
+    } else if (sd.phase == PH_BISECT) {
+        int i = 1;
+        for (int l = 0; l < sd.levels; ++l) {             // dp.py:141-162
+            const double mid = lam[i - 1];
+            if (cnt[i - 1] > target) { sd.lower = mid; i = 2 * i + 1; }
+            else { sd.upper = mid; i = 2 * i; }
+        }
+        sd.iters_left -= sd.levels;
+    }
+    if (sd.phase == PH_BISECT) {
+        skip_known_levels(sd, cb);
+        if (sd.iters_left <= 0) {
+            sd.phase = PH_DONE;
+            sd.nslots = 1;
+            lam[0] = sd.upper;                            // dp.py:164 returns the upper end
+        } else {
+            int pref = sd.levels > 0 ? sd.levels : 1;
+            if (live >= 0) pref = (live >= live_threshold) ? 1 : levels_base;
+            const int lv = min(pref, sd.iters_left);
+            sd.levels = lv;
+            sd.nslots = (1 << lv) - 1;
+            gen_tree(sd, lam, lv);
         }
     }
 }
@@ -788,44 +858,11 @@ __global__ void __launch_bounds__(256) k_chain_finish(Params P, int emit)
         return;
     }
     sd.need_lex = 0;
-    if (!emit) {                                        // the final mask-emitting solve re-evaluates `upper`
-        // reference-equivalent pass count (dp.py: 2 bracket solves + one per bisection level)
-        sd.passes += (sd.phase == PH_BISECT) ? sd.levels : sd.nslots;
-        sd.rounds += 1;
-    }
-    const long long *cnt = P.counts + (size_t)c * MAX_SLOTS;
-    double *lam = P.lam + (size_t)c * MAX_SLOTS;
-    if (sd.phase == PH_BRACKET) {
-        // dp.py:113-138: the bracket ends must give count > target (lower) and count <= target (upper)
-        if (cnt[0] <= cd.target || cnt[1] > cd.target) {
-            sd.phase = PH_HOST;                           // expansion loop handled by the host driver
-        } else {
-            sd.phase = PH_BISECT;
-        }
-    } else if (sd.phase == PH_BISECT) {
-        int i = 1;
-        for (int l = 0; l < sd.levels; ++l) {             // dp.py:141-162
-            const double mid = lam[i - 1];
-            if (cnt[i - 1] > cd.target) { sd.lower = mid; i = 2 * i + 1; }
-            else { sd.upper = mid; i = 2 * i; }
-        }
-        sd.iters_left -= sd.levels;
-    }
-    if (sd.phase == PH_BISECT) {
-        skip_known_levels(cd, sd, P.costs != nullptr);
-        if (sd.iters_left <= 0) {
-            sd.phase = PH_DONE;
-            sd.nslots = 1;
-            lam[0] = sd.upper;                            // dp.py:164 returns the upper end
-        } else {
-            int pref = sd.levels > 0 ? sd.levels : 1;
-            if (P.live_cnt) pref = (P.live_cnt[P.round_id & 1] >= P.live_threshold) ? 1 : P.levels_base;
-            const int lv = min(pref, sd.iters_left);
-            sd.levels = lv;
-            sd.nslots = (1 << lv) - 1;
-            gen_tree(sd, lam, lv);
-        }
-    }
+    // the final mask-emitting solve re-evaluates `upper`; in genome mode the group controller takes the step (k_genome_control)
+    if (!emit && !P.group)
+        search_advance(sd, P.counts + (size_t)c * MAX_SLOTS, P.lam + (size_t)c * MAX_SLOTS, cd.target,
+                       known_cost_bound(cd, P.costs != nullptr), P.live_cnt ? P.live_cnt[P.round_id & 1] : -1,
+                       P.levels_base, P.live_threshold);
     P.search[c] = sd;
 }
 
@@ -884,29 +921,136 @@ __global__ void k_chain_init(const ChromDev *chroms, SearchDev *search, double *
         sd.phase = PH_DONE; sd.lower = sd.upper = l[0];     // host stored the fixed multiplier in slot 0
         sd.iters_left = 0; sd.levels = 0; sd.nslots = 1;
     } else {
-        sd.lower = lo - cd.cost_sum - 1.0;
-        sd.upper = hi + cd.cost_sum + 1.0;
-        sd.phase = PH_BRACKET; sd.iters_left = cd.max_iter; sd.levels = levels; sd.nslots = 2;
-        l[0] = sd.lower; l[1] = sd.upper;
-        // both bracket ends have known counts (n > target and 0 <= target): the two bracket solves of dp.py:113-138 and
-        // the leading bisection levels need no DP pass
-        if (known_side(cd, sd.smin, sd.smax, sd.lower, vec) > 0 && known_side(cd, sd.smin, sd.smax, sd.upper, vec) < 0) {
-            sd.phase = PH_BISECT;
-            sd.passes = 2;
-            skip_known_levels(cd, sd, vec);
-            if (sd.iters_left <= 0) {
-                sd.phase = PH_DONE; sd.nslots = 1; l[0] = sd.upper;
-            } else {
-                const int lv = min(levels, sd.iters_left);
-                sd.levels = lv; sd.nslots = (1 << lv) - 1;
-                gen_tree(sd, l, lv);
-            }
-        }
+        search_start(sd, l, lo, hi, cd.cost_sum, cd.max_iter, known_cost_bound(cd, vec), levels);
     }
     search[c] = sd;
 }
 
 // After the bracket round, PH_BRACKET -> PH_BISECT transitions generate the first tree inside k_chain_finish.
+
+// ------------------------------------------------------------------ genome-wide budget: one controller for a group
+// The chromosomes of a call (and of every rank taking part) form one chain S = s_1 || s_2 || ..., with zero switch cost at
+// the junctions, so at any multiplier the chain's mask is the members' masks laid end to end and count(lambda) is the sum
+// of the members' counts.  The members are solved by the kernels above exactly as in a per-chromosome search; only the
+// controller step changes: k_chain_finish leaves it out (P.group), k_genome_sum adds the members' counts of every slot,
+// the caller's reducer sums those over ranks, and k_genome_control runs search_advance once on the group's state with the
+// genome target and copies the result into every member's SearchDev and multiplier row.
+struct GroupDev {
+    SearchDev sd;
+    long long target;       // floor(N * budget) of the whole genome
+    double cost_sum;        // correctly rounded sum of every switch cost of the genome
+    double cost_max;        // largest switch cost: the bound of known_side
+    int max_iter;
+    int status;             // 0, or the status a reduce reported (then sd.phase = PH_DONE)
+};
+
+// Status slot of a reduce: class k of ST_NOMEM, ST_INVALID, ST_CUDA, ST_NONFINITE (-(k+1)) adds 4096^k, so the summed slot
+// counts the failed ranks of each class (up to 4095 ranks) exactly in a double; every rank decodes the same status.
+constexpr int STATUS_FIELD_BITS = 12;
+__device__ __forceinline__ double status_field(int st)
+{
+    if (st == 0) return 0.0;
+    const int k = (st >= -4 && st < 0) ? -st - 1 : -ST_CUDA - 1;
+    return (double)(1LL << (STATUS_FIELD_BITS * k));
+}
+__host__ __device__ __forceinline__ int status_decode(double v)
+{
+    const long long x = (long long)v;
+    for (int k = 0; k < 4; ++k)
+        if ((x >> (STATUS_FIELD_BITS * k)) & ((1LL << STATUS_FIELD_BITS) - 1)) return -(k + 1);
+    return 0;
+}
+
+// every thread of the block: the group's state and multipliers into each member (their own score extremes stay)
+__device__ void group_broadcast(const Params &P, const SearchDev &g, const double *g_lam)
+{
+    for (int c = threadIdx.x; c < P.nchrom; c += blockDim.x) {
+        SearchDev sd = g;
+        sd.smin = P.search[c].smin; sd.smax = P.search[c].smax;
+        sd.need_lex = 0;
+        P.search[c] = sd;
+    }
+    const int ns = g.nslots;
+    for (int i = threadIdx.x; i < P.nchrom * ns; i += blockDim.x)
+        P.lam[(size_t)(i / ns) * MAX_SLOTS + i % ns] = g_lam[i % ns];
+}
+
+// The group's first state (one block).  member_extremes: min(S) / max(S) from the members' own (single-process calls).
+__global__ void __launch_bounds__(256) k_genome_init(Params P, GroupDev *G, double *g_lam, int levels, int member_extremes)
+{
+    __shared__ SearchDev s_g;
+    if (threadIdx.x == 0) {
+        GroupDev g = *G;
+        if (member_extremes) {
+            double lo = INFINITY, hi = -INFINITY;
+            for (int c = 0; c < P.nchrom; ++c) { lo = fmin(lo, P.search[c].smin); hi = fmax(hi, P.search[c].smax); }
+            g.sd.smin = lo; g.sd.smax = hi;
+        }
+        g.sd.need_lex = 0; g.sd.passes = 0; g.sd.rounds = 0; g.sd.pad = 0;
+        search_start(g.sd, g_lam, g.sd.smin, g.sd.smax, g.cost_sum, g.max_iter, g.cost_max, levels);
+        g.status = 0;
+        *G = g;
+        s_g = g.sd;
+    }
+    __syncthreads();
+    group_broadcast(P, s_g, g_lam);
+}
+
+// Copy the group's state (set by the host) into the members.
+__global__ void __launch_bounds__(256) k_genome_broadcast(Params P, const GroupDev *G, const double *g_lam)
+{
+    group_broadcast(P, G->sd, g_lam);
+}
+
+// red[0 .. nslots): every slot's count summed over the members (exact integers as doubles); red[nslots]: the tiles that did
+// real work this round; red[nslots + 1]: this rank's status.
+__global__ void __launch_bounds__(256) k_genome_sum(Params P, double *red, int nslots, int local_status)
+{
+    for (int s = threadIdx.x; s < nslots; s += blockDim.x) {
+        long long t = 0;
+        for (int c = 0; c < P.nchrom; ++c) t += P.counts[(size_t)c * MAX_SLOTS + s];
+        red[s] = (double)t;
+    }
+    if (threadIdx.x == 0) {
+        red[nslots] = P.live_cnt ? (double)P.live_cnt[P.round_id & 1] : 0.0;
+        red[nslots + 1] = status_field(local_status);
+    }
+}
+
+// The total selected count of the members' final masks and this rank's status, in the layout of k_genome_sum.
+__global__ void k_genome_total(const rocco_b200_chain_result *res, int nchrom, double *red, int nslots, int local_status)
+{
+    if (threadIdx.x != 0) return;
+    long long t = 0;
+    int bad = 0;
+    for (int c = 0; c < nchrom; ++c) { t += res[c].selected_count; bad |= res[c].status != 0; }
+    red[0] = (double)t;
+    red[nslots] = 0.0;
+    red[nslots + 1] = status_field(local_status ? local_status : (bad ? ST_NONFINITE : 0));
+}
+
+// The group's controller step on the reduced buffer, then the new state into every member.
+__global__ void __launch_bounds__(256) k_genome_control(Params P, GroupDev *G, const double *red, int nslots, double *g_lam,
+                                                        long long *g_cnt)
+{
+    __shared__ SearchDev s_g;
+    if (threadIdx.x == 0) {
+        GroupDev g = *G;
+        const int st = status_decode(red[nslots + 1]);
+        if (st != 0) {
+            g.status = st;
+            g.sd.phase = PH_DONE; g.sd.nslots = 1;
+        } else if (g.sd.phase == PH_BRACKET || g.sd.phase == PH_BISECT) {
+            for (int s = 0; s < g.sd.nslots; ++s) g_cnt[s] = (long long)red[s];
+            search_advance(g.sd, g_cnt, g_lam, g.target, g.cost_max, P.live_cnt ? (int)red[nslots] : -1, P.levels_base,
+                           P.live_threshold);
+        }
+        *G = g;
+        s_g = g.sd;
+    }
+    __syncthreads();
+    group_broadcast(P, s_g, g_lam);
+}
 
 // ------------------------------------------------------------------ finalize: patch undecided suffixes, objective sums
 struct FinalPart { double sum_sz; double sum_cost; long long count; long long switches; };
@@ -1078,11 +1222,43 @@ static int launch_round(Params P, bool vec, int nslots_max, int &epoch, bool any
     return 0;
 }
 
+// Genome mode of solve_batch: one multiplier searched for the chromosomes of every rank that calls with the same `search`.
+struct Genome {
+    const rocco_b200_genome_search *search;
+    rocco_b200_allreduce_fn reduce;         // nullptr: this call holds the whole genome
+    void *user;
+    rocco_b200_genome_result *out;
+};
+
 static int solve_batch(const double *d_scores, const double *d_costs, const rocco_b200_chain_task *tasks, int ntask,
-                       uint8_t *d_masks, rocco_b200_chain_result *results, int levels, cudaStream_t st)
+                       uint8_t *d_masks, rocco_b200_chain_result *results, int levels, cudaStream_t st,
+                       const Genome *G = nullptr)
 {
-    if (ntask <= 0) return 0;
-    if (!d_scores || !tasks || !d_masks || !results) return ST_INVALID;
+    if (ntask <= 0 && !G) return 0;
+    if (ntask < 0 || (ntask > 0 && (!d_scores || !tasks || !d_masks || !results))) return ST_INVALID;
+    // genome mode: the arguments every rank agrees on, checked before anything is queued
+    long long g_target = 0;
+    bool g_whole = false, g_own_extremes = false;
+    if (G) {
+        const rocco_b200_genome_search &gs = *G->search;
+        if (g_exact_search.load()) {
+            set_error("genome budget: exact search replays one chromosome's recurrence and has no meaning for a genome; "
+                      "turn it off (rocco_b200_chain_set_exact_search(0))");
+            return ST_INVALID;
+        }
+        if (gs.total_bins <= 0 || !std::isfinite(gs.cost_sum) || gs.cost_sum < 0.0 || !std::isfinite(gs.cost_max) ||
+            gs.cost_max < 0.0 || gs.max_iter < 0 || !G->out)
+            return ST_INVALID;
+        g_own_extremes = std::isnan(gs.score_min) || std::isnan(gs.score_max);
+        if (g_own_extremes ? G->reduce != nullptr
+                           : !(std::isfinite(gs.score_min) && std::isfinite(gs.score_max) && gs.score_min <= gs.score_max))
+            return ST_INVALID;
+        long long local_bins = 0;
+        for (int c = 0; c < ntask; ++c) local_bins += (long long)std::min<size_t>(tasks[c].n, (size_t)1 << 41);
+        if (G->reduce ? local_bins > gs.total_bins : local_bins != gs.total_bins) return ST_INVALID;
+        g_target = std::max<long long>(0, std::min<long long>(gs.target_count, gs.total_bins));
+        g_whole = g_target == gs.total_bins;      // dp.py:102-108: every chromosome at lambda = 0
+    }
     // levels <= 0 (default): two levels per round, dropping to ONE while more than LIVE_THRESHOLD tiles still do real work
     // (throughput-bound rounds: a 2-level tree evaluates 3 multipliers to advance 2 levels).  An explicit value is used as is.
     const bool adaptive = levels <= 0;
@@ -1104,6 +1280,7 @@ static int solve_batch(const double *d_scores, const double *d_costs, const rocc
         long long target = std::max<long long>(0, std::min<long long>(t.target_count, (long long)t.n));
         cd.target = target;
         if (t.mode == 1 && target == (long long)t.n) cd.mode = 2;    // dp.py:102-108: solve at lambda = 0
+        if (G) { cd.mode = g_whole ? 2 : 1; cd.max_iter = G->search->max_iter; }
         cd.seq = ((long long)t.n <= (long long)g_seq_max.load()) ? 1 : 0;
         cd.pad = 0;
         any_seq |= cd.seq != 0;
@@ -1113,89 +1290,246 @@ static int solve_batch(const double *d_scores, const double *d_costs, const rocc
         for (int k = 0; k < cd.ntiles; ++k) tile_chrom.push_back(c);
         if (cd.mode == 1) { any_search = true; max_iter = std::max(max_iter, t.max_iter); }
     }
+    if (G) any_search = !g_whole;     // the group's round layout comes from agreed data, also on a rank without chromosomes
     const bool vec = d_costs != nullptr;
     const int max_slots = any_search ? std::max(2, (1 << levels) - 1) : 1;
     const int slots_per_block = std::min(max_slots, 8);
 
     Arena ar(st);
+    // genome mode: the reduce buffer [max_slots counts][live tiles][status] and the group's state come first; a local failure
+    // after them is carried to the next reduce, which every rank reaches (budget.cu's Shard::local)
+    const int nred = max_slots + 2;
+    double *d_red = nullptr, *d_glam = nullptr;
+    long long *d_gcnt = nullptr;
+    GroupDev *d_group = nullptr;
+    if (G) {
+        RB_TRY(ar.alloc(&d_red, (size_t)nred));
+        RB_TRY(ar.alloc(&d_group, 1));
+        RB_TRY(ar.alloc(&d_glam, MAX_SLOTS));
+        RB_TRY(ar.alloc(&d_gcnt, MAX_SLOTS));
+    }
+    const bool carry = G && G->reduce;
+    int failed = 0;
+    auto local = [&](int s) -> int {
+        if (s == 0 || !carry) return s;
+        if (!failed) failed = s;
+        return 0;
+    };
+
     Workspace w;
-    RB_TRY(ar.alloc(&w.d_chroms, ntask));
-    RB_TRY(ar.alloc(&w.d_search, ntask));
-    RB_TRY(ar.alloc(&w.d_tile_chrom, ntiles));
-    RB_TRY(ar.alloc(&w.d_lam, (size_t)ntask * MAX_SLOTS));
-    RB_TRY(ar.alloc(&w.d_counts, (size_t)ntask * MAX_SLOTS));
-    RB_TRY(ar.alloc(&w.d_tiecnt, (size_t)ntask * MAX_SLOTS));
-    RB_TRY(ar.alloc(&w.d_near, ntask));
-    RB_TRY(ar.alloc(&w.d_flags, (size_t)max_slots * ntiles));
-    char *agg_bytes = nullptr, *incl_bytes = nullptr;
-    RB_TRY(ar.alloc(&agg_bytes, (size_t)max_slots * ntiles * sizeof(Map<VL>)));
-    RB_TRY(ar.alloc(&incl_bytes, (size_t)max_slots * ntiles * sizeof(VL)));
-    w.d_agg = agg_bytes; w.d_incl = incl_bytes;
-    RB_TRY(ar.alloc(&w.d_tout, (size_t)max_slots * ntiles));
-    RB_TRY(ar.alloc(&w.d_ticket, 1));
-    RB_TRY(ar.alloc(&w.d_zin, ntiles));
-    const int nparts = 64;
-    RB_TRY(ar.alloc(&w.d_partial, (size_t)ntask * nparts * 2));
-    RB_TRY(ar.alloc(&w.d_parts, ntiles));
-    RB_TRY(ar.alloc(&w.d_results, ntask));
-    uint8_t *d_bt = nullptr;
-    double *d_seqv = nullptr;
-    const bool exact = g_exact_search.load() != 0;
-    RB_TRY(ar.alloc(&d_bt, (any_seq || exact) ? (size_t)ntiles * TILE : 16));
-    RB_TRY(ar.alloc(&d_seqv, ntask));
-
-    // modes: 0 fixed (lambda given), 2 fixed at 0.0; both are PH_DONE from the start
-    std::vector<double> lam0((size_t)ntask * MAX_SLOTS, 0.0);
-    for (int c = 0; c < ntask; ++c) {
-        if (chroms[c].mode == 0) lam0[(size_t)c * MAX_SLOTS] = tasks[c].selection_penalty;
-        if (chroms[c].mode == 2) { chroms[c].mode = 0; lam0[(size_t)c * MAX_SLOTS] = 0.0; }
-    }
-    RB_CUDA(cudaMemcpyAsync(w.d_chroms, chroms.data(), sizeof(ChromDev) * ntask, cudaMemcpyHostToDevice, st));
-    RB_CUDA(cudaMemcpyAsync(w.d_tile_chrom, tile_chrom.data(), sizeof(int) * ntiles, cudaMemcpyHostToDevice, st));
-    RB_CUDA(cudaMemcpyAsync(w.d_lam, lam0.data(), sizeof(double) * lam0.size(), cudaMemcpyHostToDevice, st));
-    RB_CUDA(cudaMemsetAsync(w.d_flags, 0, sizeof(int) * (size_t)max_slots * ntiles, st));
-    RB_CUDA(cudaMemsetAsync(w.d_ticket, 0, sizeof(int), st));
-    RB_CUDA(cudaMemsetAsync(w.d_near, 0, sizeof(long long) * ntask, st));
-    RB_CUDA(cudaMemsetAsync(w.d_tiecnt, 0, sizeof(long long) * (size_t)ntask * MAX_SLOTS, st));
-
-    k_chain_minmax<<<dim3(ntask, nparts), 256, 0, st>>>(d_scores, w.d_chroms, w.d_search, w.d_partial);
-    RB_LAUNCH_CHECK();
-    const int init_levels = (adaptive && ntiles >= LIVE_THRESHOLD) ? 1 : levels;
-    k_chain_init<<<(ntask + 63) / 64, 64, 0, st>>>(w.d_chroms, w.d_search, w.d_lam, w.d_partial, nparts, init_levels, ntask, vec ? 1 : 0);
-    RB_LAUNCH_CHECK();
-
     Params P{};
-    P.scores = d_scores; P.costs = d_costs; P.chroms = w.d_chroms; P.search = w.d_search;
-    P.tile_chrom = w.d_tile_chrom; P.lam = w.d_lam; P.counts = w.d_counts; P.tiecnt = w.d_tiecnt;
-    P.flags = w.d_flags; P.agg = w.d_agg; P.incl = w.d_incl; P.tout = w.d_tout; P.ticket = w.d_ticket;
-    P.mask = d_masks; P.zin = w.d_zin; P.near_ties = w.d_near; P.ntiles = ntiles; P.nchrom = ntask;
-    P.slots_per_block = slots_per_block;
-    P.bt = d_bt; P.seq_value = d_seqv;
-    P.exact_mode = exact ? 1 : 0;
-    int epoch = 0;
-    // tile freezing: two state buffers (read = previous round, write = this round), the frozen outputs and hand-on values
-    int *d_fz[2] = {nullptr, nullptr};
+    const bool exact = g_exact_search.load() != 0;
     const bool freeze = any_search && !exact && g_freeze.load() != 0;
-    if (freeze) {
-        RB_TRY(ar.alloc(&d_fz[0], (size_t)ntiles));
-        RB_TRY(ar.alloc(&d_fz[1], (size_t)ntiles));
-        RB_TRY(ar.alloc(&P.fz_out, (size_t)ntiles));
-        RB_TRY(ar.alloc(&P.fz_incl, (size_t)ntiles));
-        RB_CUDA(cudaMemsetAsync(d_fz[0], 0, sizeof(int) * (size_t)ntiles, st));
-        RB_CUDA(cudaMemsetAsync(d_fz[1], 0, sizeof(int) * (size_t)ntiles, st));
-    }
-    if (adaptive && any_search) {
-        RB_TRY(ar.alloc(&P.live_cnt, (size_t)2));
-        RB_CUDA(cudaMemsetAsync(P.live_cnt, 0, sizeof(int) * 2, st));
-        P.levels_base = levels;
-        P.live_threshold = LIVE_THRESHOLD;
-    }
+    int *d_fz[2] = {nullptr, nullptr};
+    auto setup = [&]() -> int {
+        RB_TRY(ar.alloc(&w.d_chroms, ntask));
+        RB_TRY(ar.alloc(&w.d_search, ntask));
+        RB_TRY(ar.alloc(&w.d_tile_chrom, ntiles));
+        RB_TRY(ar.alloc(&w.d_lam, (size_t)ntask * MAX_SLOTS));
+        RB_TRY(ar.alloc(&w.d_counts, (size_t)ntask * MAX_SLOTS));
+        RB_TRY(ar.alloc(&w.d_tiecnt, (size_t)ntask * MAX_SLOTS));
+        RB_TRY(ar.alloc(&w.d_near, ntask));
+        RB_TRY(ar.alloc(&w.d_flags, (size_t)max_slots * ntiles));
+        char *agg_bytes = nullptr, *incl_bytes = nullptr;
+        RB_TRY(ar.alloc(&agg_bytes, (size_t)max_slots * ntiles * sizeof(Map<VL>)));
+        RB_TRY(ar.alloc(&incl_bytes, (size_t)max_slots * ntiles * sizeof(VL)));
+        w.d_agg = agg_bytes; w.d_incl = incl_bytes;
+        RB_TRY(ar.alloc(&w.d_tout, (size_t)max_slots * ntiles));
+        RB_TRY(ar.alloc(&w.d_ticket, 1));
+        RB_TRY(ar.alloc(&w.d_zin, ntiles));
+        const int nparts = 64;
+        RB_TRY(ar.alloc(&w.d_partial, (size_t)ntask * nparts * 2));
+        RB_TRY(ar.alloc(&w.d_parts, ntiles));
+        RB_TRY(ar.alloc(&w.d_results, ntask));
+        uint8_t *d_bt = nullptr;
+        double *d_seqv = nullptr;
+        RB_TRY(ar.alloc(&d_bt, (any_seq || exact) ? (size_t)ntiles * TILE : 16));
+        RB_TRY(ar.alloc(&d_seqv, ntask));
+
+        // modes: 0 fixed (lambda given), 2 fixed at 0.0; both are PH_DONE from the start
+        std::vector<double> lam0((size_t)ntask * MAX_SLOTS, 0.0);
+        for (int c = 0; c < ntask; ++c) {
+            if (chroms[c].mode == 0) lam0[(size_t)c * MAX_SLOTS] = tasks[c].selection_penalty;
+            if (chroms[c].mode == 2) { chroms[c].mode = 0; lam0[(size_t)c * MAX_SLOTS] = 0.0; }
+        }
+        if (ntask > 0) {
+            RB_CUDA(cudaMemcpyAsync(w.d_chroms, chroms.data(), sizeof(ChromDev) * ntask, cudaMemcpyHostToDevice, st));
+            RB_CUDA(cudaMemcpyAsync(w.d_tile_chrom, tile_chrom.data(), sizeof(int) * ntiles, cudaMemcpyHostToDevice, st));
+            RB_CUDA(cudaMemcpyAsync(w.d_lam, lam0.data(), sizeof(double) * lam0.size(), cudaMemcpyHostToDevice, st));
+            RB_CUDA(cudaMemsetAsync(w.d_flags, 0, sizeof(int) * (size_t)max_slots * ntiles, st));
+            RB_CUDA(cudaMemsetAsync(w.d_ticket, 0, sizeof(int), st));
+            RB_CUDA(cudaMemsetAsync(w.d_near, 0, sizeof(long long) * ntask, st));
+            RB_CUDA(cudaMemsetAsync(w.d_tiecnt, 0, sizeof(long long) * (size_t)ntask * MAX_SLOTS, st));
+            // the group sums every slot of every member: no slot may hold garbage
+            if (G) RB_CUDA(cudaMemsetAsync(w.d_counts, 0, sizeof(long long) * (size_t)ntask * MAX_SLOTS, st));
+
+            k_chain_minmax<<<dim3(ntask, nparts), 256, 0, st>>>(d_scores, w.d_chroms, w.d_search, w.d_partial);
+            RB_LAUNCH_CHECK();
+            const int init_levels = (adaptive && ntiles >= LIVE_THRESHOLD) ? 1 : levels;
+            k_chain_init<<<(ntask + 63) / 64, 64, 0, st>>>(w.d_chroms, w.d_search, w.d_lam, w.d_partial, nparts, init_levels, ntask, vec ? 1 : 0);
+            RB_LAUNCH_CHECK();
+        }
+
+        P.scores = d_scores; P.costs = d_costs; P.chroms = w.d_chroms; P.search = w.d_search;
+        P.tile_chrom = w.d_tile_chrom; P.lam = w.d_lam; P.counts = w.d_counts; P.tiecnt = w.d_tiecnt;
+        P.flags = w.d_flags; P.agg = w.d_agg; P.incl = w.d_incl; P.tout = w.d_tout; P.ticket = w.d_ticket;
+        P.mask = d_masks; P.zin = w.d_zin; P.near_ties = w.d_near; P.ntiles = ntiles; P.nchrom = ntask;
+        P.slots_per_block = slots_per_block;
+        P.bt = d_bt; P.seq_value = d_seqv;
+        P.exact_mode = exact ? 1 : 0;
+        P.group = G ? 1 : 0;
+        // tile freezing: two state buffers (read = previous round, write = this round), the frozen outputs and hand-on values
+        if (freeze) {
+            RB_TRY(ar.alloc(&d_fz[0], (size_t)ntiles));
+            RB_TRY(ar.alloc(&d_fz[1], (size_t)ntiles));
+            RB_TRY(ar.alloc(&P.fz_out, (size_t)ntiles));
+            RB_TRY(ar.alloc(&P.fz_incl, (size_t)ntiles));
+            RB_CUDA(cudaMemsetAsync(d_fz[0], 0, sizeof(int) * (size_t)ntiles, st));
+            RB_CUDA(cudaMemsetAsync(d_fz[1], 0, sizeof(int) * (size_t)ntiles, st));
+        }
+        if (adaptive && any_search) {
+            RB_TRY(ar.alloc(&P.live_cnt, (size_t)2));
+            RB_CUDA(cudaMemsetAsync(P.live_cnt, 0, sizeof(int) * 2, st));
+            P.levels_base = levels;
+            P.live_threshold = LIVE_THRESHOLD;
+        }
+        return 0;
+    };
+    RB_TRY(local(setup()));
+    int epoch = 0;
     int fz_round = 0, round_id = 0;
     auto search_round = [&](int nslots) -> int {
         P.round_id = round_id++;
         if (freeze) { P.fz_read = d_fz[fz_round & 1]; P.fz_write = d_fz[(fz_round & 1) ^ 1]; ++fz_round; }
         return launch_round<false>(P, vec, nslots, epoch, any_seq, st);
     };
+    // the final solve at the chosen multipliers, mask emitted
+    auto final_solve = [&]() -> int {
+        P.fz_read = nullptr; P.fz_write = nullptr;
+        RB_TRY((launch_round<true>(P, vec, 1, epoch, any_seq, st)));
+        {
+            RB_PROF("k_chain_finalize", st, (double)ntiles * TILE * 9.0);
+            if (vec) k_chain_finalize<true><<<ntiles, THREADS, 0, st>>>(P, w.d_parts);
+            else k_chain_finalize<false><<<ntiles, THREADS, 0, st>>>(P, w.d_parts);
+            RB_LAUNCH_CHECK();
+        }
+        k_chain_results<<<ntask, 32, 0, st>>>(P, w.d_parts, w.d_results, vec ? 1 : 0);
+        RB_LAUNCH_CHECK();
+        return 0;
+    };
+    if (G) {
+        // ---- genome mode: the members' rounds as above, the controller step on the group after one reduce per round
+        const rocco_b200_genome_search &gs = *G->search;
+        auto reduce = [&]() -> int {
+            if (!G->reduce) return 0;
+            if (G->reduce(d_red, (size_t)nred, (void *)st, G->user) != 0) {
+                set_error("genome budget: the all-reduce callback failed");
+                return ST_CUDA;
+            }
+            return 0;
+        };
+        auto another = [&](int s) -> int {                // every rank returns the status a reduce reported
+            if (!failed) set_error("genome budget: another rank failed with status %d", s);
+            return s;
+        };
+        auto group_params = [&]() { Params q = P; if (failed) q.nchrom = 0; return q; };   // a failed rank's members are left alone
+        GroupDev hg{};
+        auto read_group = [&]() -> int {
+            RB_CUDA(cudaMemcpyAsync(&hg, d_group, sizeof(GroupDev), cudaMemcpyDeviceToHost, st));
+            RB_CUDA(cudaStreamSynchronize(st));
+            return 0;
+        };
+        if (!g_whole) {
+            GroupDev g0{};
+            g0.sd.smin = gs.score_min; g0.sd.smax = gs.score_max;
+            g0.target = g_target; g0.cost_sum = gs.cost_sum; g0.cost_max = gs.cost_max; g0.max_iter = gs.max_iter;
+            // agreed data only: every rank starts from the same state
+            const int init_levels = (adaptive && (gs.total_bins + TILE - 1) / TILE >= LIVE_THRESHOLD) ? 1 : levels;
+            RB_CUDA(cudaMemcpyAsync(d_group, &g0, sizeof(GroupDev), cudaMemcpyHostToDevice, st));
+            k_genome_init<<<1, 256, 0, st>>>(group_params(), d_group, d_glam, init_levels, g_own_extremes ? 1 : 0);
+            RB_LAUNCH_CHECK();
+            RB_TRY(read_group());
+            // rounds in batches, as the per-chromosome search; the batch size depends on the group's state only, so every
+            // rank calls the reducer the same number of times
+            while (hg.sd.phase == PH_BRACKET || hg.sd.phase == PH_BISECT) {
+                const int bound = hg.sd.iters_left + (hg.sd.phase == PH_BRACKET ? 1 : 0);
+                const int batch = std::max(1, std::min(bound, 12));
+                for (int r = 0; r < batch; ++r) {
+                    if (!failed && ntask > 0) RB_TRY(local(search_round(max_slots)));
+                    k_genome_sum<<<1, 256, 0, st>>>(group_params(), d_red, max_slots, failed);
+                    RB_LAUNCH_CHECK();
+                    RB_TRY(reduce());
+                    k_genome_control<<<1, 256, 0, st>>>(group_params(), d_group, d_red, max_slots, d_glam, d_gcnt);
+                    RB_LAUNCH_CHECK();
+                }
+                RB_TRY(read_group());
+            }
+            if (hg.status) return another(hg.status);
+            // rare: bracket expansion (dp.py:119-125, 132-138) from the host, each evaluation reduced
+            if (hg.sd.phase == PH_HOST) {
+                auto eval = [&](double lamv, long long &count) -> int {
+                    GroupDev h = hg;
+                    h.sd.phase = PH_MANUAL; h.sd.nslots = 1;
+                    RB_CUDA(cudaMemcpyAsync(d_group, &h, sizeof(GroupDev), cudaMemcpyHostToDevice, st));
+                    RB_CUDA(cudaMemcpyAsync(d_glam, &lamv, sizeof(double), cudaMemcpyHostToDevice, st));
+                    k_genome_broadcast<<<1, 256, 0, st>>>(group_params(), d_group, d_glam);
+                    RB_LAUNCH_CHECK();
+                    if (!failed && ntask > 0) RB_TRY(local(launch_round<false>(P, vec, 1, epoch, any_seq, st)));
+                    k_genome_sum<<<1, 256, 0, st>>>(group_params(), d_red, 1, failed);
+                    RB_LAUNCH_CHECK();
+                    RB_TRY(reduce());
+                    double r[3];
+                    RB_CUDA(cudaMemcpyAsync(r, d_red, sizeof(r), cudaMemcpyDeviceToHost, st));
+                    RB_CUDA(cudaStreamSynchronize(st));
+                    const int s = status_decode(r[2]);
+                    if (s) return another(s);
+                    count = (long long)r[0];
+                    return 0;
+                };
+                double lower = hg.sd.lower, upper = hg.sd.upper;
+                long long cl = 0, cu = 0;
+                int passes = 0;
+                RB_TRY(eval(lower, cl)); ++passes;
+                while (cl <= g_target) { lower -= std::max(1.0, fabs(lower)); RB_TRY(eval(lower, cl)); ++passes; if (passes > 4096) return ST_INVALID; }
+                RB_TRY(eval(upper, cu)); ++passes;
+                while (cu > g_target) { upper += std::max(1.0, fabs(upper)); RB_TRY(eval(upper, cu)); ++passes; if (passes > 4096) return ST_INVALID; }
+                for (int it = 0; it < gs.max_iter; ++it) {
+                    const double mid = (lower + upper) / 2.0;
+                    long long cm = 0;
+                    RB_TRY(eval(mid, cm)); ++passes;
+                    if (cm > g_target) lower = mid; else upper = mid;
+                }
+                hg.sd.lower = lower; hg.sd.upper = upper; hg.sd.passes = passes; hg.sd.rounds = passes;
+                hg.sd.phase = PH_DONE; hg.sd.nslots = 1;
+                RB_CUDA(cudaMemcpyAsync(d_group, &hg, sizeof(GroupDev), cudaMemcpyHostToDevice, st));
+                RB_CUDA(cudaMemcpyAsync(d_glam, &hg.sd.upper, sizeof(double), cudaMemcpyHostToDevice, st));
+                k_genome_broadcast<<<1, 256, 0, st>>>(group_params(), d_group, d_glam);
+                RB_LAUNCH_CHECK();
+            }
+        }
+        // every member at the group's multiplier, then one last reduce: the genome's selected count and every rank's status
+        if (!failed && ntask > 0) RB_TRY(local(final_solve()));
+        k_genome_total<<<1, 32, 0, st>>>(failed ? nullptr : w.d_results, failed ? 0 : ntask, d_red, max_slots, failed);
+        RB_LAUNCH_CHECK();
+        RB_TRY(reduce());
+        double r[2];
+        RB_CUDA(cudaMemcpyAsync(&r[0], d_red, sizeof(double), cudaMemcpyDeviceToHost, st));
+        RB_CUDA(cudaMemcpyAsync(&r[1], d_red + max_slots + 1, sizeof(double), cudaMemcpyDeviceToHost, st));
+        if (!failed && ntask > 0)
+            RB_CUDA(cudaMemcpyAsync(results, w.d_results, sizeof(rocco_b200_chain_result) * ntask, cudaMemcpyDeviceToHost, st));
+        RB_CUDA(cudaStreamSynchronize(st));
+        const int s = status_decode(r[1]);
+        if (s) return another(s);
+        rocco_b200_genome_result &o = *G->out;
+        o.selection_penalty = g_whole ? 0.0 : hg.sd.upper;
+        o.selected_count = (long long)r[0];
+        o.dp_passes = g_whole ? 1 : hg.sd.passes;
+        o.search_rounds = g_whole ? 0 : hg.sd.rounds;
+        o.status = 0;
+        o.reserved = 0;
+        return 0;
+    }
+
 
     std::vector<SearchDev> hsearch(ntask);
     if (any_search) {
@@ -1287,17 +1621,7 @@ static int solve_batch(const double *d_scores, const double *d_costs, const rocc
         }
     }
 
-    // final solve at the chosen multiplier, mask emitted
-    P.fz_read = nullptr; P.fz_write = nullptr;
-    RB_TRY((launch_round<true>(P, vec, 1, epoch, any_seq, st)));
-    {
-        RB_PROF("k_chain_finalize", st, (double)ntiles * TILE * 9.0);
-        if (vec) k_chain_finalize<true><<<ntiles, THREADS, 0, st>>>(P, w.d_parts);
-        else k_chain_finalize<false><<<ntiles, THREADS, 0, st>>>(P, w.d_parts);
-        RB_LAUNCH_CHECK();
-    }
-    k_chain_results<<<ntask, 32, 0, st>>>(P, w.d_parts, w.d_results, vec ? 1 : 0);
-    RB_LAUNCH_CHECK();
+    RB_TRY(final_solve());
     RB_CUDA(cudaMemcpyAsync(results, w.d_results, sizeof(rocco_b200_chain_result) * ntask, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
     for (int c = 0; c < ntask; ++c)
@@ -1387,6 +1711,17 @@ extern "C" __attribute__((visibility("default"))) int rocco_b200_chain_solve_bat
 {
     return chain::solve_batch(d_scores, d_switch_costs, tasks, task_count, d_masks_out, results_out,
                               levels_per_round, (cudaStream_t)cuda_stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int rocco_b200_chain_solve_genome_dev(
+    const double *d_scores, const double *d_switch_costs, const rocco_b200_chain_task *tasks, int task_count,
+    const rocco_b200_genome_search *search, rocco_b200_allreduce_fn allreduce, void *user, uint8_t *d_masks_out,
+    rocco_b200_chain_result *results_out, rocco_b200_genome_result *genome_out, int levels_per_round, void *cuda_stream)
+{
+    if (!search || !genome_out) return ST_INVALID;
+    const chain::Genome g{search, allreduce, user, genome_out};
+    return chain::solve_batch(d_scores, d_switch_costs, tasks, task_count, d_masks_out, results_out, levels_per_round,
+                              (cudaStream_t)cuda_stream, &g);
 }
 
 extern "C" __attribute__((visibility("default"))) int rocco_b200_chain_sweep_dev(

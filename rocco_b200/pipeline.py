@@ -101,21 +101,21 @@ def solve_packed(d_scores, offsets, lengths, budgets, gammas, selection_penaltie
             ctypes.c_void_p(d_masks.data_ptr()), results, int(levels_per_round),
             ctypes.c_void_p(_stream_ptr(d_scores.device)))
     _lib.check(st, "solve_chrom_exact")
-    out = []
-    for c in range(nchrom):
-        r = results[c]
-        out.append({
-            "selection_penalty": float(r.selection_penalty),
-            "penalized_objective": float(r.penalized_objective),
-            "objective": float(r.objective),
-            "selected_count": int(r.selected_count),
-            "switch_count": int(r.switch_count),
-            "exact_tie_bins": int(r.exact_tie_bins),
-            "near_tie_bins": int(r.near_tie_bins),
-            "dp_passes": int(r.dp_passes),
-            "search_rounds": int(r.search_rounds),
-        })
-    return d_masks, out
+    return d_masks, [_chain_result_dict(results[c]) for c in range(nchrom)]
+
+
+def _chain_result_dict(r) -> dict:
+    return {
+        "selection_penalty": float(r.selection_penalty),
+        "penalized_objective": float(r.penalized_objective),
+        "objective": float(r.objective),
+        "selected_count": int(r.selected_count),
+        "switch_count": int(r.switch_count),
+        "exact_tie_bins": int(r.exact_tie_bins),
+        "near_tie_bins": int(r.near_tie_bins),
+        "dp_passes": int(r.dp_passes),
+        "search_rounds": int(r.search_rounds),
+    }
 
 
 def solve_chromosomes(scores_list, budgets, gammas, selection_penalties=None, max_iter: int = 60,
@@ -161,6 +161,214 @@ def solve_chromosomes(scores_list, budgets, gammas, selection_penalties=None, ma
     for r, off, n in zip(res, offsets, lengths):
         r["solution"] = h_masks[off:off + n].copy()
     return res
+
+
+# ------------------------------------------------------------------ genome-wide budget: one multiplier for every chromosome
+# Opt-in, and not a behaviour of the reference (which searches one multiplier per chromosome, dp.py:197-207): the search of
+# dp.py:89-164 on the concatenated chain S = s_1 || s_2 || ... with zero switch cost at the junctions (include/rocco_b200.h).
+def genome_cost_sum(lengths, gammas) -> float:
+    """Correctly rounded sum of gamma_c * (n_c - 1): the switch costs of the concatenated chain.  Summed exactly (rationals),
+    so the bracket does not depend on the order of the chromosomes or on how they are spread over ranks."""
+    from fractions import Fraction
+    return float(sum((Fraction(float(g)) * max(int(n) - 1, 0) for n, g in zip(lengths, gammas)), Fraction(0)))
+
+
+def _genome_cost_max(lengths, gammas) -> float:
+    return max([float(g) for n, g in zip(lengths, gammas) if int(n) >= 2], default=0.0)
+
+
+def _exact_search_on() -> bool:
+    lib = _lib.load()
+    prev = lib.rocco_b200_chain_set_exact_search(0)
+    lib.rocco_b200_chain_set_exact_search(prev)
+    return bool(prev)
+
+
+def _genome_problem(d_scores, offsets, lengths, gammas, genome_budget):
+    """This rank's own argument errors, or None."""
+    torch = _torch()
+    if not isinstance(d_scores, torch.Tensor) or not d_scores.is_cuda or d_scores.dtype != torch.float64 or d_scores.dim() != 1:
+        return "`d_scores` must be a one-dimensional float64 CUDA tensor"
+    if len(offsets) != len(lengths) or len(gammas) != len(lengths):
+        return "`offsets`, `lengths` and `gammas` must have one entry per chromosome"
+    if any(int(n) <= 0 for n in lengths):
+        return "`scores` cannot be empty"
+    if any(not (float(g) >= 0.0) or not np.isfinite(float(g)) for g in gammas):
+        return "switch costs (`gammas`) must be finite and >= 0"
+    if any(int(o) < 0 or int(o) + int(n) > d_scores.shape[0] for o, n in zip(offsets, lengths)):
+        return "a chromosome lies outside `d_scores`"
+    if not np.isfinite(float(genome_budget)):
+        return "`genome_budget` must be finite"
+    if _exact_search_on():
+        return "exact search replays one chromosome's recurrence and has no meaning for a genome-wide budget; turn it off"
+    return None
+
+
+def _score_extremes(d_scores, offsets, lengths):
+    """(min, max) over this rank's chromosomes, None without chromosomes; raises on a non-finite score."""
+    torch = _torch()
+    if not lengths:
+        return None
+    parts = [d_scores[int(o):int(o) + int(n)] for o, n in zip(offsets, lengths)]
+    ext = torch.stack([torch.stack([p.min(), p.max(), torch.isfinite(p).all().to(torch.float64)]) for p in parts]).cpu()
+    if not bool((ext[:, 2] > 0).all()):
+        return "non-finite"
+    return float(ext[:, 0].min()), float(ext[:, 1].max())
+
+
+def _solve_genome(d_scores, d_costs, offsets, lengths, gammas, search, levels_per_round, d_masks, reduce_fn):
+    """One rank's call of rocco_b200_chain_solve_genome_dev with the search fields already agreed.  ``reduce_fn(buf)`` sums
+    the float64 CUDA tensor ``buf`` over the ranks in place on torch's current stream (None: this call holds the genome)."""
+    torch = _torch()
+    lib = _lib.load()
+    dev = d_scores.device
+    nchrom = len(lengths)
+    tasks = (_lib.ChainTask * max(nchrom, 1))()
+    for c in range(nchrom):
+        t = tasks[c]
+        t.offset, t.n, t.gamma, t.max_iter = int(offsets[c]), int(lengths[c]), float(gammas[c]), int(search.max_iter)
+    if d_masks is None:
+        d_masks = torch.zeros(d_scores.shape[0], dtype=torch.uint8, device=dev)
+    failure = []
+
+    def _reduce(ptr, count, _stream, _user):
+        try:
+            reduce_fn(torch.as_tensor(_DeviceBuffer(ptr, count), device=dev))
+            return 0
+        except BaseException as exc:          # never let it unwind through the C frames
+            failure.append(exc)
+            return 1
+
+    cb = None if reduce_fn is None else _lib.ALLREDUCE_FN(_reduce)
+    results = (_lib.ChainResult * max(nchrom, 1))()
+    genome = _lib.GenomeResult()
+    with torch.cuda.device(dev):
+        st = lib.rocco_b200_chain_solve_genome_dev(
+            ctypes.c_void_p(d_scores.data_ptr()), None if d_costs is None else ctypes.c_void_p(d_costs.data_ptr()),
+            tasks, nchrom, ctypes.byref(search), cb, None, ctypes.c_void_p(d_masks.data_ptr()), results,
+            ctypes.byref(genome), int(levels_per_round), ctypes.c_void_p(_stream_ptr(dev)))
+    if failure:
+        raise RuntimeError(f"genome budget: the all-reduce failed: {failure[0]!r}") from failure[0]
+    if st == _lib.ST_INVALID and _lib.last_error().startswith("genome budget"):
+        raise ValueError(_lib.last_error())
+    _lib.check(st, "genome budget")
+    out = {"selection_penalty": float(genome.selection_penalty), "selected_count": int(genome.selected_count),
+           "total_bins": int(search.total_bins), "target_count": int(search.target_count),
+           "dp_passes": int(genome.dp_passes), "search_rounds": int(genome.search_rounds)}
+    return d_masks, out, [_chain_result_dict(results[c]) for c in range(nchrom)]
+
+
+def _group_size(group) -> int:
+    import torch.distributed as dist
+    return dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
+
+
+def solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_iter: int = 60, levels_per_round: int = 0,
+                        d_masks=None, group=None):
+    """One multiplier for the whole genome: the chromosomes packed in ``d_scores`` (as ``solve_packed``) and, when ``group``
+    has more than one rank, those of every other rank of it (a rank may hold none).  target = floor(N * genome_budget) over
+    all N bins; each search round's counts are summed over the ranks with one ``torch.distributed.all_reduce`` of at most
+    2^L + 1 doubles.  Returns ``(d_masks, genome, results)``: ``genome`` holds the multiplier, the genome's selected count,
+    N, the target, the DP passes and the rounds; ``results`` the per-chromosome dicts of ``solve_packed``."""
+    torch = _torch()
+    _lib.require_device()
+    problem = _genome_problem(d_scores, offsets, lengths, gammas, genome_budget)
+    nan = float("nan")
+    if _group_size(group) <= 1:
+        if problem:
+            raise ValueError(problem)
+        total = sum(int(n) for n in lengths)
+        if total == 0:
+            raise ValueError("the genome has no chromosome")
+        search = _lib.GenomeSearch(total, target_count_for_budget(total, genome_budget), genome_cost_sum(lengths, gammas),
+                                   _genome_cost_max(lengths, gammas), nan, nan, int(max_iter), 0)
+        return _solve_genome(d_scores, None, offsets, lengths, gammas, search, levels_per_round, d_masks, None)
+
+    import torch.distributed as dist
+    dev = d_scores.device if isinstance(d_scores, torch.Tensor) and d_scores.is_cuda else torch.device("cuda", torch.cuda.current_device())
+    # the reduce workspace (2^8 - 1 counts + 2 slots at most) is allocated before the ranks compare notes, so that its
+    # failure is one more problem reported to all of them
+    workspace = None
+    extremes = None
+    if problem is None:
+        try:
+            workspace = torch.empty(257, dtype=torch.float64, device=dev)
+            extremes = _score_extremes(d_scores, offsets, lengths)
+        except RuntimeError as exc:
+            problem = f"genome budget: {exc}"
+        if extremes == "non-finite":
+            problem = "genome budget: non-finite values in `d_scores`"
+    mine = {"problem": problem is not None, "n": [int(n) for n in lengths] if problem is None else [],
+            "gamma": [float(g) for g in gammas] if problem is None else [], "extremes": extremes,
+            "agreed": (float(genome_budget), int(max_iter), int(levels_per_round))}
+    every = [None] * dist.get_world_size(group)
+    dist.all_gather_object(every, mine, group=group)
+    if problem is not None:
+        raise ValueError(problem)
+    if any(r["problem"] for r in every):
+        raise ValueError("genome budget: another rank rejected its arguments")
+    if any(r["agreed"] != mine["agreed"] for r in every):
+        raise ValueError("genome budget: every rank must pass the same genome_budget, max_iter and levels_per_round")
+    all_n = [n for r in every for n in r["n"]]
+    all_g = [g for r in every for g in r["gamma"]]
+    total = sum(all_n)
+    if total == 0:
+        raise ValueError("the genome has no chromosome")
+    ext = [r["extremes"] for r in every if r["extremes"] is not None]
+    search = _lib.GenomeSearch(total, target_count_for_budget(total, genome_budget), genome_cost_sum(all_n, all_g),
+                               _genome_cost_max(all_n, all_g), min(e[0] for e in ext), max(e[1] for e in ext),
+                               int(max_iter), 0)
+
+    def reduce_fn(buf):
+        w = workspace[: buf.numel()]
+        w.copy_(buf)
+        dist.all_reduce(w, group=group)
+        buf.copy_(w)
+
+    return _solve_genome(d_scores, None, offsets, lengths, gammas, search, levels_per_round, d_masks, reduce_fn)
+
+
+def solve_genome(scores_list, genome_budget, gammas, switch_costs_list=None, max_iter: int = 60, levels_per_round: int = 0,
+                 group=None):
+    """``solve_genome_packed`` for a list of NumPy arrays or tensors; returns ``(masks, genome, results)`` with the masks as
+    NumPy arrays.  ``switch_costs_list`` (single process only; ``gammas`` is then ignored) gives each chromosome its own
+    n_c - 1 switch costs; their genome sum is ``math.fsum`` of all of them."""
+    import math
+    torch = _torch()
+    if switch_costs_list is None:
+        d_scores, offsets, lengths = pack_scores(scores_list)
+        d_masks, genome, results = solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_iter=max_iter,
+                                                       levels_per_round=levels_per_round, group=group)
+    else:
+        if _group_size(group) > 1:
+            raise ValueError("`switch_costs_list` is supported in a single process only")
+        _lib.require_device()
+        if len(switch_costs_list) != len(scores_list):
+            raise ValueError("`switch_costs_list` must have one vector per chromosome")
+        d_scores, offsets, lengths = pack_scores(scores_list)
+        costs = [np.ascontiguousarray(c, dtype=np.float64).reshape(-1) for c in switch_costs_list]
+        for c, n in zip(costs, lengths):
+            if c.shape[0] != max(n - 1, 0):
+                raise ValueError("each switch-cost vector must have n - 1 entries")
+            if c.size and not (np.all(np.isfinite(c)) and np.all(c >= 0.0)):
+                raise ValueError("switch costs must be finite and >= 0")
+        zeros = [0.0] * len(lengths)
+        problem = _genome_problem(d_scores, offsets, lengths, zeros, genome_budget)
+        if problem:
+            raise ValueError(problem)
+        total = sum(lengths)
+        if total == 0:
+            raise ValueError("the genome has no chromosome")
+        d_costs = torch.zeros_like(d_scores)
+        for c, off in zip(costs, offsets):
+            if c.size:
+                d_costs[off:off + c.shape[0]].copy_(torch.from_numpy(c))
+        flat = [float(x) for c in costs for x in c]
+        search = _lib.GenomeSearch(total, target_count_for_budget(total, genome_budget), math.fsum(flat), max(flat, default=0.0),
+                                   float("nan"), float("nan"), int(max_iter), 0)
+        d_masks, genome, results = _solve_genome(d_scores, d_costs, offsets, lengths, zeros, search, levels_per_round, None, None)
+    h_masks = d_masks.cpu().numpy()
+    return [h_masks[off:off + n].copy() for off, n in zip(offsets, lengths)], genome, results
 
 
 _URGENT: dict = {}
@@ -334,13 +542,17 @@ def _score_streams(dev, count: int):
 
 
 def run_shard(d_matrices, budgets, gammas, params=None, levels_per_round: int = 0, want_runs: bool = True,
-              score_streams: int = 1):
+              score_streams: int = 1, genome_budget=None, group=None):
     """The hot path for one rank's chromosomes, device-resident end to end:
     score every chromosome -> one batched budget search + solve -> one batched mask->runs pass.
 
     With `score_streams` > 1 chromosomes are scored from that many host threads, each on its own CUDA stream
     (measured on B200: no gain at 100 samples -- the streaming kernels already fill the device -- so the default is 1).
+    With `genome_budget` (and `budgets` None) the search is the genome-wide one of `solve_genome_packed`: one multiplier
+    for the chromosomes of every rank of `group`, and the result gains "genome".
     Returns dict(d_scores, d_masks, offsets, lengths, results, runs)."""
+    if genome_budget is not None and budgets is not None:
+        raise ValueError("pass either per-chromosome `budgets` or one `genome_budget`, not both")
     torch = _torch()
     lengths = [int(x.shape[1]) for x in d_matrices]
     offsets, total = layout_offsets(lengths)
@@ -371,10 +583,18 @@ def run_shard(d_matrices, budgets, gammas, params=None, levels_per_round: int = 
         with ThreadPoolExecutor(max_workers=score_streams) as pool:
             for ev in pool.map(work, range(score_streams)):
                 main.wait_event(ev)
-    d_masks, results = solve_packed(d_scores, offsets, lengths, budgets, gammas, levels_per_round=levels_per_round)
+    genome = None
+    if genome_budget is None:
+        d_masks, results = solve_packed(d_scores, offsets, lengths, budgets, gammas, levels_per_round=levels_per_round)
+    else:
+        d_masks, genome, results = solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas,
+                                                       levels_per_round=levels_per_round, group=group)
     runs = masks_to_runs(d_masks, offsets, lengths) if want_runs else None
-    return {"d_scores": d_scores, "d_masks": d_masks, "offsets": offsets, "lengths": lengths,
-            "results": results, "runs": runs}
+    out = {"d_scores": d_scores, "d_masks": d_masks, "offsets": offsets, "lengths": lengths,
+           "results": results, "runs": runs}
+    if genome is not None:
+        out["genome"] = genome
+    return out
 
 
 def runs_to_bed_file(path: str, chrom_names, runs, step: int, first_start: int = 0) -> str:
