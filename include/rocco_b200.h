@@ -266,6 +266,7 @@ void rocco_b200_default_score_params(rocco_b200_score_params *p);
 int rocco_b200_trend_set_mode(int mode);
 long long rocco_b200_trend_fallback_rows(void);   /* rows that took the sort path since load */
 void rocco_b200_trend_fallback_reasons(long long *out8);   /* per-reason counts (diagnostics) */
+long long rocco_b200_whittaker_exact_rows(void);   /* baseline rows solved by the exact sequential path since load */
 
 /* Optional per-locus detail outputs (device or host according to the entry point); any may be NULL. */
 typedef struct rocco_b200_score_outputs {

@@ -143,3 +143,84 @@ int oracle_whittaker_factor(size_t n, int parity, double lam, double *d, double 
     factor_system(&f, n, parity, lam);
     return 0;
 }
+
+/*
+ * Binary128 restatement of oracle_crossfit_whittaker_baseline: the same factor, the same three sweeps per parity and the
+ * same end bands, every operation in __float128 (113-bit significand, unit roundoff 2^-113 ~ 1e-34).  The float64 solve
+ * loses up to ~1e-7 of max|y| at the largest penalties the reference accepts (window 1001: lambda ~ 4.5e9); here the
+ * same loss is ~1e-27, so the result rounded once to double is the exact solve for every test of the GPU kernels.
+ * Test infrastructure only: ~0.07 s per 60000-bin row on one core.
+ */
+typedef __float128 q128;
+
+static q128 qband_main(size_t i, size_t n, int parity, q128 lam)
+{
+    const q128 w = ((i & 1U) == (size_t)parity) ? 1 : 0;
+    if (i == 0 || i == n - 1) return w + lam;
+    if (i == 1 || i == n - 2) return w + (5 * lam);
+    return w + (6 * lam);
+}
+
+static q128 qband_off1(size_t i, size_t n, q128 lam)
+{
+    return (i == 0 || i == n - 2) ? (-2 * lam) : (-4 * lam);
+}
+
+/* factor_system and solve_factored in binary128; x: masked rhs in, the parity's fit out.  buf: 5n entries. */
+static void qsolve_parity(const double *y, size_t n, int parity, q128 lam, q128 *x, q128 *buf)
+{
+    q128 *d = buf, *l1 = buf + n, *l2 = buf + 2 * n, *fw = buf + 3 * n, *dz = buf + 4 * n;
+    q128 t1, t2;
+
+    d[0] = qband_main(0, n, parity, lam);
+    l1[0] = qband_off1(0, n, lam) / d[0];
+    l2[0] = lam / d[0];
+    d[1] = qband_main(1, n, parity, lam) - ((l1[0] * l1[0]) * d[0]);
+    t1 = ((l2[0] * d[0]) * l1[0]);
+    l1[1] = (qband_off1(1, n, lam) - t1) / d[1];
+    if (n > 3) l2[1] = lam / d[1];
+    for (size_t i = 2; i < n; ++i) {
+        t1 = ((l1[i - 1] * l1[i - 1]) * d[i - 1]);
+        t2 = ((l2[i - 2] * l2[i - 2]) * d[i - 2]);
+        d[i] = qband_main(i, n, parity, lam) - t1 - t2;
+        if (i + 2 <= n) {
+            t1 = ((l2[i - 1] * d[i - 1]) * l1[i - 1]);
+            l1[i] = (qband_off1(i, n, lam) - t1) / d[i];
+        }
+        if (i + 3 <= n) l2[i] = lam / d[i];
+    }
+
+    for (size_t i = 0; i < n; ++i) x[i] = ((i & 1U) == (size_t)parity) ? (q128)y[i] : 0;
+    fw[0] = x[0];
+    fw[1] = x[1] - (l1[0] * fw[0]);
+    for (size_t i = 2; i < n; ++i) fw[i] = x[i] - l1[i - 1] * fw[i - 1] - l2[i - 2] * fw[i - 2];
+    for (size_t i = 0; i < n; ++i) dz[i] = fw[i] / d[i];
+    x[n - 1] = dz[n - 1];
+    x[n - 2] = dz[n - 2] - (l1[n - 2] * x[n - 1]);
+    for (size_t i = n - 2; i-- > 0;) x[i] = dz[i] - l1[i] * x[i + 1] - l2[i] * x[i + 2];
+}
+
+int oracle_crossfit_whittaker_baseline_exact(const double *y, size_t n, double lam, double *out)
+{
+    if (y == NULL || out == NULL) return -1;
+    if (n < 25) {
+        for (size_t i = 0; i < n; ++i) out[i] = 0.0;
+        return 0;
+    }
+    q128 *buf = (q128 *)malloc((size_t)7 * n * sizeof(q128));
+    if (buf == NULL) return -1;
+    q128 *even = buf + 5 * n, *odd = buf + 6 * n;
+    qsolve_parity(y, n, 0, (q128)lam, even, buf);
+    qsolve_parity(y, n, 1, (q128)lam, odd, buf);
+    for (size_t i = 0; i < n; ++i) out[i] = (double)((even[i] + odd[i]) / 2);
+    free(buf);
+    return 0;
+}
+
+int oracle_crossfit_whittaker_baseline_exact_matrix(const double *rows, size_t m, size_t n, double lam, double *out)
+{
+    if (rows == NULL || out == NULL) return -1;
+    for (size_t r = 0; r < m; ++r)
+        if (oracle_crossfit_whittaker_baseline_exact(rows + r * n, n, lam, out + r * n) != 0) return -1;
+    return 0;
+}

@@ -176,6 +176,7 @@ def _declare(lib):
         "rocco_b200_trend_set_mode": (c_int, [c_int]),
         "rocco_b200_trend_fallback_rows": (c_longlong, []),
         "rocco_b200_trend_fallback_reasons": (None, [c_void_p]),
+        "rocco_b200_whittaker_exact_rows": (c_longlong, []),
         "rocco_score_loci_wls_f64": (c_int, [c_void_p, c_size_t, c_size_t, POINTER(ScoreParams), POINTER(ScoreOutputs)]),
         "rocco_score_loci_wls_f32": (c_int, [c_void_p, c_size_t, c_size_t, POINTER(ScoreParams), POINTER(ScoreOutputs)]),
         "rocco_b200_score_loci_wls_dev": (

@@ -9,6 +9,8 @@ namespace score {
 // log_transform: y = log2(max(x,0)+1) - pilot[row];  write_baseline: out = baseline, else out = y - baseline.
 int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double *d_pilot, long long rows, long long n,
                    long long row_stride, double lam, int write_baseline, double *d_out, int *d_bad, cudaStream_t st);
+// Rows solved by the exact sequential path (penalties beyond the tile kernels' range, whittaker.cu) since load.
+long long whittaker_exact_rows();
 
 // Pilot offsets: per-row median of log2(max(x,0)+1) -- exact for n <= 4096, else the median of a
 // 4096-point strided sample (the offset cancels in  y - baseline(y)  up to the solver's noise).

@@ -9,9 +9,14 @@
 //    itself) and only the last two rows deviate.  The host computes a short head table, the steady
 //    pair and a 4-entry tail once per (n, lambda);
 //  * forward / backward substitution are second-order linear recurrences, i.e. IIR filters whose
-//    impulse response decays like 0.9775^k for the default window.  Each tile is solved with a
-//    halo of HALO bins on both sides from a zero state; the truncation error at the tile is
+//    impulse response decays like rho^k, rho = 0.9775 for the default window (lambda(101) = 4.67e5).  Each tile is
+//    solved with a halo of HALO bins on both sides from a zero state; the truncation error at the tile is
 //    0.9775^1280 ~ 2e-13 of the signal, below the reference's own ~1e-10 noise floor;
+//  * rho grows with lambda (1 - rho ~ 0.59 lambda^-1/4): 0.9849 at window 151, 0.9977 at window 1001, where rho^1280 is
+//    5e-2.  build_factor computes rho from the steady pair and admits the tiles only while rho^HALO and rho^1536 (the
+//    streaming kernel's truncated cross-warp sum) are <= WT_TILE_TAU = 1e-12: windows up to 105 (lambda <= 5.5e5).
+//    Above that, rows longer than the head table take k_whittaker_exact, which replays the reference's sequential solve
+//    operation for operation (the same bits as baseline_backend.c), one thread per (row, parity);
 //  * every thread owns ITEMS consecutive bins: a zero-state local sweep, a scan of the 2-vector
 //    carry across threads, then the true sweep.  Both parities run interleaved in the same thread
 //    (two independent dependency chains).
@@ -19,9 +24,10 @@
 // Kernels:
 //  * k_whittaker_stream: interior ("steady") tiles, whose coefficients are the period-2 steady state.  A
 //    persistent grid of two-CTA clusters, one cluster per tile region at a time;
-//  * k_whittaker: the first and last tile(s) of a row, which read the head and tail tables.  One CTA per
-//    region, with a general carry scan over per-chunk transitions;
-//  * k_small_rows: rows shorter than 25 bins.
+//  * k_whittaker: the first and last tile(s) of a row, which read the head and tail tables, and every tile at penalties
+//    below ~10 (WP_REDERIVE_GROWTH_MAX).  One CTA per region, with a general carry scan over per-chunk transitions;
+//  * k_small_rows: rows shorter than 25 bins;
+//  * k_whittaker_exact + k_whittaker_exact_out: penalties the tiles cannot carry (above).
 //
 // Both tile kernels fuse the reference's Python prologue: y = log2(max(x,0)+1) - pilot_row
 // (inference.py:40-47, 333-334) and the epilogue  centered = y - baseline  (inference.py:338).
@@ -32,6 +38,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <atomic>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -44,6 +51,17 @@ constexpr int WT_HALO = 1280;
 constexpr int WT_OUT = WT_REGION - 2 * WT_HALO;    // 9728 bins written per CTA
 constexpr int WT_THREADS_G = 512, WT_ITEMS_G = 24; // edge tiles (k_whittaker): one CTA per region
 constexpr int HEAD_LEN = 4096;
+// Largest decay rho^k, over the shortest distance k a truncated state is carried in the tile kernels, at which they are
+// used.  A tile's truncation error is at most about rho^k max|y| (measured in a float64 emulation of one steady tile at
+// windows 151 to 1001: 0.1 to 0.25 rho^1280 max|y|).  The reference's own float64 solve is off by ~1e-11 max|y| already
+// at the default penalty, and by more above it, so 1e-12 keeps the truncation an order of magnitude under that error:
+// the kernels stay as accurate as the reference wherever they are used.
+constexpr double WT_TILE_TAU = 1e-12;
+// The streaming kernel re-derives the forward solution right to left over a thread's WP_GEOM_ITEMS bins, which multiplies
+// its rounding by r^-WP_GEOM_ITEMS, r the smaller per-bin root modulus of the forward recurrence: 1.3 at the default
+// penalty, but 2e3 at window 3 and 1e18 at lambda = 1e-3.  Up to 64 (r >= 0.71, lambda >~ 10) that stays below 1e-14
+// of the signal; smaller penalties send the interior tiles to k_whittaker, which stores the forward solution instead.
+constexpr double WP_REDERIVE_GROWTH_MAX = 64.0;
 
 // ------------------------------------------------------------------ host: factor tables
 static void host_factor(long long n_true, long long len, int parity, double lam,
@@ -84,6 +102,7 @@ constexpr int WP_LEVELS = 9;                       // 5 in-warp levels + 4 acros
 // thread geometry of the streaming kernel (threads x bins per thread = WP_HALF): 512 x 12 (384 x 16 and a cluster of four
 // 256-thread CTAs were measured slower: fewer resident warps / no gain from the finer phases)
 constexpr int WP_GEOM_THREADS = 512, WP_GEOM_ITEMS = 12;
+constexpr int WP_CROSS_WARP_BINS = 4 * 32 * WP_GEOM_ITEMS;   // span of the streaming kernel's truncated cross-warp sum
 struct PairTab {
     double cf[2][3][2];                            // [chain][dinv, l1, l2][position parity]
     double trans[2][2][WP_LEVELS][4];              // [chain][fwd/bwd][level]: transition over ITEMS * 2^level bins
@@ -102,6 +121,9 @@ struct FactorHost {
     std::vector<double> head[2][3];      // [parity][dinv,l1,l2][head_len]
     double steady[2][3][2];              // [parity][coef][index parity]
     double tail[2][3][4];                // rows n-4 .. n-1
+    double decay[2] = {0.0, 0.0};        // [parity]: rho, the per-bin decay of the steady recurrence
+    bool tiles_exact = true;             // rho^WT_HALO and rho^WP_CROSS_WARP_BINS <= WT_TILE_TAU (always for short rows)
+    bool stream_stable = true;           // r^-WP_GEOM_ITEMS <= WP_REDERIVE_GROWTH_MAX (see above)
 };
 
 static void mat2_mul(const double *a, const double *b, double *c)   // c = a*b (row-major 2x2)
@@ -147,10 +169,24 @@ static void build_factor(long long n, double lam, FactorHost &F)
                 if (i <= n - 3) e2[k] = lam / dd[k];
                 F.tail[p][0][k - 2] = 1.0 / dd[k]; F.tail[p][1][k - 2] = e1[k]; F.tail[p][2][k - 2] = e2[k];
             }
+            // decay per bin: square root of the spectral radius of the two-step companion matrix of the forward
+            // recurrence f_i = r_i - l1[i-1] f_{i-1} - l2[i-2] f_{i-2} (the backward one is its transpose)
+            const double Se[4] = {-l1[len - 1], -l2[len - 2], 1.0, 0.0};       // step onto an even index
+            const double So[4] = {-l1[len - 2], -l2[len - 1], 1.0, 0.0};       // step onto an odd index
+            double M[4];
+            mat2_mul(So, Se, M);
+            const double tr = M[0] + M[3], det = M[0] * M[3] - M[1] * M[2], disc = tr * tr - 4.0 * det;
+            const double radius = disc < 0.0 ? sqrt(det) : 0.5 * (fabs(tr) + sqrt(disc));
+            F.decay[p] = sqrt(radius);
+            const double rmin = sqrt(fabs(det) / radius);                   // smaller per-bin root modulus
+            F.stream_stable = F.stream_stable && pow(rmin, -WP_GEOM_ITEMS) <= WP_REDERIVE_GROWTH_MAX;
         } else {
             for (int k = 0; k < 4; ++k) F.tail[p][0][k] = F.tail[p][1][k] = F.tail[p][2][k] = 0.0;
         }
     }
+    // (a NaN decay, from lambda = 0 or not finite, fails the test too)
+    for (int p = 0; p < 2 && !small; ++p)
+        F.tiles_exact = F.tiles_exact && pow(F.decay[p], WT_HALO) <= WT_TILE_TAU && pow(F.decay[p], WP_CROSS_WARP_BINS) <= WT_TILE_TAU;
     // streaming kernel: chains by region-position parity, for both alignment shift parities
     constexpr int WP_ITEMS = WP_GEOM_ITEMS, WP_WARPS = WP_GEOM_THREADS / 32;
     for (int ap = 0; ap < 2; ++ap) {
@@ -929,6 +965,102 @@ __global__ void k_small_rows(WhitParams P)
     if (bad) *P.bad = 1;
 }
 
+// ------------------------------------------------------------------ exact path: the reference's sequential solve
+// Penalties at which the tiles' truncation is not negligible (FactorHost::tiles_exact false).  One thread per (row, parity)
+// replays baseline_backend.c:142-173 over the full factor of (n, lambda, parity), which every row of the call shares:
+// the forward sweep, the division by the diagonal and the backward sweep, with the reference's roundings (no
+// contraction into FMAs).  Parity 0 solves in place in its output row, parity 1 in `scratch`; k_whittaker_exact_out then
+// forms the cross-fit average and the epilogue.  y is recomputed there with the same library log2, so both kernels see
+// the same bits, and the baseline is the reference's bit for bit.
+struct ExactFactor { const double *d[2], *l1[2], *l2[2]; };
+
+__global__ void k_whittaker_exact(WhitParams P, ExactFactor F, double *scratch, long long row0, long long rows)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= 2 * rows) return;
+    const long long row = row0 + (t >> 1), n = P.n;
+    const int p = (int)(t & 1);
+    double *x = p ? scratch + (t >> 1) * n : P.out + row * P.row_stride;
+    const double *d = F.d[p], *l1 = F.l1[p], *l2 = F.l2[p];
+    auto rhs = [&](long long i) {                     // masked rhs (oracle_baseline.c masked_rhs): keeps the signed zeros
+        const double y = load_y(P, row, i);
+        const bool on = (int)(i & 1) == p;
+        if (i < 2 || i + 2 >= n) return on ? y : 0.0;
+        return __dmul_rn(on ? 1.0 : 0.0, y);
+    };
+    double f2 = rhs(0);
+    double f1 = __dsub_rn(rhs(1), __dmul_rn(l1[0], f2));
+    x[0] = __ddiv_rn(f2, d[0]);
+    x[1] = __ddiv_rn(f1, d[1]);
+#pragma unroll 4
+    for (long long i = 2; i < n; ++i) {
+        const double f = __dsub_rn(__dsub_rn(rhs(i), __dmul_rn(l1[i - 1], f1)), __dmul_rn(l2[i - 2], f2));
+        x[i] = __ddiv_rn(f, d[i]);
+        f2 = f1; f1 = f;
+    }
+    double b1 = x[n - 1];
+    double b0 = __dsub_rn(x[n - 2], __dmul_rn(l1[n - 2], b1));
+    x[n - 2] = b0;
+#pragma unroll 4
+    for (long long i = n - 2; i-- > 0;) {
+        const double v = __dsub_rn(__dsub_rn(x[i], __dmul_rn(l1[i], b0)), __dmul_rn(l2[i], b1));
+        x[i] = v; b1 = b0; b0 = v;
+    }
+}
+
+__global__ void k_whittaker_exact_out(WhitParams P, const double *scratch, long long row0, long long rows)
+{
+    const long long total = rows * P.n;
+    int bad = 0;
+    for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < total; g += (long long)gridDim.x * blockDim.x) {
+        const long long r = g / P.n, i = g % P.n, row = row0 + r;
+        double *o = P.out + row * P.row_stride + i;
+        const double b = __dmul_rn(0.5, __dadd_rn(*o, scratch[g]));         // baseline_backend.c:296-299
+        const double y = load_y(P, row, i);                                  // NaN for a non-finite input
+        const double v = P.write_baseline ? b : __dsub_rn(y, b);
+        bad |= !isfinite(y) || !isfinite(v);
+        *o = v;
+    }
+    if (bad) *P.bad = 1;
+}
+
+static std::atomic<long long> g_exact_rows{0};
+long long whittaker_exact_rows() { return g_exact_rows.load(); }
+
+static int whittaker_exact(const WhitParams &P, double lam, cudaStream_t st)
+{
+    // scratch bounded by the factor (6 n doubles) and up to 256 MB of parity-1 rows; released when this call returns
+    const long long n = P.n, rows = P.rows;
+    Arena ar(st);
+    std::vector<double> h((size_t)6 * n);
+    ExactFactor E;
+    double *d_fac = nullptr, *d_scr = nullptr;
+    RB_TRY(ar.alloc(&d_fac, (size_t)6 * n));
+    for (int p = 0; p < 2; ++p) {
+        std::vector<double> d, l1, l2;
+        host_factor(n, n, p, lam, d, l1, l2);
+        std::copy(d.begin(), d.end(), h.begin() + (3 * p + 0) * n);
+        std::copy(l1.begin(), l1.end(), h.begin() + (3 * p + 1) * n);
+        std::copy(l2.begin(), l2.end(), h.begin() + (3 * p + 2) * n);
+        E.d[p] = d_fac + (3 * p + 0) * n; E.l1[p] = d_fac + (3 * p + 1) * n; E.l2[p] = d_fac + (3 * p + 2) * n;
+    }
+    // (pageable source: the call returns once h is staged, so h may die with this scope)
+    RB_CUDA(cudaMemcpyAsync(d_fac, h.data(), sizeof(double) * h.size(), cudaMemcpyHostToDevice, st));
+    const long long batch = std::max<long long>(1, std::min<long long>(rows, (256LL << 20) / (long long)sizeof(double) / n));
+    RB_TRY(ar.alloc(&d_scr, (size_t)(batch * n)));
+    for (long long r0 = 0; r0 < rows; r0 += batch) {
+        const long long nr = std::min(batch, rows - r0);
+        RB_PROF("k_whittaker_exact", st, (double)nr * n * ((P.in_f32 ? 4.0 : 8.0) + 8.0));
+        k_whittaker_exact<<<(unsigned)((2 * nr + 63) / 64), 64, 0, st>>>(P, E, d_scr, r0, nr);
+        RB_LAUNCH_CHECK();
+        const int blocks = (int)std::min<long long>((nr * n + 255) / 256, (long long)sm_count() * 8);
+        k_whittaker_exact_out<<<blocks, 256, 0, st>>>(P, d_scr, r0, nr);
+        RB_LAUNCH_CHECK();
+    }
+    g_exact_rows.fetch_add(rows);
+    return 0;
+}
+
 // ------------------------------------------------------------------ factor cache (device tables per (n, lambda))
 // Entries are handed out as shared_ptr: a caller keeps its tables alive across its launches whatever the cache does
 // meanwhile (eviction only drops the cache's own reference), and the device buffers are released by the destructor on
@@ -1089,9 +1221,10 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
     memcpy(P.steady, F->host.steady, sizeof(P.steady));
     memcpy(P.tail, F->host.tail, sizeof(P.tail));
     P.log2tab = F->d_log2;
+    if (!F->host.tiles_exact) return whittaker_exact(P, lam, st);
     P.tiles_per_row = (int)((n + WT_OUT - 1) / WT_OUT);
-    // Interior tiles (region inside [head_len, n-4)) take the streaming kernel; the first and last tile(s) of each row
-    // take k_whittaker.  Launches over disjoint tile sets.
+    // Interior tiles (region inside [head_len, n-4)) take the streaming kernel unless the penalty is too small for its
+    // right-to-left re-derivation; the first and last tile(s) of each row take k_whittaker.  Launches over disjoint tile sets.
     const size_t sm_general = sizeof(double) * 2 * WT_THREADS_G * (WT_ITEMS_G + 1) + sizeof(double) * 6 * WT_THREADS_G;
     static bool attr_dev[64] = {false};
     int attr_d = 0;
@@ -1106,7 +1239,7 @@ int whittaker_rows(const void *d_x, int in_f32, int log_transform, const double 
     for (int t = 0; t < P.tiles_per_row; ++t) {
         const long long o0 = (long long)t * WT_OUT, o1 = std::min(n, o0 + WT_OUT);
         const long long r0 = std::max<long long>(0, o0 - WT_HALO), r1 = std::min(n, o1 + WT_HALO);
-        const bool steady = (r0 >= P.head_len + 8) && (r1 <= n - 6) && (r1 - r0 == WT_REGION);      // (+8: room for the streaming kernel's alignment shift)
+        const bool steady = F->host.stream_stable && (r0 >= P.head_len + 8) && (r1 <= n - 6) && (r1 - r0 == WT_REGION);      // (+8: room for the streaming kernel's alignment shift)
         if (steady) { first_steady = std::min(first_steady, t); last_steady = std::max(last_steady, t); }
     }
     // general tiles: [0, first_steady) and (last_steady, tiles); steady tiles are contiguous in between

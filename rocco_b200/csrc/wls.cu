@@ -860,6 +860,7 @@ RB_API int rocco_b200_trend_set_mode(int mode)
     return score::g_trend_mode.exchange(mode == 1 ? 1 : 0);
 }
 RB_API long long rocco_b200_trend_fallback_rows(void) { return score::g_trend_fallback_rows.load(); }
+RB_API long long rocco_b200_whittaker_exact_rows(void) { return score::whittaker_exact_rows(); }
 RB_API void rocco_b200_trend_fallback_reasons(long long *out8) { for (int k = 0; k < 8; ++k) out8[k] = score::g_trend_fb_reason[k].load(); }
 
 RB_API void rocco_b200_default_score_params(rocco_b200_score_params *p)

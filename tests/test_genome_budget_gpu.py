@@ -237,7 +237,10 @@ try:
     out["nonfinite"] = "no error"
 except ValueError as exc:
     out["nonfinite"] = "ValueError"
-print("RESULT " + json.dumps(out), flush=True)
+# one write of the whole line (well under PIPE_BUF): print() writes the text and the newline separately, so the two
+# ranks' lines could interleave on the shared pipe
+sys.stdout.write("RESULT " + json.dumps(out) + "\n")
+sys.stdout.flush()
 dist.destroy_process_group()
 '''
 
