@@ -406,6 +406,10 @@ int rocco_column_stat_f64(const double *matrix, size_t m, size_t n, int stat,
                           double arg0, double arg1, double power, double *out);
 int rocco_b200_column_stat_dev(const void *d_matrix, int dtype, size_t m, size_t n, int stat,
                                double arg0, double arg1, double power, double *d_out, void *cuda_stream);
+/* Column-statistics kernel choice: 1 = the shared-memory tile kernel (radix select per rank) for every m >= 2, any other
+ * value = automatic (per-thread lists below the measured crossover, the tile kernel from it on and wherever the lists
+ * do not fit).  Both give the same values; returns the previous mode. */
+int rocco_b200_colstat_set_mode(int mode);
 
 /* ------------------------------------------------------------------ matrix assembly / input staging (SURVEY.md 8(f) rank 3)
  * The step BEFORE the hot path, on the device, so that what crosses PCIe is the decoded alignment records (or the

@@ -198,6 +198,7 @@ def _declare(lib):
         "rocco_column_stat_f64": (c_int, [c_void_p, c_size_t, c_size_t, c_int, c_double, c_double, c_double, c_void_p]),
         "rocco_b200_column_stat_dev": (
             c_int, [c_void_p, c_int, c_size_t, c_size_t, c_int, c_double, c_double, c_double, c_void_p, c_void_p]),
+        "rocco_b200_colstat_set_mode": (c_int, [c_int]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)          # AttributeError here = header/library mismatch: fail loudly

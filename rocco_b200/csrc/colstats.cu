@@ -4,14 +4,17 @@
 // np.quantile(method="nearest") / scipy.stats.tmean in a Python loop over bins / np.mean) and
 // rocco.py:307-355 (score_dispersion_chrom: scipy median_abs_deviation / iqr / np.std / tstd).
 //
-// One thread per bin.  Loads are coalesced along the bin axis (thread j reads X[i, j] for every sample i).  Median,
+// Up to a crossover in m (tile_from), one thread per bin.  Loads are coalesced along the bin axis (thread j reads X[i, j] for every sample i).  Median,
 // nearest-rank quantile, MAD and IQR read one to four ranks of the column: the thread keeps just the smallest (and / or
 // largest) values needed to reach them in a short sorted list in shared memory, [slot][thread] (conflict-free)
 // (k_colstat_ranks).  Trimmed mean / std need the whole column: it is insertion-sorted in shared memory (k_colstat).
 // All order statistics are exact.  Sums follow NumPy's own association order -- sequential over rows for axis-0
 // reductions of a C-contiguous matrix, pairwise (8 accumulators, blocks of 128) for the 1-D reductions that
 // scipy's tmean/tstd perform per column -- so means and standard deviations reproduce the reference's bits.
+// From the crossover on, and for every m those kernels cannot hold, k_colstat_tile stages a tile of bins x all samples in
+// shared memory and radix-selects each wanted rank with the whole CTA; MEAN / STD run k_colstat without shared memory.
 #include "common.cuh"
+#include "select.cuh"
 
 #include <math.h>
 
@@ -225,6 +228,197 @@ __global__ void k_colstat_ranks(Params P, PartialLists C)
     P.out[j] = np_power(result, P.power);
 }
 
+// ---- any sample count: k_colstat_tile
+// A CTA stages W consecutive bins x all m rows in shared memory, each value read from HBM once, as order-preserving
+// 64-bit keys (sign-flip; -0.0 and +0.0 share one key, as they compare equal in NumPy), column c contiguous in row order
+// at tile + c * ld (ld odd: the staging stores of one warp spread over the banks).  The wanted ranks of a column come from
+// score::block_select over the whole CTA, one column after the other; a rank already covered by the previous select's
+// run of equal keys costs nothing.  TMEAN / TSTD then sum each column in row order with np_pairwise, one thread per column.
+// Results are the bits of k_colstat / k_colstat_ranks wherever those run (up to the sign of a zero result).
+constexpr int TILE_THREADS = 256, TILE_MAX_W = 32;
+
+__device__ __forceinline__ unsigned long long dkey(double v)
+{
+    const unsigned long long b = (unsigned long long)__double_as_longlong(__dadd_rn(v, 0.0));     // -0.0 -> +0.0
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ULL);
+}
+
+__device__ __forceinline__ double dval(unsigned long long k)
+{
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffULL) : ~k));
+}
+
+struct RankCache { unsigned long long key; int below, equal; };
+
+// key of 0-based ascending rank r of the column (uniform over the CTA)
+__device__ __forceinline__ unsigned long long rank_key(const unsigned long long *col, int m, long long r, score::SelScratch &S,
+                                                       RankCache &rc)
+{
+    if (rc.equal > 0 && r >= rc.below && r < (long long)rc.below + rc.equal) return rc.key;
+    rc.key = score::block_select<TILE_THREADS, true>(col, m, (int)r, nullptr, 0ULL, S, &rc.below, &rc.equal);
+    return rc.key;
+}
+
+__global__ void __launch_bounds__(TILE_THREADS, 2) k_colstat_tile(Params P, int lw, int ld)
+{
+    extern __shared__ unsigned long long s_dyn[];          // SelScratch, then the [W][ld] key tile
+    __shared__ unsigned long long s_lim[2][TILE_MAX_W];     // TMEAN / TSTD: the limit keys of each column
+    score::SelScratch &S = score::plan_scratch(s_dyn);
+    unsigned long long *tile = s_dyn + sizeof(score::SelScratch) / sizeof(unsigned long long);
+    const int W = 1 << lw;
+    const long long j0 = (long long)blockIdx.x * W;
+    const int w = (int)min((long long)W, P.n - j0);
+    const int m = (int)P.m;
+    {                                                       // stage: a warp reads 32 / W rows of W consecutive bins
+        const int c = threadIdx.x & (W - 1), step = TILE_THREADS >> lw;
+        if (c < w) {
+            unsigned long long *col = tile + (size_t)c * ld;
+            if (P.in_f32) {
+                const float *x = reinterpret_cast<const float *>(P.x) + j0 + c;
+#pragma unroll 4
+                for (int i = threadIdx.x >> lw; i < m; i += step) col[i] = dkey((double)x[(long long)i * P.n]);
+            } else {
+                const double *x = reinterpret_cast<const double *>(P.x) + j0 + c;
+#pragma unroll 4
+                for (int i = threadIdx.x >> lw; i < m; i += step) col[i] = dkey(x[(long long)i * P.n]);
+            }
+        }
+    }
+    __syncthreads();
+    // the ranks each column needs (the same for every column): median / MAD 0-1, quantile 0, IQR 0-3, TMEAN / TSTD 0-1
+    const int stat = P.stat;
+    long long want[4];
+    double gam[2] = {0.0, 0.0};
+    int nw;
+    if (stat == ROCCO_STAT_MEDIAN || stat == ROCCO_STAT_MAD) {
+        want[0] = (m & 1) ? m / 2 : m / 2 - 1; want[1] = m / 2; nw = 2;
+    } else if (stat == ROCCO_STAT_QUANTILE) {
+        long long k = round_half_even((double)(m - 1) * P.arg0);
+        want[0] = k < 0 ? 0 : (k >= m ? m - 1 : k); nw = 1;
+    } else if (stat == ROCCO_STAT_IQR) {                   // scipy.stats.iqr, linear interpolation
+        for (int k = 0; k < 2; ++k) {
+            const double q = (k == 0 ? P.arg0 : P.arg1) / 100.0;
+            const double vi = (double)(m - 1) * q;
+            double prev = floor(vi);
+            long long ip = (long long)prev, in = ip + 1;
+            if (vi >= (double)(m - 1)) { ip = m - 1; in = m - 1; }
+            if (vi < 0) { ip = 0; in = 0; }
+            gam[k] = __dsub_rn(vi, prev);
+            want[2 * k] = ip; want[2 * k + 1] = in;
+        }
+        nw = 4;
+    } else {                                               // TMEAN / TSTD: nearest-rank limits, inclusive
+        long long kl = round_half_even((double)(m - 1) * P.arg0);
+        long long kh = round_half_even((double)(m - 1) * (1.0 - P.arg0));
+        want[0] = kl < 0 ? 0 : (kl >= m ? m - 1 : kl);
+        want[1] = kh < 0 ? 0 : (kh >= m ? m - 1 : kh);
+        nw = 2;
+    }
+    for (int c = 0; c < w; ++c) {
+        unsigned long long *col = tile + (size_t)c * ld;
+        unsigned long long key[4];
+        for (int pass = 0;; ++pass) {
+            RankCache rc{0ULL, 0, 0};
+#pragma unroll 1
+            for (int q = 0; q < nw; ++q) key[q] = rank_key(col, m, want[q], S, rc);
+            if (stat != ROCCO_STAT_MAD || pass == 1) break;
+            // MAD: the same ranks of |x - median|, rewritten in place
+            const double med = __dadd_rn(dval(key[0]), dval(key[1])) / 2.0;
+            const double mid = (m & 1) ? dval(key[1]) : med;
+            for (int i = threadIdx.x; i < m; i += TILE_THREADS) col[i] = dkey(fabs(__dsub_rn(dval(col[i]), mid)));
+            __syncthreads();
+        }
+        double result;
+        if (stat == ROCCO_STAT_MEDIAN || stat == ROCCO_STAT_MAD)
+            result = (m & 1) ? dval(key[1]) : __dadd_rn(dval(key[0]), dval(key[1])) / 2.0;
+        else if (stat == ROCCO_STAT_QUANTILE)
+            result = dval(key[0]);
+        else if (stat == ROCCO_STAT_IQR)
+            result = __dsub_rn(lerp_np(dval(key[2]), dval(key[3]), gam[1]), lerp_np(dval(key[0]), dval(key[1]), gam[0]));
+        else {
+            if (threadIdx.x == 0) { s_lim[0][c] = key[0]; s_lim[1][c] = key[1]; }
+            continue;
+        }
+        if (threadIdx.x == 0) P.out[j0 + c] = np_power(result, P.power);
+    }
+    if (stat != ROCCO_STAT_TMEAN && stat != ROCCO_STAT_TSTD) return;
+    __syncthreads();
+    const int c = threadIdx.x;
+    if (c >= w) return;
+    unsigned long long *colk = tile + (size_t)c * ld;
+    double *col = reinterpret_cast<double *>(colk);        // rewritten in place as the doubles that are summed
+    const unsigned long long klo = s_lim[0][c], khi = s_lim[1][c];
+    long long cnt = 0;
+    double result;
+    if (stat == ROCCO_STAT_TMEAN) {
+        // scipy.stats.tmean: sum over the column in row order with outsiders replaced by 0, / count
+        for (int i = 0; i < m; ++i) {
+            const unsigned long long k = colk[i];
+            const bool keep = k >= klo && k <= khi;
+            cnt += keep;
+            col[i] = keep ? dval(k) : 0.0;
+        }
+        result = cnt > 0 ? np_pairwise(col, 1, m, nullptr) / (double)cnt : NAN;
+    } else {
+        // np.std(ddof=1) of the kept values gathered in row order (write index <= read index)
+        for (int i = 0; i < m; ++i) {
+            const unsigned long long k = colk[i];
+            if (k >= klo && k <= khi) col[cnt++] = dval(k);
+        }
+        const double mean = np_pairwise(col, 1, cnt, nullptr) / (double)cnt;
+        result = cnt > 1 ? sqrt(np_pairwise(col, 1, cnt, &mean) / (double)(cnt - 1)) : NAN;
+    }
+    P.out[j0 + c] = np_power(result, P.power);
+}
+
+// largest m whose one-column tile fits in a CTA's shared memory
+static size_t tile_max_m(int smem_optin)
+{
+    const size_t avail = (size_t)smem_optin - sizeof(score::SelScratch) - 2 * TILE_MAX_W * sizeof(unsigned long long);
+    const size_t ld = avail / sizeof(unsigned long long);
+    return (ld & 1) ? ld : ld - 1;                         // ld = m | 1
+}
+
+static int run_tile(const Params &P0, cudaStream_t st)
+{
+    Params P = P0;
+    const size_t m = (size_t)P.m, n = (size_t)P.n;
+    int dev = 0, optin = 0;
+    RB_CUDA(cudaGetDevice(&dev));
+    RB_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    const size_t max_m = tile_max_m(optin);
+    if (m > max_m) {
+        set_error("column statistics support at most %zu samples (one column of 64-bit keys in shared memory)", max_m);
+        return ST_INVALID;
+    }
+    const size_t ld = m | 1, col_bytes = ld * sizeof(unsigned long long), base = sizeof(score::SelScratch);
+    const size_t limit = (size_t)optin - 2 * TILE_MAX_W * sizeof(unsigned long long);
+    // widest power of two <= 32 within 100 KB (two CTAs per SM, which is what the registers allow), but at least a 32-byte
+    // sector of every row segment (8 float32 / 4 float64 bins) when that fits at all
+    const int sector_w = P.in_f32 ? 8 : 4;
+    int lw = 5;
+    while (lw > 0 && base + ((size_t)1 << lw) * col_bytes > 100 * 1024) --lw;
+    while ((1 << lw) < sector_w && base + ((size_t)2 << lw) * col_bytes <= limit) ++lw;
+    const int W = 1 << lw;
+    const size_t smem = base + (size_t)W * col_bytes;
+    RB_CUDA(cudaFuncSetAttribute(k_colstat_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    RB_PROF("k_colstat_tile", st, (double)m * n * (P.in_f32 ? 4.0 : 8.0) + 8.0 * n);
+    k_colstat_tile<<<(unsigned)((n + W - 1) / W), TILE_THREADS, smem, st>>>(P, lw, (int)ld);
+    RB_LAUNCH_CHECK();
+    return 0;
+}
+
+// 1: k_colstat_tile for every m >= 2 (tests compare it with the other kernels); anything else: chosen from m and the statistic
+static std::atomic<int> g_colstat_mode{0};
+
+// smallest m at which k_colstat_tile takes a statistic in automatic mode even where the list kernels fit.  Until
+// tools/colstat_large.py has measured a crossover the list kernels keep every size they can hold (DESIGN.md section 3).
+static size_t tile_from(int stat, int in_f32)
+{
+    (void)stat; (void)in_f32;
+    return (size_t)1 << 62;
+}
+
 __global__ void k_single_row(Params P)
 {
     // m == 1: central tendency = row ** power; dispersion = zeros ** power (rocco.py:254-255, 318-319)
@@ -233,6 +427,16 @@ __global__ void k_single_row(Params P)
     const bool dispersion = P.stat >= ROCCO_STAT_MAD;
     const double v = dispersion ? 0.0 : ldx(P, 0, j);
     P.out[j] = np_power(v, P.power);
+}
+
+// MEAN / STD read the matrix only: k_colstat without the per-column shared-memory reservation serves any m
+static int run_moments(Params P, cudaStream_t st)
+{
+    P.tb = 128;
+    RB_PROF("k_colstat", st, (double)P.m * P.n * (P.in_f32 ? 4.0 : 8.0) + 8.0 * P.n);
+    k_colstat<<<(unsigned)((P.n + 127) / 128), 128, 0, st>>>(P);
+    RB_LAUNCH_CHECK();
+    return 0;
 }
 
 static int run(const void *d_x, int dtype, size_t m, size_t n, int stat, double arg0, double arg1, double power,
@@ -249,6 +453,8 @@ static int run(const void *d_x, int dtype, size_t m, size_t n, int stat, double 
         RB_LAUNCH_CHECK();
         return 0;
     }
+    const bool moments = stat == ROCCO_STAT_MEAN || stat == ROCCO_STAT_STD;
+    if (g_colstat_mode.load() == 1 || m >= tile_from(stat, dtype)) return moments ? run_moments(P, st) : run_tile(P, st);
     // ranks wanted by the order-statistic modes -> list capacities (ascending ranks below cap_lo, the rest from the top)
     if (stat == ROCCO_STAT_MEDIAN || stat == ROCCO_STAT_QUANTILE || stat == ROCCO_STAT_MAD || stat == ROCCO_STAT_IQR) {
         long long r_min = 0, r_max = 0;                    // smallest and largest 0-based rank read
@@ -293,7 +499,7 @@ static int run(const void *d_x, int dtype, size_t m, size_t n, int stat, double 
         const size_t budget_r = 200 * 1024;
         int tbr = 128;
         while (tbr > 32 && slots * tbr * 8 > budget_r) tbr -= 32;
-        if (slots * tbr * 8 > budget_r) { set_error("column statistics support at most %zu samples", budget_r / (8 * 32)); return ST_INVALID; }
+        if (slots * tbr * 8 > budget_r) return run_tile(P, st);            // the lists do not fit: no list kernel
         P.tb = tbr;
         const size_t smem_r = slots * tbr * sizeof(double);
         RB_CUDA(cudaFuncSetAttribute(k_colstat_ranks, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget_r));
@@ -305,7 +511,7 @@ static int run(const void *d_x, int dtype, size_t m, size_t n, int stat, double 
     const size_t budget = 192 * 1024;
     int tb = (int)std::min<size_t>(128, budget / (8 * m));
     tb = (tb / 32) * 32;
-    if (tb < 32) { set_error("column statistics support at most %zu samples", budget / (8 * 32)); return ST_INVALID; }
+    if (tb < 32) return moments ? run_moments(P, st) : run_tile(P, st);     // the column does not fit
     P.tb = tb;
     const size_t smem = (size_t)tb * m * sizeof(double);
     RB_CUDA(cudaFuncSetAttribute(k_colstat, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
@@ -325,6 +531,11 @@ RB_API int rocco_b200_column_stat_dev(const void *d_matrix, int dtype, size_t m,
                                       double power, double *d_out, void *cuda_stream)
 {
     return colstats::run(d_matrix, dtype, m, n, stat, arg0, arg1, power, d_out, (cudaStream_t)cuda_stream);
+}
+
+RB_API int rocco_b200_colstat_set_mode(int mode)
+{
+    return colstats::g_colstat_mode.exchange(mode == 1 ? 1 : 0);
 }
 
 RB_API int rocco_column_stat_f64(const double *matrix, size_t m, size_t n, int stat, double arg0, double arg1, double power,

@@ -16,7 +16,10 @@ __device__ __forceinline__ SelScratch &plan_scratch(void *raw) { return *reinter
 // Key of 0-based `rank` among the keys[i], i < cnt, that pass the filter (fkeys == nullptr, or fkeys[i] == fval).  All
 // THREADS threads call it; the result is uniform.  *below = number of filtered keys smaller than the result, *equal =
 // number equal to it.  The filtered set must hold more than `rank` keys.
-template <int THREADS>
+// RENARROW: after each pass, the next one starts at the highest bit in which the remaining candidates differ, and a
+// bucket of equal keys ends the search -- one extra scan per pass, but a column of tied values (mostly zeros in count
+// data) takes two scans instead of falling through every digit.
+template <int THREADS, bool RENARROW = false>
 __device__ unsigned long long block_select(const unsigned long long *keys, int cnt, int rank, const unsigned long long *fkeys,
                                            unsigned long long fval, SelScratch &S, int *below, int *equal)
 {
@@ -90,6 +93,25 @@ __device__ unsigned long long block_select(const unsigned long long *keys, int c
             }
             __syncthreads();
             result = S.res[2]; nequal = 1; found = true;
+        } else if (RENARROW) {
+            unsigned long long cmin = ~0ULL, cmax = 0ULL;
+            for (int i = tid; i < cnt; i += THREADS) {
+                const unsigned long long k = keys[i];
+                if ((!fkeys || fkeys[i] == fval) && (k & mask) == prefix) { cmin = min(cmin, k); cmax = max(cmax, k); }
+            }
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) {
+                cmin = min(cmin, __shfl_xor_sync(0xffffffffu, cmin, d));
+                cmax = max(cmax, __shfl_xor_sync(0xffffffffu, cmax, d));
+            }
+            if (tid == 0) { S.res[0] = ~0ULL; S.res[1] = 0ULL; }          // S.res[0..1] were last read before the histogram
+            __syncthreads();
+            if (lane == 0) { atomicMin(&S.res[0], cmin); atomicMax(&S.res[1], cmax); }
+            __syncthreads();
+            cmin = S.res[0]; cmax = S.res[1];
+            const int t2 = 64 - __clzll((long long)(cmin ^ cmax));       // < top: the candidates share the prefix
+            if (t2 == 0) { result = cmin; nequal = inside; found = true; }
+            else { top = t2; prefix = (cmin >> top) << top; mask = ~((1ULL << top) - 1ULL); }
         }
         __syncthreads();
     }

@@ -927,3 +927,159 @@ def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=
 
     return _budget_null_sharded(d_centered_local, m_total, offset, reduce_fn, d_observed_scores, params, dependence_lag_hint,
                                 num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations)
+
+
+# ------------------------------------------------------------------ column statistics on device tensors
+_DISPERSION_METHODS = ("mad", "iqr", "std", "tstd")
+
+
+def _column_stat_spec(method, quantile=0.50, tprop=0.05, rng=(25, 75)) -> tuple[int, float, float, bool]:
+    """(stat code, arg0, arg1, dispersion) of a method of ``score_central_tendency_chrom`` or ``score_dispersion_chrom``
+    (``median`` = quantile 0.5), normalised as those functions do."""
+    from .rocco import _STAT, _central_tendency_stat, _dispersion_stat, _normalize_method
+    method_ = _normalize_method(method)
+    if method_ in _DISPERSION_METHODS:
+        stat, arg0, arg1 = _dispersion_stat(method, rng, tprop)
+        return _STAT[stat], float(arg0), float(arg1), True
+    stat, arg0, arg1 = _central_tendency_stat("quantile" if method_ == "median" else method,
+                                              0.50 if method_ == "median" else quantile, tprop)
+    return _STAT[stat], float(arg0), float(arg1), False
+
+
+def _column_stat_launch(d_matrix, code: int, arg0: float, arg1: float, power: float, out):
+    torch = _torch()
+    lib = _lib.load()
+    m, n = d_matrix.shape
+    with torch.cuda.device(d_matrix.device):
+        st = lib.rocco_b200_column_stat_dev(
+            ctypes.c_void_p(d_matrix.data_ptr()), 1 if d_matrix.dtype == torch.float32 else 0, int(m), int(n), int(code),
+            float(arg0), float(arg1), float(power), ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(_stream_ptr(d_matrix.device)))
+    _lib.check(st, "column statistic")
+    return out
+
+
+def _column_matrix_problem(x) -> Optional[str]:
+    torch = _torch()
+    if not isinstance(x, torch.Tensor) or x.dim() != 2 or not x.is_cuda or not x.is_contiguous() \
+            or x.dtype not in (torch.float32, torch.float64):
+        return "the matrix must be a contiguous two-dimensional float32 or float64 CUDA tensor"
+    return None
+
+
+def column_stat_device(d_matrix, method="quantile", quantile=0.50, tprop=0.05, rng=(25, 75), power=1.0, out=None):
+    """``score_central_tendency_chrom`` / ``score_dispersion_chrom`` (by ``method``: quantile, median, tmean, mean, mad,
+    iqr, std, tstd) of a [samples, bins] float32 or float64 CUDA tensor; returns the [bins] float64 CUDA tensor (``out``
+    when given).  Inputs must be finite."""
+    torch = _torch()
+    problem = _column_matrix_problem(d_matrix)
+    if problem:
+        raise ValueError(f"`d_matrix`: {problem}")
+    code, arg0, arg1, _ = _column_stat_spec(method, quantile, tprop, rng)
+    m, n = d_matrix.shape
+    if m == 0:
+        raise ValueError("`d_matrix` must hold at least one sample")
+    if out is None:
+        out = torch.empty(n, dtype=torch.float64, device=d_matrix.device)
+    elif tuple(out.shape) != (n,) or out.dtype != torch.float64 or out.device != d_matrix.device or not out.is_contiguous():
+        raise ValueError("`out` must be a contiguous float64 tensor of one value per bin on the device of `d_matrix`")
+    if n == 0:
+        return out
+    return _column_stat_launch(d_matrix, code, arg0, arg1, power, out)
+
+
+def column_bin_ranges(n: int, ranks: int) -> list[tuple[int, int]]:
+    """The contiguous bin range [lo, hi) each rank owns in ``column_stat_sample_sharded``: equal widths rounded up to a
+    multiple of 16 bins, so only the last non-empty range is shorter; ranks past it own nothing."""
+    width = -(-(-(-int(n) // int(ranks))) // ALIGN) * ALIGN
+    return [(min(q * width, n), min((q + 1) * width, n)) for q in range(ranks)]
+
+
+def column_pack_ranges(d_rows, ranges):
+    """The send buffer of ``column_stat_sample_sharded``: the rows' [m, hi - lo] block of every bin range, row-major,
+    one after the other (one strided device copy per range)."""
+    torch = _torch()
+    m, n = d_rows.shape
+    send = torch.empty(m * n, dtype=d_rows.dtype, device=d_rows.device)
+    off = 0
+    for a, b in ranges:
+        if b > a and m > 0:
+            send[off: off + m * (b - a)].view(m, b - a).copy_(d_rows[:, a:b])
+        off += m * (b - a)
+    return send
+
+
+def column_stat_sample_sharded(d_rows_local, m_total: int, method="quantile", quantile=0.50, tprop=0.05, rng=(25, 75),
+                               power=1.0, group=None):
+    """``column_stat_device`` with the SAMPLES sharded over the ranks of ``group``: every rank passes its rows
+    ``[m_local, bins]`` (ranks in sample order, as ``score_loci_wls_sample_sharded`` takes them) and the same method and
+    arguments, and every rank returns the full [bins] float64 track.
+
+    The bins are split into one contiguous range per rank (``column_bin_ranges``).  One ``all_to_all_single`` sends each
+    rank's rows of every range to the range's owner, which then holds the complete columns ``[m_total, |range|]`` in global
+    sample order, runs the column kernel on them, and one ``all_gather_into_tensor`` hands the track to every rank.  Every
+    column is therefore reduced exactly as by the unsharded call, sums included: the result has the same bits.  With the
+    gloo backend the two collectives go through host memory."""
+    import torch.distributed as dist
+    torch = _torch()
+    x = d_rows_local
+    problem = _column_matrix_problem(x)
+    problem = f"`d_rows_local`: {problem}" if problem else None
+    try:
+        code, arg0, arg1, _ = _column_stat_spec(method, quantile, tprop, rng)
+    except ValueError as exc:
+        problem, code, arg0, arg1 = problem or str(exc), -1, 0.0, 0.0
+    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
+        if problem:
+            raise ValueError(problem)
+        if x.shape[0] != int(m_total):
+            raise ValueError(f"`m_total` ({m_total}) must equal the number of rows ({x.shape[0]}) on a single rank")
+        return column_stat_device(x, method, quantile, tprop, rng, power)
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    m, n = (int(x.shape[0]), int(x.shape[1])) if problem is None else (0, 0)
+    mine = {"problem": problem is not None, "m": m, "n": n, "dtype": str(x.dtype) if problem is None else "",
+            "agreed": (int(m_total), int(code), float(arg0), float(arg1), float(power))}
+    every = [None] * world
+    dist.all_gather_object(every, mine, group=group)
+    if problem is not None:
+        raise ValueError(problem)
+    if any(r["problem"] for r in every):
+        raise ValueError("column statistic: another rank rejected its arguments")
+    if any(r["agreed"] != mine["agreed"] for r in every):
+        raise ValueError("column statistic: every rank must pass the same m_total, method and arguments")
+    if any(r["n"] != n or r["dtype"] != mine["dtype"] for r in every):
+        raise ValueError(f"column statistic: every rank must hold the same bins and dtype, got "
+                         f"{[(r['n'], r['dtype']) for r in every]}")
+    rows = [r["m"] for r in every]
+    if sum(rows) != int(m_total) or int(m_total) == 0:
+        raise ValueError(f"column statistic: the ranks hold {sum(rows)} samples, `m_total` is {m_total}")
+    dev = x.device
+    ranges = column_bin_ranges(n, world)
+    width = max(b - a for a, b in ranges)
+    lo, hi = ranges[rank]
+    host = dist.get_backend(group) == "gloo"
+    # send: this rank's [m, |B_q|] block of every range q, back to back; receive: [m_total, |B_rank|] in sample order
+    send = column_pack_ranges(x, ranges)
+    recv = torch.empty(int(m_total) * (hi - lo), dtype=x.dtype, device="cpu" if host else dev)
+    dist.all_to_all_single(recv, send.cpu() if host else send, output_split_sizes=[r * (hi - lo) for r in rows],
+                           input_split_sizes=[m * (b - a) for a, b in ranges], group=group)
+    del send
+    # this rank's range, padded to the common width, and one status slot: a failure is raised on every rank
+    part = torch.zeros(width + 1, dtype=torch.float64, device=dev)
+    failure = None
+    if hi > lo:
+        try:
+            cols = recv.to(dev).view(int(m_total), hi - lo)
+            _column_stat_launch(cols, code, arg0, arg1, power, part[: hi - lo])
+            del cols
+        except (RuntimeError, ValueError) as exc:
+            failure = exc
+            part[width] = 1.0
+    del recv
+    full = torch.empty(world * (width + 1), dtype=torch.float64, device="cpu" if host else dev)
+    dist.all_gather_into_tensor(full, part.cpu() if host else part, group=group)
+    full = full.view(world, width + 1).to(dev)
+    if failure is not None:
+        raise failure
+    if bool((full[:, width] != 0).any()):
+        raise RuntimeError("column statistic: the kernel failed on another rank")
+    return full[:, :width].reshape(-1)[:n].contiguous()

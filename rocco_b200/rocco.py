@@ -167,26 +167,50 @@ def _column_stat(chrom_matrix: np.ndarray, stat: str, arg0: float = 0.0, arg1: f
     return out
 
 
-def score_central_tendency_chrom(chrom_matrix, method="quantile", quantile=0.50, tprop=0.05, power=1.0) -> np.ndarray:
-    r"""Return a column-wise location summary across samples (rocco.py:243-304)."""
-    chrom_matrix = np.asarray(chrom_matrix, dtype=float)
-    if chrom_matrix.ndim != 2:
-        raise ValueError("`chrom_matrix` must be a 2D array.")
-    method_ = str(method).strip().lower().replace("-", "").replace("_", "")
-    if chrom_matrix.shape[0] == 1:
-        return _column_stat(chrom_matrix, "mean", power=power)
+def _normalize_method(method) -> str:
+    return str(method).strip().lower().replace("-", "").replace("_", "")
+
+
+def _central_tendency_stat(method, quantile=0.50, tprop=0.05) -> tuple[str, float, float]:
+    """(statistic, arg0, arg1) of a ``score_central_tendency_chrom`` method with its arguments."""
+    method_ = _normalize_method(method)
     if method_ == "quantile":
         if not 0.0 <= quantile <= 1.0:
             logger.warning("`quantile` must be in [0, 1]. Using the median instead.")
             quantile = 0.50
         if quantile == 0.50:
-            return _column_stat(chrom_matrix, "median", power=power)
-        return _column_stat(chrom_matrix, "quantile", arg0=quantile, power=power)
+            return "median", 0.0, 0.0
+        return "quantile", quantile, 0.0
     if method_ == "tmean":
-        return _column_stat(chrom_matrix, "tmean", arg0=tprop, power=power)
+        return "tmean", tprop, 0.0
     if method_ == "mean":
-        return _column_stat(chrom_matrix, "mean", power=power)
+        return "mean", 0.0, 0.0
     raise ValueError(f"Central tendency method not recognized: {method}")
+
+
+def _dispersion_stat(method, rng=(25, 75), tprop=0.05) -> tuple[str, float, float]:
+    """(statistic, arg0, arg1) of a ``score_dispersion_chrom`` method with its arguments."""
+    method_ = _normalize_method(method)
+    if method_ == "mad":
+        return "mad", 0.0, 0.0
+    if method_ == "iqr":
+        return "iqr", rng[0], rng[1]
+    if method_ == "std":
+        return "std", 0.0, 0.0
+    if method_ == "tstd":
+        return "tstd", tprop, 0.0
+    raise ValueError(f"Dispersion method not recognized or could not execute: {method}")
+
+
+def score_central_tendency_chrom(chrom_matrix, method="quantile", quantile=0.50, tprop=0.05, power=1.0) -> np.ndarray:
+    r"""Return a column-wise location summary across samples (rocco.py:243-304)."""
+    chrom_matrix = np.asarray(chrom_matrix, dtype=float)
+    if chrom_matrix.ndim != 2:
+        raise ValueError("`chrom_matrix` must be a 2D array.")
+    if chrom_matrix.shape[0] == 1:
+        return _column_stat(chrom_matrix, "mean", power=power)
+    stat, arg0, arg1 = _central_tendency_stat(method, quantile, tprop)
+    return _column_stat(chrom_matrix, stat, arg0=arg0, arg1=arg1, power=power)
 
 
 def score_dispersion_chrom(chrom_matrix: np.ndarray, method: str = "mad", rng: Tuple[int, int] = (25, 75),
@@ -199,18 +223,10 @@ def score_dispersion_chrom(chrom_matrix: np.ndarray, method: str = "mad", rng: T
     chrom_matrix = np.asarray(chrom_matrix, dtype=float)
     if chrom_matrix.ndim != 2:
         raise ValueError("`chrom_matrix` must be a 2D array.")
-    method_ = str(method).strip().lower().replace("-", "").replace("_", "")
     if chrom_matrix.shape[0] == 1:
         return _column_stat(chrom_matrix, "mad", power=power)
-    if method_ == "mad":
-        return _column_stat(chrom_matrix, "mad", power=power)
-    if method_ == "iqr":
-        return _column_stat(chrom_matrix, "iqr", arg0=rng[0], arg1=rng[1], power=power)
-    if method_ == "std":
-        return _column_stat(chrom_matrix, "std", power=power)
-    if method_ == "tstd":
-        return _column_stat(chrom_matrix, "tstd", arg0=tprop, power=power)
-    raise ValueError(f"Dispersion method not recognized or could not execute: {method}")
+    stat, arg0, arg1 = _dispersion_stat(method, rng, tprop)
+    return _column_stat(chrom_matrix, stat, arg0=arg0, arg1=arg1, power=power)
 
 
 # ------------------------------------------------------------------------------------------------

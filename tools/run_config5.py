@@ -4,6 +4,7 @@ per chromosome on the rank that owns it (LPT).  Chromosomes are generated, score
 holds more than one chromosome's matrix + scratch (~35 GB).
 
     torchrun --nproc-per-node 8 tools/run_config5.py [--samples 1000] [--step-bp 20] [--chroms chr1,chr2] [--budget-null]
+                                                      [--central-tendency median]
 
 --budget-null replaces the sweep by the default CLI flow on the same layout: per chromosome the sharded scoring keeps each
 rank's centred rows, the wild-bootstrap budget null runs with the samples still sharded (2n column sums all-reduced per
@@ -23,6 +24,8 @@ ap.add_argument("--chroms", default="")
 ap.add_argument("--multipliers", type=int, default=256)
 ap.add_argument("--budget-null", action="store_true", help="budget null + EB budgets + solve instead of the sweep")
 ap.add_argument("--null-draws", type=int, default=25)
+ap.add_argument("--central-tendency", default="", help="score each chromosome by this column statistic of the sharded "
+                "samples (median, mean, tmean, quantile, ...) instead of the WLS score")
 args = ap.parse_args()
 rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 local = int(os.environ.get("LOCAL_RANK", 0))
@@ -110,6 +113,63 @@ def budget_null_run():
             "solve_ms_rank0": t_solve}))
 
 
+def central_tendency_run():
+    """bigWig-style scoring on the config-5 layout: per chromosome the column statistic of the sample-sharded matrix (one
+    all-to-all of the rows by bin range, the kernel on the owned range, one all-gather of the track), then the sweep on
+    the chromosome's owner.  The exchange and the kernel are timed apart: the exchange alone is rerun at the call's size."""
+    per = {}
+    for k, (c, n) in enumerate(zip(names, bins)):
+        x = chrom_matrix_torch(m_local, n, chrom_seed(c), dev, torch.float32, sample_stream=rank + 1)
+        if world > 1:
+            dist.barrier()
+        e = [ev() for _ in range(3)]
+        e[0].record()
+        scores = pipeline.column_stat_sample_sharded(x, m_local * world, args.central_tendency)
+        e[1].record()
+        if owner[k] == rank:
+            srt = torch.sort(scores).values
+            lo, hi = float(srt[int(0.50 * (n - 1))]), float(srt[int(0.999 * (n - 1))])
+            pipeline.sweep_multipliers(scores, HG_PARAMS[c][1], np.linspace(max(lo, 0.0), max(hi, lo), args.multipliers))
+        e[2].record()
+        torch.cuda.synchronize()
+        # the pieces: pack + all-to-all, then the kernel on the owned range of m_total rows
+        ranges = pipeline.column_bin_ranges(n, world)
+        lo_b, hi_b = ranges[rank]
+        t = [ev() for _ in range(4)]
+        t[0].record()
+        send = pipeline.column_pack_ranges(x, ranges)
+        recv = torch.empty(m_local * world * (hi_b - lo_b), dtype=x.dtype, device=dev)
+        t[1].record()
+        if world > 1:
+            dist.all_to_all_single(recv, send, [m_local * (hi_b - lo_b)] * world, [m_local * (b - a) for a, b in ranges])
+        t[2].record()
+        del send
+        if hi_b > lo_b:
+            pipeline.column_stat_device(recv.view(m_local * world, hi_b - lo_b), args.central_tendency)
+        t[3].record()
+        torch.cuda.synchronize()
+        per[c] = [n, e[0].elapsed_time(e[1]), e[1].elapsed_time(e[2]), t[0].elapsed_time(t[1]), t[1].elapsed_time(t[2]),
+                  t[2].elapsed_time(t[3])]
+        del x, recv, scores
+    keys = ("sharded_stat_ms", "sweep_ms(owner)", "pack_ms", "all_to_all_ms", "kernel_ms")
+    t = torch.tensor([per[c][1:] for c in names], dtype=torch.float64, device=dev)
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    if rank == 0:
+        mx = t.tolist()
+        tot = [sum(r[i] for r in mx) for i in range(len(keys))]
+        print(json.dumps({"config": f"hg38 @ {args.step_bp} bp x {m_local * world} samples f32, sample-sharded over {world} "
+                                    f"GPUs, column statistic {args.central_tendency!r} + {args.multipliers}-multiplier sweep",
+                          "gpu": torch.cuda.get_device_name(dev), "bins": sum(bins),
+                          "ms_max_over_ranks_total": dict(zip(keys, tot)),
+                          "chroms": {c: dict(zip(("bins",) + keys, [per[c][0]] + mx[i])) for i, c in enumerate(names)}}))
+
+
+if args.central_tendency:
+    central_tendency_run()
+    if world > 1:
+        dist.destroy_process_group()
+    sys.exit(0)
 if args.budget_null:
     budget_null_run()
     if world > 1:
