@@ -473,11 +473,13 @@ def score_params(lower_bound_z=1.0, prior_df=5.0, min_effect=None, precision_flo
     return prm
 
 
-def score_loci_wls_device(d_matrix, out_scores=None, params=None, details: bool = False):
+def score_loci_wls_device(d_matrix, out_scores=None, params=None, details: bool = False, centered_out=None):
     """score_loci_wls on a CUDA tensor [samples, bins] (float64 or float32, C-contiguous).
 
     Writes the scores into ``out_scores`` (a float64 CUDA tensor/view of length bins) or a new
-    tensor; with ``details`` also returns the per-locus detail tensors.  Nothing leaves the device."""
+    tensor; with ``details`` also returns the per-locus detail tensors.  ``centered_out`` (a contiguous float64 CUDA
+    tensor shaped like the matrix) receives the centred rows -- the input of ``budget_null_device`` -- without the
+    detail vectors being allocated.  Nothing leaves the device."""
     torch = _torch()
     lib = _lib.load()
     if d_matrix.dim() != 2 or not d_matrix.is_cuda or not d_matrix.is_contiguous():
@@ -488,6 +490,9 @@ def score_loci_wls_device(d_matrix, out_scores=None, params=None, details: bool 
     if m == 0 or n == 0:
         raise ValueError("`chrom_matrix` must be non-empty")
     dev = d_matrix.device
+    if centered_out is not None and (tuple(centered_out.shape) != (m, n) or centered_out.dtype != torch.float64
+                                     or centered_out.device != dev or not centered_out.is_contiguous()):
+        raise ValueError("`centered_out` must be a contiguous float64 tensor shaped like `d_matrix` on its device")
     if out_scores is None:
         out_scores = torch.empty(n, dtype=torch.float64, device=dev)
     out = _lib.ScoreOutputs()
@@ -497,7 +502,10 @@ def score_loci_wls_device(d_matrix, out_scores=None, params=None, details: bool 
         for k in ("mean", "raw_variance", "prior_variance", "moderated_variance", "standard_error"):
             extra[k] = torch.empty(n, dtype=torch.float64, device=dev)
             setattr(out, k, extra[k].data_ptr())
-        extra["centered_matrix"] = torch.empty((m, n), dtype=torch.float64, device=dev)
+        extra["centered_matrix"] = torch.empty((m, n), dtype=torch.float64, device=dev) if centered_out is None else centered_out
+    elif centered_out is not None:
+        extra["centered_matrix"] = centered_out
+    if "centered_matrix" in extra:
         out.centered_matrix = extra["centered_matrix"].data_ptr()
     prm = params if params is not None else score_params()
     with torch.cuda.device(dev):
@@ -541,8 +549,209 @@ def _score_streams(dev, count: int):
     return _SCORE_STREAMS[key]
 
 
+# ------------------------------------------------------------------ ROCCO's default budgets and gamma (rocco.py:1023-1143)
+# The reference's CLI without --gamma: per chromosome, score, run the wild-bootstrap budget null on the centred rows, then
+# feed every chromosome's (effective_count, effective_total_count) to the empirical-Bayes budgets and set the automatic
+# gamma from the null's autocorrelation time and the median positive score.
+DEFAULT_FLOW_ARGS = {"budget": None, "scale_chrom_budgets": 1.0, "budget_posterior_quantile": 0.01, "num_null_draws": 25,
+                     "random_seed": 0}
+
+
+def _default_flow_args(default_args) -> dict:
+    """The reference's CLI keys with their defaults, overridden by ``default_args``."""
+    args = dict(DEFAULT_FLOW_ARGS)
+    unknown = sorted(set(default_args or {}) - set(args))
+    if unknown:
+        raise ValueError(f"unknown `default_args` keys {unknown}; known: {sorted(args)}")
+    args.update(default_args or {})
+    return args
+
+
+def _chromosome_name_problem(every) -> Optional[str]:
+    """The first disagreement in the gathered ``{"names", "genome", "agreed"}`` of every rank, or None."""
+    genome = every[0]["genome"]
+    if any(r["genome"] != genome for r in every):
+        return "default flow: every rank must pass the same `genome_names`"
+    if any(r["agreed"] != every[0]["agreed"] for r in every):
+        return "default flow: every rank must pass the same default arguments and the same budget and gamma modes"
+    if len(set(genome)) != len(genome):
+        return f"default flow: `genome_names` lists {sorted({c for c in genome if genome.count(c) > 1})} more than once"
+    known = set(genome)
+    for rank, r in enumerate(every):
+        unknown = [c for c in r["names"] if c not in known]
+        if unknown:
+            return f"default flow: rank {rank} holds chromosomes missing from `genome_names`: {unknown}"
+    held = [c for r in every for c in r["names"]]
+    twice = sorted({c for c in held if held.count(c) > 1})
+    if twice:
+        return f"default flow: chromosomes held more than once: {twice}"
+    unowned = [c for c in genome if c not in set(held)]
+    if unowned:
+        return f"default flow: no rank holds {unowned}"
+    if not genome:
+        return "default flow: the genome has no chromosome"
+    return None
+
+
+def agree_chromosome_names(chrom_names, genome_names, group=None, problem=None, agreed=None) -> int:
+    """Check, on every rank of ``group`` at once, that the chromosomes the ranks hold are the genome: every name of
+    ``chrom_names`` is in ``genome_names``, no name is held twice, no name of the genome is held by nobody, and every rank
+    passed the same ``genome_names`` and ``agreed`` value.  ``problem`` is this rank's own argument error (or None).  One
+    ``all_gather_object``; every rank raises the same ``ValueError``, except that a rank with a ``problem`` raises its own.
+    Returns the number of chromosome slots of ``gather_budget_estimates``: the most any rank holds."""
+    mine = {"names": [str(c) for c in chrom_names], "genome": None if genome_names is None else [str(c) for c in genome_names],
+            "problem": problem, "agreed": agreed}
+    if _group_size(group) <= 1:
+        every = [mine]
+    else:
+        import torch.distributed as dist
+        every = [None] * dist.get_world_size(group)
+        dist.all_gather_object(every, mine, group=group)
+    if problem is not None:
+        raise ValueError(problem)
+    bad = next((r["problem"] for r in every if r["problem"] is not None), None)
+    if bad is not None:
+        raise ValueError(f"default flow: another rank rejected its arguments: {bad}")
+    if any(r["genome"] is None for r in every):
+        raise ValueError("default flow: `genome_names` is required when the chromosomes are spread over several ranks")
+    msg = _chromosome_name_problem(every)
+    if msg:
+        raise ValueError(msg)
+    return max(len(r["names"]) for r in every)
+
+
+def gather_budget_estimates(chrom_names, genome_names, rows, slots: int, group=None, failure=None, device=None) -> dict:
+    """The empirical-Bayes cache of the whole genome, in ``genome_names`` order, on every rank of ``group``.
+
+    ``rows`` holds one ``(effective_count, effective_total_count, status)`` per chromosome of ``chrom_names`` (status 0:
+    estimated; anything else: failed or not run); ``slots`` is what ``agree_chromosome_names`` returned.  One
+    ``all_gather`` of ``slots + 1`` float64 rows ``[genome index, effective_count, effective_total_count, status]`` per
+    rank (padding rows carry index -1; the last row is the rank's own status, set when it passes ``failure``, so that a
+    rank without chromosomes can report one), on the CPU for gloo and on ``device`` (default: the current CUDA device)
+    otherwise.  A status on any rank raises ``ValueError`` on every rank; the rank passing ``failure`` (its own message)
+    raises that.
+    Returns ``{name: {"budget_count_hat": effective_count, "total_count": effective_total_count}}`` in genome order, the
+    cache ``rocco._resolve_budgets`` takes: the order is data, as the optimiser's path depends on the summation order."""
+    torch = _torch()
+    genome = [str(c) for c in genome_names]
+    index = {c: g for g, c in enumerate(genome)}
+    if len(rows) != len(chrom_names) or len(chrom_names) > int(slots):
+        raise ValueError("`rows` must hold one entry per chromosome, and at most `slots`")
+    table = np.zeros((int(slots) + 1, 4), dtype=np.float64)
+    table[:, 0] = -1.0
+    for k, (c, (count, total, status)) in enumerate(zip(chrom_names, rows)):
+        table[k] = (index[str(c)], float(count), float(total), float(status))
+    table[int(slots), 3] = 0.0 if failure is None else 1.0
+    world = _group_size(group)
+    if world <= 1:
+        every = table
+    else:
+        import torch.distributed as dist
+        host = dist.get_backend(group) == "gloo"
+        dev = torch.device("cpu") if host else (device or torch.device("cuda", torch.cuda.current_device()))
+        mine = torch.from_numpy(table).to(dev)
+        parts = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(parts, mine, group=group)
+        every = torch.cat(parts).cpu().numpy()
+    if failure is not None:
+        raise ValueError(failure)
+    failed = every[(every[:, 0] >= 0) & (every[:, 3] != 0)]
+    if failed.shape[0] or np.any(every[every[:, 0] < 0, 3] != 0):
+        where = [genome[int(g)] for g in failed[:, 0]]
+        raise ValueError("default flow: another rank failed" + (f" on {where}" if where else ""))
+    by_index = {int(r[0]): r for r in every if r[0] >= 0}
+    if sorted(by_index) != list(range(len(genome))):
+        raise ValueError("default flow: the ranks' chromosomes do not cover `genome_names` exactly once")
+    return {c: {"budget_count_hat": float(by_index[g][1]), "total_count": float(by_index[g][2])} for g, c in enumerate(genome)}
+
+
+def _run_shard_defaults(d_matrices, budgets, gammas, params, levels_per_round, want_runs, score_streams, group,
+                        chrom_names, genome_names, default_args, mark):
+    """``run_shard`` with ROCCO's default budgets (``budgets`` None) and/or automatic gamma (``gammas`` None)."""
+    from .inference import _resolve_local_baseline_window
+    from .rocco import _resolve_budgets, _resolve_chrom_gamma
+    torch = _torch()
+    mark = mark or (lambda label: None)
+    nchrom = len(d_matrices)
+    # this rank's own argument errors: the name agreement reports them to every rank
+    problem = None
+    try:
+        args = _default_flow_args(default_args)
+    except ValueError as exc:
+        problem, args = str(exc), dict(DEFAULT_FLOW_ARGS)
+    names = [] if chrom_names is None else [str(c) for c in chrom_names]
+    if problem is None and score_streams > 1:
+        problem = "the default flow scores one chromosome at a time: `score_streams` must be 1"
+    if problem is None and (chrom_names is None or len(names) != nchrom):
+        problem = "`chrom_names` must name each matrix of `d_matrices`, in the same order"
+    if problem is None and any(v is not None and len(v) != nchrom for v in (budgets, gammas)):
+        problem = "`budgets` and `gammas` must have one entry per matrix of `d_matrices`"
+    if problem is None and any(not isinstance(x, torch.Tensor) or x.dim() != 2 or not x.is_cuda for x in d_matrices):
+        problem = "every matrix of `d_matrices` must be a two-dimensional CUDA tensor"
+    if genome_names is None and _group_size(group) <= 1:
+        genome_names = names
+    agreed = (tuple((k, args[k]) for k in sorted(args)), budgets is None, gammas is None)
+    slots = agree_chromosome_names(names, genome_names, group=group, problem=problem, agreed=agreed)
+
+    lengths = [int(x.shape[1]) for x in d_matrices]
+    offsets, total = layout_offsets(lengths)
+    # from here until the gather, every error of this rank goes into its status rows, so no rank is left in a collective
+    nulls, rows, failure, dev, d_scores = [], [], None, None, None
+    try:
+        dev = d_matrices[0].device if nchrom else torch.device("cuda", torch.cuda.current_device())
+        d_scores = torch.zeros(total, dtype=torch.float64, device=dev)
+        prm = params if params is not None else score_params()
+    except (ValueError, RuntimeError) as exc:
+        failure = f"default flow: setting up the scores failed: {exc}"
+    # one chromosome at a time: its centred rows live only until its null has run
+    for name, x, off, n in zip(names, d_matrices, offsets, lengths):
+        if failure is not None:
+            break
+        centered = None
+        try:
+            mark(f"score:{name}")
+            centered = torch.empty(tuple(x.shape), dtype=torch.float64, device=dev)
+            scores = score_loci_wls_device(x, out_scores=d_scores[off:off + n], params=prm, centered_out=centered)
+            window = _resolve_local_baseline_window(n, prm.baseline_window if prm.baseline_window > 0 else 101)
+            mark(f"null:{name}")
+            _, det = budget_null_device(centered, scores, params=prm, dependence_lag_hint=window,
+                                        num_null_draws=args["num_null_draws"], random_seed=args["random_seed"])
+        except (ValueError, RuntimeError) as exc:
+            failure = f"default flow: {name}: {exc}"
+            break
+        finally:
+            del centered
+        nulls.append(det)
+        rows.append((det["effective_count"], det["effective_total_count"], 0))
+    rows += [(0.0, 0.0, 1)] * (nchrom - len(rows))
+    mark("agree")
+    cache = gather_budget_estimates(names, genome_names, rows, slots, group=group, failure=failure, device=dev)
+    budget_meta = None
+    if budgets is None:
+        eb, budget_meta = _resolve_budgets(cache, args)
+        budgets = [eb[c] for c in names]
+    pairs = [_resolve_chrom_gamma(c, {"gamma": None if gammas is None else gammas[k]}, None, det)
+             for k, (c, det) in enumerate(zip(names, nulls))]
+    gammas = [g for g, _ in pairs]
+    mark("solve")
+    if nchrom:
+        d_masks, results = solve_packed(d_scores, offsets, lengths, budgets, gammas, levels_per_round=levels_per_round)
+    else:
+        d_masks, results = torch.zeros(total, dtype=torch.uint8, device=dev), []
+    mark("runs")
+    runs = None
+    if want_runs:
+        runs = masks_to_runs(d_masks, offsets, lengths) if nchrom else \
+            (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64))
+    mark("end")
+    return {"d_scores": d_scores, "d_masks": d_masks, "offsets": offsets, "lengths": lengths, "results": results,
+            "runs": runs, "budgets": list(budgets), "gammas": gammas,
+            "defaults": {"null": nulls, "gamma_meta": [m for _, m in pairs], "budget_meta": budget_meta}}
+
+
 def run_shard(d_matrices, budgets, gammas, params=None, levels_per_round: int = 0, want_runs: bool = True,
-              score_streams: int = 1, genome_budget=None, group=None):
+              score_streams: int = 1, genome_budget=None, group=None, chrom_names=None, genome_names=None,
+              default_args=None, mark=None):
     """The hot path for one rank's chromosomes, device-resident end to end:
     score every chromosome -> one batched budget search + solve -> one batched mask->runs pass.
 
@@ -550,9 +759,31 @@ def run_shard(d_matrices, budgets, gammas, params=None, levels_per_round: int = 
     (measured on B200: no gain at 100 samples -- the streaming kernels already fill the device -- so the default is 1).
     With `genome_budget` (and `budgets` None) the search is the genome-wide one of `solve_genome_packed`: one multiplier
     for the chromosomes of every rank of `group`, and the result gains "genome".
-    Returns dict(d_scores, d_masks, offsets, lengths, results, runs)."""
+    Returns dict(d_scores, d_masks, offsets, lengths, results, runs).
+
+    ROCCO's defaults (its CLI without --gamma, rocco.py:1023-1143): `budgets` None (without `genome_budget`) gives the
+    empirical-Bayes budgets, `gammas` None the automatic gamma; either needs the wild-bootstrap budget null of every
+    chromosome.  Each chromosome is scored with its centred rows kept, its null runs on them (the Whittaker window is the
+    dependence hint), and the rows are freed before the next chromosome; `score_streams` must be 1.  `chrom_names` names
+    the matrices; `genome_names` lists every chromosome of every rank of `group` in genome order (ROCCO's chromosome
+    order; default with one rank: `chrom_names`), the order in which the budgets are fitted.  `default_args` overrides
+    the CLI keys of `DEFAULT_FLOW_ARGS`.  The ranks first agree on the names (`agree_chromosome_names`), then exchange
+    their estimates in one all-gather (`gather_budget_estimates`); a failure on any rank raises ValueError on all of
+    them.  The result gains "budgets" and "gammas" (lists in `d_matrices` order) and "defaults": the null's details
+    ("null"), the gamma meta ("gamma_meta", None for a fixed gamma), both per chromosome, and the EB "budget_meta" (None
+    for explicit budgets).  A rank without chromosomes passes `d_matrices=[]` and takes part all the same.
+    `mark(label)`, when given, is called on the host as each phase begins ("score:<name>", "null:<name>", "agree",
+    "solve", "runs") and at the "end": a hook for timing with CUDA events."""
     if genome_budget is not None and budgets is not None:
         raise ValueError("pass either per-chromosome `budgets` or one `genome_budget`, not both")
+    if genome_budget is not None and (gammas is None or default_args is not None):
+        raise ValueError("`genome_budget` takes explicit `gammas`; it does not combine with the default budgets or gamma")
+    if gammas is None or (budgets is None and genome_budget is None):
+        return _run_shard_defaults(d_matrices, budgets, gammas, params, levels_per_round, want_runs, score_streams, group,
+                                   chrom_names, genome_names, default_args, mark)
+    if any(v is not None for v in (chrom_names, genome_names, default_args, mark)):
+        raise ValueError("`chrom_names`, `genome_names`, `default_args` and `mark` belong to the default flow "
+                         "(`budgets` or `gammas` None); with explicit budgets and gammas they would be ignored")
     torch = _torch()
     lengths = [int(x.shape[1]) for x in d_matrices]
     offsets, total = layout_offsets(lengths)
@@ -927,6 +1158,104 @@ def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=
 
     return _budget_null_sharded(d_centered_local, m_total, offset, reduce_fn, d_observed_scores, params, dependence_lag_hint,
                                 num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations)
+
+
+def _score_sample_sharded_agreed(x, m_total: int, prm, group, name: str):
+    """``score_loci_wls_sample_sharded(..., keep_centered=True)`` with the ranks agreeing on success first: one
+    all-reduce(MAX) of ``[failed, bins, -bins]`` comes before the accumulator all-reduce, so a rank whose per-sample stages
+    fail (non-finite rows, allocation) or whose bins differ makes every rank raise ``ValueError`` instead of leaving the
+    others waiting in the accumulator all-reduce.  Same calls and bits as ``score_loci_wls_sample_sharded`` otherwise."""
+    from .inference import _resolve_local_baseline_window
+    torch = _torch()
+    failure, acc, centered, n = None, None, None, -1
+    try:
+        n = int(x.shape[1])
+        centered = torch.empty(tuple(x.shape), dtype=torch.float64, device=x.device)
+        acc = score_partial_device(x, prm, centered_out=centered)
+    except (ValueError, RuntimeError) as exc:
+        failure = f"default flow: {name}: {exc}"
+    if _group_size(group) > 1:
+        import torch.distributed as dist
+        dev = x.device if isinstance(x, torch.Tensor) and x.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        flag = torch.tensor([0.0 if failure is None else 1.0, float(n), -float(n)], dtype=torch.float64,
+                            device="cpu" if dist.get_backend(group) == "gloo" else dev)
+        dist.all_reduce(flag, op=dist.ReduceOp.MAX, group=group)
+        failed, n_max, n_min = flag[0].item(), flag[1].item(), -flag[2].item()
+        if failure is None and failed:
+            failure = f"default flow: {name} failed on another rank"
+        elif failure is None and n_max != n_min:
+            failure = f"default flow: {name}: every rank must hold the same bins, got {int(n_min)} to {int(n_max)}"
+        if failure is None:
+            dist.all_reduce(acc, group=group)
+    if failure is not None:
+        raise ValueError(failure)
+    scores = score_finalize_device(acc, m_total, prm)
+    return scores, centered, _resolve_local_baseline_window(n, prm.baseline_window if prm.baseline_window > 0 else 101)
+
+
+def run_sample_sharded_defaults(chroms, m_total: int, params=None, default_args=None, group=None, levels_per_round: int = 0,
+                                mark=None):
+    """ROCCO's default flow (EB budgets, automatic gamma) with the SAMPLES sharded over the ranks of ``group`` (config 5).
+
+    ``chroms`` yields ``(name, d_rows_local)`` in genome order, the same chromosomes on every rank, each rank's rows of
+    the chromosome (ranks in sample order); it is consumed one chromosome at a time, so the caller can generate or load
+    each just in time.  Per chromosome: the scoring of ``score_loci_wls_sample_sharded(..., keep_centered=True)``, then
+    ``budget_null_sample_sharded`` on the centred rows with the Whittaker window as the dependence hint; the rows are
+    dropped before the next chromosome is drawn.  A failure on one rank raises ``ValueError`` on every rank: the scoring
+    agrees on success before its all-reduce (``_score_sample_sharded_agreed``) and the null carries its own status.  Every rank then holds every chromosome's details, so the EB budgets and
+    the gammas are computed on every rank from the same doubles, with no further exchange.  Each chromosome is solved on
+    its ``lpt_partition`` owner; the scores are kept on every rank until then (8 B per bin).  ``default_args``: as for
+    ``run_shard``.  ``mark(label)`` is called on the host at "score:<name>", "null:<name>", "done:<name>", "solve" and
+    "end".  Returns dict(names, lengths, budgets, gammas (dicts by name), defaults (null details and gamma meta by name,
+    budget_meta), my_names (this rank's chromosomes, genome order), d_masks, offsets, results, runs): ``my_names`` and
+    ``runs`` go straight to ``distributed.write_genome_bed``."""
+    from .rocco import _resolve_budgets, _resolve_chrom_gamma
+    args = _default_flow_args(default_args)
+    mark = mark or (lambda label: None)
+    prm = params if params is not None else score_params()
+    names, lengths, scores, nulls = [], [], [], {}
+    for name, x in chroms:
+        name = str(name)
+        if name in nulls:
+            raise ValueError(f"default flow: {name} comes twice")
+        mark(f"score:{name}")
+        s, centered, window = _score_sample_sharded_agreed(x, m_total, prm, group, name)
+        del x
+        mark(f"null:{name}")
+        _, det = budget_null_sample_sharded(centered, s, params=prm, group=group, dependence_lag_hint=window,
+                                            num_null_draws=args["num_null_draws"], random_seed=args["random_seed"])
+        del centered
+        mark(f"done:{name}")
+        names.append(name)
+        lengths.append(int(s.shape[0]))
+        scores.append(s)
+        nulls[name] = det
+    if not names:
+        raise ValueError("default flow: the genome has no chromosome")
+    cache = {c: {"budget_count_hat": nulls[c]["effective_count"], "total_count": nulls[c]["effective_total_count"]}
+             for c in names}
+    budgets, budget_meta = _resolve_budgets(cache, args)
+    pairs = {c: _resolve_chrom_gamma(c, {"gamma": None}, None, nulls[c]) for c in names}
+    gammas = {c: g for c, (g, _) in pairs.items()}
+    mark("solve")
+    import torch.distributed as dist
+    world = _group_size(group)
+    mine = lpt_partition(lengths, world)[dist.get_rank(group) if world > 1 else 0]
+    mine_scores = [scores[k] for k in mine]
+    del scores
+    my_names = [names[k] for k in mine]
+    out = {"names": names, "lengths": lengths, "budgets": budgets, "gammas": gammas, "my_names": my_names,
+           "defaults": {"null": nulls, "gamma_meta": {c: m for c, (_, m) in pairs.items()}, "budget_meta": budget_meta},
+           "d_masks": None, "offsets": [], "results": [],
+           "runs": (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64))}
+    if my_names:
+        d_scores, offsets, my_lengths = pack_scores(mine_scores)
+        del mine_scores
+        d_masks, results = solve_packed(d_scores, offsets, my_lengths, [budgets[c] for c in my_names],
+                                        [gammas[c] for c in my_names], levels_per_round=levels_per_round)
+        out.update(d_masks=d_masks, offsets=offsets, results=results, runs=masks_to_runs(d_masks, offsets, my_lengths))
+    mark("end")
+    return out
 
 
 # ------------------------------------------------------------------ column statistics on device tensors

@@ -9,7 +9,7 @@ holds more than one chromosome's matrix + scratch (~35 GB).
 --budget-null replaces the sweep by the default CLI flow on the same layout: per chromosome the sharded scoring keeps each
 rank's centred rows, the wild-bootstrap budget null runs with the samples still sharded (2n column sums all-reduced per
 scoring pass), the fractions go through the empirical-Bayes budgets and the automatic gamma (host, identical on every
-rank), and the owner rank solves each chromosome at its budget.
+rank), and the owner rank solves each chromosome at its budget: pipeline.run_sample_sharded_defaults.
 """
 import argparse, json, math, os, sys, time
 import numpy as np, torch, torch.distributed as dist
@@ -45,53 +45,50 @@ ev = lambda: torch.cuda.Event(enable_timing=True)
 
 
 def budget_null_run():
-    from rocco_b200.rocco import _resolve_budgets, _resolve_chrom_gamma
-    per_chrom, owned = {}, {}
-    for k, (c, n) in enumerate(zip(names, bins)):
-        x = chrom_matrix_torch(m_local, n, chrom_seed(c), dev, torch.float32, sample_stream=rank + 1)
-        if world > 1:
-            dist.barrier()
-        e = [ev() for _ in range(3)]
-        e[0].record()
-        scores, cent, window = pipeline.score_loci_wls_sample_sharded(x, m_local * world, prm, keep_centered=True)
-        del x
-        e[1].record()
-        frac, det = pipeline.budget_null_sample_sharded(cent, scores, params=prm, dependence_lag_hint=window,
-                                                        num_null_draws=args.null_draws)
-        e[2].record()
-        del cent
-        # the collective alone, at the estimator's size (2n sums + 4 status slots), timed after the call
-        buf = torch.zeros(2 * n + 4, dtype=torch.float64, device=dev)
-        r = [ev() for _ in range(2)]
-        if world > 1:
-            dist.all_reduce(buf)
-        r[0].record()
-        for _ in range(5):
+    """pipeline.run_sample_sharded_defaults on the config-5 layout, chromosomes generated just in time; its mark hook
+    records the per-chromosome events and, after each null, times the collective alone at the estimator's size."""
+    per_chrom, events = {}, {}
+
+    def chroms():
+        for c, n in zip(names, bins):
+            x = chrom_matrix_torch(m_local, n, chrom_seed(c), dev, torch.float32, sample_stream=rank + 1)
+            if world > 1:
+                dist.barrier()
+            yield c, x
+            del x
+
+    def mark(label):
+        e = ev()
+        e.record()
+        events[label] = e
+        if label.startswith("done:"):
+            # the collective alone, at the estimator's size (2n sums + 4 status slots), timed after the call
+            n = bins[names.index(label[5:])]
+            buf = torch.zeros(2 * n + 4, dtype=torch.float64, device=dev)
+            r = [ev() for _ in range(2)]
             if world > 1:
                 dist.all_reduce(buf)
-        r[1].record()
-        torch.cuda.synchronize()
+            r[0].record()
+            for _ in range(5):
+                if world > 1:
+                    dist.all_reduce(buf)
+            r[1].record()
+            torch.cuda.synchronize()
+            per_chrom[label[5:]] = {"all_reduce_ms": r[0].elapsed_time(r[1]) / 5}
+
+    out = pipeline.run_sample_sharded_defaults(chroms(), m_local * world, prm, default_args={"num_null_draws": args.null_draws},
+                                              mark=mark)
+    torch.cuda.synchronize()
+    for c, n in zip(names, bins):
+        det = out["defaults"]["null"][c]
         passes = 2 + int(det["num_null_draws"])
-        per_chrom[c] = {"bins": n, "score_ms": e[0].elapsed_time(e[1]), "budget_null_ms": e[1].elapsed_time(e[2]),
-                        "passes": passes, "ms_per_pass": e[1].elapsed_time(e[2]) / passes,
-                        "all_reduce_ms": r[0].elapsed_time(r[1]) / 5, "nonnull_fraction": frac, "details": det}
-        if owner[k] == rank:
-            owned[c] = scores
-        del scores
-    cache = {c: {"budget_count_hat": v["details"]["effective_count"], "total_count": v["details"]["effective_total_count"]}
-             for c, v in per_chrom.items()}
-    budgets, _ = _resolve_budgets(cache, {"budget": None, "scale_chrom_budgets": 1.0, "budget_posterior_quantile": 0.01})
-    gammas = {c: _resolve_chrom_gamma(c, {"gamma": None}, None, v["details"])[0] for c, v in per_chrom.items()}
-    t_solve = 0.0
-    solved = {}
-    if owned:
-        s0, s1 = ev(), ev()
-        s0.record()
-        res = pipeline.solve_chromosomes(list(owned.values()), [budgets[c] for c in owned], [gammas[c] for c in owned])
-        s1.record()
-        torch.cuda.synchronize()
-        t_solve = s0.elapsed_time(s1)
-        solved = {c: int(r["selected_count"]) for c, r in zip(owned, res)}
+        null_ms = events[f"null:{c}"].elapsed_time(events[f"done:{c}"])
+        per_chrom[c].update({"bins": n, "score_ms": events[f"score:{c}"].elapsed_time(events[f"null:{c}"]),
+                             "budget_null_ms": null_ms, "passes": passes, "ms_per_pass": null_ms / passes,
+                             "nonnull_fraction": det["nonnull_fraction"]})
+    t_solve = events["solve"].elapsed_time(events["end"])
+    solved = {c: int(r["selected_count"]) for c, r in zip(out["my_names"], out["results"])}
+    budgets, gammas = out["budgets"], out["gammas"]
     keys = ("score_ms", "budget_null_ms", "ms_per_pass", "all_reduce_ms")
     t = torch.tensor([[per_chrom[c][q] for q in keys] + [per_chrom[c]["passes"]] for c in names], dtype=torch.float64, device=dev)
     if world > 1:
