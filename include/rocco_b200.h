@@ -316,20 +316,25 @@ int rocco_b200_score_centered_wls_dev(const double *d_centered, size_t m, size_t
  * Dependent-wild-bootstrap estimate of a chromosome's enriched fraction (inference.py:988-1148 on top of 446-985) and
  * the inputs of the automatic gamma (rocco.py:751-789), device-resident: fit the null residual template, score it,
  * take the null centre/scale, then re-score  template x W  for up to num_null_draws Bartlett-smoothed Gaussian
- * multiplier fields W with the reference's adaptive stop.  Innovations: Philox4x32-10 keyed by random_seed (the
- * reference uses NumPy PCG64 streams: statistical parity) unless d_innovations supplies them (bit-level replay). */
+ * multiplier fields W with the reference's adaptive stop.  Innovations: Philox4x32-10 keyed by random_seed (parity with
+ * the reference is statistical), or with random_streams = 1 the reference's own NumPy PCG64 streams (same normals as the
+ * reference; see rocco_b200_numpy_normals_dev), unless d_innovations supplies them (bit-level replay). */
 typedef struct rocco_b200_budget_params {
     rocco_b200_score_params score;  /* lower_bound_z, prior_df, min_effect, precision_floor_ratio as for the scores  */
     int dependence_lag_hint;        /* <= 0: none (bandwidth round(n^(1/3)), ESS scale 101); rocco.py:1035 passes >= 25 */
     int num_null_draws;             /* 25                                                                        */
     int min_null_draws;             /* <= 0: 8 (inference.py:795-797)                                            */
     int sample_offset;              /* global index of the first local sample (sample sharding; 0 = unsharded): row r
-                                       draws the Philox stream of sample sample_offset + r                          */
+                                       draws the stream (Philox or NumPy) of sample sample_offset + r               */
     double stability_abs_tol;       /* 5e-3                                                                      */
     double stability_rel_tol;       /* 5e-2                                                                      */
     unsigned long long random_seed;
     const double *d_innovations;    /* optional DEVICE buffer [num_null_draws][m][n + 2*bandwidth] of iid N(0,1)
                                        (sharded: [num_null_draws][m_local][n + 2*bandwidth], this rank's rows)       */
+    int random_streams;             /* innovations when d_innovations is NULL: 0 = Philox4x32-10 (default), 1 = NumPy's
+                                       default_rng(random_seed + 104729 (draw + 1)).standard_normal, generated on the
+                                       device, global sample i taking normals [i L, (i + 1) L), L = n + 2*bandwidth:
+                                       the reference's own streams                                                   */
 } rocco_b200_budget_params;
 
 typedef struct rocco_b200_budget_result {
@@ -384,6 +389,19 @@ int rocco_b200_wild_multiply_dev(const double *d_template, size_t m, size_t n, i
 int rocco_budget_nonnull_fraction_f64(const double *centered, size_t m, size_t n, const double *observed_scores,
                                       const rocco_b200_budget_params *params, const double *innovations,
                                       rocco_b200_budget_result *result);
+/* NumPy streams (numpy_streams.cu).  A seed is the 128-bit integer seed_hi * 2^64 + seed_lo of default_rng(seed).
+ * rocco_b200_numpy_normals_dev writes normals [skip, skip + count) of default_rng(seed).standard_normal() to d_out
+ * (device, count >= 1), generated on the device by a parallel parse of the ziggurat's rejection stream; words_consumed
+ * (host, optional) receives how many 64-bit PCG64 outputs NumPy has drawn once it has returned normal skip + count - 1.
+ * Fast-path and wedge normals are NumPy's bits; tail normals (0.03 %) go through log1p and may differ from a host's
+ * NumPy in the last bit. */
+int rocco_b200_numpy_normals_dev(unsigned long long seed_lo, unsigned long long seed_hi, unsigned long long skip,
+                                 unsigned long long count, double *d_out, unsigned long long *words_consumed, void *cuda_stream);
+/* Host: the PCG64 state default_rng(seed) starts from: out = {state low 64, state high 64, inc low 64, inc high 64}. */
+int rocco_b200_numpy_seed_state(unsigned long long seed_lo, unsigned long long seed_hi, unsigned long long out[4]);
+/* Words per chunk of the parallel parse (default 64, clamped to 1 .. 256; <= 0: the default); results do not change.
+ * Returns the previous value. */
+int rocco_b200_numpy_streams_set_chunk_words(int words);
 /* _estimate_effective_sample_size (inference.py:446-501) of a host series. */
 int rocco_effective_sample_size_f64(const double *values, size_t n, int max_lag, double *n_eff, double *tau_int,
                                     int *lags_used);

@@ -69,7 +69,7 @@ class BudgetParams(Structure):
     _fields_ = [
         ("score", ScoreParams), ("dependence_lag_hint", c_int), ("num_null_draws", c_int), ("min_null_draws", c_int),
         ("sample_offset", c_int), ("stability_abs_tol", c_double), ("stability_rel_tol", c_double),
-        ("random_seed", c_ulonglong), ("d_innovations", c_void_p),
+        ("random_seed", c_ulonglong), ("d_innovations", c_void_p), ("random_streams", c_int),
     ]
 
 
@@ -140,6 +140,10 @@ def _declare(lib):
                                                       POINTER(BudgetResult)]),
         "rocco_b200_wild_multiply_dev": (c_int, [c_void_p, c_size_t, c_size_t, c_int, c_ulonglong, ctypes.c_uint, c_void_p, c_void_p,
                                                  c_void_p]),
+        "rocco_b200_numpy_normals_dev": (c_int, [c_ulonglong, c_ulonglong, c_ulonglong, c_ulonglong, c_void_p,
+                                                 POINTER(c_ulonglong), c_void_p]),
+        "rocco_b200_numpy_seed_state": (c_int, [c_ulonglong, c_ulonglong, POINTER(c_ulonglong)]),
+        "rocco_b200_numpy_streams_set_chunk_words": (c_int, [c_int]),
         "rocco_effective_sample_size_f64": (c_int, [c_void_p, c_size_t, c_int, dp, dp, ip]),
         "rocco_positive_score_median_f64": (c_int, [c_void_p, c_size_t, dp, llp]),
         "rocco_b200_pull_pinned": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),

@@ -5,11 +5,13 @@
 // adaptive stop), 988-1148 (observed-vs-null summary) and rocco.py:751-789 (median of the positive scores for the
 // automatic gamma).  Every draw re-runs the centred-WLS scoring chain of wls.cu / trend.cu on  template x weights.
 //
-// Random streams: the reference draws NumPy PCG64 normals (one generator per draw, samples in order).  Here the
-// innovations are counter-based -- Philox4x32-10 keyed by the seed, counter = (pair index, sample, draw) -> Box-Muller
-// in double -- so a draw is reproducible and independent of tiling, but the streams differ from NumPy's: parity with
-// the reference is statistical.  For bit-level checks the caller may pass the innovations themselves
-// (`d_innovations`), which is how tests replay the reference's own streams through these kernels.
+// Random streams: the reference draws NumPy PCG64 normals (one generator per draw, samples in order).  By default the
+// innovations here are counter-based -- Philox4x32-10 keyed by the seed, counter = (pair index, sample, draw) ->
+// Box-Muller in double -- so a draw is reproducible and independent of tiling, but the streams differ from NumPy's:
+// parity with the reference is statistical.  With random_streams = 1 the reference's own streams are generated on the
+// device (numpy_streams.cu) in groups of rows, and the FIR reads them exactly as it reads supplied innovations: the
+// field is then the reference's.  The caller may also pass the innovations themselves (`d_innovations`), which is how
+// tests replay the reference's own streams through these kernels.
 //
 // Sample sharding: the estimator also runs with the samples split over ranks (the layout of the sample-sharded scoring).
 // Everything per sample -- the template, the multiplier field (row r of a shard draws the stream of global sample
@@ -23,6 +25,7 @@
 #include <cmath>
 
 #include "common.cuh"
+#include "numpy_streams.cuh"
 #include "score.cuh"
 
 namespace rb {
@@ -424,11 +427,27 @@ struct WildScratch {
     }
 };
 
+// NumPy streams of an estimator call: draw d is default_rng(seed + 104729 (d + 1)); global sample i takes its normals
+// [i L, (i + 1) L), L = n + 2 bandwidth.  Rows are generated `rows` at a time into `buf` (at most 256 MB), each group
+// continuing the stream where the previous one stopped.
+struct NumpyField {
+    static constexpr long long MAX_BUF = 32LL << 20;      // doubles
+    double *buf = nullptr;
+    long long rows = 0;
+    npz::Scratch sc;
+    int alloc(Arena &ar, long long m, long long L, long long sample_offset)
+    {
+        rows = std::max(1LL, std::min(m, MAX_BUF / L));
+        RB_TRY(ar.alloc(&buf, (size_t)(rows * L)));
+        return sc.alloc(ar, std::max(rows, sample_offset) * L);
+    }
+};
+
 // one multiplier field applied to the template:  d_out = template x W   (inference.py:656-662); row r draws the stream of
-// sample sample_offset + r
+// sample sample_offset + r (Philox; with `np` the NumPy stream of that draw, unless d_innov is given)
 static int wild_multiply(const WildScratch &ws, const double *d_template, long long m, long long n, int bandwidth, const double *d_taps,
                          double h, unsigned long long seed, unsigned draw, unsigned sample_offset, const double *d_innov, double *d_out,
-                         int *d_bad, cudaStream_t st)
+                         int *d_bad, cudaStream_t st, NumpyField *np = nullptr)
 {
     if (n == 1) {                                         // weights are exactly one (inference.py:556-557)
         RB_CUDA(cudaMemcpyAsync(d_out, d_template, sizeof(double) * (size_t)m, cudaMemcpyDeviceToDevice, st));
@@ -447,7 +466,19 @@ static int wild_multiply(const WildScratch &ws, const double *d_template, long l
         attr_dev[dev & 63] = true;
     }
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
-    {
+    if (np && !d_innov) {
+        const long long L = n + K - 1;
+        npz::Cursor cur = npz::seed_cursor((npz::u128)seed + (npz::u128)104729 * ((npz::u128)draw + 1));
+        for (long long r0 = 0; r0 < m; r0 += np->rows) {
+            const long long r1 = std::min(m, r0 + np->rows);
+            RB_TRY(npz::generate(cur, ((long long)sample_offset + r0) * L, ((long long)sample_offset + r1) * L, np->buf, nullptr, np->sc, st));
+            RB_PROF("k_wild_fir", st, (double)(r1 - r0) * n * 8.0);
+            k_wild_fir<<<dim3((unsigned)tiles, (unsigned)(r1 - r0)), FIR_THREADS, smem, st>>>(np->buf, L, key, draw, sample_offset + (unsigned)r0,
+                                                                                             n, K, d_taps, h, d_out + r0 * n,
+                                                                                             d_part + r0 * tiles, tiles);
+            RB_LAUNCH_CHECK();
+        }
+    } else {
         RB_PROF("k_wild_fir", st, (double)m * n * 8.0);
         k_wild_fir<<<dim3((unsigned)tiles, (unsigned)m), FIR_THREADS, smem, st>>>(d_innov, n + K - 1, key, draw, sample_offset, n, K,
                                                                                   d_taps, h, d_out, d_part, tiles);
@@ -589,6 +620,8 @@ static int budget_core(const double *d_centered, long long m, long long n, const
     char *d_sort_tmp = nullptr;
     int *d_bad = nullptr;
     WildScratch wild;
+    NumpyField numpy_field;
+    const bool numpy_streams = P.random_streams == 1 && !P.d_innovations && n > 1;
     if (S.reduce) {
         // the buffers every pass needs to take part in a reduce (a failure here cannot be reported to the other ranks)
         RB_TRY(ar.alloc(&S.d_red, (size_t)(2 * n + NSTATUS)));
@@ -611,6 +644,7 @@ static int budget_core(const double *d_centered, long long m, long long n, const
         RB_TRY(ar.alloc(&d_small, 16));
         RB_TRY(ar.alloc(&d_sort_tmp, sort_track_bytes(n)));
         RB_TRY(wild.alloc(ar, m, n));
+        if (numpy_streams) RB_TRY(numpy_field.alloc(ar, m, n + 2LL * bandwidth, P.sample_offset));
         RB_TRY(ar.alloc(&d_taps, taps.size()));
         RB_CUDA(cudaMemcpyAsync(d_taps, taps.data(), sizeof(double) * taps.size(), cudaMemcpyHostToDevice, st));
         return 0;
@@ -661,7 +695,8 @@ static int budget_core(const double *d_centered, long long m, long long n, const
         const double *innov = P.d_innovations ? P.d_innovations + (size_t)d * innov_per_draw : nullptr;
         if (!S.failed)
             RB_TRY(S.local(wild_multiply(wild, d_tmpl, m, n, bandwidth, d_taps, tap_step, P.random_seed, (unsigned)d,
-                                         (unsigned)P.sample_offset, innov, d_boot, d_bad, st)));
+                                         (unsigned)P.sample_offset, innov, d_boot, d_bad, st,
+                                         numpy_streams ? &numpy_field : nullptr)));
         // the reference field is no longer needed: reuse its buffer
         RB_TRY(score_pass(S, d_boot, m, n, P.score, d_ref, nullptr, d_bad, st));
         RB_TRY(track_sums(d_ref, n, center, soft, threshold, d_part, d_small, h, st));
@@ -728,6 +763,7 @@ RB_API void rocco_b200_default_budget_params(rocco_b200_budget_params *p)
     p->stability_rel_tol = 5.0e-2;
     p->random_seed = 0;
     p->d_innovations = nullptr;
+    p->random_streams = 0;
 }
 
 RB_API int rocco_b200_budget_bandwidth(size_t n, int dependence_lag_hint) { return budget::resolve_bandwidth((long long)n, dependence_lag_hint); }
@@ -739,7 +775,7 @@ RB_API int rocco_b200_budget_nonnull_fraction_dev(const double *d_centered, size
 {
     rocco_b200_budget_params P;
     if (params) P = *params; else rocco_b200_default_budget_params(&P);
-    if (P.sample_offset < 0) return ST_INVALID;
+    if (P.sample_offset < 0 || P.random_streams < 0 || P.random_streams > 1) return ST_INVALID;
     budget::Shard whole;
     return budget::budget_core(d_centered, (long long)m, (long long)n, d_observed_scores, P, whole, result, (cudaStream_t)cuda_stream);
 }
@@ -752,6 +788,7 @@ RB_API int rocco_b200_budget_nonnull_fraction_sharded_dev(const double *d_center
     rocco_b200_budget_params P;
     if (params) P = *params; else rocco_b200_default_budget_params(&P);
     if (m_local == 0 || P.sample_offset < 0 || (size_t)P.sample_offset + m_local > m_total) return ST_INVALID;
+    if (P.random_streams < 0 || P.random_streams > 1) return ST_INVALID;
     if (!allreduce && m_local != m_total) return ST_INVALID;
     budget::Shard shard;
     shard.reduce = allreduce;
@@ -814,7 +851,7 @@ RB_API int rocco_budget_nonnull_fraction_f64(const double *centered, size_t m, s
         RB_CUDA(cudaMemcpyAsync(d_i, innovations, sizeof(double) * cnt, cudaMemcpyHostToDevice, st));
     }
     P.d_innovations = d_i;
-    if (P.sample_offset < 0) return ST_INVALID;
+    if (P.sample_offset < 0 || P.random_streams < 0 || P.random_streams > 1) return ST_INVALID;
     budget::Shard whole;
     const int status = budget::budget_core(d_c, (long long)m, (long long)n, d_o, P, whole, result, st);
     cudaStreamSynchronize(st);

@@ -213,6 +213,29 @@ def _estimate_effective_sample_size(values: np.ndarray, max_lag: int) -> tuple[f
     return float(n_eff.value), float(tau.value), int(used.value)
 
 
+RANDOM_STREAMS = {"philox": 0, "numpy": 1}
+
+
+def random_streams_code(random_streams: str, random_seed, innovations) -> int:
+    """The native code of a ``random_streams`` choice of the budget null, after checking it.
+
+    ``"philox"`` (the default): counter-based Philox4x32-10 streams keyed by ``random_seed``; the null agrees with the
+    reference in distribution.  ``"numpy"``: the reference's own streams -- draw d takes its normals from
+    ``numpy.random.default_rng(random_seed + 104729 * (d + 1))``, the samples served in order -- generated on the device,
+    so the null is the reference's.  ``"numpy"`` needs ``0 <= random_seed < 2**64`` (NumPy rejects negative seeds) and
+    excludes ``innovations``, which replace the generator."""
+    if random_streams not in RANDOM_STREAMS:
+        raise ValueError(f"`random_streams` must be one of {sorted(RANDOM_STREAMS)}, got {random_streams!r}")
+    if random_streams == "numpy":
+        if innovations is not None:
+            raise ValueError("`random_streams='numpy'` generates the innovations: do not pass `innovations` as well")
+        if int(random_seed) < 0:
+            raise ValueError("`random_seed` must be non-negative with `random_streams='numpy'` (as for numpy.random.default_rng)")
+        if int(random_seed) >= 1 << 64:
+            raise ValueError("`random_seed` must be below 2**64")
+    return RANDOM_STREAMS[random_streams]
+
+
 def _budget_params(lower_bound_z, prior_df, min_effect, precision_floor_ratio, dependence_lag_hint, num_null_draws,
                    random_seed, min_null_draws, stability_abs_tol, stability_rel_tol):
     lib = _lib.load()
@@ -260,16 +283,19 @@ def estimate_budget_nonnull_fraction_from_wild_bootstrap_null(
         dependence_lag_hint: int | None = None, num_null_draws: int = 25, random_seed: int = 0,
         progress_label: str | None = None, num_processes: int = 1, return_details: bool = False,
         min_null_draws: int | None = None, stability_abs_tol: float = 5.0e-3, stability_rel_tol: float = 5.0e-2,
-        innovations: np.ndarray | None = None) -> float | Tuple[float, Dict[str, Any]]:
+        innovations: np.ndarray | None = None, random_streams: str = "philox") -> float | Tuple[float, Dict[str, Any]]:
     r"""Conservative enriched fraction from a dependent-wild-bootstrap null (inference.py:988-1148).
 
     Same arguments, return value and details keys as the reference.  The whole estimator -- null template, fitted-null
     score field, up to ``num_null_draws`` multiplier fields each re-scored by the WLS chain, the adaptive stop, the
     observed-side summary and the ESS -- runs on the GPU in one native call; ``num_processes`` and ``progress_label``
-    are accepted and unused.  Random streams are Philox (keyed by ``random_seed``), not NumPy's PCG64: results agree
-    with the reference in distribution.  ``innovations`` (``[num_null_draws, n_samples, n_loci + 2*bandwidth]`` iid
-    N(0,1)) replaces the generator, e.g. to replay the reference's own streams.
+    are accepted and unused.  ``random_streams="philox"`` (the default) draws Philox streams keyed by ``random_seed``:
+    results agree with the reference in distribution.  ``random_streams="numpy"`` generates the reference's own NumPy
+    PCG64 streams on the device, so the draws, and the result, are the reference's (see ``random_streams_code``).
+    ``innovations`` (``[num_null_draws, n_samples, n_loci + 2*bandwidth]`` iid N(0,1)) replaces the generator, e.g. to
+    replay the reference's own streams from the host.
     """
+    streams = random_streams_code(random_streams, random_seed, innovations)
     centered = np.asarray(centered_matrix, dtype=np.float64)
     if centered.ndim == 1:
         centered = centered[np.newaxis, :]
@@ -290,6 +316,7 @@ def estimate_budget_nonnull_fraction_from_wild_bootstrap_null(
     _lib.require_device()
     prm = _budget_params(lower_bound_z, prior_df, min_effect, precision_floor_ratio, dependence_lag_hint, num_null_draws,
                          random_seed, min_null_draws, stability_abs_tol, stability_rel_tol)
+    prm.random_streams = streams
     inn = None
     if innovations is not None:
         bw = _resolve_budget_bootstrap_bandwidth(n, dependence_lag_hint)

@@ -553,8 +553,10 @@ def _score_streams(dev, count: int):
 # The reference's CLI without --gamma: per chromosome, score, run the wild-bootstrap budget null on the centred rows, then
 # feed every chromosome's (effective_count, effective_total_count) to the empirical-Bayes budgets and set the automatic
 # gamma from the null's autocorrelation time and the median positive score.
+# "random_streams": the budget null's innovations, "philox" or "numpy" (the reference's own streams: see
+# inference.random_streams_code).
 DEFAULT_FLOW_ARGS = {"budget": None, "scale_chrom_budgets": 1.0, "budget_posterior_quantile": 0.01, "num_null_draws": 25,
-                     "random_seed": 0}
+                     "random_seed": 0, "random_streams": "philox"}
 
 
 def _default_flow_args(default_args) -> dict:
@@ -564,6 +566,8 @@ def _default_flow_args(default_args) -> dict:
     if unknown:
         raise ValueError(f"unknown `default_args` keys {unknown}; known: {sorted(args)}")
     args.update(default_args or {})
+    if args["random_streams"] not in ("philox", "numpy"):
+        raise ValueError(f"`random_streams` must be 'philox' or 'numpy', got {args['random_streams']!r}")
     return args
 
 
@@ -715,7 +719,8 @@ def _run_shard_defaults(d_matrices, budgets, gammas, params, levels_per_round, w
             window = _resolve_local_baseline_window(n, prm.baseline_window if prm.baseline_window > 0 else 101)
             mark(f"null:{name}")
             _, det = budget_null_device(centered, scores, params=prm, dependence_lag_hint=window,
-                                        num_null_draws=args["num_null_draws"], random_seed=args["random_seed"])
+                                        num_null_draws=args["num_null_draws"], random_seed=args["random_seed"],
+                                        random_streams=args["random_streams"])
         except (ValueError, RuntimeError) as exc:
             failure = f"default flow: {name}: {exc}"
             break
@@ -993,14 +998,17 @@ def score_loci_wls_sample_sharded(d_matrix_local, m_total: int, params=None, gro
 
 # ------------------------------------------------------------------ budget null on device tensors (SURVEY.md 8(f) rank 1)
 def budget_null_device(d_centered, d_observed_scores=None, params=None, dependence_lag_hint=None, num_null_draws=25,
-                       random_seed=0, min_null_draws=None, stability_abs_tol=5.0e-3, stability_rel_tol=5.0e-2):
+                       random_seed=0, min_null_draws=None, stability_abs_tol=5.0e-3, stability_rel_tol=5.0e-2,
+                       random_streams="philox"):
     """``estimate_budget_nonnull_fraction_from_wild_bootstrap_null`` (inference.py:988-1148) on CUDA tensors: the centred
     matrix [samples, bins] (float64, as ``score_loci_wls_device(..., details=True)`` returns it) and optionally the observed
     scores stay on the device; returns ``(nonnull_fraction, details)`` with the reference's keys plus the positive-score
-    median/count that ``rocco._resolve_chrom_gamma`` needs."""
-    from .inference import _budget_details, _hint
+    median/count that ``rocco._resolve_chrom_gamma`` needs.  ``random_streams``: "philox" (default) or "numpy", the
+    reference's own streams generated on the device (``inference.random_streams_code``)."""
+    from .inference import _budget_details, _hint, random_streams_code
     torch = _torch()
     lib = _lib.load()
+    streams = random_streams_code(random_streams, random_seed, None)
     if d_centered.dim() != 2 or not d_centered.is_cuda or not d_centered.is_contiguous() or d_centered.dtype != torch.float64:
         raise ValueError("`d_centered` must be a contiguous two-dimensional float64 CUDA tensor")
     m, n = d_centered.shape
@@ -1019,6 +1027,7 @@ def budget_null_device(d_centered, d_observed_scores=None, params=None, dependen
     prm.stability_abs_tol = float(stability_abs_tol)
     prm.stability_rel_tol = float(stability_rel_tol)
     prm.random_seed = int(random_seed) & 0xFFFFFFFFFFFFFFFF
+    prm.random_streams = streams
     res = _lib.BudgetResult()
     dev = d_centered.device
     with torch.cuda.device(dev):
@@ -1043,14 +1052,17 @@ class _DeviceBuffer:
 
 def _budget_null_sharded(d_centered_local, m_total: int, sample_offset: int, reduce_fn, d_observed_scores=None, params=None,
                          dependence_lag_hint=None, num_null_draws=25, random_seed=0, min_null_draws=None,
-                         stability_abs_tol=5.0e-3, stability_rel_tol=5.0e-2, innovations=None):
+                         stability_abs_tol=5.0e-3, stability_rel_tol=5.0e-2, innovations=None, random_streams="philox"):
     """One rank's part of the sample-sharded estimator, shapes already agreed between the ranks.  ``reduce_fn(buf)`` sums
     the float64 CUDA tensor ``buf`` over all ranks in place, ordered on torch's current stream; it is called with the same
     length on every rank, 2 + (draws used) times.  An exception in it becomes a failed call on this rank.  ``reduce_fn=None``
-    (one rank holding every sample) is the unsharded estimator."""
-    from .inference import _budget_details, _hint
+    (one rank holding every sample) is the unsharded estimator.  ``random_streams`` as for ``budget_null_device``: with
+    "numpy", row r of this rank takes the normals of global sample ``sample_offset + r``, so the field is the same
+    whatever the sharding."""
+    from .inference import _budget_details, _hint, random_streams_code
     torch = _torch()
     lib = _lib.load()
+    streams = random_streams_code(random_streams, random_seed, innovations)
     m, n = d_centered_local.shape
     dev = d_centered_local.device
     prm = _lib.BudgetParams()
@@ -1065,6 +1077,7 @@ def _budget_null_sharded(d_centered_local, m_total: int, sample_offset: int, red
     prm.random_seed = int(random_seed) & 0xFFFFFFFFFFFFFFFF
     prm.sample_offset = int(sample_offset)
     prm.d_innovations = None if innovations is None else innovations.data_ptr()
+    prm.random_streams = streams
     failure = []
 
     def _reduce(ptr, count, _stream, _user):
@@ -1090,10 +1103,15 @@ def _budget_null_sharded(d_centered_local, m_total: int, sample_offset: int, red
     return float(res.nonnull_fraction), _budget_details(res)
 
 
-def _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint):
+def _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint,
+                            random_seed=0, random_streams="philox"):
     """This rank's own argument errors (checked before the ranks compare shapes), or None."""
-    from .inference import _resolve_budget_bootstrap_bandwidth
+    from .inference import _resolve_budget_bootstrap_bandwidth, random_streams_code
     torch = _torch()
+    try:
+        random_streams_code(random_streams, random_seed, innovations)
+    except ValueError as exc:
+        return str(exc)
     x = d_centered_local
     if x.dim() != 2 or not x.is_cuda or not x.is_contiguous() or x.dtype != torch.float64:
         return "`d_centered_local` must be a contiguous two-dimensional float64 CUDA tensor"
@@ -1110,23 +1128,26 @@ def _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, nu
 
 def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=None, group=None, dependence_lag_hint=None,
                                num_null_draws=25, random_seed=0, min_null_draws=None, stability_abs_tol=5.0e-3,
-                               stability_rel_tol=5.0e-2, innovations=None):
+                               stability_rel_tol=5.0e-2, innovations=None, random_streams="philox"):
     """``budget_null_device`` with the SAMPLES sharded over the ranks of ``group`` (BASELINE.json config 5): every rank
     passes its centred rows ``[m_local, bins]`` (e.g. from ``score_loci_wls_sample_sharded(..., keep_centered=True)``, ranks
     in sample order) and the same observed scores and arguments.  Each scoring pass all-reduces 2 x bins float64 column
     sums (plus four status slots); every rank returns the same ``(nonnull_fraction, details)``, with the keys of
     ``budget_null_device``, and raises the same exception.  ``innovations``: this rank's rows,
-    ``[draws, m_local, bins + 2*bandwidth]`` float64 on the device."""
+    ``[draws, m_local, bins + 2*bandwidth]`` float64 on the device.  ``random_streams``: as for ``budget_null_device``;
+    with "numpy" every rank generates the rows of its own samples, so the result equals the unsharded call's streams."""
     import torch.distributed as dist
     torch = _torch()
-    problem = _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint)
+    problem = _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint,
+                                      random_seed, random_streams)
     sharded = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
     if not sharded:
         if problem:
             raise ValueError(problem)
         m = d_centered_local.shape[0]
         return _budget_null_sharded(d_centered_local, m, 0, None, d_observed_scores, params, dependence_lag_hint,
-                                    num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations)
+                                    num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations,
+                                    random_streams)
     dev = d_centered_local.device if d_centered_local.is_cuda else torch.device("cuda", torch.cuda.current_device())
     m, n = (d_centered_local.shape if d_centered_local.dim() == 2 else (0, 0))
     # the reduce workspace is allocated before the ranks compare notes, so that its failure is one more problem reported
@@ -1157,7 +1178,8 @@ def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=
         buf.copy_(w)
 
     return _budget_null_sharded(d_centered_local, m_total, offset, reduce_fn, d_observed_scores, params, dependence_lag_hint,
-                                num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations)
+                                num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations,
+                                random_streams)
 
 
 def _score_sample_sharded_agreed(x, m_total: int, prm, group, name: str):
@@ -1223,7 +1245,8 @@ def run_sample_sharded_defaults(chroms, m_total: int, params=None, default_args=
         del x
         mark(f"null:{name}")
         _, det = budget_null_sample_sharded(centered, s, params=prm, group=group, dependence_lag_hint=window,
-                                            num_null_draws=args["num_null_draws"], random_seed=args["random_seed"])
+                                            num_null_draws=args["num_null_draws"], random_seed=args["random_seed"],
+                                            random_streams=args["random_streams"])
         del centered
         mark(f"done:{name}")
         names.append(name)

@@ -1,14 +1,15 @@
 """ROCCO's default flow (budget null -> EB budgets -> automatic gamma -> solve) on the synthetic config-4 genome, timed by
 phase, next to the fixed-parameter step on the same matrices.
 
-    python tools/default_flow.py [--samples 100] [--step-bp 50] [--chroms chr1,chr21] [--draws 25]
+    python tools/default_flow.py [--samples 100] [--step-bp 50] [--chroms chr1,chr21] [--draws 25] [--random-streams numpy]
     torchrun --nproc-per-node 8 tools/default_flow.py
 
 hg38 @ 50 bp x 100 samples float64, the chromosomes LPT-packed over the ranks and resident in HBM (as bench.py lays them
 out).  pipeline.run_shard(budgets=None, gammas=None) runs once untimed, then once with its `mark` hook recording a CUDA
 event at each phase boundary; the genome BED is written by distributed.write_genome_bed.  Phase times are the maximum
 over ranks.  The fixed-parameter step (HG_PARAMS budgets and gammas, run_shard + genome BED) is timed on the same
-matrices in the same process: median of --fixed-steps after one warm-up.  One JSON line on rank 0's stdout.
+matrices in the same process: median of --fixed-steps after one warm-up.  --random-streams picks the null's innovations:
+Philox (default) or the reference's own NumPy streams generated on the device.  One JSON line on rank 0's stdout.
 """
 import argparse, json, math, os, shutil, subprocess, sys, tempfile, time
 import numpy as np, torch, torch.distributed as dist
@@ -22,6 +23,8 @@ ap.add_argument("--step-bp", type=int, default=50)
 ap.add_argument("--chroms", default="")
 ap.add_argument("--draws", type=int, default=25, help="num_null_draws (the reference's default is 25)")
 ap.add_argument("--fixed-steps", type=int, default=3)
+ap.add_argument("--random-streams", choices=("philox", "numpy"), default="philox",
+                help="the budget null's innovations: Philox, or the reference's NumPy PCG64 streams")
 args = ap.parse_args()
 rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 local = int(os.environ.get("LOCAL_RANK", 0))
@@ -75,7 +78,7 @@ def default_flow(events=None):
             e.record()
             events.append((label, e))
     out = pipeline.run_shard(d_mats, None, None, params=prm, chrom_names=my_names, genome_names=names,
-                             default_args={"num_null_draws": args.draws}, mark=mark)
+                             default_args={"num_null_draws": args.draws, "random_streams": args.random_streams}, mark=mark)
     mark("bed")
     t0 = time.perf_counter()
     tot = write_bed(out)
@@ -146,6 +149,7 @@ if rank == 0:
     line = {
         "config": f"hg38 @ {args.step_bp} bp x {args.samples} samples f64 resident, chromosomes LPT-sharded over {world} GPU(s), "
                   f"ROCCO default flow (budget null with up to {args.draws} draws -> EB budgets -> automatic gamma -> solve)",
+        "random_streams": args.random_streams,
         "gpus": [e["card"] for e in every], "bins": int(sum(bins)),
         "default_flow_ms_max_over_ranks": dict(zip(keys, vec[:nb])),
         "null_ms_by_chrom_max_over_ranks": dict(zip(names, vec[nb:nb + len(names)])),

@@ -4,12 +4,14 @@ per chromosome on the rank that owns it (LPT).  Chromosomes are generated, score
 holds more than one chromosome's matrix + scratch (~35 GB).
 
     torchrun --nproc-per-node 8 tools/run_config5.py [--samples 1000] [--step-bp 20] [--chroms chr1,chr2] [--budget-null]
-                                                      [--central-tendency median]
+                                                      [--random-streams numpy] [--central-tendency median]
 
 --budget-null replaces the sweep by the default CLI flow on the same layout: per chromosome the sharded scoring keeps each
 rank's centred rows, the wild-bootstrap budget null runs with the samples still sharded (2n column sums all-reduced per
 scoring pass), the fractions go through the empirical-Bayes budgets and the automatic gamma (host, identical on every
 rank), and the owner rank solves each chromosome at its budget: pipeline.run_sample_sharded_defaults.
+--random-streams numpy draws the null's innovations from the reference's own NumPy streams, each rank generating the rows
+of its samples.
 """
 import argparse, json, math, os, sys, time
 import numpy as np, torch, torch.distributed as dist
@@ -24,6 +26,7 @@ ap.add_argument("--chroms", default="")
 ap.add_argument("--multipliers", type=int, default=256)
 ap.add_argument("--budget-null", action="store_true", help="budget null + EB budgets + solve instead of the sweep")
 ap.add_argument("--null-draws", type=int, default=25)
+ap.add_argument("--random-streams", choices=("philox", "numpy"), default="philox", help="with --budget-null: the null's innovations")
 ap.add_argument("--central-tendency", default="", help="score each chromosome by this column statistic of the sharded "
                 "samples (median, mean, tmean, quantile, ...) instead of the WLS score")
 args = ap.parse_args()
@@ -76,8 +79,9 @@ def budget_null_run():
             torch.cuda.synchronize()
             per_chrom[label[5:]] = {"all_reduce_ms": r[0].elapsed_time(r[1]) / 5}
 
-    out = pipeline.run_sample_sharded_defaults(chroms(), m_local * world, prm, default_args={"num_null_draws": args.null_draws},
-                                              mark=mark)
+    out = pipeline.run_sample_sharded_defaults(chroms(), m_local * world, prm, mark=mark,
+                                              default_args={"num_null_draws": args.null_draws,
+                                                            "random_streams": args.random_streams})
     torch.cuda.synchronize()
     for c, n in zip(names, bins):
         det = out["defaults"]["null"][c]
@@ -102,7 +106,7 @@ def budget_null_run():
         mx = t.tolist()
         print(json.dumps({
             "config": f"hg38 @ {args.step_bp} bp x {m_local * world} samples f32, sample-sharded over {world} GPUs, budget null + "
-                      "EB budgets + auto gamma + solve", "gpu": torch.cuda.get_device_name(dev),
+                      f"EB budgets + auto gamma + solve ({args.random_streams} streams)", "gpu": torch.cuda.get_device_name(dev),
             "chroms": {c: {"bins": per_chrom[c]["bins"], "budget": budgets[c], "gamma": gammas[c],
                            "nonnull_fraction": per_chrom[c]["nonnull_fraction"],
                            "ms_max_over_ranks": dict(zip(keys, mx[i][:4])), "passes_max_over_ranks": int(mx[i][4]),
