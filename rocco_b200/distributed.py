@@ -8,8 +8,10 @@ Works with NCCL (GPUs) and gloo (CPU tests) alike; with world size 1 nothing is 
 """
 from __future__ import annotations
 
+import contextlib
 from typing import Sequence
 
+from . import _lib
 from .pipeline import lpt_partition
 from .rocco import _merge_bed_records
 
@@ -19,11 +21,86 @@ def _dist():
     return dist
 
 
-def world() -> tuple[int, int]:
+def world(group=None) -> tuple[int, int]:
+    """(rank, size) of this process in ``group`` (default: the whole world); (0, 1) without an initialised process group."""
     dist = _dist()
     if dist.is_available() and dist.is_initialized():
-        return dist.get_rank(), dist.get_world_size()
+        return dist.get_rank(group), dist.get_world_size(group)
     return 0, 1
+
+
+def collective_device(group, device=None):
+    """Where the tensors of a collective on ``group`` live: the CPU for gloo, otherwise ``device`` (default: the current
+    CUDA device)."""
+    import torch
+    if _dist().get_backend(group) == "gloo":
+        return torch.device("cpu")
+    return device if device is not None else torch.device("cuda", torch.cuda.current_device())
+
+
+def agree(problem, facts: dict, group, what: str) -> list:
+    """Every rank's ``facts`` in rank order, from one ``all_gather_object`` of ``{"problem": problem, **facts}`` over
+    ``group`` (with one rank: ``[facts]`` and no collective).  ``problem`` is this rank's own argument error, or None.
+    A rank with a problem raises ``ValueError(problem)`` and every other rank a ``ValueError`` that names it, so all
+    ranks leave together instead of some entering a collective that the others never reach.  Checks across the
+    gathered facts are the caller's."""
+    size = world(group)[1]
+    if size <= 1:
+        if problem is not None:
+            raise ValueError(problem)
+        return [facts]
+    every = [None] * size
+    _dist().all_gather_object(every, {"problem": problem, **facts}, group=group)
+    if problem is not None:
+        raise ValueError(problem)
+    bad = next((r["problem"] for r in every if r["problem"] is not None), None)
+    if bad is not None:
+        raise ValueError(f"{what}: another rank rejected its arguments: {bad}")
+    return [{k: v for k, v in r.items() if k != "problem"} for r in every]
+
+
+class _DeviceBuffer:
+    """A raw float64 device buffer as a torch tensor (``__cuda_array_interface__``, no copy)."""
+
+    def __init__(self, ptr: int, count: int):
+        self.__cuda_array_interface__ = {"shape": (int(count),), "typestr": "<f8", "data": (int(ptr), False),
+                                          "strides": None, "version": 2}
+
+
+@contextlib.contextmanager
+def allreduce_callback(reduce_fn, device, what: str):
+    """``reduce_fn(buf)`` as the native ``rocco_b200_allreduce_fn`` (None when ``reduce_fn`` is None), for one native
+    call made inside the ``with`` block.  ``buf`` is the library's float64 buffer as a tensor on ``device``.  An
+    exception in ``reduce_fn`` fails the callback instead of unwinding through the C frames, and leaving the block raises
+    it as ``RuntimeError`` -- before the caller looks at the native status, which then only reports the failed reduce."""
+    import torch
+    failure = []
+
+    def call(ptr, count, _stream, _user):
+        try:
+            reduce_fn(torch.as_tensor(_DeviceBuffer(ptr, count), device=device))
+            return 0
+        except BaseException as exc:
+            failure.append(exc)
+            return 1
+
+    yield None if reduce_fn is None else _lib.ALLREDUCE_FN(call)
+    if failure:
+        raise RuntimeError(f"{what}: the all-reduce failed: {failure[0]!r}") from failure[0]
+
+
+def workspace_allreduce(workspace, group):
+    """A ``reduce_fn`` for ``allreduce_callback``: sums ``buf`` over ``group`` in place through ``workspace``, a float64
+    CUDA tensor at least as long as any ``buf``, allocated by the caller before the ranks agree (so that its failure is
+    reported to every rank)."""
+    dist = _dist()
+
+    def reduce_fn(buf):
+        w = workspace[: buf.numel()]
+        w.copy_(buf)
+        dist.all_reduce(w, group=group)
+        buf.copy_(w)
+    return reduce_fn
 
 
 def shard_chromosomes(bin_counts: Sequence[int]) -> list[int]:

@@ -16,6 +16,7 @@ import numpy as np
 from . import _baseline as _baseline_native
 from . import _lib
 from . import _wls as _wls_native
+from .pipeline import score_params
 
 logger = logging.getLogger(__name__)
 
@@ -120,14 +121,7 @@ def score_loci_wls(chrom_matrix: np.ndarray, lower_bound_z: float = 1.0, prior_d
     m, n = matrix_in.shape
     lib = _lib.load()
     _lib.require_device()
-
-    prm = _lib.ScoreParams()
-    lib.rocco_b200_default_score_params(ctypes.byref(prm))
-    prm.lower_bound_z = float(lower_bound_z)
-    prm.prior_df = float(prior_df)
-    prm.use_min_effect = 0 if min_effect is None else 1
-    prm.min_effect = 0.0 if min_effect is None else max(float(min_effect), 0.0)
-    prm.precision_floor_ratio = float(max(precision_floor_ratio, 0.0))
+    prm = score_params(lower_bound_z, prior_df, min_effect, precision_floor_ratio)
 
     names = ("scores", "mean", "raw_variance", "prior_variance", "moderated_variance", "standard_error")
     bufs = {k: np.zeros(n, dtype=np.float64) for k in (names if return_details else names[:1])}
@@ -236,22 +230,23 @@ def random_streams_code(random_streams: str, random_seed, innovations) -> int:
     return RANDOM_STREAMS[random_streams]
 
 
-def _budget_params(lower_bound_z, prior_df, min_effect, precision_floor_ratio, dependence_lag_hint, num_null_draws,
-                   random_seed, min_null_draws, stability_abs_tol, stability_rel_tol):
-    lib = _lib.load()
+def budget_params(score, dependence_lag_hint=None, num_null_draws=25, min_null_draws=None, stability_abs_tol=5.0e-3,
+                  stability_rel_tol=5.0e-2, random_seed=0, random_streams="philox", sample_offset=0, d_innovations=None):
+    """The native parameters of the budget null: the ``ScoreParams`` ``score`` and the null's settings, as the estimator
+    entries take them.  ``sample_offset``: global index of this rank's first sample (sample sharding); ``d_innovations``:
+    a CUDA tensor of supplied innovations, or None.  Raises ``ValueError`` as ``random_streams_code``."""
     prm = _lib.BudgetParams()
-    lib.rocco_b200_default_budget_params(ctypes.byref(prm))
-    prm.score.lower_bound_z = float(lower_bound_z)
-    prm.score.prior_df = float(prior_df)
-    prm.score.use_min_effect = 0 if min_effect is None else 1
-    prm.score.min_effect = 0.0 if min_effect is None else max(float(min_effect), 0.0)
-    prm.score.precision_floor_ratio = float(max(precision_floor_ratio, 0.0))
+    _lib.load().rocco_b200_default_budget_params(ctypes.byref(prm))
+    prm.score = score
     prm.dependence_lag_hint = _hint(dependence_lag_hint)
     prm.num_null_draws = int(max(1, num_null_draws))
     prm.min_null_draws = 0 if min_null_draws is None else int(max(1, min_null_draws))
     prm.stability_abs_tol = float(stability_abs_tol)
     prm.stability_rel_tol = float(stability_rel_tol)
     prm.random_seed = int(random_seed) & 0xFFFFFFFFFFFFFFFF
+    prm.random_streams = random_streams_code(random_streams, random_seed, d_innovations)
+    prm.sample_offset = int(sample_offset)
+    prm.d_innovations = None if d_innovations is None else d_innovations.data_ptr()
     return prm
 
 
@@ -295,7 +290,7 @@ def estimate_budget_nonnull_fraction_from_wild_bootstrap_null(
     ``innovations`` (``[num_null_draws, n_samples, n_loci + 2*bandwidth]`` iid N(0,1)) replaces the generator, e.g. to
     replay the reference's own streams from the host.
     """
-    streams = random_streams_code(random_streams, random_seed, innovations)
+    random_streams_code(random_streams, random_seed, innovations)     # budget_params does not see host innovations
     centered = np.asarray(centered_matrix, dtype=np.float64)
     if centered.ndim == 1:
         centered = centered[np.newaxis, :]
@@ -314,9 +309,8 @@ def estimate_budget_nonnull_fraction_from_wild_bootstrap_null(
             raise ValueError("`observed_scores` must have the same number of loci as `centered_matrix`")
     lib = _lib.load()
     _lib.require_device()
-    prm = _budget_params(lower_bound_z, prior_df, min_effect, precision_floor_ratio, dependence_lag_hint, num_null_draws,
-                         random_seed, min_null_draws, stability_abs_tol, stability_rel_tol)
-    prm.random_streams = streams
+    prm = budget_params(score_params(lower_bound_z, prior_df, min_effect, precision_floor_ratio), dependence_lag_hint,
+                        num_null_draws, min_null_draws, stability_abs_tol, stability_rel_tol, random_seed, random_streams)
     inn = None
     if innovations is not None:
         bw = _resolve_budget_bootstrap_bandwidth(n, dependence_lag_hint)

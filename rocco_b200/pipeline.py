@@ -219,6 +219,7 @@ def _score_extremes(d_scores, offsets, lengths):
 def _solve_genome(d_scores, d_costs, offsets, lengths, gammas, search, levels_per_round, d_masks, reduce_fn):
     """One rank's call of rocco_b200_chain_solve_genome_dev with the search fields already agreed.  ``reduce_fn(buf)`` sums
     the float64 CUDA tensor ``buf`` over the ranks in place on torch's current stream (None: this call holds the genome)."""
+    from .distributed import allreduce_callback
     torch = _torch()
     lib = _lib.load()
     dev = d_scores.device
@@ -229,26 +230,13 @@ def _solve_genome(d_scores, d_costs, offsets, lengths, gammas, search, levels_pe
         t.offset, t.n, t.gamma, t.max_iter = int(offsets[c]), int(lengths[c]), float(gammas[c]), int(search.max_iter)
     if d_masks is None:
         d_masks = torch.zeros(d_scores.shape[0], dtype=torch.uint8, device=dev)
-    failure = []
-
-    def _reduce(ptr, count, _stream, _user):
-        try:
-            reduce_fn(torch.as_tensor(_DeviceBuffer(ptr, count), device=dev))
-            return 0
-        except BaseException as exc:          # never let it unwind through the C frames
-            failure.append(exc)
-            return 1
-
-    cb = None if reduce_fn is None else _lib.ALLREDUCE_FN(_reduce)
     results = (_lib.ChainResult * max(nchrom, 1))()
     genome = _lib.GenomeResult()
-    with torch.cuda.device(dev):
+    with torch.cuda.device(dev), allreduce_callback(reduce_fn, dev, "genome budget") as cb:
         st = lib.rocco_b200_chain_solve_genome_dev(
             ctypes.c_void_p(d_scores.data_ptr()), None if d_costs is None else ctypes.c_void_p(d_costs.data_ptr()),
             tasks, nchrom, ctypes.byref(search), cb, None, ctypes.c_void_p(d_masks.data_ptr()), results,
             ctypes.byref(genome), int(levels_per_round), ctypes.c_void_p(_stream_ptr(dev)))
-    if failure:
-        raise RuntimeError(f"genome budget: the all-reduce failed: {failure[0]!r}") from failure[0]
     if st == _lib.ST_INVALID and _lib.last_error().startswith("genome budget"):
         raise ValueError(_lib.last_error())
     _lib.check(st, "genome budget")
@@ -258,11 +246,6 @@ def _solve_genome(d_scores, d_costs, offsets, lengths, gammas, search, levels_pe
     return d_masks, out, [_chain_result_dict(results[c]) for c in range(nchrom)]
 
 
-def _group_size(group) -> int:
-    import torch.distributed as dist
-    return dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
-
-
 def solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_iter: int = 60, levels_per_round: int = 0,
                         d_masks=None, group=None):
     """One multiplier for the whole genome: the chromosomes packed in ``d_scores`` (as ``solve_packed``) and, when ``group``
@@ -270,11 +253,12 @@ def solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_i
     all N bins; each search round's counts are summed over the ranks with one ``torch.distributed.all_reduce`` of at most
     2^L + 1 doubles.  Returns ``(d_masks, genome, results)``: ``genome`` holds the multiplier, the genome's selected count,
     N, the target, the DP passes and the rounds; ``results`` the per-chromosome dicts of ``solve_packed``."""
+    from .distributed import agree, workspace_allreduce, world
     torch = _torch()
     _lib.require_device()
     problem = _genome_problem(d_scores, offsets, lengths, gammas, genome_budget)
     nan = float("nan")
-    if _group_size(group) <= 1:
+    if world(group)[1] <= 1:
         if problem:
             raise ValueError(problem)
         total = sum(int(n) for n in lengths)
@@ -284,7 +268,6 @@ def solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_i
                                    _genome_cost_max(lengths, gammas), nan, nan, int(max_iter), 0)
         return _solve_genome(d_scores, None, offsets, lengths, gammas, search, levels_per_round, d_masks, None)
 
-    import torch.distributed as dist
     dev = d_scores.device if isinstance(d_scores, torch.Tensor) and d_scores.is_cuda else torch.device("cuda", torch.cuda.current_device())
     # the reduce workspace (2^8 - 1 counts + 2 slots at most) is allocated before the ranks compare notes, so that its
     # failure is one more problem reported to all of them
@@ -298,15 +281,9 @@ def solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_i
             problem = f"genome budget: {exc}"
         if extremes == "non-finite":
             problem = "genome budget: non-finite values in `d_scores`"
-    mine = {"problem": problem is not None, "n": [int(n) for n in lengths] if problem is None else [],
-            "gamma": [float(g) for g in gammas] if problem is None else [], "extremes": extremes,
-            "agreed": (float(genome_budget), int(max_iter), int(levels_per_round))}
-    every = [None] * dist.get_world_size(group)
-    dist.all_gather_object(every, mine, group=group)
-    if problem is not None:
-        raise ValueError(problem)
-    if any(r["problem"] for r in every):
-        raise ValueError("genome budget: another rank rejected its arguments")
+    mine = {} if problem else {"n": [int(n) for n in lengths], "gamma": [float(g) for g in gammas], "extremes": extremes,
+                               "agreed": (float(genome_budget), int(max_iter), int(levels_per_round))}
+    every = agree(problem, mine, group, "genome budget")
     if any(r["agreed"] != mine["agreed"] for r in every):
         raise ValueError("genome budget: every rank must pass the same genome_budget, max_iter and levels_per_round")
     all_n = [n for r in every for n in r["n"]]
@@ -318,14 +295,8 @@ def solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_i
     search = _lib.GenomeSearch(total, target_count_for_budget(total, genome_budget), genome_cost_sum(all_n, all_g),
                                _genome_cost_max(all_n, all_g), min(e[0] for e in ext), max(e[1] for e in ext),
                                int(max_iter), 0)
-
-    def reduce_fn(buf):
-        w = workspace[: buf.numel()]
-        w.copy_(buf)
-        dist.all_reduce(w, group=group)
-        buf.copy_(w)
-
-    return _solve_genome(d_scores, None, offsets, lengths, gammas, search, levels_per_round, d_masks, reduce_fn)
+    return _solve_genome(d_scores, None, offsets, lengths, gammas, search, levels_per_round, d_masks,
+                         workspace_allreduce(workspace, group))
 
 
 def solve_genome(scores_list, genome_budget, gammas, switch_costs_list=None, max_iter: int = 60, levels_per_round: int = 0,
@@ -334,13 +305,14 @@ def solve_genome(scores_list, genome_budget, gammas, switch_costs_list=None, max
     NumPy arrays.  ``switch_costs_list`` (single process only; ``gammas`` is then ignored) gives each chromosome its own
     n_c - 1 switch costs; their genome sum is ``math.fsum`` of all of them."""
     import math
+    from .distributed import world
     torch = _torch()
     if switch_costs_list is None:
         d_scores, offsets, lengths = pack_scores(scores_list)
         d_masks, genome, results = solve_genome_packed(d_scores, offsets, lengths, genome_budget, gammas, max_iter=max_iter,
                                                        levels_per_round=levels_per_round, group=group)
     else:
-        if _group_size(group) > 1:
+        if world(group)[1] > 1:
             raise ValueError("`switch_costs_list` is supported in a single process only")
         _lib.require_device()
         if len(switch_costs_list) != len(scores_list):
@@ -603,19 +575,10 @@ def agree_chromosome_names(chrom_names, genome_names, group=None, problem=None, 
     passed the same ``genome_names`` and ``agreed`` value.  ``problem`` is this rank's own argument error (or None).  One
     ``all_gather_object``; every rank raises the same ``ValueError``, except that a rank with a ``problem`` raises its own.
     Returns the number of chromosome slots of ``gather_budget_estimates``: the most any rank holds."""
+    from .distributed import agree
     mine = {"names": [str(c) for c in chrom_names], "genome": None if genome_names is None else [str(c) for c in genome_names],
-            "problem": problem, "agreed": agreed}
-    if _group_size(group) <= 1:
-        every = [mine]
-    else:
-        import torch.distributed as dist
-        every = [None] * dist.get_world_size(group)
-        dist.all_gather_object(every, mine, group=group)
-    if problem is not None:
-        raise ValueError(problem)
-    bad = next((r["problem"] for r in every if r["problem"] is not None), None)
-    if bad is not None:
-        raise ValueError(f"default flow: another rank rejected its arguments: {bad}")
+            "agreed": agreed}
+    every = agree(problem, mine, group, "default flow")
     if any(r["genome"] is None for r in every):
         raise ValueError("default flow: `genome_names` is required when the chromosomes are spread over several ranks")
     msg = _chromosome_name_problem(every)
@@ -636,6 +599,7 @@ def gather_budget_estimates(chrom_names, genome_names, rows, slots: int, group=N
     raises that.
     Returns ``{name: {"budget_count_hat": effective_count, "total_count": effective_total_count}}`` in genome order, the
     cache ``rocco._resolve_budgets`` takes: the order is data, as the optimiser's path depends on the summation order."""
+    from .distributed import collective_device, world
     torch = _torch()
     genome = [str(c) for c in genome_names]
     index = {c: g for g, c in enumerate(genome)}
@@ -646,15 +610,13 @@ def gather_budget_estimates(chrom_names, genome_names, rows, slots: int, group=N
     for k, (c, (count, total, status)) in enumerate(zip(chrom_names, rows)):
         table[k] = (index[str(c)], float(count), float(total), float(status))
     table[int(slots), 3] = 0.0 if failure is None else 1.0
-    world = _group_size(group)
-    if world <= 1:
+    size = world(group)[1]
+    if size <= 1:
         every = table
     else:
         import torch.distributed as dist
-        host = dist.get_backend(group) == "gloo"
-        dev = torch.device("cpu") if host else (device or torch.device("cuda", torch.cuda.current_device()))
-        mine = torch.from_numpy(table).to(dev)
-        parts = [torch.empty_like(mine) for _ in range(world)]
+        mine = torch.from_numpy(table).to(collective_device(group, device))
+        parts = [torch.empty_like(mine) for _ in range(size)]
         dist.all_gather(parts, mine, group=group)
         every = torch.cat(parts).cpu().numpy()
     if failure is not None:
@@ -672,6 +634,7 @@ def gather_budget_estimates(chrom_names, genome_names, rows, slots: int, group=N
 def _run_shard_defaults(d_matrices, budgets, gammas, params, levels_per_round, want_runs, score_streams, group,
                         chrom_names, genome_names, default_args, mark):
     """``run_shard`` with ROCCO's default budgets (``budgets`` None) and/or automatic gamma (``gammas`` None)."""
+    from .distributed import world
     from .inference import _resolve_local_baseline_window
     from .rocco import _resolve_budgets, _resolve_chrom_gamma
     torch = _torch()
@@ -692,7 +655,7 @@ def _run_shard_defaults(d_matrices, budgets, gammas, params, levels_per_round, w
         problem = "`budgets` and `gammas` must have one entry per matrix of `d_matrices`"
     if problem is None and any(not isinstance(x, torch.Tensor) or x.dim() != 2 or not x.is_cuda for x in d_matrices):
         problem = "every matrix of `d_matrices` must be a two-dimensional CUDA tensor"
-    if genome_names is None and _group_size(group) <= 1:
+    if genome_names is None and world(group)[1] <= 1:
         genome_names = names
     agreed = (tuple((k, args[k]) for k in sorted(args)), budgets is None, gammas is None)
     slots = agree_chromosome_names(names, genome_names, group=group, problem=problem, agreed=agreed)
@@ -980,12 +943,13 @@ def score_loci_wls_sample_sharded(d_matrix_local, m_total: int, params=None, gro
     the input of ``budget_null_sample_sharded``) and the resolved Whittaker window, which is the
     ``dependence_lag_hint`` the reference's CLI hands the budget null (rocco.py:1035)."""
     import torch.distributed as dist
+    from .distributed import world
     torch = _torch()
     centered = None
     if keep_centered:
         centered = torch.empty(tuple(d_matrix_local.shape), dtype=torch.float64, device=d_matrix_local.device)
     acc = score_partial_device(d_matrix_local, params, centered_out=centered)
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    if world(group)[1] > 1:
         dist.all_reduce(acc, group=group)
     result = score_finalize_device(acc, m_total, params, details=details)
     if not keep_centered:
@@ -1005,29 +969,16 @@ def budget_null_device(d_centered, d_observed_scores=None, params=None, dependen
     scores stay on the device; returns ``(nonnull_fraction, details)`` with the reference's keys plus the positive-score
     median/count that ``rocco._resolve_chrom_gamma`` needs.  ``random_streams``: "philox" (default) or "numpy", the
     reference's own streams generated on the device (``inference.random_streams_code``)."""
-    from .inference import _budget_details, _hint, random_streams_code
+    from .inference import _budget_details, budget_params
     torch = _torch()
     lib = _lib.load()
-    streams = random_streams_code(random_streams, random_seed, None)
-    if d_centered.dim() != 2 or not d_centered.is_cuda or not d_centered.is_contiguous() or d_centered.dtype != torch.float64:
-        raise ValueError("`d_centered` must be a contiguous two-dimensional float64 CUDA tensor")
+    problem = _budget_null_problem(d_centered, d_observed_scores, None, num_null_draws, dependence_lag_hint, random_seed,
+                                   random_streams)
+    if problem:
+        raise ValueError(problem)
     m, n = d_centered.shape
-    if m == 0 or n == 0:
-        raise ValueError("`centered_matrix` must contain at least one locus")
-    if d_observed_scores is not None and (d_observed_scores.numel() != n or d_observed_scores.dtype != torch.float64
-                                          or not d_observed_scores.is_cuda or not d_observed_scores.is_contiguous()):
-        raise ValueError("`observed_scores` must have the same number of loci as `centered_matrix`")
-    prm = _lib.BudgetParams()
-    lib.rocco_b200_default_budget_params(ctypes.byref(prm))
-    if params is not None:
-        prm.score = params
-    prm.dependence_lag_hint = _hint(dependence_lag_hint)
-    prm.num_null_draws = int(max(1, num_null_draws))
-    prm.min_null_draws = 0 if min_null_draws is None else int(max(1, min_null_draws))
-    prm.stability_abs_tol = float(stability_abs_tol)
-    prm.stability_rel_tol = float(stability_rel_tol)
-    prm.random_seed = int(random_seed) & 0xFFFFFFFFFFFFFFFF
-    prm.random_streams = streams
+    prm = budget_params(params if params is not None else score_params(), dependence_lag_hint, num_null_draws,
+                        min_null_draws, stability_abs_tol, stability_rel_tol, random_seed, random_streams)
     res = _lib.BudgetResult()
     dev = d_centered.device
     with torch.cuda.device(dev):
@@ -1042,14 +993,6 @@ def budget_null_device(d_centered, d_observed_scores=None, params=None, dependen
 
 
 # ------------------------------------------------------------------ budget null with the samples sharded over ranks
-class _DeviceBuffer:
-    """A raw float64 device buffer as a torch tensor (``__cuda_array_interface__``, no copy)."""
-
-    def __init__(self, ptr: int, count: int):
-        self.__cuda_array_interface__ = {"shape": (int(count),), "typestr": "<f8", "data": (int(ptr), False),
-                                          "strides": None, "version": 2}
-
-
 def _budget_null_sharded(d_centered_local, m_total: int, sample_offset: int, reduce_fn, d_observed_scores=None, params=None,
                          dependence_lag_hint=None, num_null_draws=25, random_seed=0, min_null_draws=None,
                          stability_abs_tol=5.0e-3, stability_rel_tol=5.0e-2, innovations=None, random_streams="philox"):
@@ -1059,70 +1002,48 @@ def _budget_null_sharded(d_centered_local, m_total: int, sample_offset: int, red
     (one rank holding every sample) is the unsharded estimator.  ``random_streams`` as for ``budget_null_device``: with
     "numpy", row r of this rank takes the normals of global sample ``sample_offset + r``, so the field is the same
     whatever the sharding."""
-    from .inference import _budget_details, _hint, random_streams_code
+    from .distributed import allreduce_callback
+    from .inference import _budget_details, budget_params
     torch = _torch()
     lib = _lib.load()
-    streams = random_streams_code(random_streams, random_seed, innovations)
+    prm = budget_params(params if params is not None else score_params(), dependence_lag_hint, num_null_draws,
+                        min_null_draws, stability_abs_tol, stability_rel_tol, random_seed, random_streams,
+                        sample_offset=sample_offset, d_innovations=innovations)
     m, n = d_centered_local.shape
     dev = d_centered_local.device
-    prm = _lib.BudgetParams()
-    lib.rocco_b200_default_budget_params(ctypes.byref(prm))
-    if params is not None:
-        prm.score = params
-    prm.dependence_lag_hint = _hint(dependence_lag_hint)
-    prm.num_null_draws = int(max(1, num_null_draws))
-    prm.min_null_draws = 0 if min_null_draws is None else int(max(1, min_null_draws))
-    prm.stability_abs_tol = float(stability_abs_tol)
-    prm.stability_rel_tol = float(stability_rel_tol)
-    prm.random_seed = int(random_seed) & 0xFFFFFFFFFFFFFFFF
-    prm.sample_offset = int(sample_offset)
-    prm.d_innovations = None if innovations is None else innovations.data_ptr()
-    prm.random_streams = streams
-    failure = []
-
-    def _reduce(ptr, count, _stream, _user):
-        try:
-            reduce_fn(torch.as_tensor(_DeviceBuffer(ptr, count), device=dev))
-            return 0
-        except BaseException as exc:          # never let it unwind through the C frames
-            failure.append(exc)
-            return 1
-
-    cb = None if reduce_fn is None else _lib.ALLREDUCE_FN(_reduce)
     res = _lib.BudgetResult()
-    with torch.cuda.device(dev):
+    with torch.cuda.device(dev), allreduce_callback(reduce_fn, dev, "budget null") as cb:
         st = lib.rocco_b200_budget_nonnull_fraction_sharded_dev(
             ctypes.c_void_p(d_centered_local.data_ptr()), m, n, int(m_total),
             None if d_observed_scores is None else ctypes.c_void_p(d_observed_scores.data_ptr()),
             ctypes.byref(prm), cb, None, ctypes.byref(res), ctypes.c_void_p(_stream_ptr(dev)))
-    if failure:
-        raise RuntimeError(f"budget null: the all-reduce failed: {failure[0]!r}") from failure[0]
     if st == _lib.ST_NONFINITE:
         raise ValueError("Budget initialization produced non-finite values")
     _lib.check(st, "budget null")
     return float(res.nonnull_fraction), _budget_details(res)
 
 
-def _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint,
-                            random_seed=0, random_streams="philox"):
-    """This rank's own argument errors (checked before the ranks compare shapes), or None."""
+def _budget_null_problem(d_centered, d_observed_scores, innovations, num_null_draws, dependence_lag_hint, random_seed,
+                         random_streams):
+    """The argument errors of ``budget_null_device`` and of one rank of ``budget_null_sample_sharded`` (checked there
+    before the ranks compare shapes), or None."""
     from .inference import _resolve_budget_bootstrap_bandwidth, random_streams_code
     torch = _torch()
     try:
         random_streams_code(random_streams, random_seed, innovations)
     except ValueError as exc:
         return str(exc)
-    x = d_centered_local
+    x = d_centered
     if x.dim() != 2 or not x.is_cuda or not x.is_contiguous() or x.dtype != torch.float64:
-        return "`d_centered_local` must be a contiguous two-dimensional float64 CUDA tensor"
+        return "the centred rows must be a contiguous two-dimensional float64 CUDA tensor"
     m, n = x.shape
     if m == 0 or n == 0:
-        return "`centered_matrix` must contain at least one sample and one locus on every rank"
+        return "`centered_matrix` must contain at least one sample and one locus"
     for name, t, shape in (("observed_scores", d_observed_scores, (n,)),
                            ("innovations", innovations, (int(max(1, num_null_draws)), m,
                                                          n + 2 * _resolve_budget_bootstrap_bandwidth(n, dependence_lag_hint)))):
         if t is not None and (tuple(t.shape) != shape or t.dtype != torch.float64 or t.device != x.device or not t.is_contiguous()):
-            return f"`{name}` must be a contiguous float64 tensor of shape {shape} on the device of `d_centered_local`"
+            return f"`{name}` must be a contiguous float64 tensor of shape {shape} on the device of the centred rows"
     return None
 
 
@@ -1136,12 +1057,12 @@ def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=
     ``budget_null_device``, and raises the same exception.  ``innovations``: this rank's rows,
     ``[draws, m_local, bins + 2*bandwidth]`` float64 on the device.  ``random_streams``: as for ``budget_null_device``;
     with "numpy" every rank generates the rows of its own samples, so the result equals the unsharded call's streams."""
-    import torch.distributed as dist
+    from .distributed import agree, workspace_allreduce, world
     torch = _torch()
-    problem = _sharded_budget_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint,
-                                      random_seed, random_streams)
-    sharded = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
-    if not sharded:
+    problem = _budget_null_problem(d_centered_local, d_observed_scores, innovations, num_null_draws, dependence_lag_hint,
+                                   random_seed, random_streams)
+    rank, size = world(group)
+    if size <= 1:
         if problem:
             raise ValueError(problem)
         m = d_centered_local.shape[0]
@@ -1157,29 +1078,13 @@ def budget_null_sample_sharded(d_centered_local, d_observed_scores=None, params=
             workspace = torch.empty(2 * n + 4, dtype=torch.float64, device=dev)
         except RuntimeError as exc:
             problem = f"could not allocate the reduce workspace: {exc}"
-    world = dist.get_world_size(group)
-    mine = torch.tensor([int(m), int(n), 0 if problem is None else 1], dtype=torch.int64, device=dev)
-    every = [torch.empty_like(mine) for _ in range(world)]
-    dist.all_gather(every, mine, group=group)
-    rows = torch.stack(every).cpu().tolist()
-    if problem is not None:
-        raise ValueError(problem)
-    if any(r[2] for r in rows):
-        raise ValueError("budget null: another rank rejected its arguments")
-    if any(r[1] != n for r in rows):
-        raise ValueError(f"budget null: every rank must hold the same loci, got bins {[r[1] for r in rows]}")
-    rank = dist.get_rank(group)
-    offset, m_total = sum(r[0] for r in rows[:rank]), sum(r[0] for r in rows)
-
-    def reduce_fn(buf):
-        w = workspace[: buf.numel()]
-        w.copy_(buf)
-        dist.all_reduce(w, group=group)
-        buf.copy_(w)
-
-    return _budget_null_sharded(d_centered_local, m_total, offset, reduce_fn, d_observed_scores, params, dependence_lag_hint,
-                                num_null_draws, random_seed, min_null_draws, stability_abs_tol, stability_rel_tol, innovations,
-                                random_streams)
+    rows = agree(problem, {"m": int(m), "n": int(n)}, group, "budget null")
+    if any(r["n"] != n for r in rows):
+        raise ValueError(f"budget null: every rank must hold the same loci, got bins {[r['n'] for r in rows]}")
+    offset, m_total = sum(r["m"] for r in rows[:rank]), sum(r["m"] for r in rows)
+    return _budget_null_sharded(d_centered_local, m_total, offset, workspace_allreduce(workspace, group), d_observed_scores,
+                                params, dependence_lag_hint, num_null_draws, random_seed, min_null_draws, stability_abs_tol,
+                                stability_rel_tol, innovations, random_streams)
 
 
 def _score_sample_sharded_agreed(x, m_total: int, prm, group, name: str):
@@ -1187,6 +1092,7 @@ def _score_sample_sharded_agreed(x, m_total: int, prm, group, name: str):
     all-reduce(MAX) of ``[failed, bins, -bins]`` comes before the accumulator all-reduce, so a rank whose per-sample stages
     fail (non-finite rows, allocation) or whose bins differ makes every rank raise ``ValueError`` instead of leaving the
     others waiting in the accumulator all-reduce.  Same calls and bits as ``score_loci_wls_sample_sharded`` otherwise."""
+    from .distributed import collective_device, world
     from .inference import _resolve_local_baseline_window
     torch = _torch()
     failure, acc, centered, n = None, None, None, -1
@@ -1196,11 +1102,10 @@ def _score_sample_sharded_agreed(x, m_total: int, prm, group, name: str):
         acc = score_partial_device(x, prm, centered_out=centered)
     except (ValueError, RuntimeError) as exc:
         failure = f"default flow: {name}: {exc}"
-    if _group_size(group) > 1:
+    if world(group)[1] > 1:
         import torch.distributed as dist
-        dev = x.device if isinstance(x, torch.Tensor) and x.is_cuda else torch.device("cuda", torch.cuda.current_device())
         flag = torch.tensor([0.0 if failure is None else 1.0, float(n), -float(n)], dtype=torch.float64,
-                            device="cpu" if dist.get_backend(group) == "gloo" else dev)
+                            device=collective_device(group, x.device if isinstance(x, torch.Tensor) and x.is_cuda else None))
         dist.all_reduce(flag, op=dist.ReduceOp.MAX, group=group)
         failed, n_max, n_min = flag[0].item(), flag[1].item(), -flag[2].item()
         if failure is None and failed:
@@ -1231,6 +1136,7 @@ def run_sample_sharded_defaults(chroms, m_total: int, params=None, default_args=
     "end".  Returns dict(names, lengths, budgets, gammas (dicts by name), defaults (null details and gamma meta by name,
     budget_meta), my_names (this rank's chromosomes, genome order), d_masks, offsets, results, runs): ``my_names`` and
     ``runs`` go straight to ``distributed.write_genome_bed``."""
+    from .distributed import world
     from .rocco import _resolve_budgets, _resolve_chrom_gamma
     args = _default_flow_args(default_args)
     mark = mark or (lambda label: None)
@@ -1261,9 +1167,8 @@ def run_sample_sharded_defaults(chroms, m_total: int, params=None, default_args=
     pairs = {c: _resolve_chrom_gamma(c, {"gamma": None}, None, nulls[c]) for c in names}
     gammas = {c: g for c, (g, _) in pairs.items()}
     mark("solve")
-    import torch.distributed as dist
-    world = _group_size(group)
-    mine = lpt_partition(lengths, world)[dist.get_rank(group) if world > 1 else 0]
+    rank, size = world(group)
+    mine = lpt_partition(lengths, size)[rank]
     mine_scores = [scores[k] for k in mine]
     del scores
     my_names = [names[k] for k in mine]
@@ -1372,6 +1277,7 @@ def column_stat_sample_sharded(d_rows_local, m_total: int, method="quantile", qu
     column is therefore reduced exactly as by the unsharded call, sums included: the result has the same bits.  With the
     gloo backend the two collectives go through host memory."""
     import torch.distributed as dist
+    from .distributed import agree, collective_device, world
     torch = _torch()
     x = d_rows_local
     problem = _column_matrix_problem(x)
@@ -1380,22 +1286,17 @@ def column_stat_sample_sharded(d_rows_local, m_total: int, method="quantile", qu
         code, arg0, arg1, _ = _column_stat_spec(method, quantile, tprop, rng)
     except ValueError as exc:
         problem, code, arg0, arg1 = problem or str(exc), -1, 0.0, 0.0
-    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
+    rank, size = world(group)
+    if size <= 1:
         if problem:
             raise ValueError(problem)
         if x.shape[0] != int(m_total):
             raise ValueError(f"`m_total` ({m_total}) must equal the number of rows ({x.shape[0]}) on a single rank")
         return column_stat_device(x, method, quantile, tprop, rng, power)
-    world, rank = dist.get_world_size(group), dist.get_rank(group)
     m, n = (int(x.shape[0]), int(x.shape[1])) if problem is None else (0, 0)
-    mine = {"problem": problem is not None, "m": m, "n": n, "dtype": str(x.dtype) if problem is None else "",
+    mine = {"m": m, "n": n, "dtype": str(x.dtype) if problem is None else "",
             "agreed": (int(m_total), int(code), float(arg0), float(arg1), float(power))}
-    every = [None] * world
-    dist.all_gather_object(every, mine, group=group)
-    if problem is not None:
-        raise ValueError(problem)
-    if any(r["problem"] for r in every):
-        raise ValueError("column statistic: another rank rejected its arguments")
+    every = agree(problem, mine, group, "column statistic")
     if any(r["agreed"] != mine["agreed"] for r in every):
         raise ValueError("column statistic: every rank must pass the same m_total, method and arguments")
     if any(r["n"] != n or r["dtype"] != mine["dtype"] for r in every):
@@ -1405,14 +1306,14 @@ def column_stat_sample_sharded(d_rows_local, m_total: int, method="quantile", qu
     if sum(rows) != int(m_total) or int(m_total) == 0:
         raise ValueError(f"column statistic: the ranks hold {sum(rows)} samples, `m_total` is {m_total}")
     dev = x.device
-    ranges = column_bin_ranges(n, world)
+    ranges = column_bin_ranges(n, size)
     width = max(b - a for a, b in ranges)
     lo, hi = ranges[rank]
-    host = dist.get_backend(group) == "gloo"
+    cdev = collective_device(group, dev)
     # send: this rank's [m, |B_q|] block of every range q, back to back; receive: [m_total, |B_rank|] in sample order
     send = column_pack_ranges(x, ranges)
-    recv = torch.empty(int(m_total) * (hi - lo), dtype=x.dtype, device="cpu" if host else dev)
-    dist.all_to_all_single(recv, send.cpu() if host else send, output_split_sizes=[r * (hi - lo) for r in rows],
+    recv = torch.empty(int(m_total) * (hi - lo), dtype=x.dtype, device=cdev)
+    dist.all_to_all_single(recv, send.to(cdev), output_split_sizes=[r * (hi - lo) for r in rows],
                            input_split_sizes=[m * (b - a) for a, b in ranges], group=group)
     del send
     # this rank's range, padded to the common width, and one status slot: a failure is raised on every rank
@@ -1427,9 +1328,9 @@ def column_stat_sample_sharded(d_rows_local, m_total: int, method="quantile", qu
             failure = exc
             part[width] = 1.0
     del recv
-    full = torch.empty(world * (width + 1), dtype=torch.float64, device="cpu" if host else dev)
-    dist.all_gather_into_tensor(full, part.cpu() if host else part, group=group)
-    full = full.view(world, width + 1).to(dev)
+    full = torch.empty(size * (width + 1), dtype=torch.float64, device=cdev)
+    dist.all_gather_into_tensor(full, part.to(cdev), group=group)
+    full = full.view(size, width + 1).to(dev)
     if failure is not None:
         raise failure
     if bool((full[:, width] != 0).any()):

@@ -226,10 +226,14 @@ from rocco_b200 import pipeline
 from rocco_b200.synth import chrom_matrix_numpy
 
 rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
-local = int(os.environ["LOCAL_RANK"])
+backend = os.environ["ROCCO_B200_BACKEND"]
+local = int(os.environ["LOCAL_RANK"]) % torch.cuda.device_count()     # gloo: both ranks may share one device
 torch.cuda.set_device(local)
 dev = torch.device("cuda", local)
-dist.init_process_group("nccl", device_id=dev)
+if backend == "nccl":
+    dist.init_process_group("nccl", device_id=dev)
+else:
+    dist.init_process_group("gloo")
 m, n = 8, 120_001
 x = chrom_matrix_numpy(m, n, seed=23)
 prm = pipeline.score_params(prior_df=6.0)
@@ -247,7 +251,14 @@ for dtype, draws, min_draws in ((np.float64, 8, 8), (np.float32, 8, 8), (np.floa
     out["runs"].append({"dtype": np.dtype(dtype).name, "fixed_draws": min_draws is not None, "window": window,
                         "window_unsharded": extra["local_baseline_window"], "identical_across_ranks": all(e == every[0] for e in every),
                         "frac": frac, "det": det, "unsharded_frac": w_frac, "unsharded": w_det})
-print("RESULT " + json.dumps(out), flush=True)
+# a rank-local argument problem (float32 rows on rank 1) raises on both ranks before any reduce
+try:
+    pipeline.budget_null_sample_sharded(cent.float() if rank == 1 else cent, scores, **kw)
+    out["local_problem"] = "no error"
+except ValueError as exc:
+    out["local_problem"] = str(exc)
+sys.stdout.write("RESULT " + json.dumps(out) + "\n")
+sys.stdout.flush()
 dist.destroy_process_group()
 '''
 
@@ -262,9 +273,18 @@ def test_two_rank_nccl_sample_sharded_budget_null(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
+    _two_rank_sample_sharded_budget_null(tmp_path, "nccl")
+
+
+def test_two_rank_gloo_sample_sharded_budget_null(tmp_path):
+    """Both ranks may share one GPU: the reduces of CUDA tensors go through the host."""
+    _two_rank_sample_sharded_budget_null(tmp_path, "gloo")
+
+
+def _two_rank_sample_sharded_budget_null(tmp_path, backend):
     script = tmp_path / "worker.py"
     script.write_text(WORKER)
-    env = dict(os.environ, ROCCO_B200_REPO=REPO)
+    env = dict(os.environ, ROCCO_B200_REPO=REPO, ROCCO_B200_BACKEND=backend)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", str(_free_port()), str(script)]
     res = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=900)
@@ -280,3 +300,6 @@ def test_two_rank_nccl_sample_sharded_budget_null(tmp_path):
                 n = run["det"]["num_loci"]
                 assert abs(run["frac"] - run["unsharded_frac"]) <= 2.0 / n
                 assert_close_details(run["det"], run["unsharded"], n, what=run["dtype"])
+    by_rank = {r["rank"]: r["local_problem"] for r in rows}
+    assert "float64" in by_rank[1] and "another rank" not in by_rank[1], by_rank
+    assert "another rank" in by_rank[0] and by_rank[1] in by_rank[0], by_rank
